@@ -1,9 +1,10 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the trace-and-shade hot path (BASELINE.json: Mrays/s and frames/s at 1920x1080).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--frames F] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--frames F] [--workload NAME] [--dump-outputs DIR]
 
-One JSON line on stdout (rank 0).  A "step" is one pass of the hot path over one batch of F camera frames per GPU.
+One JSON line on stdout (rank 0).  A "step" is one pass of the hot path over one batch of F camera frames per GPU; every
+timed loop (headline, e2e, copy-only ceiling and the `secondary` workloads) runs K steps.
 Workload "config2" (default) is BASELINE.json configs[1]: the reference's default scene at 1920x1080, reflection depth
 20 (Default::scrnshotRefections), 1 sample/pixel, default camera; the F frames of a step are successive frames of one
 reference process (the randDir stream continues from frame to frame), so every frame is a full config-2 render.
@@ -29,6 +30,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the tree may be read-only; the benchmark leaves nothing in it
 
 W, H, DEPTH = 1920, 1080, 20
 CENSUS_FLOP_PER_PIXEL = 1301.7          # SURVEY.md §8(d), config 2 (our own census build counts 1270.9, see DESIGN.md)
@@ -80,7 +82,39 @@ def parse():
     ap.add_argument("--workload", default="config2")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the configs 3 / 4 / 5 measurements of the `secondary` object")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the headline's last timed step rendered (rank 0's frames) to DIR/*.npy, see dump_outputs()")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "ours" or a.workload != "config2"):
+        ap.error("--dump-outputs applies to the headline workload (--impl ours --workload config2)")
+    return a
+
+
+DUMP_SAMPLE_PIXELS = 1 << 20
+
+
+def dump_outputs(frames):
+    """frames: the [F, H, W] ARGB (0x00RRGGBB) frames one step returns, as a device tensor.  The whole step is F x 24.9 MB as
+    float32 channels, so what --dump-outputs stores is (<= 50 MB in all, float32, R, G, B in 0 ... 255):
+      last_frame_rgb     [H, W, 3]  the step's last frame, whole
+      step_sample_rgb    [N, 3]     pixels drawn from all F frames at a fixed seeded set of positions (N <= 2^20) ...
+      step_sample_index  [N, 3]     ... and those positions: frame, row, column"""
+    import numpy as np
+    import torch
+
+    def rgb(argb):
+        return np.stack([(argb >> s) & 255 for s in (16, 8, 0)], axis=-1).astype(np.float32)
+
+    F = frames.shape[0]
+    pos = np.unique(np.random.default_rng(20261020).integers(0, F * H * W, DUMP_SAMPLE_PIXELS))
+    flat = frames.reshape(-1)
+    sample = flat[torch.from_numpy(pos).to(flat.device)].cpu().numpy()
+    f, rest = np.divmod(pos, H * W)
+    y, x = np.divmod(rest, W)
+    return {"last_frame_rgb": rgb(frames[F - 1].cpu().numpy()), "step_sample_rgb": rgb(sample),
+            "step_sample_index": np.stack([f, y, x], axis=-1).astype(np.float32)}
 
 
 # ----------------------------------------------------------------------------------------------------------------------
@@ -191,7 +225,7 @@ def run_reference(args):
     cores = os.cpu_count() or 1
     binary = "ref_render_fast"
     if not O.have_ref(binary):
-        print(json.dumps({"impl": "reference", "unavailable": "oracle/_ref/%s was not built (needs /root/reference at build time)" % binary}))
+        print(json.dumps({"impl": "reference", "unavailable": "oracle/_ref/%s was not built (needs the reference tree, RFX_REFERENCE_SRC, at build time)" % binary}))
         return
     rays = canonical_rays_per_frame()
     F = args.frames
@@ -298,6 +332,7 @@ def run_ours(args):
     e1.record(stream)
     barrier()
     sampler.end()
+    dumped = dump_outputs(out_dev) if args.dump_outputs and rank == 0 else None    # before the next render overwrites out_dev
     ms = maxreduce(e0.elapsed_time(e1))
     st = ctx.stats()
     rays_total = sumreduce(float(st["rays"]))
@@ -352,12 +387,11 @@ def run_ours(args):
         copy_step()
     barrier()
     t0 = time.perf_counter()
-    KC = max(3, K // 2)
-    for _ in range(KC):
+    for _ in range(K):
         copy_step()
     torch.cuda.synchronize()
     copy_s = maxreduce(time.perf_counter() - t0)
-    d2h_ceiling_fps = KC * F * world / copy_s
+    d2h_ceiling_fps = K * F * world / copy_s
     if world > 1:
         dist.barrier()
     st2 = ctx.stats()
@@ -384,10 +418,10 @@ def run_ours(args):
         sys.path.insert(0, os.path.join(ROOT, "tools"))
         import bench_extra
         env = bench_extra.Env()
-        secondary = {"config3_split_8k_frame": bench_extra.config3(env, steps=10, warmup=3),
-                     "config5_orbit_240_frames": bench_extra.config5(env, steps=3, warmup=3)}
+        secondary = {"config3_split_8k_frame": bench_extra.config3(env, steps=K, warmup=3),
+                     "config5_orbit_240_frames": bench_extra.config5(env, steps=K, warmup=3)}
         if world == 1:
-            secondary["config4_1024_spheres_depth_sweep"] = bench_extra.config4(env, steps=5, fp32_peak_tflops=fp32_peak)
+            secondary["config4_1024_spheres_depth_sweep"] = bench_extra.config4(env, steps=K, fp32_peak_tflops=fp32_peak)
 
     if rank != 0:
         if world > 1:
@@ -447,6 +481,10 @@ def run_ours(args):
         "device": info["name"],
     }
     print(json.dumps(line))
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if world > 1:
         dist.destroy_process_group()
 

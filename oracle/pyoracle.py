@@ -1,7 +1,7 @@
 """TEST INFRASTRUCTURE — NOT PRODUCT CODE.
 
 ctypes front end for the CPU oracle (oracle/librfx_oracle.so, our C restatement) and a subprocess front end for
-the unmodified reference (oracle/_ref/ref_render*, built from /root/reference by oracle/Makefile).
+the unmodified reference (oracle/_ref/ref_render*, built by oracle/Makefile from the tree $RFX_REFERENCE_SRC names).
 
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / ``--impl reference`` legs may import this.
 """
@@ -15,10 +15,11 @@ import tempfile
 
 import numpy as np
 
+from reflaxman_b200.build import REFERENCE_SRC   # where the unmodified reference's src/common lies, if anywhere
+
 HERE = os.path.dirname(os.path.abspath(__file__))
 PORT_SO = os.path.join(HERE, "librfx_oracle.so")
 REF_DIR = os.path.join(HERE, "_ref")
-REFERENCE_SRC = "/root/reference/src/common"
 
 _fp = C.POINTER(C.c_float)
 _u32p = C.POINTER(C.c_uint32)
@@ -36,11 +37,11 @@ class Counters(C.Structure):
 
 
 def build(ref=True, quiet=True):
-    """Compile the port (always) and, when /root/reference is present, the reference binaries."""
+    """Compile the port (always) and, when the reference tree is present, the reference binaries."""
     targets = ["port"]
     if ref and os.path.isdir(REFERENCE_SRC):
         targets.append("ref")
-    subprocess.run(["make", "-C", HERE, *targets], check=True,
+    subprocess.run(["make", "-C", HERE, *targets, "REF=" + REFERENCE_SRC], check=True,
                    stdout=subprocess.DEVNULL if quiet else None)
 
 

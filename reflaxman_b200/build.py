@@ -60,13 +60,14 @@ def build_shim_harness(force=False):
 
 
 SHIM_PULSE = os.path.join(HERE, "..", "build", "shim_pulse_headless")
-REFERENCE_SRC = "/root/reference/src/common"
+# src/common of an upstream ReflaxMan checkout: the unmodified reference, which this repository does not contain
+REFERENCE_SRC = os.environ.get("RFX_REFERENCE_SRC", "")
 
 
 def build_shim_pulse(force=False):
     """The reference's UI controller — Pulse.cpp and BasePlatformInterface.cpp, compiled UNCHANGED from where they lie —
     against the shim headers, linked with the CUDA library and the headless platform stub: a front end running on the GPU
-    path (SURVEY §8 f-2).  Needs the reference tree (build container); the binary travels to the GPU box with build/.
+    path (SURVEY §8 f-2).  Needs the reference tree (REFERENCE_SRC).
     Returns the path, or None when neither the tree nor a prebuilt binary exists."""
     import shutil
     import tempfile

@@ -49,6 +49,16 @@ def load_golden(name):
     return g
 
 
+def full_size_hashes():
+    """{case: (sha256 of the reference's ARGB image, sha256 of its float image)} for the frames too large to store"""
+    want = {}
+    with open(os.path.join(GOLDEN_DIR, "full_size_sha256.txt")) as f:
+        for line in f:
+            p = line.split()
+            want[p[0]] = (p[2], p[4])
+    return want
+
+
 def replay(engine, g):
     """engine: object with set_image_size / render(cam, refl, samples, additive) / read_rgbf|resolve.
     Returns [(rgbf, argb)] per dumped frame, following oracle/ref_harness.cpp's frame loop."""

@@ -1,5 +1,5 @@
-"""Generates tests/golden/*.npz from the UNMODIFIED reference (oracle/_ref/ref_render, built from /root/reference by
-oracle/Makefile).  Run in the build container only:  python tests/golden/make_golden.py
+"""Generates tests/golden/*.npz from the UNMODIFIED reference (oracle/_ref/ref_render, built by oracle/Makefile
+from the tree RFX_REFERENCE_SRC names).  Run in the build container only:  python tests/golden/make_golden.py
 
 Each vector stores the inputs needed to replay it (scene name, camera floats, size, depth, samples, seed) and the
 reference's outputs (ARGB, and the float image for the small cases), zlib-compressed by numpy.
@@ -50,7 +50,7 @@ CASES = [
 def main(only=None):
     """only: names of the cases to (re)generate (default: everything, ~3 minutes)"""
     O.build(ref=True)
-    assert O.have_ref(), "oracle/_ref/ref_render missing: /root/reference not available?"
+    assert O.have_ref(), "oracle/_ref/ref_render missing: set RFX_REFERENCE_SRC to the reference's src/common"
     index = {}
     if not only or "plane_probe" in only:
         # Plane::trace is unreachable through Scene: the reference's own function probed directly (oracle/ref_plane_probe.cpp)

@@ -9,7 +9,6 @@ round-1 advisor findings.  Everything goes through the C ABI (ctypes).
   * renderRange's chunk loop (huge SSAA factors): driven at small sizes by lowering "max_calls_per_launch".
 """
 import hashlib
-import os
 
 import numpy as np
 import pytest
@@ -30,15 +29,6 @@ def _ctx(capi, scene, W, H, seed):
     c = capi.Context(0)
     c.load_scene(scene); c.set_seeds(seed, seed); c.set_image_size(W, H)
     return c
-
-
-def _reference_hashes():
-    want = {}
-    with open(os.path.join(cases.GOLDEN_DIR, "full_size_sha256.txt")) as f:
-        for line in f:
-            p = line.split()
-            want[p[0]] = (p[2], p[4])
-    return want
 
 
 def test_config3_full_size_whole_chunked_split_oracle_reference(capi, oracle):
@@ -91,7 +81,7 @@ def test_config3_full_size_whole_chunked_split_oracle_reference(capi, oracle):
     _, oargb = o.resolve()
     stp = cases.assert_parity(whole, oargb, "config 3 vs oracle")
     assert st["rays"] == o.counters["rays"] and seeds_after[0] == int(o.seeds[0])
-    ref_hash = _reference_hashes()["default_7680x4320_d20_seed12345"][0]
+    ref_hash = cases.full_size_hashes()["default_7680x4320_d20_seed12345"][0]
     exact = hashlib.sha256(whole.tobytes()).hexdigest() == ref_hash
     print("config 3 parity:", stp, "sha256 equals the reference's:", exact)
     assert hashlib.sha256(oargb.tobytes()).hexdigest() == ref_hash

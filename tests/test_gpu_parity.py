@@ -1,10 +1,12 @@
 """GPU parity tests (-m gpu): the CUDA path, called through the C ABI, against
   (1) the golden vectors generated from the unmodified reference (committed fixtures),
   (2) the CPU oracle on the same seeded inputs at sizes it finishes in seconds,
-  (3) the unmodified reference binary when oracle/_ref travelled to the box.
+  (3) the unmodified reference's config-2 frame, identified by its stored hash.
 Bar (BASELINE.json): <= 1 LSB/channel on >= 99.9 % of pixels, none > 4 LSB.  The only arithmetic that may differ is
 powf (CUDA vs glibc); everything else is expected to be identical, so we also require identical hit-path signatures
 and report the exact-match fraction."""
+import hashlib
+
 import numpy as np
 import pytest
 
@@ -82,16 +84,17 @@ def test_signatures_and_rays_match_oracle_config1(capi, oracle, path):
 
 
 def test_gpu_vs_reference_binary_config2(capi, oracle):
-    """config 2 (1920x1080, depth 20, seed 12345) against the unmodified reference itself."""
-    if not oracle.have_ref():
-        pytest.skip("oracle/_ref/ref_render did not travel to this box")
+    """config 2 (1920x1080, depth 20, seed 12345) against the unmodified reference's frame: the oracle's frame hashes to the
+    reference's (tests/golden/full_size_sha256.txt), so it is that frame, bit for bit."""
     W, H = 1920, 1080
-    info, imgs = oracle.run_reference(W, H, refl=20, seed=12345)
+    ref_hash = cases.full_size_hashes()["default_%dx%d_d20_seed12345" % (W, H)][0]
+    _, ref_argb = oracle.OracleRender(S.default_scene(), W, H, seed=12345).render(S.default_camera(), 20).resolve()
+    assert hashlib.sha256(ref_argb.tobytes()).hexdigest() == ref_hash
     c = capi.Context(0)
     try:
         c.load_scene(S.default_scene()); c.set_seeds(12345, 12345); c.set_image_size(W, H)
         c.render(S.default_camera(), 20)
-        st = cases.assert_parity(c.read_argb(), imgs[0][1], "config 2 vs reference")
+        st = cases.assert_parity(c.read_argb(), ref_argb, "config 2 vs reference")
         print("config 2 parity:", st)
     finally:
         c.close()

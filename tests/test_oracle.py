@@ -45,11 +45,7 @@ def test_oracle_thread_count_invariance(oracle):
 
 def test_oracle_config1_hash(oracle):
     """config 1 (1024x768, depth 20, seed 12345): the port's images hash to what the reference produced."""
-    want = {}
-    with open(os.path.join(cases.GOLDEN_DIR, "full_size_sha256.txt")) as f:
-        for line in f:
-            p = line.split()
-            want[p[0]] = (p[2], p[4])
+    want = cases.full_size_hashes()
     r = oracle.OracleRender(S.default_scene(), 1024, 768, seed=12345).render(S.default_camera(), 20)
     rgbf, argb = r.resolve()
     assert hashlib.sha256(argb.tobytes()).hexdigest() == want["default_1024x768_d20_seed12345"][0]
@@ -61,11 +57,7 @@ def test_oracle_config1_hash(oracle):
 def test_oracle_config3_hash(oracle):
     """config 3's frame (7680x4320, depth 20, seed 12345, a reference screenshot preset): the port's 8-bit image hashes to what
     the unmodified reference produced — the GPU tests at that size compare against the port."""
-    want = {}
-    with open(os.path.join(cases.GOLDEN_DIR, "full_size_sha256.txt")) as f:
-        for line in f:
-            p = line.split()
-            want[p[0]] = (p[2], p[4])
+    want = cases.full_size_hashes()
     r = oracle.OracleRender(S.default_scene(), 7680, 4320, seed=12345).render(S.default_camera(), 20)
     rgbf, argb = r.resolve()
     assert hashlib.sha256(argb.tobytes()).hexdigest() == want["default_7680x4320_d20_seed12345"][0]

@@ -13,10 +13,10 @@ import pytest
 
 import cases
 from reflaxman_b200 import scenes as S
+from reflaxman_b200.build import REFERENCE_SRC as REF
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SHIM = os.path.join(ROOT, "reflaxman_b200", "shim")
-REF = "/root/reference/src/common"
 
 
 def test_reference_harness_source_builds_against_shim(rfx_lib):
@@ -28,7 +28,7 @@ def test_reference_harness_source_builds_against_shim(rfx_lib):
 def test_reference_pulse_compiles_unchanged_against_shim():
     """Pulse.cpp is the only client of Render upstream (reference Pulse.cpp:38-457)."""
     if not os.path.isdir(REF):
-        pytest.skip("reference tree not present on this box")
+        pytest.skip("RFX_REFERENCE_SRC does not name the reference's src/common")
     with tempfile.TemporaryDirectory() as td:
         for f in ("Pulse.h", "Pulse.cpp", "BasePlatformInterface.h", "BasePlatformInterface.cpp", "defaults.h"):
             os.symlink(os.path.join(REF, f), os.path.join(td, f))       # the reference's own files, untouched
@@ -44,7 +44,7 @@ def test_reference_pulse_links_against_shim_and_library(rfx_lib):
     from reflaxman_b200 import build
     exe = build.build_shim_pulse(force=os.path.isdir(REF))
     if exe is None:
-        pytest.skip("no reference tree and no prebuilt build/shim_pulse_headless on this box")
+        pytest.skip("no reference tree (RFX_REFERENCE_SRC) and no prebuilt build/shim_pulse_headless")
     assert os.access(exe, os.X_OK)
 
 
@@ -69,7 +69,7 @@ def test_pulse_runs_headless_on_the_gpu_path(rfx_lib, oracle, tmp_path):
     from reflaxman_b200 import build
     exe = build.build_shim_pulse()
     if exe is None:
-        pytest.skip("build/shim_pulse_headless was not built (needs /root/reference at build time)")
+        pytest.skip("build/shim_pulse_headless was not built (needs the reference tree, RFX_REFERENCE_SRC, at build time)")
     inter, hud, bmp, info = _run_pulse(exe, str(tmp_path / "gpu"))
     g = np.load(os.path.join(cases.GOLDEN_DIR, "pulse_headless.npz"))
     assert hud == str(g["hud"]), (hud, str(g["hud"]))
