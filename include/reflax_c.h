@@ -56,6 +56,7 @@ typedef struct rfx_stats
    * (k_trace_small_any), blob batch kernel (k_trace_blob<MULTI>), blob general kernel (k_trace) */
   uint64_t launches_small_fast, launches_small_any, launches_blob_fast, launches_blob_any;
   uint64_t light_grids;     /* lights of the uploaded scene whose shadow queries use a candidate grid (not a counter: survives rfx_stats_reset) */
+  uint64_t bvh_triangles;   /* triangles of the uploaded scene under a bounding-volume hierarchy, 0 = they are walked one by one (not a counter) */
 } rfx_stats;
 
 typedef struct rfx_device_info
@@ -87,6 +88,12 @@ RFX_API int rfx_add_sphere(rfx_ctx * ctx, const float center[3], float radius, i
                            float reflectivity, float transparency);                             /* Scene::addSphere, Scene.cpp:29-39 -> object index */
 RFX_API int rfx_add_triangle(rfx_ctx * ctx, const float v[9], int mtype, const float rgb[3], float reflectivity,
                              float transparency);                                               /* Scene::addTriangle, Scene.cpp:41-46 -> object index */
+/* an indexed triangle mesh: triangle k = rfx_add_triangle(xyz[idx[3k]], xyz[idx[3k+1]], xyz[idx[3k+2]]), added in order with one
+ * material (xyz = n_vertices x 3 floats, idx = n_tris x 3 vertex indices).  Returns the object index of the first triangle; the others
+ * follow it.  An index >= n_vertices, a NULL pointer or n_tris = 0 adds nothing and returns RFX_ERR_ARG.  Mesh triangles are ordinary
+ * objects (rfx_set_triangle_texture applies to each). */
+RFX_API int rfx_add_mesh(rfx_ctx * ctx, uint32_t n_vertices, const float * xyz, uint32_t n_tris, const uint32_t * idx, int mtype,
+                         const float rgb[3], float reflectivity, float transparency);
 RFX_API int rfx_set_triangle_texture(rfx_ctx * ctx, int object, int texture, const float uv[6]); /* Triangle::setTexture, Triangle.cpp:110-120 (u1,v1,u2,v2,u3,v3) */
 RFX_API int rfx_add_plane(rfx_ctx * ctx, const float pos[3], const float norm[3], int mtype, const float rgb[3],
                           float reflectivity, float transparency);                              /* Plane::Plane, Plane.cpp:9-14 (no Scene::addPlane exists upstream) */
@@ -132,6 +139,11 @@ RFX_API int rfx_selftest_primary_bounds_host(const float cam[13], uint32_t width
 RFX_API int rfx_selftest_light_grid_host(const float light[4], int n_spheres, const float * spheres, const float box[6], float reach_diagonal,
                                          float uv[8], int32_t dims[2], uint32_t * cell_start, uint64_t cell_cap, int32_t * items, uint64_t item_cap,
                                          uint64_t counts[2]);
+/* diagnostic, pure host function: the boxes of the triangle hierarchy (rfx_set_bvh_mode).  tris = n x (v0[3], axTrans[9] row-major: what
+ * Triangle::trace reads); reach = lo[3], hi[3] of every ray origin.  boxes out = n x (lo[3], hi[3]): each holds every point at which the
+ * float32 test of Triangle.cpp:56-68 can accept a ray from inside reach (a zero-area triangle's test accepts the unit triangle its
+ * identity basis describes, not its vertices), inflated by that test's rounding noise and by 1e-6 of the reach diagonal. */
+RFX_API int rfx_selftest_tri_bounds_host(int n, const float * tris, const float reach[6], float * boxes);
 /* diagnostic, pure host function: the screen grid of a path's first query (option "eye_grid") for cam = eye[3], view[9], fov and
  * spheres = n_spheres x (cx, cy, cz, r^2): dims = {nx, ny, shift} (cells of 2^shift pixels; {0, 0, 0}: no grid for this camera),
  * counts = {nx*ny + 1, items}, cell_start / items (sphere indices, cell after cell) filled when their capacities suffice. */
@@ -202,16 +214,17 @@ RFX_API int rfx_enable_profiling(rfx_ctx * ctx, int on);
  * in between (default 8).  "light_grids": scenes with a sphere hierarchy answer the shadow queries of far lights from a 2-D grid of
  * candidate spheres across the light's direction instead of walking the hierarchy (default 1).  "eye_grid": the same scenes take the
  * candidates of a path's first query (origin = eye) from a screen grid binned per camera out of the spheres' primary-ray bounds
- * (default 1).  Frames are bit-identical under
- * every setting. */
+ * (default 1).  Both grids list spheres only: triangles are tested after them, through their own hierarchy when the scene has one
+ * (rfx_set_bvh_mode).  Frames are bit-identical under every setting. */
 RFX_API int rfx_set_option(rfx_ctx * ctx, const char * name, int64_t value);
 /* kernel selection: 0 = automatic (constant-bank kernels when the scene fits, the blob kernels otherwise),
  * 1 = constant-bank kernel if it fits, 2 = always the blob kernels (tile / wavefront kernels for row-aligned slices, the general
  * one otherwise), 3 = always the general blob kernel.  Results are identical; tests use it. */
 RFX_API int rfx_force_path(rfx_ctx * ctx, int path);
-/* acceleration structure of the blob kernels: 0 = automatic (bounding-volume hierarchy over the spheres when there are more than
- * 32 and the scene holds no unbounded plane), 1 = always, 2 = never (the reference's brute-force list walk).  Results are
- * identical; tests compare them. */
+/* acceleration structures of the blob kernels: 0 = automatic (a bounding-volume hierarchy over the spheres when there are more than
+ * 32 and the scene holds no unbounded plane; one over the triangles, walked after the spheres, when there are more than 32 triangles
+ * and no plane), 1 = always (spheres: whenever there are any; triangles: whenever there are any and no plane), 2 = never (the
+ * reference's brute-force list walk).  Results are identical; tests compare them. */
 RFX_API int rfx_set_bvh_mode(rfx_ctx * ctx, int mode);
 /* cost-ordered tile scheduling of the constant-bank fast kernel: launches record which tiles held long paths (every
  * "tile_order_period"-th launch over a grid) and the following launches over the same grid start those first (1 = on, the

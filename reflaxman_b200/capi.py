@@ -21,7 +21,8 @@ _u32p = C.POINTER(C.c_uint32)
 class RfxStats(C.Structure):
     _fields_ = [(n, C.c_uint64) for n in ("rays", "bounces", "shadow_rays", "samples", "kernel_launches",
                                           "h2d_bytes", "d2h_bytes", "trace_kernels")] + [("trace_kernel_ms", C.c_double)] + \
-               [(n, C.c_uint64) for n in ("launches_small_fast", "launches_small_any", "launches_blob_fast", "launches_blob_any", "light_grids")]
+               [(n, C.c_uint64) for n in ("launches_small_fast", "launches_small_any", "launches_blob_fast", "launches_blob_any", "light_grids",
+                                          "bvh_triangles")]
 
     def as_dict(self):
         return {n: (float if n == "trace_kernel_ms" else int)(getattr(self, n)) for n, _ in self._fields_}
@@ -43,6 +44,7 @@ SYMBOLS = [
     ("rfx_add_light", C.c_int, [C.c_void_p, _fp, C.c_float, _fp, C.c_float]),
     ("rfx_add_sphere", C.c_int, [C.c_void_p, _fp, C.c_float, C.c_int, _fp, C.c_float, C.c_float]),
     ("rfx_add_triangle", C.c_int, [C.c_void_p, _fp, C.c_int, _fp, C.c_float, C.c_float]),
+    ("rfx_add_mesh", C.c_int, [C.c_void_p, C.c_uint32, _fp, C.c_uint32, _u32p, C.c_int, _fp, C.c_float, C.c_float]),
     ("rfx_set_triangle_texture", C.c_int, [C.c_void_p, C.c_int, C.c_int, _fp]),
     ("rfx_add_plane", C.c_int, [C.c_void_p, _fp, _fp, C.c_int, _fp, C.c_float, C.c_float]),
     ("rfx_add_texture_argb", C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, _u32p]),
@@ -56,6 +58,7 @@ SYMBOLS = [
     ("rfx_selftest_primary_bounds_host", C.c_int, [_fp, C.c_uint32, C.c_uint32, C.c_int, _fp, C.c_int, _fp, C.POINTER(C.c_int32)]),
     ("rfx_selftest_light_grid_host", C.c_int, [_fp, C.c_int, _fp, _fp, C.c_float, _fp, C.POINTER(C.c_int32), _u32p, C.c_uint64,
                                               C.POINTER(C.c_int32), C.c_uint64, C.POINTER(C.c_uint64)]),
+    ("rfx_selftest_tri_bounds_host", C.c_int, [C.c_int, _fp, _fp, _fp]),
     ("rfx_selftest_eye_grid_host", C.c_int, [_fp, C.c_uint32, C.c_uint32, C.c_int, _fp, C.POINTER(C.c_int32), _u32p, C.c_uint64,
                                             C.POINTER(C.c_int32), C.c_uint64, C.POINTER(C.c_uint64)]),
     ("rfx_set_image_size", C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32]),
@@ -161,6 +164,18 @@ def light_grid_host(light, spheres, box, reach_diagonal):
     return uv.reshape(2, 4), int(dims[0]), int(dims[1]), cells, items[:int(counts[1])]
 
 
+def tri_bounds_host(tris, reach):
+    """Pure host function (no GPU): the boxes of the triangle hierarchy.  tris [n][12] = (v0[3], axTrans[9] row-major), reach = (lo[3], hi[3])
+    of every ray origin.  Returns boxes [n][6] = (lo[3], hi[3])."""
+    L = load()
+    tr = np.ascontiguousarray(np.asarray(tris, np.float32).reshape(-1, 12))
+    rc_ = np.ascontiguousarray(np.asarray(reach, np.float32).reshape(6))
+    out = np.zeros((len(tr), 6), np.float32)
+    if L.rfx_selftest_tri_bounds_host(len(tr), tr.ctypes.data_as(_fp), rc_.ctypes.data_as(_fp), out.ctypes.data_as(_fp)) != 0:
+        raise RfxError("rfx_selftest_tri_bounds_host failed")
+    return out
+
+
 def eye_grid_host(cam, width, height, spheres):
     """Pure host function (no GPU): the screen grid of the first query for ``cam`` and spheres [n][4] = (cx, cy, cz, r^2).
     Returns None when the camera gets no grid, else (nx, ny, shift, cell_start, items)."""
@@ -241,11 +256,21 @@ class Context:
                 idx = self._ck(self.L.rfx_add_triangle(self.h, _f(v)[1], mt, _f(col)[1], C.c_float(refl), C.c_float(tr)), "rfx_add_triangle")
                 if tex >= 0:
                     self._ck(self.L.rfx_set_triangle_texture(self.h, idx, tex_ids[tex], _f(uv)[1]), "rfx_set_triangle_texture")
+            elif ob[0] == "mesh":
+                _, xyz, idx, mt, col, refl, tr = ob
+                self.add_mesh(xyz, idx, mt, col, refl, tr)
             elif ob[0] == "plane":
                 _, pos, nrm, mt, col, refl, tr = ob
                 self._ck(self.L.rfx_add_plane(self.h, _f(pos)[1], _f(nrm)[1], mt, _f(col)[1], C.c_float(refl), C.c_float(tr)), "rfx_add_plane")
             else:
                 raise ValueError(ob[0])
+
+    def add_mesh(self, xyz, idx, mtype, rgb, refl, transp):
+        """rfx_add_mesh: xyz [N][3] vertices, idx [M][3] vertex indices; returns the object index of the first of the M triangles."""
+        v = np.ascontiguousarray(xyz, dtype=np.float32).reshape(-1, 3)
+        ix = np.ascontiguousarray(idx, dtype=np.uint32).reshape(-1, 3)
+        return self._ck(self.L.rfx_add_mesh(self.h, v.shape[0], v.ctypes.data_as(_fp), ix.shape[0], ix.ctypes.data_as(_u32p), mtype,
+                                            _f(rgb)[1], C.c_float(refl), C.c_float(transp)), "rfx_add_mesh")
 
     def add_texture(self, argb):
         if argb is None:
@@ -418,7 +443,8 @@ class Context:
         self._ck(self.L.rfx_force_path(self.h, path), "rfx_force_path")
 
     def set_bvh_mode(self, mode):
-        """0 automatic (hierarchy over the spheres when there are more than 32), 1 always, 2 never (list walk)."""
+        """0 automatic (hierarchies over the spheres / the triangles when there are more than 32 of them and no plane), 1 always,
+        2 never (list walk)."""
         self._ck(self.L.rfx_set_bvh_mode(self.h, mode), "rfx_set_bvh_mode")
 
     def set_tile_ordering(self, on=True):

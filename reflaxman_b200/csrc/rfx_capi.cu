@@ -68,11 +68,16 @@ void invertColumns(H3 u, H3 v, H3 n, float out[9])
 
 template <typename T> inline size_t align16(T v) { return ((size_t)v + 15) & ~(size_t)15; }
 
-// ---- bounding-volume hierarchy over the spheres of big scenes (SURVEY f-3) ---------------------------------------------
-// Median split on the widest centroid axis, leaves of <= 4 spheres, boxes inflated by `margin`.  The hierarchy only
-// selects which spheres receive the exact reference test on the device; it never decides a hit.
+// ---- bounding-volume hierarchies over the spheres and over the triangles of big scenes (SURVEY f-3) ---------------------------
+// Median split on the widest centroid axis, leaves of <= 4 primitives, each primitive's box inflated by its margin.  A hierarchy
+// only selects which primitives receive the exact reference test on the device; it never decides a hit.
 struct BvhNode { float lo[3], hi[3]; int a, b; };
-struct BvhPrim { float c[3], r, m; int index; };   // m: this sphere's box margin (see uploadScene)
+struct BvhPrim
+{
+  float c[3], r, m;         // spheres: centre (the split key), radius, box margin (see uploadScene); triangles: c = centre of the box
+  int index;                // position in the sorted sphere / triangle array (the split's tie-break)
+  float lo[3], hi[3];       // the box: spheres c -/+ r -/+ m, triangles buildTriBoxes
+};
 
 int buildBvhRec(std::vector<BvhNode> & nodes, std::vector<BvhPrim> & prims, int begin, int end, int depth, int & maxDepth)
 {
@@ -83,8 +88,8 @@ int buildBvhRec(std::vector<BvhNode> & nodes, std::vector<BvhPrim> & prims, int 
   for (int i = begin; i < end; i++)
     for (int k = 0; k < 3; k++)
     {
-      lo[k] = std::min(lo[k], prims[i].c[k] - prims[i].r - prims[i].m);
-      hi[k] = std::max(hi[k], prims[i].c[k] + prims[i].r + prims[i].m);
+      lo[k] = std::min(lo[k], prims[i].lo[k]);
+      hi[k] = std::max(hi[k], prims[i].hi[k]);
       clo[k] = std::min(clo[k], prims[i].c[k]);
       chi[k] = std::max(chi[k], prims[i].c[k]);
     }
@@ -106,6 +111,109 @@ int buildBvhRec(std::vector<BvhNode> & nodes, std::vector<BvhPrim> & prims, int 
   n.b = buildBvhRec(nodes, prims, mid, end, depth + 1, maxDepth);
   nodes[me] = n;
   return me;
+}
+
+// Device form of a hierarchy: refs (leaf: ~(first slot), 4 slots per leaf in node order; inner node: its pair-node index) and the
+// pair nodes {lo_a.xyz, ref_a} {hi_a.xyz, ref_b} {lo_b.xyz, -} {hi_b.xyz, -}, 4 float4 each, written to pairs
+size_t bvhRefs(const std::vector<BvhNode> & nodes, std::vector<int> & ref)
+{
+  size_t nLeaves = 0;
+  for (const BvhNode & n : nodes) nLeaves += n.b < 0;
+  ref.resize(nodes.size());
+  int inner = 0, lf = 0;
+  for (size_t i = 0; i < nodes.size(); i++) ref[i] = nodes[i].b < 0 ? ~(4 * lf++) : inner++;
+  return nLeaves;
+}
+
+void writePairNode(const std::vector<BvhNode> & nodes, const std::vector<int> & ref, size_t i, float4 * pairs)
+{
+  const BvhNode & ca = nodes[nodes[i].a], & cb = nodes[nodes[i].b];
+  float4 * w = pairs + 4 * (size_t)ref[i];
+  w[0] = make_float4(ca.lo[0], ca.lo[1], ca.lo[2], 0.0f); w[1] = make_float4(ca.hi[0], ca.hi[1], ca.hi[2], 0.0f);
+  w[2] = make_float4(cb.lo[0], cb.lo[1], cb.lo[2], 0.0f); w[3] = make_float4(cb.hi[0], cb.hi[1], cb.hi[2], 0.0f);
+  memcpy(&w[0].w, &ref[nodes[i].a], 4); memcpy(&w[1].w, &ref[nodes[i].b], 4);
+}
+
+// Boxes of the triangle hierarchy.  The box of a triangle must hold every point X = o + t d at which the float test of
+// Triangle.cpp:56-68 (rfx_trace_blob.cu intersectBlob) can accept it.  That is not the triangle the user gave: the test reads
+// M = axTrans = inverse[v2-v0 | v1-v0 | -n] as rounded to float, and a triangle of zero area (n = 0) gets M = identity
+// (invertColumns), which accepts a unit right triangle at v0.  So the box starts from the EFFECTIVE triangle
+// E = {v0 + u a + v b : u, v >= 0, u + v <= 1} with [a | b | c] = A = M^-1 (binary64), and is inflated by the test's rounding noise.
+//
+// Margin.  With u = 2^-24, p = o - v0, M_k the rows of M and U, V, W the exact coordinates M (X - v0) of the exact point X = o + t d
+// (t the float root the test computed), the test's float ox, rx (row 0), oy, ry (row 1), oz, rz (row 2) carry errors of at most
+// 4u|M_k||p| and 3u|M_k||d| (three-term dot products after the subtraction p), so
+//   |u_f - U| <= 4u|M_0||p| + 4u|M_0||t d| + u(1 + u)   (one more rounding each for t * rx and the sum; |u_f| <= 1 when accepted)
+//   |W|       <= 5u|M_2||p| + 3u|M_2||t d|              (t = fl(-oz / rz) leaves |oz + t rz| <= u|oz| in the float values)
+// and likewise for v_f with M_1.  X = v0 + U a + V b + W c therefore lies within
+//   dev <= 5u kappa (|p| + |t d|) + 1.01u(|a| + |b|),   kappa = |a||M_0| + |b||M_1| + |c||M_2|   (>= 3: M_k . A_k = 1)
+// of the point v0 + u_f a + v_f b, which is in E up to u(|a| + |b|) (u_f + v_f < 1 is a rounded sum).  (kappa is at most sqrt(3) times
+// the condition number |M||A|, and much smaller for a small triangle, whose unit normal column c meets a unit row M_2.)  Let R be the
+// diagonal of the box that holds every ray origin and every E (the reach box the sphere margins use, joined with the boxes of all E):
+// |p| <= R and |t d| = |X - o| <= R + dev, so
+//   dev <= 5u kappa (2R + dev) + 2.1u|A|,   i.e. dev <= 20u kappa R + 4.2u|A|   while 5u kappa <= 1/2   (|A|: Frobenius norm).
+// The box is E's inflated by m = 64u (kappa R + |A|) (three times the bound: A is formed in binary64, drop points overshoot their
+// surface by a rounding) plus 1e-6 R for the device's fused slab test (as for the spheres), rounded outwards to float.  A triangle
+// with 16u kappa > 1/2 (a sliver: kappa above 2^19), or whose M or A is not finite, gets the whole box of reach instead: every
+// query from inside it then tests that triangle, which is slow but exact.
+// tris: n x (v0[3], ax[9]); reach: lo[3], hi[3]; boxes out: n x (lo[3], hi[3]).  Returns R.
+double buildTriBoxes(int n, const float * tris, const float reach[6], float * boxes)
+{
+  const double u = 1.0 / 16777216.0;
+  std::vector<double> e((size_t)n * 8);   // per triangle: E's box (lo xyz, hi xyz), |A|, kappa (negative: no finite E)
+  double ulo[3] = { reach[0], reach[1], reach[2] }, uhi[3] = { reach[3], reach[4], reach[5] };
+  for (int i = 0; i < n; i++)
+  {
+    const float * t = tris + 12 * (size_t)i;
+    double M[9], A[9];
+    bool ok = true;
+    for (int k = 0; k < 9; k++) { M[k] = t[3 + k]; ok = ok && std::isfinite(M[k]); }
+    for (int k = 0; k < 3; k++) ok = ok && std::isfinite((double)t[k]);
+    double det = 0;
+    if (ok)
+    {
+      A[0] = M[4] * M[8] - M[5] * M[7]; A[1] = M[2] * M[7] - M[1] * M[8]; A[2] = M[1] * M[5] - M[2] * M[4];
+      A[3] = M[5] * M[6] - M[3] * M[8]; A[4] = M[0] * M[8] - M[2] * M[6]; A[5] = M[2] * M[3] - M[0] * M[5];
+      A[6] = M[3] * M[7] - M[4] * M[6]; A[7] = M[1] * M[6] - M[0] * M[7]; A[8] = M[0] * M[4] - M[1] * M[3];
+      det = M[0] * A[0] + M[1] * A[3] + M[2] * A[6];
+      ok = std::isfinite(det) && det != 0.0;
+    }
+    double * r = &e[8 * (size_t)i];
+    r[7] = -1.0;
+    if (!ok) continue;
+    double na = 0, kappa = 0;
+    for (int k = 0; k < 9; k++) { A[k] /= det; na += A[k] * A[k]; }
+    na = sqrt(na);
+    for (int k = 0; k < 3; k++)   // |column k of A| * |row k of M|
+      kappa += sqrt(A[k] * A[k] + A[3 + k] * A[3 + k] + A[6 + k] * A[6 + k]) * sqrt(M[3 * k] * M[3 * k] + M[3 * k + 1] * M[3 * k + 1] + M[3 * k + 2] * M[3 * k + 2]);
+    bool fin = std::isfinite(na) && std::isfinite(kappa);
+    for (int k = 0; k < 3; k++)
+    {
+      const double v0 = t[k], pa = v0 + A[3 * k], pb = v0 + A[3 * k + 1];   // v0, v0 + a, v0 + b (a, b: columns 0 and 1 of A)
+      r[k] = std::min(v0, std::min(pa, pb)); r[3 + k] = std::max(v0, std::max(pa, pb));
+      fin = fin && std::isfinite(r[k]) && std::isfinite(r[3 + k]);
+    }
+    if (!fin) continue;
+    r[6] = na; r[7] = kappa;
+    for (int k = 0; k < 3; k++) { ulo[k] = std::min(ulo[k], r[k]); uhi[k] = std::max(uhi[k], r[3 + k]); }
+  }
+  const double dx = uhi[0] - ulo[0], dy = uhi[1] - ulo[1], dz = uhi[2] - ulo[2];
+  const double R = sqrt(dx * dx + dy * dy + dz * dz);
+  auto down = [](double v) { float f = (float)v; if ((double)f > v) f = nextafterf(f, -FLT_MAX); return f; };
+  auto up = [](double v) { float f = (float)v; if ((double)f < v) f = nextafterf(f, FLT_MAX); return f; };
+  for (int i = 0; i < n; i++)
+  {
+    const double * r = &e[8 * (size_t)i];
+    float * b = boxes + 6 * (size_t)i;
+    if (!(r[7] >= 0.0) || !(16.0 * u * r[7] <= 0.5))
+    {
+      for (int k = 0; k < 3; k++) { b[k] = down(ulo[k]); b[3 + k] = up(uhi[k]); }
+      continue;
+    }
+    const double m = 64.0 * u * (r[7] * R + r[6]) + 1e-6 * R;
+    for (int k = 0; k < 3; k++) { b[k] = down(r[k] - m); b[3 + k] = up(r[3 + k] + m); }
+  }
+  return R;
 }
 
 } // namespace
@@ -164,7 +272,10 @@ struct rfx_ctx
   bool eyeGridOn = true;                    // rfx_set_option "eye_grid"
   uint64_t eyeGridBuilds = 0;
   int lightGridsBuilt = 0;                  // lights of the uploaded scene that have a grid
-  int bvhMode = 0;                          // 0 auto (spheres > 32), 1 always, 2 never — tests compare both
+  int bvhMode = 0;                          // 0 auto (spheres > 32, triangles > 32), 1 always, 2 never — tests compare both
+  float4 * dTriNodes = nullptr; size_t triNodesCap = 0;   // hierarchy over the triangles: leaf slots, then pair nodes (uploadScene)
+  int * dTriPrims = nullptr; size_t triPrimsCap = 0;
+  uint64_t triBvhTris = 0;                  // triangles under that hierarchy in the uploaded scene (0: list walk)
 
   // ---- camera + render state (reference Render.h:9-27)
   float eye[3] = { 0, 0, 0 }, view[9] = { 1, 0, 0, 0, 1, 0, 0, 0, 1 }, fov = 1.0f;
@@ -264,7 +375,8 @@ Material makeMaterial(int mtype, const float rgb[3], float refl, float transp, i
 // and s is bounded because P must lie in B: C - s*l is within r + m + 1.01 sigma diag(B) of P, so s is at most the distance from C
 // backwards along l to the boundary of B inflated by that much.  The grid cell of proj(P) therefore lists every sphere a shadow ray
 // from P can hit; the any-hit query tests that list with the reference's exact arithmetic instead of walking the hierarchy, and its
-// answer — is the light occluded — is the same.  (Triangles and planes are few and are tested directly, as before.)
+// answer — is the light occluded — is the same.  (Triangles and planes are tested after the list, as before: one by one, or through
+// the triangle hierarchy.)
 struct LightGridHost
 {
   LightGrid g;
@@ -421,6 +533,8 @@ int uploadScene(rfx_ctx * ctx, cudaStream_t st)
   h.offPlanes = (uint32_t)off; off = align16(off + sizeof(Plane) * pla.size());
   h.offMats = (uint32_t)off; off = align16(off + sizeof(Material) * ctx->objs.size());
   h.offTex = (uint32_t)off; off = align16(off + sizeof(TexRef) * ctx->tex.size());
+  // the header addresses the blob with 32-bit offsets (every earlier offset is below off)
+  if (off > (size_t)UINT32_MAX) return fail(ctx, RFX_ERR_ARG, "scene too large: the blob exceeds 4 GB");
   h.bytes = (uint32_t)off;
   h.byteLut = ctx->dLut;
   h.bvhPrims = nullptr;
@@ -436,9 +550,15 @@ int uploadScene(rfx_ctx * ctx, cudaStream_t st)
   // below, which are sized for ray origins inside a bounded region, could not be guaranteed (the reference's Scene cannot hold
   // planes at all; mode 1 builds the hierarchy regardless, for tests)
   const bool wantBvh = ctx->bvhMode == 1 ? !sph.empty() : ctx->bvhMode == 2 ? false : (sph.size() > 32 && pla.empty());
-  if (wantBvh)
+  // the hierarchy over the triangles: the same automatic rule; mode 1 builds it for any triangle, but never next to a plane (its
+  // margins need bounded drop points)
+  const bool wantTriBvh = pla.empty() && (ctx->bvhMode == 1 ? !tri.empty() : ctx->bvhMode == 2 ? false : tri.size() > 32);
+  ctx->triBvhTris = 0;
+  h.triPrims = nullptr; h.triLeaf = nullptr; h.triPairs = nullptr; h.triRoot = 0;
+  float lo[3] = { ctx->eye[0], ctx->eye[1], ctx->eye[2] }, hi[3] = { ctx->eye[0], ctx->eye[1], ctx->eye[2] };
+  double R = 0.0;
+  if (wantBvh || wantTriBvh)
   {
-    std::vector<BvhPrim> prims(sph.size());
     // Box margins.  The hierarchy must never cull a sphere the reference's exact test (Sphere.cpp:49-57) would report, and that
     // test is noisy: with v = origin - centre, disc = b*b - 4a*c carries an absolute rounding error of at most ~40 * 2^-24 * a|v|^2
     // (three-term dot products, the square, the product), while a ray that misses the sphere by m has disc = 4a(r^2 - m^2).  A
@@ -448,7 +568,6 @@ int uploadScene(rfx_ctx * ctx, cudaStream_t st)
     // test (fused arithmetic with clamped reciprocals: a box plane moves by at most 2^-22 |origin| along its axis).  (Planes are unbounded: a drop point
     // on a plane can lie outside the box; the reference's Scene cannot hold planes, and rfx_set_camera re-flattens the scene
     // when the eye leaves the box.)
-    float lo[3] = { ctx->eye[0], ctx->eye[1], ctx->eye[2] }, hi[3] = { ctx->eye[0], ctx->eye[1], ctx->eye[2] };
     for (int k = 0; k < 3; k++)
       if (ctx->extraOrigins[k] <= ctx->extraOrigins[3 + k])   // origins of explicit ray lists (rfx_trace_rays)
       {
@@ -476,8 +595,12 @@ int uploadScene(rfx_ctx * ctx, cudaStream_t st)
       lo[k] -= pad; hi[k] += pad;
     }
     const double dx = (double)hi[0] - lo[0], dy = (double)hi[1] - lo[1], dz = (double)hi[2] - lo[2];
-    const double R = sqrt(dx * dx + dy * dy + dz * dz);
+    R = sqrt(dx * dx + dy * dy + dz * dz);
     for (int k = 0; k < 3; k++) { ctx->bvhReach[k] = lo[k]; ctx->bvhReach[3 + k] = hi[k]; }
+  }
+  if (wantBvh)
+  {
+    std::vector<BvhPrim> prims(sph.size());
     for (size_t i = 0; i < sph.size(); i++)
     {
       BvhPrim & p = prims[i];
@@ -486,25 +609,21 @@ int uploadScene(rfx_ctx * ctx, cudaStream_t st)
       p.index = (int)i;
       const double noise = std::min(3e-7 * R * R / std::max((double)p.r, 1e-30), 7.7e-4 * R);
       p.m = (float)(2.0 * noise + 1e-6 * R);
+      for (int k = 0; k < 3; k++) { p.lo[k] = p.c[k] - p.r - p.m; p.hi[k] = p.c[k] + p.r + p.m; }
     }
     std::vector<BvhNode> nodes;
     int maxDepth = 0;
     buildBvhRec(nodes, prims, 0, (int)prims.size(), 0, maxDepth);
-    if (maxDepth <= BLOB_MAX_BVH_DEPTH)   // the traversal stacks hold 24 entries; a median split of the <= 12 800 spheres a 200 KB blob can carry is 13 deep
+    if (maxDepth <= BLOB_MAX_BVH_DEPTH)   // the traversal stacks hold 24 entries; a median split of 2^20 spheres is 18 deep
     {
       // The device form, one allocation: leaf records — every leaf is 4 slots of (cx, cy, cz, r^2), NaN in the unused ones, so a
       // whole leaf is tested without indirection — then the "pair nodes": an inner node carries both children's boxes,
       // {lo_a.xyz, ref_a} {hi_a.xyz, ref_b} {lo_b.xyz, -} {hi_b.xyz, -}, ref >= 0: pair node index, ref < 0: ~(first slot of a leaf).
       // bvhPrims[4 * leaf + k] = position of that slot's sphere in the sorted sphere array (materials, tie-break order).
-      size_t nLeaves = 0;
-      for (const BvhNode & n : nodes) nLeaves += n.b < 0;
+      std::vector<int> ref;
+      const size_t nLeaves = bvhRefs(nodes, ref);
       const size_t nInner = nodes.size() - nLeaves;
       std::vector<float4> packed(nLeaves * 4 + nInner * 4);
-      std::vector<int> ref(nodes.size());
-      {
-        int inner = 0, lf = 0;
-        for (size_t i = 0; i < nodes.size(); i++) ref[i] = nodes[i].b < 0 ? ~(4 * lf++) : inner++;
-      }
       std::vector<int> order(nLeaves * 4, -1);
       const float qnan = std::numeric_limits<float>::quiet_NaN();
       size_t leaf = 0;
@@ -526,14 +645,7 @@ int uploadScene(rfx_ctx * ctx, cudaStream_t st)
           }
           leaf++;
         }
-        else
-        {
-          const BvhNode & ca = nodes[nodes[i].a], & cb = nodes[nodes[i].b];
-          float4 * w = &packed[nLeaves * 4 + 4 * (size_t)ref[i]];
-          w[0] = make_float4(ca.lo[0], ca.lo[1], ca.lo[2], 0.0f); w[1] = make_float4(ca.hi[0], ca.hi[1], ca.hi[2], 0.0f);
-          w[2] = make_float4(cb.lo[0], cb.lo[1], cb.lo[2], 0.0f); w[3] = make_float4(cb.hi[0], cb.hi[1], cb.hi[2], 0.0f);
-          memcpy(&w[0].w, &ref[nodes[i].a], 4); memcpy(&w[1].w, &ref[nodes[i].b], 4);
-        }
+        else writePairNode(nodes, ref, i, &packed[nLeaves * 4]);
       }
       int rc;
       if ((rc = ensure(ctx, ctx->dBvhNodes, ctx->bvhNodesCap, packed.size())) != RFX_OK) return rc;
@@ -618,7 +730,68 @@ int uploadScene(rfx_ctx * ctx, cudaStream_t st)
       }
     }
   }
-  if (off > 200 * 1024) return fail(ctx, RFX_ERR_ARG, "scene too large for the shared-memory resident layout (200 KB)");
+  if (wantTriBvh)
+  {
+    // The hierarchy over the triangles (buildTriBoxes has the boxes and their margins).  Device form, one allocation: leaf slots of
+    // 3 float4 each (4 per leaf, the layout of SmallScene::triPk; unused slots all zero, which the exact test's gate |rz| > 2^-63
+    // rejects), then the pair nodes; triPrims[slot] = the slot's position in the sorted triangle array (-1 unused).
+    std::vector<float> tv(tri.size() * 12), boxes(tri.size() * 6);
+    for (size_t i = 0; i < tri.size(); i++) { memcpy(&tv[12 * i], tri[i]->tri.v0, 12); memcpy(&tv[12 * i + 3], tri[i]->tri.ax, 36); }
+    buildTriBoxes((int)tri.size(), tv.data(), ctx->bvhReach, boxes.data());
+    std::vector<BvhPrim> prims(tri.size());
+    for (size_t i = 0; i < tri.size(); i++)
+    {
+      BvhPrim & p = prims[i];
+      memset(&p, 0, sizeof(p));
+      p.index = (int)i;
+      for (int k = 0; k < 3; k++)
+      {
+        p.lo[k] = boxes[6 * i + k]; p.hi[k] = boxes[6 * i + 3 + k];
+        p.c[k] = 0.5f * p.lo[k] + 0.5f * p.hi[k];
+      }
+    }
+    std::vector<BvhNode> nodes;
+    int maxDepth = 0;
+    buildBvhRec(nodes, prims, 0, (int)prims.size(), 0, maxDepth);
+    if (maxDepth <= BLOB_MAX_BVH_DEPTH)   // deeper (not seen from a median split below ~2^22 triangles): the list walk
+    {
+      std::vector<int> ref;
+      const size_t nLeaves = bvhRefs(nodes, ref), nInner = nodes.size() - nLeaves;
+      std::vector<float4> packed(nLeaves * 12 + nInner * 4, make_float4(0.0f, 0.0f, 0.0f, 0.0f));
+      std::vector<int> order(nLeaves * 4, -1);
+      size_t leaf = 0;
+      for (size_t i = 0; i < nodes.size(); i++)
+      {
+        if (nodes[i].b < 0)
+        {
+          for (int k = 0; k < -nodes[i].b; k++)
+          {
+            const int ti = prims[nodes[i].a + k].index;
+            const Triangle & t = tri[ti]->tri;
+            float4 * w = &packed[12 * leaf + 3 * k];
+            w[0] = make_float4(t.v0[0], t.v0[1], t.v0[2], t.ax[6]);
+            w[1] = make_float4(t.ax[7], t.ax[8], t.ax[0], t.ax[1]);
+            w[2] = make_float4(t.ax[2], t.ax[3], t.ax[4], t.ax[5]);
+            order[4 * leaf + k] = ti;
+          }
+          leaf++;
+        }
+        else writePairNode(nodes, ref, i, &packed[nLeaves * 12]);
+      }
+      int rc;
+      if ((rc = ensure(ctx, ctx->dTriNodes, ctx->triNodesCap, packed.size())) != RFX_OK) return rc;
+      if ((rc = ensure(ctx, ctx->dTriPrims, ctx->triPrimsCap, order.size())) != RFX_OK) return rc;
+      CK(cudaMemcpyAsync(ctx->dTriNodes, packed.data(), packed.size() * sizeof(float4), cudaMemcpyHostToDevice, st));
+      CK(cudaMemcpyAsync(ctx->dTriPrims, order.data(), order.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+      CK(cudaStreamSynchronize(st));
+      ctx->stats.h2d_bytes += packed.size() * sizeof(float4) + order.size() * sizeof(int);
+      h.triPrims = ctx->dTriPrims;
+      h.triLeaf = ctx->dTriNodes;
+      h.triPairs = ctx->dTriNodes + nLeaves * 12;
+      h.triRoot = ref[0];
+      ctx->triBvhTris = tri.size();
+    }
+  }
 
   std::vector<unsigned char> blob(off, 0);
   memcpy(blob.data(), &h, sizeof(h));
@@ -920,6 +1093,7 @@ int renderRange(rfx_ctx * ctx, uint64_t p0, uint64_t p1, uint32_t * argbOut, boo
       w.sigOut = ctx->sigOn ? ctx->dSig : nullptr;
       w.counters = ctx->dCounters;
       w.lightGrids = ctx->lightGridsBuilt > 0;
+      w.triBvh = ctx->triBvhTris > 0;
       cudaEvent_t evA = nullptr, evB = nullptr;
       if (ctx->profiling)
       {
@@ -1052,7 +1226,7 @@ void rfx_destroy(rfx_ctx * ctx)
   for (HostTex & t : ctx->tex) if (t.dev) cudaFree(t.dev);
   cudaFree(ctx->dBlob); cudaFree(ctx->dLut); cudaFree(ctx->dImage); cudaFree(ctx->dSig); cudaFree(ctx->dRng);
   cudaFree(ctx->dRngPrefix); cudaFree(ctx->dRngLocate); cudaFree(ctx->dSampleStates); cudaFree(ctx->dStatus);
-  cudaFree(ctx->dCounters); cudaFree(ctx->dRays); cudaFree(ctx->dBvhNodes); cudaFree(ctx->dBvhPrims); cudaFree(ctx->dEyeCells); cudaFree(ctx->dEyeSpheres); cudaFree(ctx->dEyeIndex); cudaFree(ctx->dLightGrids); cudaFree(ctx->dGridCells); cudaFree(ctx->dGridSpheres); cudaFree(ctx->dGridIndex); cudaFree(ctx->dTileLists[0]); cudaFree(ctx->dTileLists[1]); cudaFree(ctx->dTileCounts);
+  cudaFree(ctx->dCounters); cudaFree(ctx->dRays); cudaFree(ctx->dBvhNodes); cudaFree(ctx->dBvhPrims); cudaFree(ctx->dTriNodes); cudaFree(ctx->dTriPrims); cudaFree(ctx->dEyeCells); cudaFree(ctx->dEyeSpheres); cudaFree(ctx->dEyeIndex); cudaFree(ctx->dLightGrids); cudaFree(ctx->dGridCells); cudaFree(ctx->dGridSpheres); cudaFree(ctx->dGridIndex); cudaFree(ctx->dTileLists[0]); cudaFree(ctx->dTileLists[1]); cudaFree(ctx->dTileCounts);
   for (cudaEvent_t e : ctx->evPool) cudaEventDestroy(e);
   cudaFree(ctx->dResolve); cudaFree(ctx->dQueue); cudaFree(ctx->dQueueCtl); cudaFree(ctx->dOwnBlocks);
   for (int i = 0; i < rfx_ctx::FRAME_SLOTS; i++)
@@ -1152,6 +1326,25 @@ int rfx_add_triangle(rfx_ctx * ctx, const float v[9], int mtype, const float rgb
   return (int)ctx->objs.size() - 1;
 }
 
+int rfx_add_mesh(rfx_ctx * ctx, uint32_t n_vertices, const float * xyz, uint32_t n_tris, const uint32_t * idx, int mtype, const float rgb[3],
+                 float refl, float transp)
+{
+  if (!ctx || !xyz || !idx || !rgb || n_tris == 0) return fail(ctx, RFX_ERR_ARG, "rfx_add_mesh: NULL argument or no triangle");
+  if ((uint64_t)ctx->objs.size() + n_tris > (uint64_t)INT32_MAX) return fail(ctx, RFX_ERR_ARG, "rfx_add_mesh: too many objects");
+  for (uint64_t k = 0; k < 3ull * n_tris; k++)
+    if (idx[k] >= n_vertices) return fail(ctx, RFX_ERR_ARG, "rfx_add_mesh: vertex index out of range");
+  const int first = (int)ctx->objs.size();
+  ctx->objs.reserve(ctx->objs.size() + n_tris);
+  for (uint32_t k = 0; k < n_tris; k++)
+  {
+    float v[9];
+    for (int j = 0; j < 3; j++) memcpy(v + 3 * j, xyz + 3 * (size_t)idx[3 * (size_t)k + j], 12);
+    const int rc = rfx_add_triangle(ctx, v, mtype, rgb, refl, transp);
+    if (rc < 0) return rc;
+  }
+  return first;
+}
+
 int rfx_set_triangle_texture(rfx_ctx * ctx, int object, int texture, const float uv[6])
 {
   if (!ctx || !uv) return fail(ctx, RFX_ERR_ARG, "rfx_set_triangle_texture: NULL argument");
@@ -1213,8 +1406,8 @@ int rfx_set_camera(rfx_ctx * ctx, const float eye[3], const float view[9], float
   memcpy(ctx->eye, eye, sizeof(float) * 3);
   memcpy(ctx->view, view, sizeof(float) * 9);
   ctx->fov = fov;
-  // the BVH's box margins were sized for ray origins inside bvhReach (uploadScene): an eye outside it re-flattens the scene
-  if (ctx->bvhDepth > 0)
+  // the hierarchies' box margins were sized for ray origins inside bvhReach (uploadScene): an eye outside it re-flattens the scene
+  if (ctx->bvhDepth > 0 || ctx->triBvhTris > 0)
     for (int k = 0; k < 3; k++)
       if (!(eye[k] >= ctx->bvhReach[k] && eye[k] <= ctx->bvhReach[3 + k])) ctx->sceneDirty = true;
   return RFX_OK;
@@ -1320,6 +1513,13 @@ int rfx_selftest_light_grid_host(const float light[4], int n_spheres, const floa
   counts[0] = lg.cellStart.size(); counts[1] = lg.index.size();
   if (cell_start && cell_cap >= lg.cellStart.size()) memcpy(cell_start, lg.cellStart.data(), lg.cellStart.size() * sizeof(uint32_t));
   if (items && item_cap >= lg.index.size() && !lg.index.empty()) memcpy(items, lg.index.data(), lg.index.size() * sizeof(int32_t));
+  return RFX_OK;
+}
+
+int rfx_selftest_tri_bounds_host(int n, const float * tris, const float reach[6], float * boxes)
+{
+  if (n < 0 || (n && (!tris || !boxes)) || !reach) return RFX_ERR_ARG;
+  buildTriBoxes(n, tris, reach, boxes);
   return RFX_OK;
 }
 
@@ -1534,6 +1734,7 @@ int rfx_render_strips(rfx_ctx * ctx, uint32_t strip_rows, uint32_t world, uint32
   w.sampleStates = ctx->dSampleStates;
   w.image = nullptr; w.argbOut = argb_device; w.sigOut = nullptr; w.counters = ctx->dCounters;
   w.lightGrids = ctx->lightGridsBuilt > 0;
+  w.triBvh = ctx->triBvhTris > 0;
   cudaEvent_t evA = nullptr, evB = nullptr;
   if (ctx->profiling)
   {
@@ -1700,9 +1901,9 @@ int rfx_trace_rays(rfx_ctx * ctx, int n, const float * origins, const float * ra
   int rc;
   if ((rc = useStream(ctx, st)) != RFX_OK) return rc;
   if ((rc = uploadScene(ctx, st)) != RFX_OK) return rc;
-  if (ctx->bvhDepth > 0)
+  if (ctx->bvhDepth > 0 || ctx->triBvhTris > 0)
   {
-    // the hierarchy's box margins are sized for ray origins inside bvhReach: origins outside it widen the region and re-flatten
+    // the hierarchies' box margins are sized for ray origins inside bvhReach: origins outside it widen the region and re-flatten
     bool outside = false;
     for (int i = 0; i < n; i++)
       for (int k = 0; k < 3; k++)
@@ -1728,7 +1929,7 @@ int rfx_trace_rays(rfx_ctx * ctx, int n, const float * origins, const float * ra
   CK(cudaMemcpyAsync(dO, origins, (size_t)n * 12, cudaMemcpyHostToDevice, st));
   CK(cudaMemcpyAsync(dR, rays, (size_t)n * 12, cudaMemcpyHostToDevice, st));
   ctx->stats.h2d_bytes += (uint64_t)n * 24;
-  ctx->stats.kernel_launches += launchTraceBlobRays(ctx->dBlob, n, dO, dR, reflect_num, ctx->dSampleStates, dC, ctx->dCounters, st);
+  ctx->stats.kernel_launches += launchTraceBlobRays(ctx->dBlob, n, dO, dR, reflect_num, ctx->dSampleStates, dC, ctx->dCounters, st, ctx->triBvhTris > 0);
   CK(cudaGetLastError());
   CK(cudaMemcpyAsync(rgb, dC, (size_t)n * 12, cudaMemcpyDeviceToHost, st));
   CK(cudaStreamSynchronize(st));
@@ -1898,6 +2099,7 @@ int rfx_get_stats(rfx_ctx * ctx, rfx_stats * out)
   }
   ctx->evUsed = 0;
   ctx->stats.light_grids = (uint64_t)ctx->lightGridsBuilt;
+  ctx->stats.bvh_triangles = ctx->triBvhTris;
   *out = ctx->stats;
   return RFX_OK;
 }

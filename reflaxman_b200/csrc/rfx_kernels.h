@@ -96,6 +96,7 @@ struct TraceWork
   unsigned long long * counters;// device [32][2] striped {bounces, shadowRays}
   TileOrder order;              // fast constant-bank kernel only
   bool lightGrids = false;      // blob scenes: the header carries candidate grids for some light (picks the kernel instantiation)
+  bool triBvh = false;          // blob scenes: the header carries a hierarchy over the triangles (picks the kernel instantiation)
   EyeGrid eyeGrid = { nullptr, nullptr, nullptr, 0, 0, 0 };
 };
 // blob scenes (rfx_trace_blob.cu).  launchTraceBlobFast: row-aligned slices (one sample per pixel, grid SSAA, additive jitter; ARGB
@@ -116,7 +117,7 @@ int launchTraceBlobFast(const TraceWork & w, cudaStream_t st, void * queueRecord
 int launchTraceBlobAny(const TraceWork & w, cudaStream_t st);     // every renderNext mode: ragged slices, block preview, signatures
 // Scene::trace for a list of rays (rfx_trace_rays): rays[i] uses sampleStates[i]
 int launchTraceBlobRays(const void * sceneBlob, int n, const float * origins, const float * rays, int reflNum,
-                        const uint32_t * sampleStates, float * rgbOut, unsigned long long * counters, cudaStream_t st);
+                        const uint32_t * sampleStates, float * rgbOut, unsigned long long * counters, cudaStream_t st, bool triBvh);
 // small scenes: constant-bank resident; *fastGrid (optional) receives the CTA count of the fast kernel's grid, 0 when the
 // general kernel ran (the caller keeps tile-order history only for fast launches)
 int launchTraceSmall(const SmallScene & sc, const TraceWork & w, cudaStream_t st, uint32_t * fastGrid = nullptr);

@@ -98,12 +98,63 @@ __device__ __forceinline__ void consider(Hit & best, float dist, int idx, int or
   }
 }
 
+// The pair-node walk of a hierarchy (the spheres' and the triangles'), in the scope of intersectBlob: the slab-test terms ix, iy, iz,
+// oxi, oyi, ozi, the pruning distance reachT (refreshed from best.dist after every leaf), invLen, the per-thread stack and STRIDE.
+// SMEM_: the nodes are in shared memory; PAIRS / ROOT: nodes and root ref; LEAF(slot): the exact test of a leaf's slots;
+// OPEN: false once an any-hit query has its occluder (the walk ends).
+#define RFX_BLOB_WALK(SMEM_, PAIRS, ROOT, LEAF, OPEN)                                                                          \
+  {                                                                                                                          \
+    constexpr int DONE = (int)0x80000000;                                                                                    \
+    const float4 * __restrict__ pn = (PAIRS);                                                                                \
+    int cur = (ROOT);                                                                                                        \
+    int sp = 1;                                                                                                              \
+    stack[0] = DONE;                                                                                                         \
+    _Pragma("unroll 1")                                                                                                      \
+    while (cur != DONE)                                                                                                      \
+    {                                                                                                                        \
+      _Pragma("unroll 1")                                                                                                    \
+      while (cur >= 0)                                                                                                       \
+      {                                                                                                                      \
+        const float4 * q = pn + 4 * cur;                                                                                     \
+        const float4 n0 = SMEM_ ? q[0] : __ldg(q), n1 = SMEM_ ? q[1] : __ldg(q + 1), n2 = SMEM_ ? q[2] : __ldg(q + 2), n3 = SMEM_ ? q[3] : __ldg(q + 3); \
+        const float ax1 = __fmaf_rn(n0.x, ix, oxi), ax2 = __fmaf_rn(n1.x, ix, oxi);                                          \
+        const float ay1 = __fmaf_rn(n0.y, iy, oyi), ay2 = __fmaf_rn(n1.y, iy, oyi);                                          \
+        const float az1 = __fmaf_rn(n0.z, iz, ozi), az2 = __fmaf_rn(n1.z, iz, ozi);                                          \
+        const float bx1 = __fmaf_rn(n2.x, ix, oxi), bx2 = __fmaf_rn(n3.x, ix, oxi);                                          \
+        const float by1 = __fmaf_rn(n2.y, iy, oyi), by2 = __fmaf_rn(n3.y, iy, oyi);                                          \
+        const float bz1 = __fmaf_rn(n2.z, iz, ozi), bz2 = __fmaf_rn(n3.z, iz, ozi);                                          \
+        const float tminA = fmaxf(fmaxf(fminf(ax1, ax2), fminf(ay1, ay2)), fmaxf(fminf(az1, az2), 0.0f));                    \
+        const float tmaxA = fminf(fminf(fmaxf(ax1, ax2), fmaxf(ay1, ay2)), fmaxf(az1, az2));                                 \
+        const float tminB = fmaxf(fmaxf(fminf(bx1, bx2), fminf(by1, by2)), fmaxf(fminf(bz1, bz2), 0.0f));                    \
+        const float tmaxB = fminf(fminf(fmaxf(bx1, bx2), fmaxf(by1, by2)), fmaxf(bz1, bz2));                                 \
+        const bool hitA = tminA <= tmaxA && !(tminA > reachT);                                                               \
+        const bool hitB = tminB <= tmaxB && !(tminB > reachT);                                                               \
+        int ra = __float_as_int(n0.w), rb = __float_as_int(n1.w);                                                            \
+        if (hitA && hitB)                                                                                                    \
+        {                                                                                                                    \
+          if (tminB < tminA) { const int t = ra; ra = rb; rb = t; }                                                          \
+          stack[sp * STRIDE] = rb; sp++;                                                                                     \
+          cur = ra;                                                                                                          \
+        }                                                                                                                    \
+        else if (hitA) cur = ra;                                                                                             \
+        else if (hitB) cur = rb;                                                                                             \
+        else cur = stack[(--sp) * STRIDE];                                                                                   \
+      }                                                                                                                      \
+      if (cur == DONE) break;                                                                                                \
+      LEAF(~cur)                                                                                                             \
+      reachT = (best.dist * 1.001f + 1e-2f) * invLen;                                                                        \
+      cur = (OPEN) ? stack[(--sp) * STRIDE] : DONE;                                                                          \
+    }                                                                                                                        \
+  }
+
 // All objects against one ray; `skip` = object the query ignores (-1 none); anyHit = shadow query (stop at the first hit).
 // STRIDE: threads of the CTA (the traversal stack is one column per thread).  SMEM: bvh points at the CTA's shared-memory copy of
 // the hierarchy (leaf sphere records, then pair nodes), else at the global arrays (read-only path).
 // grid: the candidate grid of the light this (shadow) query runs towards, NULL for bounce queries and for lights that have none.
 // GRIDS = false compiles the candidate-list branch out (the queue-driven kernel, see traceBlob).
-template <int STRIDE, bool SMEM, bool GRIDS>
+// TRIS: the scene has a hierarchy over its triangles (h.triPairs) and the triangles are walked through it instead of one by one;
+// the host picks the instantiation by scene, so the kernels of scenes without one are compiled as before.
+template <int STRIDE, bool SMEM, bool GRIDS, bool TRIS = false>
 __device__ __forceinline__ void intersectBlob(const BlobView & sc, int * __restrict__ stack, V3 o, V3 d, int skip, bool anyHit, Hit & best,
                                               const uint32_t * __restrict__ cellStart, const float4 * __restrict__ itemSphere,
                                               const int * __restrict__ itemIndex, int cell)
@@ -208,47 +259,7 @@ __device__ __forceinline__ void intersectBlob(const BlobView & sc, int * __restr
     // one) and only defers the other to the stack; "while-while": every lane walks to its next leaf, then the warp tests its
     // leaves together.  The bottom stack entry is the end marker.  (Single-box nodes, if-if order and far-child-first were
     // measured slower: profiles/README.md.)
-    constexpr int DONE = (int)0x80000000;
-    const float4 * __restrict__ pn = sc.bvhPairs;
-    int cur = h.bvhRoot;
-    int sp = 1;
-    stack[0] = DONE;
-#pragma unroll 1
-    while (cur != DONE)
-    {
-#pragma unroll 1
-      while (cur >= 0)
-      {
-        const float4 * q = pn + 4 * cur;
-        const float4 n0 = SMEM ? q[0] : __ldg(q), n1 = SMEM ? q[1] : __ldg(q + 1), n2 = SMEM ? q[2] : __ldg(q + 2), n3 = SMEM ? q[3] : __ldg(q + 3);
-        const float ax1 = __fmaf_rn(n0.x, ix, oxi), ax2 = __fmaf_rn(n1.x, ix, oxi);
-        const float ay1 = __fmaf_rn(n0.y, iy, oyi), ay2 = __fmaf_rn(n1.y, iy, oyi);
-        const float az1 = __fmaf_rn(n0.z, iz, ozi), az2 = __fmaf_rn(n1.z, iz, ozi);
-        const float bx1 = __fmaf_rn(n2.x, ix, oxi), bx2 = __fmaf_rn(n3.x, ix, oxi);
-        const float by1 = __fmaf_rn(n2.y, iy, oyi), by2 = __fmaf_rn(n3.y, iy, oyi);
-        const float bz1 = __fmaf_rn(n2.z, iz, ozi), bz2 = __fmaf_rn(n3.z, iz, ozi);
-        const float tminA = fmaxf(fmaxf(fminf(ax1, ax2), fminf(ay1, ay2)), fmaxf(fminf(az1, az2), 0.0f));
-        const float tmaxA = fminf(fminf(fmaxf(ax1, ax2), fmaxf(ay1, ay2)), fmaxf(az1, az2));
-        const float tminB = fmaxf(fmaxf(fminf(bx1, bx2), fminf(by1, by2)), fmaxf(fminf(bz1, bz2), 0.0f));
-        const float tmaxB = fminf(fminf(fmaxf(bx1, bx2), fmaxf(by1, by2)), fmaxf(bz1, bz2));
-        const bool hitA = tminA <= tmaxA && !(tminA > reachT);
-        const bool hitB = tminB <= tmaxB && !(tminB > reachT);
-        int ra = __float_as_int(n0.w), rb = __float_as_int(n1.w);
-        if (hitA && hitB)
-        {
-          if (tminB < tminA) { const int t = ra; ra = rb; rb = t; }
-          stack[sp * STRIDE] = rb; sp++;
-          cur = ra;
-        }
-        else if (hitA) cur = ra;
-        else if (hitB) cur = rb;
-        else cur = stack[(--sp) * STRIDE];
-      }
-      if (cur == DONE) break;
-      RFX_BLOB_LEAF(~cur)
-      reachT = (best.dist * 1.001f + 1e-2f) * invLen;
-      cur = open ? stack[(--sp) * STRIDE] : DONE;
-    }
+    RFX_BLOB_WALK(SMEM, sc.bvhPairs, h.bvhRoot, RFX_BLOB_LEAF, open)
   }
 #undef RFX_BLOB_LEAF
 #undef RFX_BLOB_TAIL
@@ -258,38 +269,100 @@ __device__ __forceinline__ void intersectBlob(const BlobView & sc, int * __restr
   // ---- triangles (Triangle.cpp:53-108): third matrix row first; t = -oz/rz > 2^-63 needs oz, rz nonzero of opposite sign
   const float rzMin = open ? RFX_VSN : __int_as_float(0x7F800000);
   bool openT = open;
-#pragma unroll 1
-  for (int k = 0; k < h.nTris; k++)
+  // the exact test of the list walk below (same operations in the same order) for one leaf slot of the hierarchy; the slot's
+  // position K in the sorted triangle array is read behind the gate, so the skip test comes after it
+#define RFX_BLOB_TRI(K, V0X, V0Y, V0Z, A0, A1, A2, A3, A4, A5, A6, A7, A8)                                     \
+  {                                                                                                            \
+    const float px = o.x - (V0X), py = o.y - (V0Y), pz = o.z - (V0Z);                                          \
+    const float oz = (px * (A6) + py * (A7)) + pz * (A8);                                                      \
+    const float rz = (d.x * (A6) + d.y * (A7)) + d.z * (A8);                                                   \
+    if ((__float_as_int(oz) ^ __float_as_int(rz)) < 0 && fabsf(rz) > rzMin && fabsf(oz) > 0.0f && openT)      \
+    {                                                                                                          \
+      const int ti = h.nSpheres + (K);                                                                         \
+      const float t = -oz / rz;                                       /* Triangle.cpp:61 */                    \
+      if (t > RFX_VSN && ti != skip)                                                                           \
+      {                                                                                                        \
+        const float ox = (px * (A0) + py * (A1)) + pz * (A2);                                                  \
+        const float rx = (d.x * (A0) + d.y * (A1)) + d.z * (A2);                                               \
+        const float oy = (px * (A3) + py * (A4)) + pz * (A5);                                                  \
+        const float ry = (d.x * (A3) + d.y * (A4)) + d.z * (A5);                                               \
+        const float u = ox + t * rx;                                  /* Triangle.cpp:65-66 */                 \
+        const float v = oy + t * ry;                                                                           \
+        if (u >= 0.0f && v >= 0.0f && u + v < 1.0f)                                                           \
+        {                                                                                                      \
+          const float fx = d.x * t, fy = d.y * t, fz = d.z * t;                                                \
+          const float sq = (fx * fx + fy * fy) + fz * fz;                                                      \
+          if (sq > RFX_DELTA * RFX_DELTA)                                                                      \
+          {                                                                                                    \
+            consider(best, sqrtf(sq), ti, sc.mats[ti].order, t, u, v);                                         \
+            if (anyHit) openT = false;                                                                         \
+          }                                                                                                    \
+        }                                                                                                      \
+      }                                                                                                        \
+    }                                                                                                          \
+  }
+  if (TRIS && h.triPairs != nullptr)
   {
-    const int ti = h.nSpheres + k;
-    const Triangle & tr = sc.tris[k];
-    const float px = o.x - tr.v0[0], py = o.y - tr.v0[1], pz = o.z - tr.v0[2];
-    const float oz = (px * tr.ax[6] + py * tr.ax[7]) + pz * tr.ax[8];
-    const float rz = (d.x * tr.ax[6] + d.y * tr.ax[7]) + d.z * tr.ax[8];
-    if ((__float_as_int(oz) ^ __float_as_int(rz)) < 0 && fabsf(rz) > rzMin && fabsf(oz) > 0.0f && ti != skip && openT)
+    // The hierarchy over the triangles (rfx_capi.cu buildTriBoxes: every box holds every point the exact test below can accept,
+    // with margin) selects which triangles get that test, as the sphere hierarchy does.  A leaf is 4 slots of 3 float4 (unused
+    // slots have a zero third row: the gate stays shut); the slot's position in the sorted triangle array is read only behind the
+    // gate.  The stack is free again (the sphere walk has ended); a sphere hit already prunes the boxes behind it.
+    if (openT)
     {
-      const float t = -oz / rz;                                       // Triangle.cpp:61
-      if (t > RFX_VSN)
+      const float ix = fminf(fmaxf(1.0f / d.x, -1e30f), 1e30f), iy = fminf(fmaxf(1.0f / d.y, -1e30f), 1e30f), iz = fminf(fmaxf(1.0f / d.z, -1e30f), 1e30f);
+      const float oxi = -(o.x * ix), oyi = -(o.y * iy), ozi = -(o.z * iz);
+      const float invLen = 1.0f / sqrtf(a);
+      float reachT = (best.dist * 1.001f + 1e-2f) * invLen;
+#define RFX_TRI_LEAF(CA)                                                                                       \
+      {                                                                                                        \
+        _Pragma("unroll 1")                                                                                    \
+        for (int j = (CA); j < (CA) + 4; j++)                                                                  \
+        {                                                                                                      \
+          const float4 * lt = h.triLeaf + 3 * j;                                                               \
+          const float4 q0 = __ldg(lt), q1 = __ldg(lt + 1), q2 = __ldg(lt + 2);                                 \
+          RFX_BLOB_TRI(__ldg(h.triPrims + j), q0.x, q0.y, q0.z, q1.z, q1.w, q2.x, q2.y, q2.z, q2.w, q0.w, q1.x, q1.y) \
+        }                                                                                                      \
+      }
+      RFX_BLOB_WALK(false, h.triPairs, h.triRoot, RFX_TRI_LEAF, openT)
+#undef RFX_TRI_LEAF
+    }
+  }
+  else
+  {
+#pragma unroll 1
+    for (int k = 0; k < h.nTris; k++)
+    {
+      const int ti = h.nSpheres + k;
+      const Triangle & tr = sc.tris[k];
+      const float px = o.x - tr.v0[0], py = o.y - tr.v0[1], pz = o.z - tr.v0[2];
+      const float oz = (px * tr.ax[6] + py * tr.ax[7]) + pz * tr.ax[8];
+      const float rz = (d.x * tr.ax[6] + d.y * tr.ax[7]) + d.z * tr.ax[8];
+      if ((__float_as_int(oz) ^ __float_as_int(rz)) < 0 && fabsf(rz) > rzMin && fabsf(oz) > 0.0f && ti != skip && openT)
       {
-        const float ox = (px * tr.ax[0] + py * tr.ax[1]) + pz * tr.ax[2];
-        const float rx = (d.x * tr.ax[0] + d.y * tr.ax[1]) + d.z * tr.ax[2];
-        const float oy = (px * tr.ax[3] + py * tr.ax[4]) + pz * tr.ax[5];
-        const float ry = (d.x * tr.ax[3] + d.y * tr.ax[4]) + d.z * tr.ax[5];
-        const float u = ox + t * rx;                                  // Triangle.cpp:65-66
-        const float v = oy + t * ry;
-        if (u >= 0.0f && v >= 0.0f && u + v < 1.0f)
+        const float t = -oz / rz;                                       // Triangle.cpp:61
+        if (t > RFX_VSN)
         {
-          const float fx = d.x * t, fy = d.y * t, fz = d.z * t;
-          const float sq = (fx * fx + fy * fy) + fz * fz;
-          if (sq > RFX_DELTA * RFX_DELTA)
+          const float ox = (px * tr.ax[0] + py * tr.ax[1]) + pz * tr.ax[2];
+          const float rx = (d.x * tr.ax[0] + d.y * tr.ax[1]) + d.z * tr.ax[2];
+          const float oy = (px * tr.ax[3] + py * tr.ax[4]) + pz * tr.ax[5];
+          const float ry = (d.x * tr.ax[3] + d.y * tr.ax[4]) + d.z * tr.ax[5];
+          const float u = ox + t * rx;                                  // Triangle.cpp:65-66
+          const float v = oy + t * ry;
+          if (u >= 0.0f && v >= 0.0f && u + v < 1.0f)
           {
-            consider(best, sqrtf(sq), ti, sc.mats[ti].order, t, u, v);
-            if (anyHit) openT = false;
+            const float fx = d.x * t, fy = d.y * t, fz = d.z * t;
+            const float sq = (fx * fx + fy * fy) + fz * fz;
+            if (sq > RFX_DELTA * RFX_DELTA)
+            {
+              consider(best, sqrtf(sq), ti, sc.mats[ti].order, t, u, v);
+              if (anyHit) openT = false;
+            }
           }
         }
       }
     }
   }
+#undef RFX_BLOB_TRI
 
   // ---- planes (Plane.cpp:36-73)
 #pragma unroll 1
@@ -352,7 +425,7 @@ constexpr int MODE_QUEUE = 2;       // paths come from the queue; a lane whose p
 // only part of it) — that kernel keeps walking the hierarchy for every query.  profiles/r2_grid has the measurements.
 // Kernels that serve the batch path are instantiated both ways and the host picks by scene, because the grid branch costs a scene
 // without far lights 4-5 % although it is never taken (registers across the walk).
-template <bool SIG, int MODE, int STRIDE = BLOB_THREADS, bool SMEM = false, bool GRIDS = (MODE != MODE_QUEUE)>
+template <bool SIG, int MODE, int STRIDE = BLOB_THREADS, bool SMEM = false, bool GRIDS = (MODE != MODE_QUEUE), bool TRIS = false>
 __device__ __forceinline__ bool traceBlob(const BlobView & sc, int * __restrict__ stack, V3 & qo, V3 & qd, int reflNumber, V3 randDir,
                                           V3 & mul, V3 & pix, uint32_t & events, uint32_t & sig, QueueFeed * feed = nullptr, int firstSegments = 1,
                                           const EyeGrid * eyeGrid = nullptr, int eyeCell = -1)   // candidates of the first query (origin = eye), or NULL
@@ -432,7 +505,7 @@ __device__ __forceinline__ bool traceBlob(const BlobView & sc, int * __restrict_
       cellStart = eyeGrid->cellStart; itemSphere = eyeGrid->itemSphere; itemIndex = eyeGrid->itemIndex;
       cell = eyeCell;
     }
-    intersectBlob<STRIDE, SMEM, GRIDS>(sc, stack, qo, qd, shadowQuery ? hidx : -1, shadowQuery, hit, cellStart, itemSphere, itemIndex, cell);
+    intersectBlob<STRIDE, SMEM, GRIDS, TRIS>(sc, stack, qo, qd, shadowQuery ? hidx : -1, shadowQuery, hit, cellStart, itemSphere, itemIndex, cell);
 
     bool ended = false;
     if (!shadowQuery)
@@ -593,13 +666,13 @@ __device__ __forceinline__ bool traceBlob(const BlobView & sc, int * __restrict_
 }
 
 // one whole Scene::trace call
-template <bool SIG, bool GRIDS = true>
+template <bool SIG, bool GRIDS = true, bool TRIS = false>
 __device__ __forceinline__ V3 tracePath(const BlobView & sc, int * __restrict__ stack, V3 origin, V3 ray, int reflNumber, V3 randDir, uint32_t & events, uint32_t & sig,
                                         const EyeGrid * eyeGrid = nullptr, int eyeCell = -1)
 {
   V3 qo = origin, qd = ray, mul = mk(1.0f, 1.0f, 1.0f), pix = mk(0.0f, 0.0f, 0.0f);
   events = 0;
-  traceBlob<SIG, MODE_PATH, BLOB_THREADS, false, GRIDS>(sc, stack, qo, qd, reflNumber, randDir, mul, pix, events, sig, nullptr, 1, eyeGrid, eyeCell);
+  traceBlob<SIG, MODE_PATH, BLOB_THREADS, false, GRIDS, TRIS>(sc, stack, qo, qd, reflNumber, randDir, mul, pix, events, sig, nullptr, 1, eyeGrid, eyeCell);
   return pix;
 }
 
@@ -620,7 +693,7 @@ __device__ __forceinline__ void flushBlobCounters(unsigned long long * __restric
 // K2 for row-aligned slices of blob scenes.  MULTI = false: one sample per pixel, no jitter (the batch path of the bench).
 // MULTI = true: the same tiling for grid SSAA (Render.cpp:174-196: the thread walks its s*s samples in the reference's ssx, ssy
 // order so the sum is formed in the same order) and additive jitter / accumulation (Render.cpp:177-178, :196-207).
-template <bool MULTI, bool GRIDS>
+template <bool MULTI, bool GRIDS, bool TRIS = false>
 __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob(const unsigned char * __restrict__ sceneBlob, const __grid_constant__ FrameParams fp,
                                                                 const uint32_t * __restrict__ sampleStates, uint32_t * __restrict__ argbOut,
                                                                 unsigned long long * __restrict__ counters, uint32_t y0, uint32_t y1,
@@ -651,7 +724,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob
       V3 rd;
       rngTriple(s, rd.x, rd.y, rd.z);
       uint32_t events = 0, sig = 0;
-      c = tracePath<false, GRIDS>(sc, stackMem + threadIdx.x, eye, ray, fp.reflNum, rd, events, sig, eg, eyeCell);   // one sample: colour / 1 == colour
+      c = tracePath<false, GRIDS, TRIS>(sc, stackMem + threadIdx.x, eye, ray, fp.reflNum, rd, events, sig, eg, eyeCell);   // one sample: colour / 1 == colour
       nBounces = events & 0xFFFFu; nShadow = events >> 16;
     }
     else
@@ -680,7 +753,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob
                           (px * fp.view[3] + py * fp.view[4]) + fp.rz * fp.view[5],
                           (px * fp.view[6] + py * fp.view[7]) + fp.rz * fp.view[8]);
         uint32_t events = 0, sig = 0;
-        const V3 one = tracePath<false, GRIDS>(sc, stackMem + threadIdx.x, eye, ray, fp.reflNum, rd, events, sig, eg, eyeCell);
+        const V3 one = tracePath<false, GRIDS, TRIS>(sc, stackMem + threadIdx.x, eye, ray, fp.reflNum, rd, events, sig, eg, eyeCell);
         nBounces += events & 0xFFFFu; nShadow += events >> 16;
         c = vadd(c, one);
       }
@@ -728,7 +801,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob
 // queue-driven kernel, and what bounds both is SIMT divergence inside the traversal — the queue-driven kernel issues at
 // 11.5 of 32 lanes although every lane holds a path (ncu, profiles/r2_s7) — not idle lanes and not the L1 pipeline (the
 // shared-memory copy of the hierarchy is worth 1.5 %).
-template <bool GRIDS>
+template <bool GRIDS, bool TRIS = false>
 __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_blob_wave_first(const unsigned char * __restrict__ sceneBlob, const __grid_constant__ FrameParams fp,
                                                                      const uint32_t * __restrict__ sampleStates, uint32_t * __restrict__ argbOut,
                                                                      unsigned long long * __restrict__ counters, uint32_t y0, uint32_t y1, PathQueue queue,
@@ -759,7 +832,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_blob_wave_
     V3 rd;
     rngTriple(s, rd.x, rd.y, rd.z);
     uint32_t sig = 0;
-    alive = !traceBlob<false, MODE_FIRST, BLOB_THREADS, false, GRIDS>(sc, stackMem + threadIdx.x, qo, qd, fp.reflNum, rd, mul, pix, events, sig, nullptr, firstSegments, eg, eyeCell);
+    alive = !traceBlob<false, MODE_FIRST, BLOB_THREADS, false, GRIDS, TRIS>(sc, stackMem + threadIdx.x, qo, qd, fp.reflNum, rd, mul, pix, events, sig, nullptr, firstSegments, eg, eyeCell);
     if (!alive)
     {
       argbOut[q] = packArgb(pix.x, pix.y, pix.z);
@@ -785,7 +858,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_blob_wave_
   flushBlobCounters(counters, nBounces, nShadow, (blockIdx.y * gridDim.x + blockIdx.x) * (BLOB_THREADS / 32) + warp);
 }
 
-template <int THREADS, bool SMEM>
+template <int THREADS, bool SMEM, bool TRIS = false>
 __global__ void __launch_bounds__(THREADS, SMEM ? 2 : RFX_BLOB_MINBLOCKS) k_blob_wave_rest(const unsigned char * __restrict__ sceneBlob, int reflNum,
                                                                     uint32_t * __restrict__ argbSlice,
                                                                     unsigned long long * __restrict__ counters, PathQueue queue)
@@ -814,12 +887,13 @@ __global__ void __launch_bounds__(THREADS, SMEM ? 2 : RFX_BLOB_MINBLOCKS) k_blob
   feed.doneBounces = 0; feed.doneShadow = 0;
   V3 qo = mk(0.0f, 0.0f, 0.0f), qd = qo, mul = qo, pix = qo;
   uint32_t events = 0, sig = 0;
-  traceBlob<false, MODE_QUEUE, THREADS, SMEM>(sc, stackMem + threadIdx.x, qo, qd, reflNum, qo, mul, pix, events, sig, &feed);
+  traceBlob<false, MODE_QUEUE, THREADS, SMEM, false, TRIS>(sc, stackMem + threadIdx.x, qo, qd, reflNum, qo, mul, pix, events, sig, &feed);
   flushBlobCounters(counters, feed.doneBounces, feed.doneShadow, blockIdx.x * (THREADS / 32) + (threadIdx.x >> 5));
 }
 
 // ---- general kernel: every mode of Render::renderNext for blob scenes (arbitrary pixel slices, block preview, signatures; grid SSAA,
 // additive jitter, float image) — the blob counterpart of k_trace_small_any.  One thread per pixel (or per block origin).
+template <bool TRIS = false>
 __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob_any(const unsigned char * __restrict__ sceneBlob, const __grid_constant__ FrameParams fp,
                                                                     const uint32_t * __restrict__ sampleStates, float * __restrict__ image,
                                                                     uint32_t * __restrict__ argbOut, uint32_t * __restrict__ sigOut,
@@ -903,7 +977,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob
                         (px * fp.view[3] + py * fp.view[4]) + fp.rz * fp.view[5],
                         (px * fp.view[6] + py * fp.view[7]) + fp.rz * fp.view[8]);
       uint32_t events = 0;
-      const V3 c = tracePath<true>(sc, stackMem + threadIdx.x, eye, ray, fp.reflNum, rd, events, sig, eg, eyeCell);
+      const V3 c = tracePath<true, true, TRIS>(sc, stackMem + threadIdx.x, eye, ray, fp.reflNum, rd, events, sig, eg, eyeCell);
       nBounces += events & 0xFFFFu; nShadow += events >> 16;
       fin = blockMode ? c : vadd(fin, c);
       if (++ssy == sn) { ssy = 0; ssx++; }                  // ssx outer, ssy inner: the reference's summation order
@@ -935,6 +1009,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob
 }
 
 // ---- Scene::trace for an explicit ray list (rfx_trace_rays): ray i uses sampleStates[i]
+template <bool TRIS = false>
 __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob_rays(const unsigned char * __restrict__ sceneBlob, int n,
                                                                      const float * __restrict__ origins, const float * __restrict__ rays, int reflNum,
                                                                      const uint32_t * __restrict__ sampleStates, float * __restrict__ rgbOut,
@@ -949,7 +1024,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob
     uint32_t s = sampleStates[i], sig = 0;
     V3 rd;
     rngTriple(s, rd.x, rd.y, rd.z);
-    const V3 c = tracePath<false>(sc, stackMem + threadIdx.x, mk(origins[3 * i], origins[3 * i + 1], origins[3 * i + 2]),
+    const V3 c = tracePath<false, true, TRIS>(sc, stackMem + threadIdx.x, mk(origins[3 * i], origins[3 * i + 1], origins[3 * i + 2]),
                                   mk(rays[3 * i], rays[3 * i + 1], rays[3 * i + 2]), reflNum, rd, events, sig);
     rgbOut[3 * i] = c.x; rgbOut[3 * i + 1] = c.y; rgbOut[3 * i + 2] = c.z;
   }
@@ -986,28 +1061,44 @@ int launchTraceBlobFast(const TraceWork & w, cudaStream_t st, void * queueRecord
     if (cudaMemsetAsync(queueCounters, 0, 2 * sizeof(uint32_t), st) != cudaSuccess) return 0;
     PathQueue q;
     q.records = reinterpret_cast<uint4 *>(queueRecords); q.count = queueCounters; q.cursor = queueCounters + 1;
-    if (w.lightGrids || w.eyeGrid.cellStart != nullptr) k_blob_wave_first<true><<<grid, BLOB_THREADS, 0, st>>>(blob, fp, w.sampleStates, w.argbOut, w.counters, y0, y1, q, firstSegments, w.eyeGrid);
-    else k_blob_wave_first<false><<<grid, BLOB_THREADS, 0, st>>>(blob, fp, w.sampleStates, w.argbOut, w.counters, y0, y1, q, firstSegments, w.eyeGrid);
+#define RFX_LAUNCH_FIRST(G, T) k_blob_wave_first<G, T><<<grid, BLOB_THREADS, 0, st>>>(blob, fp, w.sampleStates, w.argbOut, w.counters, y0, y1, q, firstSegments, w.eyeGrid)
+    const bool gridsFirst = w.lightGrids || w.eyeGrid.cellStart != nullptr;
+    if (w.triBvh) { if (gridsFirst) RFX_LAUNCH_FIRST(true, true); else RFX_LAUNCH_FIRST(false, true); }
+    else if (gridsFirst) RFX_LAUNCH_FIRST(true, false);
+    else RFX_LAUNCH_FIRST(false, false);
+#undef RFX_LAUNCH_FIRST
     // the hierarchy in shared memory when it fits next to the stacks of two 512-thread CTAs per SM
     const size_t stackBytes512 = (size_t)BLOB_STACK * 512 * sizeof(int), bvhBytes = (size_t)bvhFloat4 * sizeof(float4);
     if (bvhFloat4 && stackBytes512 + bvhBytes <= 100 * 1024)
     {
-      if (cudaFuncSetAttribute(k_blob_wave_rest<512, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(stackBytes512 + bvhBytes)) != cudaSuccess) return 0;
-      k_blob_wave_rest<512, true><<<persistentCtas / 4, 512, stackBytes512 + bvhBytes, st>>>(blob, fp.reflNum, w.argbOut + fp.p0, w.counters, q);
+      // (the triangle hierarchy, if any, stays in global memory and L1)
+      const auto kRest = w.triBvh ? k_blob_wave_rest<512, true, true> : k_blob_wave_rest<512, true, false>;
+      if (cudaFuncSetAttribute(kRest, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(stackBytes512 + bvhBytes)) != cudaSuccess) return 0;
+      kRest<<<persistentCtas / 4, 512, stackBytes512 + bvhBytes, st>>>(blob, fp.reflNum, w.argbOut + fp.p0, w.counters, q);
     }
     else
-      k_blob_wave_rest<BLOB_THREADS, false><<<persistentCtas, BLOB_THREADS, (size_t)BLOB_STACK * BLOB_THREADS * sizeof(int), st>>>(blob, fp.reflNum, w.argbOut + fp.p0, w.counters, q);
+    {
+      const auto kRest = w.triBvh ? k_blob_wave_rest<BLOB_THREADS, false, true> : k_blob_wave_rest<BLOB_THREADS, false, false>;
+      kRest<<<persistentCtas, BLOB_THREADS, (size_t)BLOB_STACK * BLOB_THREADS * sizeof(int), st>>>(blob, fp.reflNum, w.argbOut + fp.p0, w.counters, q);
+    }
     return 2;
   }
   // 128-bit framebuffer stores need a 16-byte aligned frame: a caller's offset sub-buffer goes to the general kernel
   if (w.argbOut && (fp.W & 3u) == 0u && (reinterpret_cast<uintptr_t>(w.argbOut) & 15u) != 0u) return 0;
   const bool multi = !(fp.sampleNum == 1 && !fp.jitter);
-#define RFX_LAUNCH_BLOB(M, G) k_trace_blob<M, G><<<grid, BLOB_THREADS, 0, st>>>(blob, fp, w.sampleStates, w.argbOut, w.counters, y0, y1, w.image, w.eyeGrid)
+#define RFX_LAUNCH_BLOB(M, G, T) k_trace_blob<M, G, T><<<grid, BLOB_THREADS, 0, st>>>(blob, fp, w.sampleStates, w.argbOut, w.counters, y0, y1, w.image, w.eyeGrid)
   const bool grids = w.lightGrids || w.eyeGrid.cellStart != nullptr;
-  if (!multi && grids) RFX_LAUNCH_BLOB(false, true);
-  else if (!multi) RFX_LAUNCH_BLOB(false, false);
-  else if (grids) RFX_LAUNCH_BLOB(true, true);
-  else RFX_LAUNCH_BLOB(true, false);
+  if (w.triBvh)
+  {
+    if (!multi && grids) RFX_LAUNCH_BLOB(false, true, true);
+    else if (!multi) RFX_LAUNCH_BLOB(false, false, true);
+    else if (grids) RFX_LAUNCH_BLOB(true, true, true);
+    else RFX_LAUNCH_BLOB(true, false, true);
+  }
+  else if (!multi && grids) RFX_LAUNCH_BLOB(false, true, false);
+  else if (!multi) RFX_LAUNCH_BLOB(false, false, false);
+  else if (grids) RFX_LAUNCH_BLOB(true, true, false);
+  else RFX_LAUNCH_BLOB(true, false, false);
 #undef RFX_LAUNCH_BLOB
   return 1;
 }
@@ -1036,16 +1127,18 @@ int launchTraceBlobAny(const TraceWork & w, cudaStream_t st)
   }
   if (nThreads == 0) return 0;
   const uint32_t blocks = (uint32_t)((nThreads + BLOB_THREADS - 1) / BLOB_THREADS);
-  k_trace_blob_any<<<blocks, BLOB_THREADS, 0, st>>>(reinterpret_cast<const unsigned char *>(w.sceneBlob), fp, w.sampleStates, w.image, w.argbOut, w.sigOut,
-                                                    w.counters, tiled, w.eyeGrid);
+  const auto kAny = w.triBvh ? k_trace_blob_any<true> : k_trace_blob_any<false>;
+  kAny<<<blocks, BLOB_THREADS, 0, st>>>(reinterpret_cast<const unsigned char *>(w.sceneBlob), fp, w.sampleStates, w.image, w.argbOut, w.sigOut,
+                                        w.counters, tiled, w.eyeGrid);
   return 1;
 }
 
 int launchTraceBlobRays(const void * sceneBlob, int n, const float * origins, const float * rays, int reflNum,
-                        const uint32_t * sampleStates, float * rgbOut, unsigned long long * counters, cudaStream_t st)
+                        const uint32_t * sampleStates, float * rgbOut, unsigned long long * counters, cudaStream_t st, bool triBvh)
 {
   if (n <= 0) return 0;
-  k_trace_blob_rays<<<(n + BLOB_THREADS - 1) / BLOB_THREADS, BLOB_THREADS, 0, st>>>(reinterpret_cast<const unsigned char *>(sceneBlob), n, origins, rays, reflNum,
+  const auto kRays = triBvh ? k_trace_blob_rays<true> : k_trace_blob_rays<false>;
+  kRays<<<(n + BLOB_THREADS - 1) / BLOB_THREADS, BLOB_THREADS, 0, st>>>(reinterpret_cast<const unsigned char *>(sceneBlob), n, origins, rays, reflNum,
                                                                                     sampleStates, rgbOut, counters);
   return 1;
 }

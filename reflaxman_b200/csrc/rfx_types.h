@@ -78,6 +78,13 @@ struct SceneHeader
   const float4 * bvhLeafSph;        // the same slots as (cx, cy, cz, r^2), NaN = unused: a leaf is 4 contiguous records
   uint32_t bvhFloat4;               // float4 count of [leaf records | pair nodes], contiguous from bvhLeafSph (what a CTA copies to shared memory)
   const LightGrid * lightGrids;     // [nLights] when the hierarchy exists and some light is far enough for a grid, else NULL
+  // hierarchy over the triangles (rfx_capi.cu buildTriBoxes), walked after the spheres; triPairs == NULL: list walk.  Same pair-node
+  // format and leaf refs as the sphere hierarchy; a leaf slot is 3 float4 {v0.xyz, ax6} {ax7, ax8, ax0, ax1} {ax2, ax3, ax4, ax5}
+  // (as SmallScene::triPk), all zero in unused slots (ax row 3 = 0: |rz| > 2^-63 never holds)
+  const int * triPrims;             // position in the sorted triangle array of each leaf slot, 4 slots per leaf (-1 = unused)
+  const float4 * triLeaf;           // 3 float4 per slot, then the pair nodes
+  const float4 * triPairs;
+  int triRoot;
 };
 
 // Small scenes travel as a kernel parameter (constant bank): see rfx_trace_small.cu

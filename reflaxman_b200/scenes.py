@@ -9,7 +9,11 @@ A scene is a plain dict of float32 data (no classes), mirroring what the referen
      "lights": [(origin[3], radius, rgb[3], power), ...],
      "objects": [("sphere", center[3], radius, mtype, rgb[3], refl, transp) |
                  ("tri", v[9], mtype, rgb[3], refl, transp, tex_index_or_-1, uv[6]) |
-                 ("plane", pos[3], norm[3], mtype, rgb[3], refl, transp), ...]}   # insertion order matters (ties)
+                 ("plane", pos[3], norm[3], mtype, rgb[3], refl, transp) |
+                 ("mesh", xyz[N,3], idx[M,3], mtype, rgb[3], refl, transp), ...]}   # insertion order matters (ties)
+
+A "mesh" is M triangles with one material, triangle k = vertices xyz[idx[k]] (rfx_add_mesh); :func:`expand_meshes` turns it into
+the M "tri" objects it stands for, which is what the reference's Scene (it has no mesh call) and the oracle take.
 
 Material types follow reference Material.h:8: 0 = mtMetal, 1 = mtDielectric.
 Nothing here touches the GPU; :mod:`reflaxman_b200.capi` uploads a scene through the C ABI.
@@ -115,6 +119,50 @@ def synthetic_scene(n_side=32, floor=None, skybox=None, seed=0x9E3779B9, back_wa
         "lights": [((11.8e9, 4.26e9, 3.08e9), 3.48e8, (1.0, 1.0, 0.95), 0.85)],
         "objects": objs,
     }
+
+
+def torus_mesh(n_u, n_v, major=2.2, minor=0.6, center=(0.0, 2.6, 0.0), tilt=1.0):
+    """An indexed torus of 2 * n_u * n_v triangles: n_u segments around the ring, n_v around the tube, the ring's axis tilted by
+    ``tilt`` radians about x.  Returns (xyz float32 [n_u * n_v, 3], idx uint32 [2 * n_u * n_v, 3]); the triangles face outwards."""
+    u = 2.0 * np.pi * np.arange(n_u) / n_u
+    v = 2.0 * np.pi * np.arange(n_v) / n_v
+    uu, vv = np.meshgrid(u, v, indexing="ij")
+    ring = major + minor * np.cos(vv)
+    x, y, z = ring * np.cos(uu), minor * np.sin(vv), ring * np.sin(uu)
+    c, s = math.cos(tilt), math.sin(tilt)
+    y, z = c * y - s * z, s * y + c * z
+    xyz = np.stack([x + center[0], y + center[1], z + center[2]], axis=-1).reshape(-1, 3).astype(np.float32)
+    i, j = np.meshgrid(np.arange(n_u), np.arange(n_v), indexing="ij")
+    a = i * n_v + j
+    b = ((i + 1) % n_u) * n_v + j
+    cc = ((i + 1) % n_u) * n_v + (j + 1) % n_v
+    d = i * n_v + (j + 1) % n_v
+    idx = np.stack([np.stack([a, cc, b], axis=-1), np.stack([a, d, cc], axis=-1)], axis=2).reshape(-1, 3).astype(np.uint32)
+    return xyz, idx
+
+
+def mesh_scene(n_u, n_v, spheres=0, floor=None, skybox=None):
+    """A reflective metal torus of 2 * n_u * n_v triangles (:func:`torus_mesh`) in view of the default camera, over the textured floor
+    and back wall of :func:`synthetic_scene`; ``spheres`` = n_side > 0 keeps that scene's n_side^2 spheres too."""
+    base = synthetic_scene(max(spheres, 1), floor=floor, skybox=skybox)
+    objs = [ob for ob in base["objects"] if spheres or ob[0] != "sphere"]
+    xyz, idx = torus_mesh(n_u, n_v)
+    objs.append(("mesh", xyz, idx, MT_METAL, (0.95, 0.8, 0.55), 0.85, 0.0))
+    base["objects"] = objs
+    return base
+
+
+def expand_meshes(scene):
+    """The same scene with every "mesh" object replaced by its triangles, in order (untextured "tri" objects)."""
+    objs = []
+    for ob in scene["objects"]:
+        if ob[0] != "mesh":
+            objs.append(ob)
+            continue
+        _, xyz, idx, mt, col, refl, tr = ob
+        v = np.asarray(xyz, np.float32)[np.asarray(idx, np.int64)].reshape(-1, 9)
+        objs.extend(("tri", tuple(float(x) for x in row), mt, col, refl, tr, -1, (0.0, 0.0, 0.0, 0.0, 0.0, 0.0)) for row in v)
+    return dict(scene, objects=objs)
 
 
 def synthetic_texture(w, h, seed, alpha=True):
