@@ -1,4 +1,4 @@
-// rfx_kernels.h — launch interface between the C-ABI host layer (rfx_capi.cu) and the sm_100a kernels (rfx_kernels.cu: K1 and K3;
+// rfx_kernels.h — launch interface between the C-ABI host layer (rfx_capi.cu, rfx_scene.cpp) and the sm_100a kernels (rfx_kernels.cu: K1 and K3;
 // rfx_trace_small.cu, rfx_trace_blob.cu: K2).
 #pragma once
 #include <cuda_runtime.h>

@@ -9,7 +9,7 @@
 // It is the structure of the constant-bank kernel (rfx_trace_small.cu) applied to the scene blob in global memory:
 //   * Scene::trace as a per-lane state machine with ONE traversal site: the query in flight is the bounce segment (closest
 //     hit) or the shadow ray of light li (any hit).
-//   * The BVH over the spheres (built by rfx_capi.cu, every box inflated beyond the rounding noise of the exact test) only
+//   * The BVH over the spheres (built by rfx_scene.cpp, every box inflated beyond the rounding noise of the exact test) only
 //     selects which spheres get the reference's exact test.  It is walked over PAIR NODES (both children's boxes in the parent,
 //     four 16-byte loads per trip): the walk continues into the nearer hit child in a register and defers the other one to a
 //     stack in shared memory (one column per thread); "while-while" order — every lane walks to its next leaf, then the warp
@@ -17,7 +17,7 @@
 //     the constant-bank kernel.  The slab test is the one piece of arithmetic here that is not the reference's, so it is fused.
 //   * Shadow queries towards a FAR light do not walk the hierarchy: their rays are nearly parallel, so the host bins the spheres'
 //     (inflated) shadows on a plane across the light's direction and the query tests the candidate list of its origin's cell with
-//     the exact arithmetic (LightGrid, rfx_capi.cu buildLightGrid) — an any-hit query only asks whether something is hit.
+//     the exact arithmetic (LightGrid, rfx_scene.cpp buildLightGrid) — an any-hit query only asks whether something is hit.
 //   * Neither does the FIRST query of a path: every path starts at the eye, so the host bins the spheres' primary-ray screen bounds
 //     into 32x32-pixel cells per camera (EyeGrid, buildEyeGrid) and the 32 lanes of a tile walk the same short list.
 //     (Both lists go through the same branch of intersectBlob; the queue-driven kernel is compiled without it: traceBlob.)
@@ -244,7 +244,7 @@ __device__ __forceinline__ void intersectBlob(const BlobView & sc, int * __restr
   }
   else
   {
-    // Slab test.  The hierarchy only selects candidates for the exact test and its boxes carry margins (rfx_capi.cu), so — unlike
+    // Slab test.  The hierarchy only selects candidates for the exact test and its boxes carry margins (rfx_scene.cpp), so — unlike
     // everything the reference computes — this arithmetic may be fused: t = box * (1/d) - origin * (1/d) is one FFMA per plane
     // instead of a subtraction and a multiplication.  Its error moves a box plane by at most 2^-22 |origin| along the axis, which
     // the margins' 1e-6 * R term covers.  The reciprocals are clamped to +-1e30 so that an axis-parallel ray (1/0 = inf) gives
@@ -303,7 +303,7 @@ __device__ __forceinline__ void intersectBlob(const BlobView & sc, int * __restr
   }
   if (TRIS && h.triPairs != nullptr)
   {
-    // The hierarchy over the triangles (rfx_capi.cu buildTriBoxes: every box holds every point the exact test below can accept,
+    // The hierarchy over the triangles (rfx_scene.cpp buildTriBoxes: every box holds every point the exact test below can accept,
     // with margin) selects which triangles get that test, as the sphere hierarchy does.  A leaf is 4 slots of 3 float4 (unused
     // slots have a zero third row: the gate stays shut); the slot's position in the sorted triangle array is read only behind the
     // gate.  The stack is free again (the sphere walk has ended); a sphere hit already prunes the boxes behind it.
@@ -477,7 +477,7 @@ __device__ __forceinline__ bool traceBlob(const BlobView & sc, int * __restrict_
     }
     Hit hit;
     hit.dist = FLT_MAX; hit.idx = -1; hit.order = 0x7FFFFFFF; hit.t = 0; hit.u = 0; hit.v = 0;
-    // Candidate lists.  A shadow query towards a far light: the cell of its origin in the light's grid (rfx_capi.cu, buildLightGrid;
+    // Candidate lists.  A shadow query towards a far light: the cell of its origin in the light's grid (rfx_scene.cpp, buildLightGrid;
     // an origin outside the grid lies outside every sphere's inflated shadow).  The first query of a path: the screen cell of its
     // pixel in the camera's grid (buildEyeGrid).  Everything else walks the hierarchy.
     const uint32_t * cellStart = nullptr;

@@ -1,4 +1,4 @@
-// rfx_types.h — POD records shared by the host flattening code (rfx_capi.cu) and the sm_100a kernels (rfx_kernels.cu).
+// rfx_types.h — POD records shared by the host flattening code (rfx_scene.cpp) and the sm_100a kernels (rfx_kernels.cu).
 //
 // HBM layout of a scene ("scene blob", one contiguous allocation, read in place by k_trace):
 //   SceneHeader | Light[nLights] | float4 sphere[nSpheres] (cx,cy,cz,r^2) | Triangle[nTris] | Plane[nPlanes] |
@@ -50,7 +50,7 @@ struct TexRef
   uint32_t w, h;
 };
 
-// Shadow-ray candidates of one far light (built by rfx_capi.cu next to the hierarchy, walked by rfx_trace_blob.cu).  Every shadow ray
+// Shadow-ray candidates of one far light (built by rfx_scene.cpp next to the hierarchy, walked by rfx_trace_blob.cu).  Every shadow ray
 // towards the light is nearly parallel to the direction from the scene to the light, so the spheres it can hit are the ones whose
 // (inflated) shadow on a plane across that direction covers the ray's origin: a 2-D grid of candidate lists over that plane.
 struct LightGrid
@@ -78,7 +78,7 @@ struct SceneHeader
   const float4 * bvhLeafSph;        // the same slots as (cx, cy, cz, r^2), NaN = unused: a leaf is 4 contiguous records
   uint32_t bvhFloat4;               // float4 count of [leaf records | pair nodes], contiguous from bvhLeafSph (what a CTA copies to shared memory)
   const LightGrid * lightGrids;     // [nLights] when the hierarchy exists and some light is far enough for a grid, else NULL
-  // hierarchy over the triangles (rfx_capi.cu buildTriBoxes), walked after the spheres; triPairs == NULL: list walk.  Same pair-node
+  // hierarchy over the triangles (rfx_scene.cpp buildTriBoxes), walked after the spheres; triPairs == NULL: list walk.  Same pair-node
   // format and leaf refs as the sphere hierarchy; a leaf slot is 3 float4 {v0.xyz, ax6} {ax7, ax8, ax0, ax1} {ax2, ax3, ax4, ax5}
   // (as SmallScene::triPk), all zero in unused slots (ax row 3 = 0: |rz| > 2^-63 never holds)
   const int * triPrims;             // position in the sorted triangle array of each leaf slot, 4 slots per leaf (-1 = unused)

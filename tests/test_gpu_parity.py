@@ -573,7 +573,7 @@ def _with_lights(scene, lights):
 @pytest.mark.parametrize("case", ["far", "overhead", "grazing", "far+near", "near", "two_far"])
 def test_light_grid_equals_hierarchy_walk(capi, case):
     """Scenes with a sphere hierarchy answer the shadow queries of far lights from a grid of candidate spheres across the light's
-    direction (rfx_capi.cu buildLightGrid) instead of walking the hierarchy.  The query is an any-hit query (Scene.cpp:131-143), so
+    direction (rfx_scene.cpp buildLightGrid) instead of walking the hierarchy.  The query is an any-hit query (Scene.cpp:131-143), so
     a complete candidate list gives the same answer: frames, ray counts and the stream position are identical with the grids
     on and off — far light (config 4's), straight overhead, grazing (long shadows), a far and a near light together (the near
     one keeps the hierarchy), near light only (no grid), two far lights; tile kernel, wavefront pair and general kernel."""
@@ -655,7 +655,7 @@ def test_light_grid_random_scenes(capi, seed):
 @pytest.mark.parametrize("which", ["grid16", "cloud"])
 def test_eye_grid_equals_hierarchy_walk(capi, which):
     """Scenes with a sphere hierarchy take the candidates of a path's FIRST query (origin = eye) from a screen grid the host bins per
-    camera out of the spheres' primary-ray bounds (rfx_capi.cu buildEyeGrid) instead of walking the hierarchy.  Cameras all over the
+    camera out of the spheres' primary-ray bounds (rfx_scene.cpp binEyeGrid) instead of walking the hierarchy.  Cameras all over the
     place — orbit, inside spheres, under the floor, looking away, fov 0.3..2.6: frames, ray counts and stream positions are identical
     with the grid on and off; tile kernel (depth 1 and 2), wavefront pair (depth 6), 2x2 SSAA through the Render API, and the general
     kernel on ragged renderNext slices with identical hit-path signatures."""

@@ -1,7 +1,7 @@
 """CPU tests of the two host-side bound computations the kernels' skipping rests on (pure host functions of the C-ABI library: no
 GPU, no context), each against the kernels' float32 expressions evaluated op for op in numpy:
   * primary-ray screen bounds (rfx_trace_small.cu makePrimaryCull): no pixel outside an object's rectangle passes its accept test;
-  * shadow-ray candidate grids of far lights (rfx_capi.cu buildLightGrid): every sphere a jittered shadow ray passes the gate of is
+  * shadow-ray candidate grids of far lights (rfx_scene.cpp buildLightGrid): every sphere a jittered shadow ray passes the gate of is
     listed in the grid cell of the ray's origin."""
 import math
 import os

@@ -170,7 +170,7 @@ def check(eye, view, fov, W, H, spheres, tris, offsets=((0.0, 0.0),)):
 
 
 def scene_arrays(scene):
-    """spheres and triangles of a scenes.py dict as the kernel sees them (float32 flattening of rfx_capi.cu restated in numpy)."""
+    """spheres and triangles of a scenes.py dict as the kernel sees them (float32 flattening of rfx_scene.cpp restated in numpy)."""
     sph, tris = [], []
     for ob in scene["objects"]:
         if ob[0] == "sphere":
