@@ -223,7 +223,7 @@ RFX_API int rfx_set_option(rfx_ctx * ctx, const char * name, int64_t value);
 RFX_API int rfx_force_path(rfx_ctx * ctx, int path);
 /* acceleration structures of the blob kernels: 0 = automatic (a bounding-volume hierarchy over the spheres when there are more than
  * 32 and the scene holds no unbounded plane; one over the triangles, walked after the spheres, when there are more than 32 triangles
- * and no plane), 1 = always (spheres: whenever there are any; triangles: whenever there are any and no plane), 2 = never (the
+ * and no plane), 1 = always (whenever there are any spheres / triangles and no plane), 2 = never (the
  * reference's brute-force list walk).  Results are identical; tests compare them. */
 RFX_API int rfx_set_bvh_mode(rfx_ctx * ctx, int mode);
 /* cost-ordered tile scheduling of the constant-bank fast kernel: launches record which tiles held long paths (every

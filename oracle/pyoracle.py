@@ -19,6 +19,7 @@ from reflaxman_b200.build import REFERENCE_SRC   # where the unmodified referenc
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 PORT_SO = os.path.join(HERE, "librfx_oracle.so")
+POWCR_SO = os.path.join(HERE, "librfx_oracle_powcr.so")   # both power sites as the GPU computes them (RFXO_POW_CR)
 REF_DIR = os.path.join(HERE, "_ref")
 
 _fp = C.POINTER(C.c_float)
@@ -58,7 +59,7 @@ def lib(path=None):
         return _lib
     so = path or PORT_SO
     if not os.path.exists(so):
-        build(ref=False)
+        build(ref=False)   # `make port` builds every port library, the default one and the variants
     L = C.CDLL(so)
     L.rfxo_scene_new.restype = C.c_void_p
     L.rfxo_scene_new.argtypes = [_fp, C.c_float]
@@ -72,6 +73,7 @@ def lib(path=None):
     L.rfxo_get_triangle.argtypes = [C.c_void_p, C.c_int, _fp, _fp, _fp]
     L.rfxo_get_env.argtypes = [C.c_void_p, _fp, _fp]
     L.rfxo_trace_one.argtypes = [C.c_void_p, _fp, _fp, C.c_int, _fp, _fp, _u32p]
+    L.rfxo_trace_many.argtypes = [C.c_void_p, C.c_int, _fp, _fp, C.c_int, _fp, _fp, _u32p]
     L.rfxo_rand_dirs.argtypes = [_u32p, C.c_uint64, _fp]
     L.rfxo_plane_probe.argtypes = [_fp, C.c_int, _fp]
     L.rfxo_render_pass.restype = C.c_int
@@ -83,6 +85,17 @@ def lib(path=None):
     if path is None:
         _lib = L
     return L
+
+
+_lib_powcr = None
+
+
+def lib_powcr():
+    """The oracle built with -DRFXO_POW_CR (cached apart from :func:`lib`): the GPU's arithmetic, powers included."""
+    global _lib_powcr
+    if _lib_powcr is None:
+        _lib_powcr = lib(POWCR_SO)
+    return _lib_powcr
 
 
 def _f(a):
@@ -195,6 +208,21 @@ def rand_dirs(seed, n):
     out = np.zeros((n, 3), np.float32)
     lib().rfxo_rand_dirs(s.ctypes.data_as(_u32p), n, out.ctypes.data_as(_fp))
     return out, int(s[0])
+
+
+def trace_many(scene, origins, rays, refl, seed, L=None):
+    """Scene::trace for a ray list, as rfx_trace_rays runs it: ray i takes the i-th direction of the stream that starts at
+    ``seed``.  ``scene``: an :class:`OracleScene` or a scenes.py dict.  Returns (rgb [n, 3], signatures [n], stream end state)."""
+    sc = scene if isinstance(scene, OracleScene) else OracleScene(scene, L)
+    o = np.ascontiguousarray(origins, dtype=np.float32).reshape(-1, 3)
+    r = np.ascontiguousarray(rays, dtype=np.float32).reshape(-1, 3)
+    n = o.shape[0]
+    dirs, end = rand_dirs(seed, n)
+    rgb = np.zeros((n, 3), np.float32)
+    sig = np.zeros(n, np.uint32)
+    sc.L.rfxo_trace_many(sc.h, n, o.ctypes.data_as(_fp), r.ctypes.data_as(_fp), refl, dirs.ctypes.data_as(_fp),
+                         rgb.ctypes.data_as(_fp), sig.ctypes.data_as(_u32p))
+    return rgb, sig, end
 
 
 def plane_probe(inputs):

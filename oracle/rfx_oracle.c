@@ -46,6 +46,15 @@ static inline float MUL(float a, float b) { CNT(1); return a * b; }
 static inline float DIV(float a, float b) { CNT(2); return a / b; }
 static inline float SQRT(float a) { CNT(3); return sqrtf(a); }
 static inline float POWF(float a, float b) { CNT(4); return powf(a, b); }
+#ifdef RFXO_POW_CR
+/* -DRFXO_POW_CR: each power site computes what the GPU computes there (rfx_device.cuh): the specular power as the correctly
+ * rounded x^y, the Fresnel cube as the binary64 cube rounded once.  Per site, not by exponent: the specular exponent can be 3. */
+static inline float POW_SPEC(float a, float b) { CNT(4); return (float)pow((double)a, (double)b); }
+static inline float POW_CUBE(float a) { CNT(4); const double d = (double)a; return (float)((d * d) * d); }
+#else
+static inline float POW_SPEC(float a, float b) { return POWF(a, b); }
+static inline float POW_CUBE(float a) { return POWF(a, 3.0f); }
+#endif
 
 #define VSN 1.08420217248550443e-19f /* sqrtf(FLT_MIN) = 2^-63 exactly, trace_math.h:17 */
 #define DELTA 0.0001f                /* trace_math.h:18 */
@@ -607,7 +616,7 @@ static C3 scene_trace(const rfxo_scene * s, V3 origin, V3 ray, int reflNumber, V
                 if (lightRadius > VSN)
                 {
                   k->spec_pow++;
-                  specPower = MUL(POWF(specPower, ADD(1, DIV(MUL(MUL(3, hit.mat.reflectivity), dropToLightLen), lightRadius))), hit.mat.reflectivity);
+                  specPower = MUL(POW_SPEC(specPower, ADD(1, DIV(MUL(MUL(3, hit.mat.reflectivity), dropToLightLen), lightRadius))), hit.mat.reflectivity);
                   sumSpecColor = c_add(sumSpecColor, c_scale(lightColor, specPower));
                 }
               }
@@ -626,7 +635,7 @@ static C3 scene_trace(const rfxo_scene * s, V3 origin, V3 ray, int reflNumber, V
         const float a = MUL(rayLen, normLen);
         const float dropAngleCos = (a > VSN) ? clampf(DIV(v_dot(ray, v_neg(hit.norm)), a), 0.0f, 1.0f) : 0.0f;
         k->fresnel_pow++;
-        const float rf = ADD(0.2f, MUL(0.8f, POWF(SUB(1.0f, dropAngleCos), 3.0f)));
+        const float rf = ADD(0.2f, MUL(0.8f, POW_CUBE(SUB(1.0f, dropAngleCos))));
         finColor = c_add(c_mul(c_scale(color, SUB(1.0f, rf)), sumLightColor), sumSpecColor);
         finColor = c_mul(finColor, mulColor);
         mulColor = c_scale(mulColor, rf);
@@ -667,6 +676,16 @@ void rfxo_trace_one(const rfxo_scene * s, const float origin[3], const float ray
   const C3 c = scene_trace(s, v3(origin[0], origin[1], origin[2]), v3(ray[0], ray[1], ray[2]), refl, v3(randDir[0], randDir[1], randDir[2]), &k, &h);
   rgb[0] = c.r; rgb[1] = c.g; rgb[2] = c.b;
   if (sig) *sig = h;
+}
+
+/* n independent Scene::trace calls (rfx_trace_rays' operation): ray i from origins[3i] along rays[3i] with randDirs[3i];
+ * rgb and sig (may be NULL) receive 3 floats / one signature per ray */
+void rfxo_trace_many(const rfxo_scene * s, int n, const float * origins, const float * rays, int refl, const float * randDirs,
+                     float * rgb, uint32_t * sig)
+{
+  for (int i = 0; i < n; i++)
+    rfxo_trace_one(s, origins + 3 * (size_t)i, rays + 3 * (size_t)i, refl, randDirs + 3 * (size_t)i, rgb + 3 * (size_t)i,
+                   sig ? sig + i : NULL);
 }
 
 /* Plane::trace (Plane.cpp:36-73) on n independent (pos, norm, origin, ray) inputs of 12 floats each, for the pin against the

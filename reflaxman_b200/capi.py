@@ -443,8 +443,8 @@ class Context:
         self._ck(self.L.rfx_force_path(self.h, path), "rfx_force_path")
 
     def set_bvh_mode(self, mode):
-        """0 automatic (hierarchies over the spheres / the triangles when there are more than 32 of them and no plane), 1 always,
-        2 never (list walk)."""
+        """0 automatic (hierarchies over the spheres / the triangles when there are more than 32 of them and no plane), 1 always
+        (whenever there are any and no plane), 2 never (list walk)."""
         self._ck(self.L.rfx_set_bvh_mode(self.h, mode), "rfx_set_bvh_mode")
 
     def set_tile_ordering(self, on=True):

@@ -469,8 +469,9 @@ int buildSceneImage(const HostScene & s, SceneImage & img, std::string & err)
 
   // automatic mode: more than 32 spheres, and no planes — a drop point on an (unbounded) plane can lie anywhere, so the box margins
   // below, which are sized for ray origins inside a bounded region, could not be guaranteed (the reference's Scene cannot hold
-  // planes at all; mode 1 builds the hierarchy regardless, for tests)
-  const bool wantBvh = s.bvhMode == 1 ? !sph.empty() : s.bvhMode == 2 ? false : (sph.size() > 32 && pla.empty());
+  // planes at all).  Mode 1 builds it for any sphere, but never next to a plane either: a bounce off the plane far outside the
+  // reach box would walk boxes whose margins do not cover its origin and could lose an occluder or a hit the list walk finds.
+  const bool wantBvh = pla.empty() && (s.bvhMode == 1 ? !sph.empty() : s.bvhMode == 2 ? false : sph.size() > 32);
   // the hierarchy over the triangles: the same automatic rule; mode 1 builds it for any triangle, but never next to a plane (its
   // margins need bounded drop points)
   const bool wantTriBvh = pla.empty() && (s.bvhMode == 1 ? !tri.empty() : s.bvhMode == 2 ? false : tri.size() > 32);

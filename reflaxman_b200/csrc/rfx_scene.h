@@ -50,7 +50,7 @@ struct HostScene
   std::vector<HostObj> objs;
   std::vector<HostTex> tex;                 // uploaded before the image is built: TexRef and SmallScene carry their device pointers
   int skyTex = -1;
-  int bvhMode = 0;                          // 0 auto (spheres > 32, triangles > 32), 1 always, 2 never — tests compare both
+  int bvhMode = 0;                          // 0 auto (spheres > 32, triangles > 32), 1 always, 2 never (no plane: 0, 1) — tests compare them
   bool lightGridsOn = true;                 // rfx_set_option "light_grids"
   // ray origins the hierarchies' box margins must cover (besides every drop point)
   float eye[3] = { 0, 0, 0 };               // the camera's

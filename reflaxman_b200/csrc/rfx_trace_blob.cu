@@ -252,8 +252,9 @@ __device__ __forceinline__ void intersectBlob(const BlobView & sc, int * __restr
     const float ix = fminf(fmaxf(1.0f / d.x, -1e30f), 1e30f), iy = fminf(fmaxf(1.0f / d.y, -1e30f), 1e30f), iz = fminf(fmaxf(1.0f / d.z, -1e30f), 1e30f);
     const float oxi = -(o.x * ix), oyi = -(o.y * iy), ozi = -(o.z * iz);
     // a box whose entry lies beyond the closest hit so far cannot improve it: compared in ray-parameter space, with generous slack
-    // (0.1 % + 0.01 length units; +inf while there is no hit and in any-hit queries); refreshed after every leaf
-    const float invLen = 1.0f / sqrtf(a);
+    // (0.1 % + 0.01 length units; +inf while there is no hit and in any-hit queries); refreshed after every leaf.  |d|^2 overflows
+    // for |d| > ~1.8e19: 1/sqrtf(inf) = 0 would make reachT 0 after the first hit and prune every box ahead, so such rays prune nothing
+    const float invLen = (a < FLT_MAX) ? 1.0f / sqrtf(a) : __int_as_float(0x7F800000);
     float reachT = (best.dist * 1.001f + 1e-2f) * invLen;
     // pair nodes: one trip tests both children of an inner node; the walk continues into a hit child in a register (the nearer
     // one) and only defers the other to the stack; "while-while": every lane walks to its next leaf, then the warp tests its
@@ -311,7 +312,7 @@ __device__ __forceinline__ void intersectBlob(const BlobView & sc, int * __restr
     {
       const float ix = fminf(fmaxf(1.0f / d.x, -1e30f), 1e30f), iy = fminf(fmaxf(1.0f / d.y, -1e30f), 1e30f), iz = fminf(fmaxf(1.0f / d.z, -1e30f), 1e30f);
       const float oxi = -(o.x * ix), oyi = -(o.y * iy), ozi = -(o.z * iz);
-      const float invLen = 1.0f / sqrtf(a);
+      const float invLen = (a < FLT_MAX) ? 1.0f / sqrtf(a) : __int_as_float(0x7F800000);   // as in the sphere walk
       float reachT = (best.dist * 1.001f + 1e-2f) * invLen;
 #define RFX_TRI_LEAF(CA)                                                                                       \
       {                                                                                                        \
