@@ -47,6 +47,7 @@ struct rfx_ctx
 {
   int device = 0;
   cudaStream_t stream = nullptr, copyStream[2] = { nullptr, nullptr }, lastStream = nullptr;
+  bool frameBatch = true;                   // rfx_set_option "frame_batch": rfx_render_frames_device renders runs of one camera in batched launches
   int copyStreams = 1;                      // D2H streams rfx_render_frames alternates between (rfx_set_option "copy_streams")
   cudaDeviceProp prop;
   mutable std::string err;
@@ -394,8 +395,9 @@ int profileStart(rfx_ctx * ctx, cudaStream_t st, cudaEvent_t & stop)
 
 // render pixels [p0, p1) of the frame latched by render_begin
 // preStates: random states already ranked for exactly [p0, p1) (batch path ranks several frames per K1 pass); NULL = rank here
+// frames > 1: that many whole frames of the latched camera in one launch (fastBatchOk), states and ARGB frames one after the other
 int renderRange(rfx_ctx * ctx, uint64_t p0, uint64_t p1, uint32_t * argbOut, bool writeImage, cudaStream_t st,
-                const uint32_t * preStates = nullptr)
+                const uint32_t * preStates = nullptr, uint32_t frames = 1)
 {
   int rc;
   const int sn = ctx->sampleNum;
@@ -423,6 +425,7 @@ int renderRange(rfx_ctx * ctx, uint64_t p0, uint64_t p1, uint32_t * argbOut, boo
     {
       if (!preStates && (rc = rankSamples(ctx, nCalls, false, st)) != RFX_OK) return rc;
       TraceWork w = traceWork(ctx, cur, end, firstRank, preStates ? preStates : ctx->dSampleStates.p, writeImage ? ctx->dImage.p : nullptr, argbOut);
+      w.frames = frames;
       cudaEvent_t evStop;
       if ((rc = profileStart(ctx, st, evStop)) != RFX_OK) return rc;
       const bool useSmall = ctx->forcePath >= 2 ? false : ctx->image.smallOk;
@@ -452,7 +455,7 @@ int renderRange(rfx_ctx * ctx, uint64_t p0, uint64_t p1, uint32_t * argbOut, boo
       }
       if (evStop) CK(cudaEventRecord(evStop, st));
       CK(cudaGetLastError());
-      ctx->stats.samples += nCalls;
+      ctx->stats.samples += nCalls * frames;
       if (ctx->snap.jitter && sn > 0) ctx->seedRender = lcgJumpHost(ctx->seedRender, 2 * (end - cur));
     }
     cur = end;
@@ -1184,14 +1187,29 @@ int rfx_render_frames_device(rfx_ctx * ctx, int n_frames, const float * cams, in
     const int g = std::min(group, n_frames - f0);
     const bool pre = perFrame <= ctx->maxCallsPerLaunch;
     if (pre && (rc = rankSamples(ctx, perFrame * g, false, st)) != RFX_OK) return rc;
-    for (int f = f0; f < f0 + g; f++)
+    for (int f = f0; f < f0 + g;)
     {
-      if ((rc = beginFrame(ctx, cams + 13 * (size_t)f, reflect_num, sample_num)) != RFX_OK) return rc;
+      const float * cam = cams + 13 * (size_t)f;
+      if ((rc = beginFrame(ctx, cam, reflect_num, sample_num)) != RFX_OK) return rc;
       if (ctx->sceneDirty && (rc = uploadScene(ctx, st)) != RFX_OK) return rc;   // this frame's eye left the box the BVH margins were sized for
-      if ((rc = renderRange(ctx, 0, total, argb_device + (size_t)f * total, false, st,
-                            pre ? ctx->dSampleStates.p + (size_t)(f - f0) * perFrame : nullptr)) != RFX_OK) return rc;
+      uint32_t * out = argb_device + (size_t)f * total;
+      const uint32_t * states = pre ? ctx->dSampleStates.p + (size_t)(f - f0) * perFrame : nullptr;
+      // the following frames that repeat this camera (bit for bit) share their first segments: one launch renders up to
+      // RFX_FRAME_BATCH of them (k_trace_small, BATCH)
+      int n = 1;
+      if (ctx->frameBatch && pre)
+        while (n < std::min(RFX_FRAME_BATCH, f0 + g - f) && memcmp(cam, cam + 13 * (size_t)n, 13 * sizeof(float)) == 0) n++;
+      if (n > 1)
+      {
+        // a repeat whose eye would re-flatten the scene (outside the box the hierarchy margins were sized for) renders on its own
+        if ((rc = rfx_set_camera(ctx, cam, cam + 3, cam[12])) != RFX_OK) return rc;
+        const bool useSmall = ctx->forcePath >= 2 ? false : ctx->image.smallOk;
+        if (ctx->sceneDirty || !useSmall || !fastBatchOk(traceWork(ctx, 0, total, 0, states, nullptr, out))) n = 1;
+      }
+      if ((rc = renderRange(ctx, 0, total, out, false, st, states, (uint32_t)n)) != RFX_OK) return rc;
       ctx->cursor = total;
       ctx->inProgress = false;
+      f += n;
     }
   }
   return RFX_OK;
@@ -1348,6 +1366,12 @@ int rfx_set_option(rfx_ctx * ctx, const char * name, int64_t value)
   if (!strcmp(name, "blob_smem_bvh"))
   {
     ctx->blobSmemBvh = value != 0;
+    return RFX_OK;
+  }
+  if (!strcmp(name, "frame_batch"))
+  {
+    if (value != 0 && value != 1) return fail(ctx, RFX_ERR_ARG, "rfx_set_option: frame_batch must be 0 or 1");
+    ctx->frameBatch = value != 0;
     return RFX_OK;
   }
   if (!strcmp(name, "copy_streams"))

@@ -95,6 +95,8 @@ struct TraceWork
   uint32_t * sigOut;            // optional per-pixel hit-path signature
   unsigned long long * counters;// device [32][2] striped {bounces, shadowRays}
   TileOrder order;              // fast constant-bank kernel only
+  uint32_t frames = 1;          // fast constant-bank kernel: consecutive frames of this one camera (fastBatchOk); frame f's states
+                                // and ARGB frame lie f whole frames after sampleStates / argbOut
   bool lightGrids = false;      // blob scenes: the header carries candidate grids for some light (picks the kernel instantiation)
   bool triBvh = false;          // blob scenes: the header carries a hierarchy over the triangles (picks the kernel instantiation)
   EyeGrid eyeGrid = { nullptr, nullptr, nullptr, 0, 0, 0 };
@@ -123,6 +125,11 @@ int launchTraceBlobRays(const void * sceneBlob, int n, const float * origins, co
 int launchTraceSmall(const SmallScene & sc, const TraceWork & w, cudaStream_t st, uint32_t * fastGrid = nullptr);
 // CTA count the fast kernel would use for this work, 0 if the work does not qualify for it
 uint32_t fastGridSize(const TraceWork & w);
+#ifndef RFX_FRAME_BATCH
+#define RFX_FRAME_BATCH 16      // most frames of one camera a fast-kernel launch renders (rfx_render_frames_device)
+#endif
+// whether the fast kernel can render several frames of this work's camera in one launch (whole one-sample ARGB frames)
+bool fastBatchOk(const TraceWork & w);
 // per launch of the fast kernel: pixel rectangles outside of which no primary ray can hit sphere i (rect[i]) / triangle k
 // (rect[SMALL_MAX_SPHERES + k]); rfx_trace_small.cu has the derivation
 struct PrimaryCull

@@ -241,9 +241,18 @@ __device__ __forceinline__ void intersectSmall(const SmallScene & sc, V3 o, V3 d
 // ---- Scene::trace (reference Scene.cpp:73-236) ------------------------------------------------------------------------
 // `events` counts bounce-loop iterations in its low half and shadow rays in its high half (one register instead of two).
 // RANGED: `first` is the object range of the path's first query (the tile's PrimaryCull answer); every later query sees everything.
-template <bool SIG, int FEAT, bool RANGED = false>
+//
+// BATCH (frames of one camera, see k_trace_small): everything a path computes before it first reads randDir — the first query
+// and the hit set-up — is the same in every frame.  SEG_FIRST runs that first segment only and leaves its state in `cache`
+// (PATH_WORDS words at a stride of SMALL_THREADS, shared memory); SEG_RESUME starts from that state at the choice of the first
+// light, with this frame's randDir.  A primary miss stores its finished colour (hslot = -1).  Same operations, same operands.
+constexpr int SEG_WHOLE = 0, SEG_FIRST = 1, SEG_RESUME = 2;
+constexpr int PATH_WORDS = 17;
+constexpr int SMALL_THREADS = RFX_SMALL_THREADS;
+
+template <bool SIG, int FEAT, bool RANGED = false, bool BATCH = false>
 __device__ __forceinline__ V3 traceSmall(const SmallScene & sc, V3 origin, V3 ray, int reflNumber, V3 randDir, uint32_t & events, uint32_t & sig,
-                                         const ObjRange first = ObjRange())
+                                         const ObjRange first = ObjRange(), int mode = SEG_WHOLE, float * cache = nullptr)
 {
   V3 mul = mk(1.0f, 1.0f, 1.0f);
   V3 pix = mk(0.0f, 0.0f, 0.0f);
@@ -263,16 +272,31 @@ __device__ __forceinline__ V3 traceSmall(const SmallScene & sc, V3 origin, V3 ra
   float rfs = 0.0f;         // weight of the reflected continuation (Scene.cpp:196 / :207), negated for metals (one register
                             // for the weight and the material type; the weight is in [0.2, 1], never zero)
   ObjRange range = first;
+  constexpr int S = SMALL_THREADS;
+  bool resume = false;
+  if (BATCH && mode == SEG_RESUME)
+  {
+    events++;                                                            // the first bounce-loop iteration, run once per batch
+    color = mk(cache[9 * S], cache[10 * S], cache[11 * S]);
+    hslot = __float_as_int(cache[16 * S]);
+    if (hslot < 0) return color;                                         // primary miss: the finished colour
+    qo = mk(cache[0], cache[S], cache[2 * S]);
+    norm = mk(cache[3 * S], cache[4 * S], cache[5 * S]);
+    reflect = mk(cache[6 * S], cache[7 * S], cache[8 * S]);
+    normLen = cache[12 * S]; reflectLen = cache[13 * S]; mrefl = cache[14 * S]; rfs = cache[15 * S];
+    resume = true;
+  }
 
   for (;;)
   {
+    V3 sumLight = (FEAT & F_LIGHTS) ? carryLight : mk(0.0f, 0.0f, 0.0f);
+    V3 sumSpec = (FEAT & F_LIGHTS) ? carrySpec : mk(0.0f, 0.0f, 0.0f);
+    if (BATCH && resume) { resume = false; goto chooseLight; }   // (a forward jump inside the loop body: one intersection call site)
     Best hit;
     hit.dist = FLT_MAX; hit.slot = -1; hit.order = 0x7FFFFFFF; hit.t = 0; hit.u = 0; hit.v = 0;
     intersectSmall<FEAT, RANGED>(sc, qo, qd, shadowQuery ? hslot : -1, shadowQuery, hit, range);
     if (RANGED) { range.s0 = 0; range.s1 = sc.nS << 4; range.t0 = 0; range.t1 = sc.nT * 48; }   // rematerialised from the constant bank
 
-    V3 sumLight = (FEAT & F_LIGHTS) ? carryLight : mk(0.0f, 0.0f, 0.0f);
-    V3 sumSpec = (FEAT & F_LIGHTS) ? carrySpec : mk(0.0f, 0.0f, 0.0f);
     if (!shadowQuery)
     {
       // ---- closest hit of the bounce segment (origin = qo, ray = qd), Scene.cpp:80-112
@@ -285,6 +309,7 @@ __device__ __forceinline__ V3 traceSmall(const SmallScene & sc, V3 origin, V3 ra
         const V3 sky = texSampleRef((FEAT & F_TEXELS) && sc.skyTex >= 0 ? &sc.tex[sc.skyTex] : nullptr, sc.byteLut, u, v);
         pix = mk(clamp01(pix.x + (mul.x * sky.x) * sc.env[0]), clamp01(pix.y + (mul.y * sky.y) * sc.env[1]),
                  clamp01(pix.z + (mul.z * sky.z) * sc.env[2]));            // Scene.cpp:230-231
+        if (BATCH && mode == SEG_FIRST) { cache[9 * S] = pix.x; cache[10 * S] = pix.y; cache[11 * S] = pix.z; cache[16 * S] = __int_as_float(-1); }
         break;
       }
       if (SIG) RFX_SIG(sig, hit.order + 1);
@@ -332,6 +357,16 @@ __device__ __forceinline__ V3 traceSmall(const SmallScene & sc, V3 origin, V3 ra
       sumLight = mk(0.0f, 0.0f, 0.0f);
       sumSpec = mk(0.0f, 0.0f, 0.0f);
       li = 0;
+      if (BATCH && mode == SEG_FIRST)
+      {
+        cache[0] = qo.x; cache[S] = qo.y; cache[2 * S] = qo.z;
+        cache[3 * S] = norm.x; cache[4 * S] = norm.y; cache[5 * S] = norm.z;
+        cache[6 * S] = reflect.x; cache[7 * S] = reflect.y; cache[8 * S] = reflect.z;
+        cache[9 * S] = color.x; cache[10 * S] = color.y; cache[11 * S] = color.z;
+        cache[12 * S] = normLen; cache[13 * S] = reflectLen; cache[14 * S] = mrefl; cache[15 * S] = rfs;
+        cache[16 * S] = __int_as_float(hslot);
+        return pix;
+      }
     }
     else
     {
@@ -376,6 +411,7 @@ __device__ __forceinline__ V3 traceSmall(const SmallScene & sc, V3 origin, V3 ra
     }
 
     // ---- next light that faces the surface gets a shadow query, Scene.cpp:118-129
+  chooseLight:
     bool cast = false;
     const int nL = (FEAT & F_LIGHTS) ? sc.nL : ((sc.nL > 0 && !shadowQuery) ? 1 : 0);   // one light: an answered query is the last
     for (; li < nL; li++)
@@ -389,6 +425,13 @@ __device__ __forceinline__ V3 traceSmall(const SmallScene & sc, V3 origin, V3 ra
         break;
       }
     }
+#ifdef RFX_DEBUG_FIRST_SEGMENT
+    // debug build (tools/first_segment_prize.py): the path ends after its first hit set-up and first-light choice; the colour
+    // folds in everything that set-up produced so that none of it is dead code
+    if (!shadowQuery)
+      return mk(color.x * rfs + qd.x + norm.x + reflect.x, color.y * mrefl + qd.y + normLen + reflect.y,
+                color.z + qd.z + reflectLen + (float)(li + hslot) + norm.z + reflect.z + qo.x);
+#endif
     if (cast)
     {
       if (FEAT & F_LIGHTS) { carryLight = sumLight; carrySpec = sumSpec; }
@@ -576,7 +619,6 @@ PrimaryCull makePrimaryCull(const SmallScene & sc, const FrameParams & fp)
 }
 
 // ---- K2 ----------------------------------------------------------------------------------------------------------------
-constexpr int SMALL_THREADS = RFX_SMALL_THREADS;
 
 __device__ __forceinline__ void flushCounters(unsigned long long * __restrict__ counters, uint32_t nBounces, uint32_t nShadow, uint32_t warpId)
 {
@@ -608,12 +650,19 @@ __device__ __forceinline__ unsigned smId() { unsigned s; asm volatile("mov.u32 %
 // blockIdx.y = tile row, blockIdx.x * warps + warp = tile column.  MULTI = false: one sample per pixel, no jitter, ARGB
 // output only (the bench path).  MULTI = true: the same tiling and scheduling for grid SSAA (Render.cpp:174-196), additive
 // jitter and accumulation, and the float image of the Render API.
-template <int FEAT, bool MULTI, bool STRIPS>
+//
+// BATCH: nFrames frames of one camera (whole frames, one sample, ARGB).  Each lane runs its pixel's first segment once (SEG_FIRST,
+// state in shared memory), then every frame from there with that frame's random state; frame f reads its states and writes its
+// ARGB one frame further on (sampleStates / argbOut + f * W * rows).  The frames run one after the other for the whole warp, so
+// that the bounce and shadow trips of a tile stay aligned; the tile's cost class is its longest path over all frames.
+template <int FEAT, bool MULTI, bool STRIPS, bool BATCH = false>
 __global__ void __launch_bounds__(SMALL_THREADS, MULTI ? 7 : RFX_SMALL_MINBLOCKS) k_trace_small(const __grid_constant__ SmallScene sc, const __grid_constant__ FrameParams fp,
                                                                const uint32_t * __restrict__ sampleStates, uint32_t * __restrict__ argbOut,
                                                                unsigned long long * __restrict__ counters, uint32_t y0, uint32_t y1,
-                                                               const TileOrder ord, float * __restrict__ image, const __grid_constant__ PrimaryCull pc)
+                                                               const TileOrder ord, float * __restrict__ image, const __grid_constant__ PrimaryCull pc,
+                                                               uint32_t nFrames)
 {
+  static_assert(!BATCH || (!MULTI && !STRIPS), "frame batches are whole one-sample frames");
   // which tile group does this CTA render: index order, or the previous launch's cost order (expensive classes first)
   uint32_t bx = blockIdx.x, by = blockIdx.y;
   if (ord.zeroCounts && (blockIdx.x | blockIdx.y) == 0u && threadIdx.x < TILE_CLASSES) ord.zeroCounts[threadIdx.x] = 0u;   // for the next launch
@@ -676,57 +725,75 @@ __global__ void __launch_bounds__(SMALL_THREADS, MULTI ? 7 : RFX_SMALL_MINBLOCKS
     const uint32_t mt = (m >> SMALL_MAX_SPHERES) & ((1u << sc.nT) - 1u);
     if (mt) { first.t0 = (__ffs(mt) - 1) * 48; first.t1 = (32 - __clz(mt)) * 48; }
   }
-  uint32_t events = 0;                                                   // MULTI: of the longest call in the low half (cost class)
-  uint32_t nBounces = 0, nShadow = 0;                                    // MULTI: totals over the calls
-  uint32_t packed = 0, qOut = 0;
-  if (valid && !MULTI)
-  {
-    const uint32_t q = y * fp.W + x;                                     // < 2^32 for every frame size the API accepts
-    uint32_t s = __ldg(sampleStates + (q - y0 * fp.W));
-    const float rx = float(x) - fp.wHalf;                                // Render.cpp:154-155
-    const float ry = float(y) - fp.hHalf;
-    const V3 ray = mk((rx * fp.view[0] + ry * fp.view[1]) + fp.rz * fp.view[2],
-                      (rx * fp.view[3] + ry * fp.view[4]) + fp.rz * fp.view[5],
-                      (rx * fp.view[6] + ry * fp.view[7]) + fp.rz * fp.view[8]);
-    V3 rd;
-    rngTriple(s, rd.x, rd.y, rd.z);
-    uint32_t sig = 0;
-    const V3 c = traceSmall<false, FEAT, RFX_PRIMARY_CULL != 0>(sc, mk(fp.eye[0], fp.eye[1], fp.eye[2]), ray, fp.reflNum, rd, events, sig, first);
-#ifdef RFX_DEBUG_DEPTH
-    packed = events;           // debug build (tools/depth_stats.py): bounce-loop iterations | shadow rays << 16 instead of the colour
-#else
-    packed = packArgb(c.x, c.y, c.z);
-#endif
-    qOut = q;
-    nBounces = events & 0xFFFFu; nShadow = events >> 16;
-  }
-  // Framebuffer store of the one-sample path.
-  //  * Frame in local HBM: the four lanes of a tile row hold four consecutive pixels; the first of them stores all four as one
-  //    128-bit word (16-byte aligned when W is a multiple of 4 and the frame is), so a warp writes its 4x8 tile with 8 STG.128;
-  //    L2 merges them into lines.
-  //  * Split frame (rfx_render_strips): argbOut may be ANOTHER GPU's framebuffer (peer mapping), and then every store
-  //    instruction leaves this GPU as NVLink write packets.  Eight 16-byte pieces per instruction (one per tile row) throttled
-  //    the 7-to-1 gather of an 8K frame to 0.70 ms against 0.48 ms with local stores (profiles/r2_s2), so a tile group that lies
-  //    inside the image is staged in shared memory and written by whole row segments — warp w stores rows 2w and 2w+1, 16
-  //    consecutive pixels (64 contiguous bytes) per half warp — after the CTA barrier the tile scheduler needs anyway.
-  //    (For local frames the staging costs 0.8 % — measured — so they keep the direct stores: STRIPS is a template parameter and
-  //    the whole-frame instantiations carry none of this.)
+  uint32_t events = 0;                                                   // of the longest call / frame in the low half (cost class)
+  uint32_t nBounces = 0, nShadow = 0;                                    // totals over the calls / frames
   constexpr uint32_t GROUP_W = (SMALL_THREADS / 32) * RFX_TILE_W, STAGE_STRIDE = GROUP_W + 4;   // +4 words: conflict-free column writes
   __shared__ uint32_t sStage[(MULTI || !STRIPS) ? 1 : RFX_TILE_H * STAGE_STRIDE];
+  __shared__ float sPath[BATCH ? PATH_WORDS * SMALL_THREADS : 1];
   const bool staged = RFX_STRIP_STAGING && !MULTI && STRIPS && xCta + GROUP_W <= fp.W && yTop + RFX_TILE_H <= y1;   // uniform over the CTA
   if (!MULTI)
   {
-    if (staged) sStage[(lane / RFX_TILE_W) * STAGE_STRIDE + warp * RFX_TILE_W + (lane % RFX_TILE_W)] = packed;
-    else
+    const uint32_t q = y * fp.W + x;                                     // < 2^32 for every frame size the API accepts
+    const size_t frameStride = (size_t)(y1 - y0) * fp.W;
+#pragma unroll 1
+    for (int f = BATCH ? -1 : 0; f < (BATCH ? (int)nFrames : 1); f++)   // BATCH: f = -1 is the first segment
     {
-      const uint32_t p1 = __shfl_down_sync(0xffffffffu, packed, 1), p2 = __shfl_down_sync(0xffffffffu, packed, 2), p3 = __shfl_down_sync(0xffffffffu, packed, 3);
-      const uint32_t validMask = __ballot_sync(0xffffffffu, valid);
-      const bool rowOfFour = RFX_TILE_W % 4u == 0u && (fp.W & 3u) == 0u && ((validMask >> (lane & ~3u)) & 0xFu) == 0xFu;
-      if (rowOfFour)
+      ObjRange range = first;                                          // BATCH: every query of a frame sees every object
+      if (BATCH && f >= 0) { range.s0 = 0; range.s1 = sc.nS << 4; range.t0 = 0; range.t1 = sc.nT * 48; }
+      uint32_t packed = 0;
+      if (valid)
       {
-        if ((lane & 3u) == 0u) *reinterpret_cast<uint4 *>(argbOut + qOut) = make_uint4(packed, p1, p2, p3);
+        V3 rd = mk(0.0f, 0.0f, 0.0f);                                    // (the first segment reads no randDir)
+        if (f >= 0)
+        {
+          uint32_t s = __ldg(sampleStates + (size_t)f * frameStride + (q - y0 * fp.W));
+          rngTriple(s, rd.x, rd.y, rd.z);
+        }
+        const float rx = float(x) - fp.wHalf;                            // Render.cpp:154-155
+        const float ry = float(y) - fp.hHalf;
+        const V3 ray = mk((rx * fp.view[0] + ry * fp.view[1]) + fp.rz * fp.view[2],
+                          (rx * fp.view[3] + ry * fp.view[4]) + fp.rz * fp.view[5],
+                          (rx * fp.view[6] + ry * fp.view[7]) + fp.rz * fp.view[8]);
+        uint32_t ev = 0, sig = 0;
+        const V3 c = traceSmall<false, FEAT, RFX_PRIMARY_CULL != 0, BATCH>(sc, mk(fp.eye[0], fp.eye[1], fp.eye[2]), ray, fp.reflNum, rd, ev, sig,
+                                                                         range,
+                                                                         !BATCH ? SEG_WHOLE : f < 0 ? SEG_FIRST : SEG_RESUME, sPath + threadIdx.x);
+#ifdef RFX_DEBUG_DEPTH
+        packed = ev;               // debug build (tools/depth_stats.py): bounce-loop iterations | shadow rays << 16 instead of the colour
+#else
+        packed = packArgb(c.x, c.y, c.z);
+#endif
+        if (f >= 0)
+        {
+          nBounces += ev & 0xFFFFu; nShadow += ev >> 16;
+          events = max(events, ev & 0xFFFFu);
+        }
       }
-      else if (valid) argbOut[qOut] = packed;
+      if (BATCH && f < 0) { __syncwarp(); continue; }                    // every lane of the tile starts frame 0 together
+      // Framebuffer store of the one-sample path.
+      //  * Frame in local HBM: the four lanes of a tile row hold four consecutive pixels; the first of them stores all four as one
+      //    128-bit word (16-byte aligned when W is a multiple of 4 and the frame is), so a warp writes its 4x8 tile with 8 STG.128;
+      //    L2 merges them into lines.
+      //  * Split frame (rfx_render_strips): argbOut may be ANOTHER GPU's framebuffer (peer mapping), and then every store
+      //    instruction leaves this GPU as NVLink write packets.  Eight 16-byte pieces per instruction (one per tile row) throttled
+      //    the 7-to-1 gather of an 8K frame to 0.70 ms against 0.48 ms with local stores (profiles/r2_s2), so a tile group that lies
+      //    inside the image is staged in shared memory and written by whole row segments — warp w stores rows 2w and 2w+1, 16
+      //    consecutive pixels (64 contiguous bytes) per half warp — after the CTA barrier the tile scheduler needs anyway.
+      //    (For local frames the staging costs 0.8 % — measured — so they keep the direct stores: STRIPS is a template parameter and
+      //    the whole-frame instantiations carry none of this.)
+      if (staged) sStage[(lane / RFX_TILE_W) * STAGE_STRIDE + warp * RFX_TILE_W + (lane % RFX_TILE_W)] = packed;
+      else
+      {
+        uint32_t * out = argbOut + (BATCH ? (size_t)f * frameStride : 0) + (valid ? q : 0u);
+        const uint32_t p1 = __shfl_down_sync(0xffffffffu, packed, 1), p2 = __shfl_down_sync(0xffffffffu, packed, 2), p3 = __shfl_down_sync(0xffffffffu, packed, 3);
+        const uint32_t validMask = __ballot_sync(0xffffffffu, valid);
+        const bool rowOfFour = RFX_TILE_W % 4u == 0u && (fp.W & 3u) == 0u && ((validMask >> (lane & ~3u)) & 0xFu) == 0xFu;
+        if (rowOfFour)
+        {
+          if ((lane & 3u) == 0u) *reinterpret_cast<uint4 *>(out) = make_uint4(packed, p1, p2, p3);
+        }
+        else if (valid) *out = packed;
+      }
     }
   }
   if (valid && MULTI)
@@ -974,6 +1041,12 @@ uint32_t fastGridSize(const TraceWork & w)
   return g.x <= 65535u ? g.x * g.y : 0;
 }
 
+bool fastBatchOk(const TraceWork & w)
+{
+  const FrameParams & fp = w.fp;
+  return fastGridSize(w) && fp.sampleNum == 1 && !fp.jitter && !w.image && w.argbOut && !fp.stripWorld && fp.p0 == 0 && fp.p1 == (uint64_t)fp.W * fp.H;
+}
+
 int launchTraceSmall(const SmallScene & sc, const TraceWork & w, cudaStream_t st, uint32_t * fastGrid)
 {
   if (fastGrid) *fastGrid = 0;
@@ -1005,8 +1078,13 @@ int launchTraceSmall(const SmallScene & sc, const TraceWork & w, cudaStream_t st
         const bool multi = fp.sampleNum != 1 || fp.jitter || w.image != nullptr;
         const uint32_t y0 = (uint32_t)(fp.p0 / fp.W), y1 = (uint32_t)(fp.p1 / fp.W);
         const PrimaryCull pc = RFX_PRIMARY_CULL ? makePrimaryCull(sc, fp) : PrimaryCull();
-#define RFX_LAUNCH_SMALL(F, M, S, IMG) k_trace_small<F, M, S><<<grid, SMALL_THREADS, 0, st>>>(sc, fp, w.sampleStates, w.argbOut, w.counters, y0, y1, w.order, IMG, pc)
-        if (fp.stripWorld)
+#define RFX_LAUNCH_SMALL(F, M, S, IMG) k_trace_small<F, M, S><<<grid, SMALL_THREADS, 0, st>>>(sc, fp, w.sampleStates, w.argbOut, w.counters, y0, y1, w.order, IMG, pc, 1u)
+        if (w.frames > 1)   // the caller checked fastBatchOk
+        {
+          if (lean) k_trace_small<0, false, false, true><<<grid, SMALL_THREADS, 0, st>>>(sc, fp, w.sampleStates, w.argbOut, w.counters, y0, y1, w.order, nullptr, pc, w.frames);
+          else k_trace_small<F_ALL, false, false, true><<<grid, SMALL_THREADS, 0, st>>>(sc, fp, w.sampleStates, w.argbOut, w.counters, y0, y1, w.order, nullptr, pc, w.frames);
+        }
+        else if (fp.stripWorld)
         {
           if (lean && !multi) RFX_LAUNCH_SMALL(0, false, true, nullptr);
           else if (!multi) RFX_LAUNCH_SMALL(F_ALL, false, true, nullptr);
