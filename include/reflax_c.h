@@ -57,6 +57,7 @@ typedef struct rfx_stats
   uint64_t launches_small_fast, launches_small_any, launches_blob_fast, launches_blob_any;
   uint64_t light_grids;     /* lights of the uploaded scene whose shadow queries use a candidate grid (not a counter: survives rfx_stats_reset) */
   uint64_t bvh_triangles;   /* triangles of the uploaded scene under a bounding-volume hierarchy, 0 = they are walked one by one (not a counter) */
+  uint64_t bvh_spheres;     /* spheres of the uploaded scene under a bounding-volume hierarchy, 0 = they are walked one by one (not a counter) */
 } rfx_stats;
 
 typedef struct rfx_device_info
@@ -144,6 +145,15 @@ RFX_API int rfx_selftest_light_grid_host(const float light[4], int n_spheres, co
  * float32 test of Triangle.cpp:56-68 can accept a ray from inside reach (a zero-area triangle's test accepts the unit triangle its
  * identity basis describes, not its vertices), inflated by that test's rounding noise and by 1e-6 of the reach diagonal. */
 RFX_API int rfx_selftest_tri_bounds_host(int n, const float * tris, const float reach[6], float * boxes);
+/* diagnostic, pure host function: the hierarchies' boxes in a scene with a plane, where a ray can start anywhere.  spheres = n_spheres x
+ * (cx, cy, cz, r), tris = n_tris x (v0[3], axTrans[9]), reach = lo[3], hi[3] of the box the margins are sized for (every centre and
+ * vertex inside).  Out: sphere_boxes, tri_boxes = n x (lo[3], hi[3]) (a sliver or non-finite triangle, which no margin holds from far
+ * origins, gets (-inf, +inf): it is tested after the walk, by every query); reaches = the sphere reach box, then the triangle reach box
+ * (reach joined with every effective triangle); grow = {sphere growth, triangle growth}.  A query from origin o grows every box it
+ * tests by grow * (sum of o's per-axis distances outside the reach box of that kind), which keeps each box around every point the
+ * float32 tests of Sphere.cpp:49-57 / Triangle.cpp:56-68 can accept. */
+RFX_API int rfx_selftest_far_bounds_host(int n_spheres, const float * spheres, int n_tris, const float * tris, const float reach[6],
+                                         float * sphere_boxes, float * tri_boxes, float reaches[12], float grow[2]);
 /* diagnostic, pure host function: the screen grid of a path's first query (option "eye_grid") for cam = eye[3], view[9], fov and
  * spheres = n_spheres x (cx, cy, cz, r^2): dims = {nx, ny, shift} (cells of 2^shift pixels; {0, 0, 0}: no grid for this camera),
  * counts = {nx*ny + 1, items}, cell_start / items (sphere indices, cell after cell) filled when their capacities suffice. */
@@ -215,16 +225,17 @@ RFX_API int rfx_enable_profiling(rfx_ctx * ctx, int on);
  * candidate spheres across the light's direction instead of walking the hierarchy (default 1).  "eye_grid": the same scenes take the
  * candidates of a path's first query (origin = eye) from a screen grid binned per camera out of the spheres' primary-ray bounds
  * (default 1).  Both grids list spheres only: triangles are tested after them, through their own hierarchy when the scene has one
- * (rfx_set_bvh_mode).  Frames are bit-identical under every setting. */
+ * (rfx_set_bvh_mode).  Scenes with a plane get no light grids (a shadow ray can start anywhere on the plane); their eye grid is built.  Frames are bit-identical under every setting. */
 RFX_API int rfx_set_option(rfx_ctx * ctx, const char * name, int64_t value);
 /* kernel selection: 0 = automatic (constant-bank kernels when the scene fits, the blob kernels otherwise),
  * 1 = constant-bank kernel if it fits, 2 = always the blob kernels (tile / wavefront kernels for row-aligned slices, the general
  * one otherwise), 3 = always the general blob kernel.  Results are identical; tests use it. */
 RFX_API int rfx_force_path(rfx_ctx * ctx, int path);
 /* acceleration structures of the blob kernels: 0 = automatic (a bounding-volume hierarchy over the spheres when there are more than
- * 32 and the scene holds no unbounded plane; one over the triangles, walked after the spheres, when there are more than 32 triangles
- * and no plane), 1 = always (whenever there are any spheres / triangles and no plane), 2 = never (the
- * reference's brute-force list walk).  Results are identical; tests compare them. */
+ * 32; one over the triangles, walked after the spheres, when there are more than 32 triangles), 1 = always (whenever there are any
+ * spheres / triangles), 2 = never (the reference's brute-force list walk).  In a scene with a plane a ray can start anywhere on it: a
+ * query from outside the box the margins are sized for grows the boxes it tests with its distance from that box, and slivers are
+ * tested after the walk (rfx_selftest_far_bounds_host).  Results are identical; tests compare them. */
 RFX_API int rfx_set_bvh_mode(rfx_ctx * ctx, int mode);
 /* cost-ordered tile scheduling of the constant-bank fast kernel: launches record which tiles held long paths (every
  * "tile_order_period"-th launch over a grid) and the following launches over the same grid start those first (1 = on, the

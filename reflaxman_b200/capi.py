@@ -22,7 +22,7 @@ class RfxStats(C.Structure):
     _fields_ = [(n, C.c_uint64) for n in ("rays", "bounces", "shadow_rays", "samples", "kernel_launches",
                                           "h2d_bytes", "d2h_bytes", "trace_kernels")] + [("trace_kernel_ms", C.c_double)] + \
                [(n, C.c_uint64) for n in ("launches_small_fast", "launches_small_any", "launches_blob_fast", "launches_blob_any", "light_grids",
-                                          "bvh_triangles")]
+                                          "bvh_triangles", "bvh_spheres")]
 
     def as_dict(self):
         return {n: (float if n == "trace_kernel_ms" else int)(getattr(self, n)) for n, _ in self._fields_}
@@ -59,6 +59,7 @@ SYMBOLS = [
     ("rfx_selftest_light_grid_host", C.c_int, [_fp, C.c_int, _fp, _fp, C.c_float, _fp, C.POINTER(C.c_int32), _u32p, C.c_uint64,
                                               C.POINTER(C.c_int32), C.c_uint64, C.POINTER(C.c_uint64)]),
     ("rfx_selftest_tri_bounds_host", C.c_int, [C.c_int, _fp, _fp, _fp]),
+    ("rfx_selftest_far_bounds_host", C.c_int, [C.c_int, _fp, C.c_int, _fp, _fp, _fp, _fp, _fp, _fp]),
     ("rfx_selftest_eye_grid_host", C.c_int, [_fp, C.c_uint32, C.c_uint32, C.c_int, _fp, C.POINTER(C.c_int32), _u32p, C.c_uint64,
                                             C.POINTER(C.c_int32), C.c_uint64, C.POINTER(C.c_uint64)]),
     ("rfx_set_image_size", C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32]),
@@ -174,6 +175,26 @@ def tri_bounds_host(tris, reach):
     if L.rfx_selftest_tri_bounds_host(len(tr), tr.ctypes.data_as(_fp), rc_.ctypes.data_as(_fp), out.ctypes.data_as(_fp)) != 0:
         raise RfxError("rfx_selftest_tri_bounds_host failed")
     return out
+
+
+def far_bounds_host(spheres, tris, reach):
+    """Pure host function (no GPU): the hierarchies' boxes in a scene with a plane.  spheres [n][4] = (cx, cy, cz, r), tris [m][12] =
+    (v0[3], axTrans[9] row-major), reach = (lo[3], hi[3]) of the box the margins are sized for.  Returns (sphere_boxes [n][6],
+    tri_boxes [m][6] (slivers and non-finite triangles: (-inf, +inf), tested after the walk), sphere_reach [6], tri_reach [6],
+    (grow_spheres, grow_triangles)): a query from origin o grows every box by grow * (sum of o's per-axis distances outside the
+    reach box of its kind)."""
+    L = load()
+    sp = np.ascontiguousarray(np.asarray(spheres, np.float32).reshape(-1, 4))
+    tr = np.ascontiguousarray(np.asarray(tris, np.float32).reshape(-1, 12))
+    rc_ = np.ascontiguousarray(np.asarray(reach, np.float32).reshape(6))
+    sb = np.zeros((max(len(sp), 1), 6), np.float32)
+    tb = np.zeros((max(len(tr), 1), 6), np.float32)
+    reaches = np.zeros(12, np.float32)
+    grow = np.zeros(2, np.float32)
+    if L.rfx_selftest_far_bounds_host(len(sp), sp.ctypes.data_as(_fp), len(tr), tr.ctypes.data_as(_fp), rc_.ctypes.data_as(_fp), sb.ctypes.data_as(_fp),
+                                      tb.ctypes.data_as(_fp), reaches.ctypes.data_as(_fp), grow.ctypes.data_as(_fp)) != 0:
+        raise RfxError("rfx_selftest_far_bounds_host failed")
+    return sb[:len(sp)], tb[:len(tr)], reaches[:6], reaches[6:], (float(grow[0]), float(grow[1]))
 
 
 def eye_grid_host(cam, width, height, spheres):
@@ -443,8 +464,9 @@ class Context:
         self._ck(self.L.rfx_force_path(self.h, path), "rfx_force_path")
 
     def set_bvh_mode(self, mode):
-        """0 automatic (hierarchies over the spheres / the triangles when there are more than 32 of them and no plane), 1 always
-        (whenever there are any and no plane), 2 never (list walk)."""
+        """0 automatic (hierarchies over the spheres / the triangles when there are more than 32 of them), 1 always (whenever there
+        are any), 2 never (list walk).  In scenes with a plane, queries from outside the box the margins are sized for grow the boxes
+        they test (far_bounds_host)."""
         self._ck(self.L.rfx_set_bvh_mode(self.h, mode), "rfx_set_bvh_mode")
 
     def set_tile_ordering(self, on=True):

@@ -91,6 +91,7 @@ struct rfx_ctx
   uint64_t eyeGridBuilds = 0;
   DevArray<float4> dTriNodes;               // hierarchy over the triangles: leaf slots, then pair nodes
   DevArray<int> dTriPrims;
+  DevArray<int> dTriAlways;                 // plane scenes: triangles tested after the triangle walk (SceneHeader::triAlways)
 
   // ---- camera + render state (reference Render.h:9-27); the eye is scene.eye
   float view[9] = { 1, 0, 0, 0, 1, 0, 0, 0, 1 }, fov = 1.0f;
@@ -224,6 +225,11 @@ int uploadScene(rfx_ctx * ctx, cudaStream_t st)
     h.triPrims = ctx->dTriPrims.p;
     h.triLeaf = ctx->dTriNodes.p;
     h.triPairs = ctx->dTriNodes.p + img.triBvh.leafFloat4;
+  }
+  if (!img.triAlways.empty())
+  {
+    if ((rc = upload(ctx, ctx->dTriAlways, img.triAlways, st)) != RFX_OK) return rc;
+    h.triAlways = ctx->dTriAlways.p;
   }
   if ((rc = upload(ctx, ctx->dBlob, img.blob, st)) != RFX_OK) return rc;
   CK(cudaStreamSynchronize(st));   // every copy above read from img, which the next upload overwrites
@@ -376,6 +382,7 @@ TraceWork traceWork(const rfx_ctx * ctx, uint64_t p0, uint64_t p1, uint64_t firs
   w.counters = ctx->dCounters.p;
   w.lightGrids = ctx->image.lightGridsBuilt > 0;
   w.triBvh = ctx->image.triBvhTris > 0;
+  w.far = ctx->image.far;
   return w;
 }
 
@@ -1110,7 +1117,8 @@ int rfx_trace_rays(rfx_ctx * ctx, int n, const float * origins, const float * ra
   CK(cudaMemcpyAsync(dO, origins, (size_t)n * 12, cudaMemcpyHostToDevice, st));
   CK(cudaMemcpyAsync(dR, rays, (size_t)n * 12, cudaMemcpyHostToDevice, st));
   ctx->stats.h2d_bytes += (uint64_t)n * 24;
-  ctx->stats.kernel_launches += launchTraceBlobRays(ctx->dBlob.p, n, dO, dR, reflect_num, ctx->dSampleStates.p, dC, ctx->dCounters.p, st, ctx->image.triBvhTris > 0);
+  ctx->stats.kernel_launches += launchTraceBlobRays(ctx->dBlob.p, n, dO, dR, reflect_num, ctx->dSampleStates.p, dC, ctx->dCounters.p, st, ctx->image.triBvhTris > 0,
+                                                    ctx->image.far);
   CK(cudaGetLastError());
   CK(cudaMemcpyAsync(rgb, dC, (size_t)n * 12, cudaMemcpyDeviceToHost, st));
   CK(cudaStreamSynchronize(st));
@@ -1290,6 +1298,7 @@ int rfx_get_stats(rfx_ctx * ctx, rfx_stats * out)
   ctx->evUsed = 0;
   ctx->stats.light_grids = (uint64_t)ctx->image.lightGridsBuilt;
   ctx->stats.bvh_triangles = ctx->image.triBvhTris;
+  ctx->stats.bvh_spheres = ctx->image.bvhSpheres;
   *out = ctx->stats;
   return RFX_OK;
 }

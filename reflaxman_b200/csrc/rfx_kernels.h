@@ -99,6 +99,7 @@ struct TraceWork
                                 // and ARGB frame lie f whole frames after sampleStates / argbOut
   bool lightGrids = false;      // blob scenes: the header carries candidate grids for some light (picks the kernel instantiation)
   bool triBvh = false;          // blob scenes: the header carries a hierarchy over the triangles (picks the kernel instantiation)
+  bool far = false;             // blob scenes: the scene has a plane and a hierarchy, so a query can start outside the reach box (FAR)
   EyeGrid eyeGrid = { nullptr, nullptr, nullptr, 0, 0, 0 };
 };
 // blob scenes (rfx_trace_blob.cu).  launchTraceBlobFast: row-aligned slices (one sample per pixel, grid SSAA, additive jitter; ARGB
@@ -119,7 +120,7 @@ int launchTraceBlobFast(const TraceWork & w, cudaStream_t st, void * queueRecord
 int launchTraceBlobAny(const TraceWork & w, cudaStream_t st);     // every renderNext mode: ragged slices, block preview, signatures
 // Scene::trace for a list of rays (rfx_trace_rays): rays[i] uses sampleStates[i]
 int launchTraceBlobRays(const void * sceneBlob, int n, const float * origins, const float * rays, int reflNum,
-                        const uint32_t * sampleStates, float * rgbOut, unsigned long long * counters, cudaStream_t st, bool triBvh);
+                        const uint32_t * sampleStates, float * rgbOut, unsigned long long * counters, cudaStream_t st, bool triBvh, bool far);
 // small scenes: constant-bank resident; *fastGrid (optional) receives the CTA count of the fast kernel's grid, 0 when the
 // general kernel ran (the caller keeps tile-order history only for fast launches)
 int launchTraceSmall(const SmallScene & sc, const TraceWork & w, cudaStream_t st, uint32_t * fastGrid = nullptr);

@@ -198,7 +198,11 @@ void packBvh(const std::vector<BvhNode> & nodes, const std::vector<BvhPrim> & pr
 // with 16u kappa > 1/2 (a sliver: kappa above 2^19), or whose M or A is not finite, gets the whole box of reach instead: every
 // query from inside it then tests that triangle, which is slow but exact.
 // tris: n x (v0[3], ax[9]); reach: lo[3], hi[3]; boxes out: n x (lo[3], hi[3]).  Returns R.
-double buildTriBoxes(int n, const float * tris, const float reach[6], float * boxes)
+// farOrigins (scenes with a plane, see farGrowthSpheres): a sliver or non-finite triangle gets the box (-inf, +inf) instead, which marks it
+// as tested after the walk and kept out of the hierarchy; triReach receives the box R is the diagonal of and kappaMax the largest
+// kappa of the triangles that keep a finite box (0 when there is none).
+double buildTriBoxes(int n, const float * tris, const float reach[6], float * boxes, bool farOrigins = false, double triReach[6] = nullptr,
+                     double * kappaMax = nullptr)
 {
   const double u = 1.0 / 16777216.0;
   std::vector<double> e((size_t)n * 8);   // per triangle: E's box (lo xyz, hi xyz), |A|, kappa (negative: no finite E)
@@ -242,19 +246,65 @@ double buildTriBoxes(int n, const float * tris, const float reach[6], float * bo
   const double R = sqrt(dx * dx + dy * dy + dz * dz);
   auto down = [](double v) { float f = (float)v; if ((double)f > v) f = nextafterf(f, -FLT_MAX); return f; };
   auto up = [](double v) { float f = (float)v; if ((double)f < v) f = nextafterf(f, FLT_MAX); return f; };
+  double kmax = 0.0;
   for (int i = 0; i < n; i++)
   {
     const double * r = &e[8 * (size_t)i];
     float * b = boxes + 6 * (size_t)i;
     if (!(r[7] >= 0.0) || !(16.0 * u * r[7] <= 0.5))
     {
-      for (int k = 0; k < 3; k++) { b[k] = down(ulo[k]); b[3 + k] = up(uhi[k]); }
+      for (int k = 0; k < 3; k++)
+        if (farOrigins) { b[k] = -std::numeric_limits<float>::infinity(); b[3 + k] = std::numeric_limits<float>::infinity(); }
+        else { b[k] = down(ulo[k]); b[3 + k] = up(uhi[k]); }
       continue;
     }
+    kmax = std::max(kmax, r[7]);
     const double m = 64.0 * u * (r[7] * R + r[6]) + 1e-6 * R;
     for (int k = 0; k < 3; k++) { b[k] = down(r[k] - m); b[3 + k] = up(r[3 + k] + m); }
   }
+  if (triReach)
+    for (int k = 0; k < 3; k++) { triReach[k] = ulo[k]; triReach[3 + k] = uhi[k]; }
+  if (kappaMax) *kappaMax = kmax;
   return R;
+}
+
+// ---- origins outside the reach box (scenes with a plane) ------------------------------------------------------------------------
+// The margins above hold for every query whose origin lies in the reach box.  A bounce or shadow ray that starts on an unbounded
+// plane can start anywhere; from an origin at Euclidean distance delta outside the box they are too small by at most an amount
+// linear in delta, so such a query grows every box it tests by grow * delta_1 (delta_1 >= delta: the sum of the per-axis excesses,
+// evaluated on the device rounding upwards), and a query from inside the box grows nothing.
+//   Spheres (sphereMargin).  Every centre lies in the reach box, so |v| = |origin - centre| <= R + delta, and the noise bound is
+//   h(R + delta) with h(x) = min(3e-7 x^2 / r, 7.7e-4 x).  h is quadratic up to x* = 7.7e-4 r / 3e-7, where its slope is
+//   6e-7 x* / r = 2 * 7.7e-4, and linear with slope 7.7e-4 beyond: h(R + delta) <= h(R) + 2 * 7.7e-4 * delta for every r.  The
+//   margin is twice h, so it needs 4 * 7.7e-4 * delta more; the slab test's own error (2^-22 |origin| along an axis) grows by
+//   2^-22 delta < 1e-6 delta.  growS = 4 * 7.7e-4 + 1e-6.
+//   Triangles (buildTriBoxes).  With R the diagonal of the triangle reach box (the reach box joined with every E, which holds v0):
+//   |p| <= R + delta and |t d| <= R + delta + dev, so dev <= 20u kappa (R + delta) + 4.2u|A| under the same condition 5u kappa <= 1/2,
+//   which does not involve R.  The margin keeps its factor 3 when it grows by 64u kappa delta, plus 1e-6 delta for the slab test:
+//   growT = 64u kappa_max + 1e-6, kappa_max over the triangles in the hierarchy (at most 2^19: growT <= 2).  Slivers and non-finite
+//   triangles have no such bound: in plane scenes they stay out of the hierarchy and every query tests them after the walk.
+// The device widens the slab interval of every box by G |1/d_k| per axis (G = grow * delta_1, rounded upwards; the bounds rounded
+// outwards), which is the fused slab test of the box grown by G on every side, with the same clamped reciprocals.
+float roundUp(double v) { float f = (float)v; if ((double)f < v) f = nextafterf(f, FLT_MAX); return f; }
+float farGrowthSpheres() { return roundUp(4.0 * 7.7e-4 + 1e-6); }
+float farGrowthTris(double kappaMax) { return roundUp(64.0 / 16777216.0 * kappaMax + 1e-6); }
+
+// a box (lo xyz, hi xyz) rounded outwards to float
+void roundOutwards(const double in[6], float out[6])
+{
+  for (int k = 0; k < 3; k++)
+  {
+    out[k] = (float)in[k]; if ((double)out[k] > in[k]) out[k] = nextafterf(out[k], -FLT_MAX);
+    out[3 + k] = (float)in[3 + k]; if ((double)out[3 + k] < in[3 + k]) out[3 + k] = nextafterf(out[3 + k], FLT_MAX);
+  }
+}
+
+// the box of a sphere in the hierarchy: centre -/+ (r + sphereMargin(r, R)); returns the margin
+float sphereBox(const float c[3], float r, double R, float lo[3], float hi[3])
+{
+  const float m = sphereMargin(r, R);
+  for (int k = 0; k < 3; k++) { lo[k] = c[k] - r - m; hi[k] = c[k] + r + m; }
+  return m;
 }
 
 // ---- shadow-ray candidate grids (LightGrid) ---------------------------------------------------------------------------------------
@@ -378,8 +428,8 @@ bool buildLightGrid(const Light & L, const std::vector<const HostObj *> & sph, c
   return true;
 }
 
-// The grids of every far light, concatenated into img.  B: the box of every drop point — all objects (planes are excluded by the
-// automatic hierarchy rule; with planes present no grid is built), padded for the rounding of a drop point.  prims: the sphere
+// The grids of every far light, concatenated into img.  B: the box of every drop point — all objects (with planes present no grid is
+// built: a drop point on a plane can lie anywhere), padded for the rounding of a drop point.  prims: the sphere
 // hierarchy's, in the order its build left them.
 void buildLightGrids(const std::vector<Light> & lights, const std::vector<const HostObj *> & sph, const std::vector<const HostObj *> & tri,
                      const std::vector<BvhPrim> & prims, SceneImage & img)
@@ -462,25 +512,25 @@ int buildSceneImage(const HostScene & s, SceneImage & img, std::string & err)
   h.bytes = (uint32_t)off;
   img.sphBvh.nodes.clear(); img.sphBvh.prims.clear(); img.triBvh.nodes.clear(); img.triBvh.prims.clear();
   img.grids.clear(); img.gridCells.clear(); img.gridSpheres.clear(); img.gridIndex.clear();
-  img.lightGridsBuilt = 0; img.bvhDepth = 0; img.bvhFloat4 = 0; img.triBvhTris = 0;
+  img.lightGridsBuilt = 0; img.bvhDepth = 0; img.bvhFloat4 = 0; img.triBvhTris = 0; img.bvhSpheres = 0;
+  img.triAlways.clear(); img.far = false;
   memset(img.reach, 0, sizeof(img.reach));
   img.spheres.resize(sph.size());
   for (size_t i = 0; i < sph.size(); i++) img.spheres[i] = make_float4(sph[i]->center[0], sph[i]->center[1], sph[i]->center[2], sph[i]->sqRadius);
 
-  // automatic mode: more than 32 spheres, and no planes — a drop point on an (unbounded) plane can lie anywhere, so the box margins
-  // below, which are sized for ray origins inside a bounded region, could not be guaranteed (the reference's Scene cannot hold
-  // planes at all).  Mode 1 builds it for any sphere, but never next to a plane either: a bounce off the plane far outside the
-  // reach box would walk boxes whose margins do not cover its origin and could lose an occluder or a hit the list walk finds.
-  const bool wantBvh = pla.empty() && (s.bvhMode == 1 ? !sph.empty() : s.bvhMode == 2 ? false : sph.size() > 32);
-  // the hierarchy over the triangles: the same automatic rule; mode 1 builds it for any triangle, but never next to a plane (its
-  // margins need bounded drop points)
-  const bool wantTriBvh = pla.empty() && (s.bvhMode == 1 ? !tri.empty() : s.bvhMode == 2 ? false : tri.size() > 32);
+  // automatic mode: more than 32 spheres; mode 1: any.  The box margins below are sized for ray origins inside a bounded reach box;
+  // next to an (unbounded) plane a drop point can lie anywhere, and a query from outside the box grows the boxes it tests by an
+  // amount linear in its distance from the box (farGrowthSpheres): the kernels instantiated with FAR.
+  const bool wantBvh = s.bvhMode == 1 ? !sph.empty() : s.bvhMode == 2 ? false : sph.size() > 32;
+  // the hierarchy over the triangles: the same rule
+  const bool wantTriBvh = s.bvhMode == 1 ? !tri.empty() : s.bvhMode == 2 ? false : tri.size() > 32;
+  const bool farOrigins = !pla.empty();
   double R = 0.0;
   if (wantBvh || wantTriBvh)
   {
     // The reach box: every possible ray origin — the camera eye and all drop points (on spheres and triangles) — and every centre.
     // Its diagonal R bounds |origin - centre| in the box margins.  (Planes are unbounded: a drop point on a plane can lie outside the
-    // box; the reference's Scene cannot hold planes, and rfx_set_camera re-flattens the scene when the eye leaves the box.)
+    // box, and the queries from there grow the boxes (farGrowthSpheres); rfx_set_camera re-flattens the scene when the eye leaves the box.)
     float lo[3] = { s.eye[0], s.eye[1], s.eye[2] }, hi[3] = { s.eye[0], s.eye[1], s.eye[2] };
     for (int k = 0; k < 3; k++)
       if (s.extraOrigins[k] <= s.extraOrigins[3 + k])   // origins of explicit ray lists (rfx_trace_rays)
@@ -521,8 +571,7 @@ int buildSceneImage(const HostScene & s, SceneImage & img, std::string & err)
       memcpy(p.c, sph[i]->center, sizeof(p.c));
       p.r = sph[i]->radius;
       p.index = (int)i;
-      p.m = sphereMargin(p.r, R);
-      for (int k = 0; k < 3; k++) { p.lo[k] = p.c[k] - p.r - p.m; p.hi[k] = p.c[k] + p.r + p.m; }
+      p.m = sphereBox(p.c, p.r, R, p.lo, p.hi);
     }
     std::vector<BvhNode> nodes;
     int maxDepth = 0;
@@ -536,19 +585,24 @@ int buildSceneImage(const HostScene & s, SceneImage & img, std::string & err)
       img.bvhFloat4 = (uint32_t)img.sphBvh.nodes.size();
       h.bvhRoot = img.sphBvh.root;
       h.bvhFloat4 = img.bvhFloat4;
+      img.bvhSpheres = sph.size();
       if (s.lightGridsOn && pla.empty() && !s.lights.empty()) buildLightGrids(s.lights, sph, tri, prims, img);
     }
   }
   if (wantTriBvh)
   {
-    // The hierarchy over the triangles (buildTriBoxes has the boxes and their margins)
+    // The hierarchy over the triangles (buildTriBoxes has the boxes and their margins).  In plane scenes the triangles without a
+    // finite box are tested one by one after the walk instead (h.triAlways).
     std::vector<float> tv(tri.size() * 12), boxes(tri.size() * 6);
     for (size_t i = 0; i < tri.size(); i++) { memcpy(&tv[12 * i], tri[i]->tri.v0, 12); memcpy(&tv[12 * i + 3], tri[i]->tri.ax, 36); }
-    buildTriBoxes((int)tri.size(), tv.data(), img.reach, boxes.data());
-    std::vector<BvhPrim> prims(tri.size());
+    double triReach[6], kappaMax = 0.0;
+    buildTriBoxes((int)tri.size(), tv.data(), img.reach, boxes.data(), farOrigins, triReach, &kappaMax);
+    std::vector<BvhPrim> prims;
+    std::vector<int> always;
     for (size_t i = 0; i < tri.size(); i++)
     {
-      BvhPrim & p = prims[i];
+      if (farOrigins && std::isinf(boxes[6 * i])) { always.push_back((int)i); continue; }
+      BvhPrim p;
       memset(&p, 0, sizeof(p));
       p.index = (int)i;
       for (int k = 0; k < 3; k++)
@@ -556,18 +610,29 @@ int buildSceneImage(const HostScene & s, SceneImage & img, std::string & err)
         p.lo[k] = boxes[6 * i + k]; p.hi[k] = boxes[6 * i + 3 + k];
         p.c[k] = 0.5f * p.lo[k] + 0.5f * p.hi[k];
       }
+      prims.push_back(p);
     }
     std::vector<BvhNode> nodes;
     int maxDepth = 0;
-    buildBvhRec(nodes, prims, 0, (int)prims.size(), 0, maxDepth);
-    if (maxDepth <= BLOB_MAX_BVH_DEPTH)   // deeper (not seen from a median split below ~2^22 triangles): the list walk
+    if (!prims.empty()) buildBvhRec(nodes, prims, 0, (int)prims.size(), 0, maxDepth);
+    if (!prims.empty() && maxDepth <= BLOB_MAX_BVH_DEPTH)   // deeper (not seen from a median split below ~2^22 triangles): the list walk
     {
       // leaf slots of 3 float4 each (the layout of SmallScene::triPk), all zero in the unused ones, which the exact test's gate
       // |rz| > 2^-63 rejects
       packBvh(nodes, prims, 3, 0.0f, [&](int i, float4 * w) { packTriangle(tri[i]->tri, w); }, img.triBvh);
       h.triRoot = img.triBvh.root;
       img.triBvhTris = tri.size();
+      img.triAlways = always;
+      h.nTriAlways = (int)always.size();
+      roundOutwards(triReach, h.triReach);
+      h.growT = farGrowthTris(kappaMax);
     }
+  }
+  if (farOrigins && (img.bvhSpheres || img.triBvhTris))
+  {
+    img.far = true;
+    memcpy(h.sphReach, img.reach, sizeof(h.sphReach));
+    h.growS = farGrowthSpheres();
   }
 
   img.blob.assign(off, 0);
@@ -751,6 +816,23 @@ int rfx_selftest_tri_bounds_host(int n, const float * tris, const float reach[6]
 {
   if (n < 0 || (n && (!tris || !boxes)) || !reach) return RFX_ERR_ARG;
   buildTriBoxes(n, tris, reach, boxes);
+  return RFX_OK;
+}
+
+int rfx_selftest_far_bounds_host(int n_spheres, const float * spheres, int n_tris, const float * tris, const float reach[6],
+                                 float * sphere_boxes, float * tri_boxes, float reaches[12], float grow[2])
+{
+  if (n_spheres < 0 || n_tris < 0 || (n_spheres && (!spheres || !sphere_boxes)) || (n_tris && (!tris || !tri_boxes)) || !reach || !reaches || !grow)
+    return RFX_ERR_ARG;
+  // as buildSceneImage: R from the float reach box, the triangle boxes under the plane-scene rule
+  const double dx = (double)reach[3] - reach[0], dy = (double)reach[4] - reach[1], dz = (double)reach[5] - reach[2];
+  const double R = sqrt(dx * dx + dy * dy + dz * dz);
+  for (int i = 0; i < n_spheres; i++) sphereBox(spheres + 4 * i, spheres[4 * i + 3], R, sphere_boxes + 6 * i, sphere_boxes + 6 * i + 3);
+  double triReach[6], kappaMax = 0.0;
+  buildTriBoxes(n_tris, tris, reach, tri_boxes, true, triReach, &kappaMax);
+  memcpy(reaches, reach, 6 * sizeof(float));
+  roundOutwards(triReach, reaches + 6);
+  grow[0] = farGrowthSpheres(); grow[1] = farGrowthTris(kappaMax);
   return RFX_OK;
 }
 

@@ -50,7 +50,7 @@ struct HostScene
   std::vector<HostObj> objs;
   std::vector<HostTex> tex;                 // uploaded before the image is built: TexRef and SmallScene carry their device pointers
   int skyTex = -1;
-  int bvhMode = 0;                          // 0 auto (spheres > 32, triangles > 32), 1 always, 2 never (no plane: 0, 1) — tests compare them
+  int bvhMode = 0;                          // 0 auto (spheres > 32, triangles > 32), 1 always, 2 never — tests compare them
   bool lightGridsOn = true;                 // rfx_set_option "light_grids"
   // ray origins the hierarchies' box margins must cover (besides every drop point)
   float eye[3] = { 0, 0, 0 };               // the camera's
@@ -86,6 +86,9 @@ struct SceneImage
   int bvhDepth = 0;                         // depth of the sphere hierarchy (0: none)
   uint32_t bvhFloat4 = 0;                   // SceneHeader::bvhFloat4
   uint64_t triBvhTris = 0;                  // triangles under the triangle hierarchy (0: list walk)
+  uint64_t bvhSpheres = 0;                  // spheres under the sphere hierarchy (0: list walk)
+  std::vector<int> triAlways;               // SceneHeader::triAlways (plane scenes: triangles tested after the walk)
+  bool far = false;                         // the scene has a plane and a hierarchy: the kernels instantiated with FAR
 };
 
 // flattens the host scene into img, rebuilt in place: its arrays keep their memory from the last image (a re-flatten of a big scene then

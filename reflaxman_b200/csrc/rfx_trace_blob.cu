@@ -3,6 +3,7 @@
 //   k_blob_wave_first<GRIDS> + k_blob_wave_rest   one-sample ARGB frames of reflection depth >= 3 as a two-kernel wavefront (below)
 //   k_trace_blob_any                       arbitrary pixel slices, block preview, signature runs
 //   k_trace_blob_rays                      Scene::trace for an explicit ray list (rfx_trace_rays)
+// Every one of them also comes with FAR = true, for scenes with a plane and a hierarchy (queries from outside the reach box grow boxes).
 // All of them run ONE restatement of Scene::trace, traceBlob<SIG, MODE> (round 1 kept a second one, k_trace in rfx_kernels.cu, with two
 // inlined traversals; it is gone).
 //
@@ -30,6 +31,8 @@
 // Scene.cpp:73-236, Render.cpp:136-215.
 #include "rfx_kernels.h"
 #include "rfx_device.cuh"
+
+#include <type_traits>
 
 namespace rfx
 {
@@ -100,9 +103,12 @@ __device__ __forceinline__ void consider(Hit & best, float dist, int idx, int or
 
 // The pair-node walk of a hierarchy (the spheres' and the triangles'), in the scope of intersectBlob: the slab-test terms ix, iy, iz,
 // oxi, oyi, ozi, the pruning distance reachT (refreshed from best.dist after every leaf), invLen, the per-thread stack and STRIDE.
-// SMEM_: the nodes are in shared memory; PAIRS / ROOT: nodes and root ref; LEAF(slot): the exact test of a leaf's slots;
-// OPEN: false once an any-hit query has its occluder (the walk ends).
-#define RFX_BLOB_WALK(SMEM_, PAIRS, ROOT, LEAF, OPEN)                                                                          \
+// SMEM_: the nodes are in shared memory; FAR_: every slab interval is widened by gx, gy, gz (the query's box growth times |ix|,
+// |iy|, |iz|: the box grown on every side, see farGrowth), its bounds rounded outwards; PAIRS / ROOT: nodes and root ref;
+// LEAF(slot): the exact test of a leaf's slots; OPEN: false once an any-hit query has its occluder (the walk ends).
+#define RFX_WIDEN_LO(F, T, G) ((F) ? __fsub_rd((T), (G)) : (T))
+#define RFX_WIDEN_HI(F, T, G) ((F) ? __fadd_ru((T), (G)) : (T))
+#define RFX_BLOB_WALK(SMEM_, FAR_, PAIRS, ROOT, LEAF, OPEN)                                                                    \
   {                                                                                                                          \
     constexpr int DONE = (int)0x80000000;                                                                                    \
     const float4 * __restrict__ pn = (PAIRS);                                                                                \
@@ -123,10 +129,14 @@ __device__ __forceinline__ void consider(Hit & best, float dist, int idx, int or
         const float bx1 = __fmaf_rn(n2.x, ix, oxi), bx2 = __fmaf_rn(n3.x, ix, oxi);                                          \
         const float by1 = __fmaf_rn(n2.y, iy, oyi), by2 = __fmaf_rn(n3.y, iy, oyi);                                          \
         const float bz1 = __fmaf_rn(n2.z, iz, ozi), bz2 = __fmaf_rn(n3.z, iz, ozi);                                          \
-        const float tminA = fmaxf(fmaxf(fminf(ax1, ax2), fminf(ay1, ay2)), fmaxf(fminf(az1, az2), 0.0f));                    \
-        const float tmaxA = fminf(fminf(fmaxf(ax1, ax2), fmaxf(ay1, ay2)), fmaxf(az1, az2));                                 \
-        const float tminB = fmaxf(fmaxf(fminf(bx1, bx2), fminf(by1, by2)), fmaxf(fminf(bz1, bz2), 0.0f));                    \
-        const float tmaxB = fminf(fminf(fmaxf(bx1, bx2), fmaxf(by1, by2)), fmaxf(bz1, bz2));                                 \
+        const float tminA = fmaxf(fmaxf(RFX_WIDEN_LO(FAR_, fminf(ax1, ax2), gx), RFX_WIDEN_LO(FAR_, fminf(ay1, ay2), gy)),               \
+                                  fmaxf(RFX_WIDEN_LO(FAR_, fminf(az1, az2), gz), 0.0f));                                           \
+        const float tmaxA = fminf(fminf(RFX_WIDEN_HI(FAR_, fmaxf(ax1, ax2), gx), RFX_WIDEN_HI(FAR_, fmaxf(ay1, ay2), gy)),               \
+                                  RFX_WIDEN_HI(FAR_, fmaxf(az1, az2), gz));                                                        \
+        const float tminB = fmaxf(fmaxf(RFX_WIDEN_LO(FAR_, fminf(bx1, bx2), gx), RFX_WIDEN_LO(FAR_, fminf(by1, by2), gy)),               \
+                                  fmaxf(RFX_WIDEN_LO(FAR_, fminf(bz1, bz2), gz), 0.0f));                                           \
+        const float tmaxB = fminf(fminf(RFX_WIDEN_HI(FAR_, fmaxf(bx1, bx2), gx), RFX_WIDEN_HI(FAR_, fmaxf(by1, by2), gy)),               \
+                                  RFX_WIDEN_HI(FAR_, fmaxf(bz1, bz2), gz));                                                        \
         const bool hitA = tminA <= tmaxA && !(tminA > reachT);                                                               \
         const bool hitB = tminB <= tmaxB && !(tminB > reachT);                                                               \
         int ra = __float_as_int(n0.w), rb = __float_as_int(n1.w);                                                            \
@@ -147,6 +157,17 @@ __device__ __forceinline__ void consider(Hit & best, float dist, int idx, int or
     }                                                                                                                        \
   }
 
+// Box growth of a query from origin o in a scene with a plane (rfx_scene.cpp, the comment above farGrowthSpheres): grow times the
+// sum of o's per-axis distances outside the reach box (lo xyz, hi xyz), rounded upwards; 0 from inside the box (and for a NaN origin,
+// which no exact test accepts).
+__device__ __forceinline__ float farGrowth(const float * __restrict__ box, float grow, V3 o)
+{
+  const float ex = fmaxf(fmaxf(__fsub_ru(box[0], o.x), __fsub_ru(o.x, box[3])), 0.0f);
+  const float ey = fmaxf(fmaxf(__fsub_ru(box[1], o.y), __fsub_ru(o.y, box[4])), 0.0f);
+  const float ez = fmaxf(fmaxf(__fsub_ru(box[2], o.z), __fsub_ru(o.z, box[5])), 0.0f);
+  return __fmul_ru(grow, __fadd_ru(__fadd_ru(ex, ey), ez));
+}
+
 // All objects against one ray; `skip` = object the query ignores (-1 none); anyHit = shadow query (stop at the first hit).
 // STRIDE: threads of the CTA (the traversal stack is one column per thread).  SMEM: bvh points at the CTA's shared-memory copy of
 // the hierarchy (leaf sphere records, then pair nodes), else at the global arrays (read-only path).
@@ -154,7 +175,9 @@ __device__ __forceinline__ void consider(Hit & best, float dist, int idx, int or
 // GRIDS = false compiles the candidate-list branch out (the queue-driven kernel, see traceBlob).
 // TRIS: the scene has a hierarchy over its triangles (h.triPairs) and the triangles are walked through it instead of one by one;
 // the host picks the instantiation by scene, so the kernels of scenes without one are compiled as before.
-template <int STRIDE, bool SMEM, bool GRIDS, bool TRIS = false>
+// FAR: the scene has a plane, so the origin can lie outside the box the hierarchies' margins are sized for: the query grows the
+// boxes it tests (farGrowth) and tests the triangles that are in no box (h.triAlways) after the triangle walk.
+template <int STRIDE, bool SMEM, bool GRIDS, bool TRIS = false, bool FAR = false>
 __device__ __forceinline__ void intersectBlob(const BlobView & sc, int * __restrict__ stack, V3 o, V3 d, int skip, bool anyHit, Hit & best,
                                               const uint32_t * __restrict__ cellStart, const float4 * __restrict__ itemSphere,
                                               const int * __restrict__ itemIndex, int cell)
@@ -256,11 +279,17 @@ __device__ __forceinline__ void intersectBlob(const BlobView & sc, int * __restr
     // for |d| > ~1.8e19: 1/sqrtf(inf) = 0 would make reachT 0 after the first hit and prune every box ahead, so such rays prune nothing
     const float invLen = (a < FLT_MAX) ? 1.0f / sqrtf(a) : __int_as_float(0x7F800000);
     float reachT = (best.dist * 1.001f + 1e-2f) * invLen;
+    float gx = 0.0f, gy = 0.0f, gz = 0.0f;
+    if (FAR)
+    {
+      const float g = farGrowth(h.sphReach, h.growS, o);
+      gx = __fmul_ru(g, fabsf(ix)); gy = __fmul_ru(g, fabsf(iy)); gz = __fmul_ru(g, fabsf(iz));
+    }
     // pair nodes: one trip tests both children of an inner node; the walk continues into a hit child in a register (the nearer
     // one) and only defers the other to the stack; "while-while": every lane walks to its next leaf, then the warp tests its
     // leaves together.  The bottom stack entry is the end marker.  (Single-box nodes, if-if order and far-child-first were
     // measured slower: profiles/README.md.)
-    RFX_BLOB_WALK(SMEM, sc.bvhPairs, h.bvhRoot, RFX_BLOB_LEAF, open)
+    RFX_BLOB_WALK(SMEM, FAR, sc.bvhPairs, h.bvhRoot, RFX_BLOB_LEAF, open)
   }
 #undef RFX_BLOB_LEAF
 #undef RFX_BLOB_TAIL
@@ -314,6 +343,12 @@ __device__ __forceinline__ void intersectBlob(const BlobView & sc, int * __restr
       const float oxi = -(o.x * ix), oyi = -(o.y * iy), ozi = -(o.z * iz);
       const float invLen = (a < FLT_MAX) ? 1.0f / sqrtf(a) : __int_as_float(0x7F800000);   // as in the sphere walk
       float reachT = (best.dist * 1.001f + 1e-2f) * invLen;
+      float gx = 0.0f, gy = 0.0f, gz = 0.0f;
+      if (FAR)
+      {
+        const float g = farGrowth(h.triReach, h.growT, o);
+        gx = __fmul_ru(g, fabsf(ix)); gy = __fmul_ru(g, fabsf(iy)); gz = __fmul_ru(g, fabsf(iz));
+      }
 #define RFX_TRI_LEAF(CA)                                                                                       \
       {                                                                                                        \
         _Pragma("unroll 1")                                                                                    \
@@ -324,8 +359,19 @@ __device__ __forceinline__ void intersectBlob(const BlobView & sc, int * __restr
           RFX_BLOB_TRI(__ldg(h.triPrims + j), q0.x, q0.y, q0.z, q1.z, q1.w, q2.x, q2.y, q2.z, q2.w, q0.w, q1.x, q1.y) \
         }                                                                                                      \
       }
-      RFX_BLOB_WALK(false, h.triPairs, h.triRoot, RFX_TRI_LEAF, openT)
+      RFX_BLOB_WALK(false, FAR, h.triPairs, h.triRoot, RFX_TRI_LEAF, openT)
 #undef RFX_TRI_LEAF
+      if (FAR)
+      {
+        // the triangles no box holds from far origins (slivers, non-finite bases), one by one
+#pragma unroll 1
+        for (int j = 0; j < h.nTriAlways && openT; j++)
+        {
+          const int k = __ldg(h.triAlways + j);
+          const Triangle & tr = sc.tris[k];
+          RFX_BLOB_TRI(k, tr.v0[0], tr.v0[1], tr.v0[2], tr.ax[0], tr.ax[1], tr.ax[2], tr.ax[3], tr.ax[4], tr.ax[5], tr.ax[6], tr.ax[7], tr.ax[8])
+        }
+      }
     }
   }
   else
@@ -426,7 +472,7 @@ constexpr int MODE_QUEUE = 2;       // paths come from the queue; a lane whose p
 // only part of it) — that kernel keeps walking the hierarchy for every query.  profiles/r2_grid has the measurements.
 // Kernels that serve the batch path are instantiated both ways and the host picks by scene, because the grid branch costs a scene
 // without far lights 4-5 % although it is never taken (registers across the walk).
-template <bool SIG, int MODE, int STRIDE = BLOB_THREADS, bool SMEM = false, bool GRIDS = (MODE != MODE_QUEUE), bool TRIS = false>
+template <bool SIG, int MODE, int STRIDE = BLOB_THREADS, bool SMEM = false, bool GRIDS = (MODE != MODE_QUEUE), bool TRIS = false, bool FAR = false>
 __device__ __forceinline__ bool traceBlob(const BlobView & sc, int * __restrict__ stack, V3 & qo, V3 & qd, int reflNumber, V3 randDir,
                                           V3 & mul, V3 & pix, uint32_t & events, uint32_t & sig, QueueFeed * feed = nullptr, int firstSegments = 1,
                                           const EyeGrid * eyeGrid = nullptr, int eyeCell = -1)   // candidates of the first query (origin = eye), or NULL
@@ -506,7 +552,7 @@ __device__ __forceinline__ bool traceBlob(const BlobView & sc, int * __restrict_
       cellStart = eyeGrid->cellStart; itemSphere = eyeGrid->itemSphere; itemIndex = eyeGrid->itemIndex;
       cell = eyeCell;
     }
-    intersectBlob<STRIDE, SMEM, GRIDS, TRIS>(sc, stack, qo, qd, shadowQuery ? hidx : -1, shadowQuery, hit, cellStart, itemSphere, itemIndex, cell);
+    intersectBlob<STRIDE, SMEM, GRIDS, TRIS, FAR>(sc, stack, qo, qd, shadowQuery ? hidx : -1, shadowQuery, hit, cellStart, itemSphere, itemIndex, cell);
 
     bool ended = false;
     if (!shadowQuery)
@@ -667,13 +713,13 @@ __device__ __forceinline__ bool traceBlob(const BlobView & sc, int * __restrict_
 }
 
 // one whole Scene::trace call
-template <bool SIG, bool GRIDS = true, bool TRIS = false>
+template <bool SIG, bool GRIDS = true, bool TRIS = false, bool FAR = false>
 __device__ __forceinline__ V3 tracePath(const BlobView & sc, int * __restrict__ stack, V3 origin, V3 ray, int reflNumber, V3 randDir, uint32_t & events, uint32_t & sig,
                                         const EyeGrid * eyeGrid = nullptr, int eyeCell = -1)
 {
   V3 qo = origin, qd = ray, mul = mk(1.0f, 1.0f, 1.0f), pix = mk(0.0f, 0.0f, 0.0f);
   events = 0;
-  traceBlob<SIG, MODE_PATH, BLOB_THREADS, false, GRIDS, TRIS>(sc, stack, qo, qd, reflNumber, randDir, mul, pix, events, sig, nullptr, 1, eyeGrid, eyeCell);
+  traceBlob<SIG, MODE_PATH, BLOB_THREADS, false, GRIDS, TRIS, FAR>(sc, stack, qo, qd, reflNumber, randDir, mul, pix, events, sig, nullptr, 1, eyeGrid, eyeCell);
   return pix;
 }
 
@@ -694,7 +740,7 @@ __device__ __forceinline__ void flushBlobCounters(unsigned long long * __restric
 // K2 for row-aligned slices of blob scenes.  MULTI = false: one sample per pixel, no jitter (the batch path of the bench).
 // MULTI = true: the same tiling for grid SSAA (Render.cpp:174-196: the thread walks its s*s samples in the reference's ssx, ssy
 // order so the sum is formed in the same order) and additive jitter / accumulation (Render.cpp:177-178, :196-207).
-template <bool MULTI, bool GRIDS, bool TRIS = false>
+template <bool MULTI, bool GRIDS, bool TRIS = false, bool FAR = false>
 __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob(const unsigned char * __restrict__ sceneBlob, const __grid_constant__ FrameParams fp,
                                                                 const uint32_t * __restrict__ sampleStates, uint32_t * __restrict__ argbOut,
                                                                 unsigned long long * __restrict__ counters, uint32_t y0, uint32_t y1,
@@ -725,7 +771,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob
       V3 rd;
       rngTriple(s, rd.x, rd.y, rd.z);
       uint32_t events = 0, sig = 0;
-      c = tracePath<false, GRIDS, TRIS>(sc, stackMem + threadIdx.x, eye, ray, fp.reflNum, rd, events, sig, eg, eyeCell);   // one sample: colour / 1 == colour
+      c = tracePath<false, GRIDS, TRIS, FAR>(sc, stackMem + threadIdx.x, eye, ray, fp.reflNum, rd, events, sig, eg, eyeCell);   // one sample: colour / 1 == colour
       nBounces = events & 0xFFFFu; nShadow = events >> 16;
     }
     else
@@ -754,7 +800,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob
                           (px * fp.view[3] + py * fp.view[4]) + fp.rz * fp.view[5],
                           (px * fp.view[6] + py * fp.view[7]) + fp.rz * fp.view[8]);
         uint32_t events = 0, sig = 0;
-        const V3 one = tracePath<false, GRIDS, TRIS>(sc, stackMem + threadIdx.x, eye, ray, fp.reflNum, rd, events, sig, eg, eyeCell);
+        const V3 one = tracePath<false, GRIDS, TRIS, FAR>(sc, stackMem + threadIdx.x, eye, ray, fp.reflNum, rd, events, sig, eg, eyeCell);
         nBounces += events & 0xFFFFu; nShadow += events >> 16;
         c = vadd(c, one);
       }
@@ -802,7 +848,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob
 // queue-driven kernel, and what bounds both is SIMT divergence inside the traversal — the queue-driven kernel issues at
 // 11.5 of 32 lanes although every lane holds a path (ncu, profiles/r2_s7) — not idle lanes and not the L1 pipeline (the
 // shared-memory copy of the hierarchy is worth 1.5 %).
-template <bool GRIDS, bool TRIS = false>
+template <bool GRIDS, bool TRIS = false, bool FAR = false>
 __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_blob_wave_first(const unsigned char * __restrict__ sceneBlob, const __grid_constant__ FrameParams fp,
                                                                      const uint32_t * __restrict__ sampleStates, uint32_t * __restrict__ argbOut,
                                                                      unsigned long long * __restrict__ counters, uint32_t y0, uint32_t y1, PathQueue queue,
@@ -833,7 +879,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_blob_wave_
     V3 rd;
     rngTriple(s, rd.x, rd.y, rd.z);
     uint32_t sig = 0;
-    alive = !traceBlob<false, MODE_FIRST, BLOB_THREADS, false, GRIDS, TRIS>(sc, stackMem + threadIdx.x, qo, qd, fp.reflNum, rd, mul, pix, events, sig, nullptr, firstSegments, eg, eyeCell);
+    alive = !traceBlob<false, MODE_FIRST, BLOB_THREADS, false, GRIDS, TRIS, FAR>(sc, stackMem + threadIdx.x, qo, qd, fp.reflNum, rd, mul, pix, events, sig, nullptr, firstSegments, eg, eyeCell);
     if (!alive)
     {
       argbOut[q] = packArgb(pix.x, pix.y, pix.z);
@@ -859,7 +905,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_blob_wave_
   flushBlobCounters(counters, nBounces, nShadow, (blockIdx.y * gridDim.x + blockIdx.x) * (BLOB_THREADS / 32) + warp);
 }
 
-template <int THREADS, bool SMEM, bool TRIS = false>
+template <int THREADS, bool SMEM, bool TRIS = false, bool FAR = false>
 __global__ void __launch_bounds__(THREADS, SMEM ? 2 : RFX_BLOB_MINBLOCKS) k_blob_wave_rest(const unsigned char * __restrict__ sceneBlob, int reflNum,
                                                                     uint32_t * __restrict__ argbSlice,
                                                                     unsigned long long * __restrict__ counters, PathQueue queue)
@@ -888,13 +934,13 @@ __global__ void __launch_bounds__(THREADS, SMEM ? 2 : RFX_BLOB_MINBLOCKS) k_blob
   feed.doneBounces = 0; feed.doneShadow = 0;
   V3 qo = mk(0.0f, 0.0f, 0.0f), qd = qo, mul = qo, pix = qo;
   uint32_t events = 0, sig = 0;
-  traceBlob<false, MODE_QUEUE, THREADS, SMEM, false, TRIS>(sc, stackMem + threadIdx.x, qo, qd, reflNum, qo, mul, pix, events, sig, &feed);
+  traceBlob<false, MODE_QUEUE, THREADS, SMEM, false, TRIS, FAR>(sc, stackMem + threadIdx.x, qo, qd, reflNum, qo, mul, pix, events, sig, &feed);
   flushBlobCounters(counters, feed.doneBounces, feed.doneShadow, blockIdx.x * (THREADS / 32) + (threadIdx.x >> 5));
 }
 
 // ---- general kernel: every mode of Render::renderNext for blob scenes (arbitrary pixel slices, block preview, signatures; grid SSAA,
 // additive jitter, float image) — the blob counterpart of k_trace_small_any.  One thread per pixel (or per block origin).
-template <bool TRIS = false>
+template <bool TRIS = false, bool FAR = false>
 __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob_any(const unsigned char * __restrict__ sceneBlob, const __grid_constant__ FrameParams fp,
                                                                     const uint32_t * __restrict__ sampleStates, float * __restrict__ image,
                                                                     uint32_t * __restrict__ argbOut, uint32_t * __restrict__ sigOut,
@@ -978,7 +1024,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob
                         (px * fp.view[3] + py * fp.view[4]) + fp.rz * fp.view[5],
                         (px * fp.view[6] + py * fp.view[7]) + fp.rz * fp.view[8]);
       uint32_t events = 0;
-      const V3 c = tracePath<true, true, TRIS>(sc, stackMem + threadIdx.x, eye, ray, fp.reflNum, rd, events, sig, eg, eyeCell);
+      const V3 c = tracePath<true, true, TRIS, FAR>(sc, stackMem + threadIdx.x, eye, ray, fp.reflNum, rd, events, sig, eg, eyeCell);
       nBounces += events & 0xFFFFu; nShadow += events >> 16;
       fin = blockMode ? c : vadd(fin, c);
       if (++ssy == sn) { ssy = 0; ssx++; }                  // ssx outer, ssy inner: the reference's summation order
@@ -1010,7 +1056,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob
 }
 
 // ---- Scene::trace for an explicit ray list (rfx_trace_rays): ray i uses sampleStates[i]
-template <bool TRIS = false>
+template <bool TRIS = false, bool FAR = false>
 __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob_rays(const unsigned char * __restrict__ sceneBlob, int n,
                                                                      const float * __restrict__ origins, const float * __restrict__ rays, int reflNum,
                                                                      const uint32_t * __restrict__ sampleStates, float * __restrict__ rgbOut,
@@ -1025,11 +1071,18 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob
     uint32_t s = sampleStates[i], sig = 0;
     V3 rd;
     rngTriple(s, rd.x, rd.y, rd.z);
-    const V3 c = tracePath<false, true, TRIS>(sc, stackMem + threadIdx.x, mk(origins[3 * i], origins[3 * i + 1], origins[3 * i + 2]),
+    const V3 c = tracePath<false, true, TRIS, FAR>(sc, stackMem + threadIdx.x, mk(origins[3 * i], origins[3 * i + 1], origins[3 * i + 2]),
                                   mk(rays[3 * i], rays[3 * i + 1], rays[3 * i + 2]), reflNum, rd, events, sig);
     rgbOut[3 * i] = c.x; rgbOut[3 * i + 1] = c.y; rgbOut[3 * i + 2] = c.z;
   }
   flushBlobCounters(counters, events & 0xFFFFu, events >> 16, blockIdx.x * (BLOB_THREADS / 32) + (threadIdx.x >> 5));
+}
+
+// calls f(std::true_type()) or f(std::false_type()): a run-time flag picks a kernel instantiation
+template <typename F> inline void withFlag(bool b, F && f)
+{
+  if (b) f(std::true_type());
+  else f(std::false_type());
 }
 
 } // namespace
@@ -1062,45 +1115,34 @@ int launchTraceBlobFast(const TraceWork & w, cudaStream_t st, void * queueRecord
     if (cudaMemsetAsync(queueCounters, 0, 2 * sizeof(uint32_t), st) != cudaSuccess) return 0;
     PathQueue q;
     q.records = reinterpret_cast<uint4 *>(queueRecords); q.count = queueCounters; q.cursor = queueCounters + 1;
-#define RFX_LAUNCH_FIRST(G, T) k_blob_wave_first<G, T><<<grid, BLOB_THREADS, 0, st>>>(blob, fp, w.sampleStates, w.argbOut, w.counters, y0, y1, q, firstSegments, w.eyeGrid)
     const bool gridsFirst = w.lightGrids || w.eyeGrid.cellStart != nullptr;
-    if (w.triBvh) { if (gridsFirst) RFX_LAUNCH_FIRST(true, true); else RFX_LAUNCH_FIRST(false, true); }
-    else if (gridsFirst) RFX_LAUNCH_FIRST(true, false);
-    else RFX_LAUNCH_FIRST(false, false);
-#undef RFX_LAUNCH_FIRST
+    withFlag(gridsFirst, [&](auto G) { withFlag(w.triBvh, [&](auto T) { withFlag(w.far, [&](auto F) {
+      k_blob_wave_first<decltype(G)::value, decltype(T)::value, decltype(F)::value><<<grid, BLOB_THREADS, 0, st>>>(blob, fp, w.sampleStates, w.argbOut, w.counters, y0, y1, q, firstSegments, w.eyeGrid);
+    }); }); });
     // the hierarchy in shared memory when it fits next to the stacks of two 512-thread CTAs per SM
     const size_t stackBytes512 = (size_t)BLOB_STACK * 512 * sizeof(int), bvhBytes = (size_t)bvhFloat4 * sizeof(float4);
-    if (bvhFloat4 && stackBytes512 + bvhBytes <= 100 * 1024)
-    {
-      // (the triangle hierarchy, if any, stays in global memory and L1)
-      const auto kRest = w.triBvh ? k_blob_wave_rest<512, true, true> : k_blob_wave_rest<512, true, false>;
-      if (cudaFuncSetAttribute(kRest, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(stackBytes512 + bvhBytes)) != cudaSuccess) return 0;
-      kRest<<<persistentCtas / 4, 512, stackBytes512 + bvhBytes, st>>>(blob, fp.reflNum, w.argbOut + fp.p0, w.counters, q);
-    }
-    else
-    {
-      const auto kRest = w.triBvh ? k_blob_wave_rest<BLOB_THREADS, false, true> : k_blob_wave_rest<BLOB_THREADS, false, false>;
-      kRest<<<persistentCtas, BLOB_THREADS, (size_t)BLOB_STACK * BLOB_THREADS * sizeof(int), st>>>(blob, fp.reflNum, w.argbOut + fp.p0, w.counters, q);
-    }
-    return 2;
+    bool ok = true;
+    withFlag(w.triBvh, [&](auto T) { withFlag(w.far, [&](auto F) {
+      if (bvhFloat4 && stackBytes512 + bvhBytes <= 100 * 1024)
+      {
+        // (the triangle hierarchy, if any, stays in global memory and L1)
+        const auto kRest = k_blob_wave_rest<512, true, decltype(T)::value, decltype(F)::value>;
+        if (cudaFuncSetAttribute(kRest, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(stackBytes512 + bvhBytes)) != cudaSuccess) { ok = false; return; }
+        kRest<<<persistentCtas / 4, 512, stackBytes512 + bvhBytes, st>>>(blob, fp.reflNum, w.argbOut + fp.p0, w.counters, q);
+      }
+      else
+        k_blob_wave_rest<BLOB_THREADS, false, decltype(T)::value, decltype(F)::value><<<persistentCtas, BLOB_THREADS, (size_t)BLOB_STACK * BLOB_THREADS * sizeof(int), st>>>(
+            blob, fp.reflNum, w.argbOut + fp.p0, w.counters, q);
+    }); });
+    return ok ? 2 : 0;
   }
   // 128-bit framebuffer stores need a 16-byte aligned frame: a caller's offset sub-buffer goes to the general kernel
   if (w.argbOut && (fp.W & 3u) == 0u && (reinterpret_cast<uintptr_t>(w.argbOut) & 15u) != 0u) return 0;
   const bool multi = !(fp.sampleNum == 1 && !fp.jitter);
-#define RFX_LAUNCH_BLOB(M, G, T) k_trace_blob<M, G, T><<<grid, BLOB_THREADS, 0, st>>>(blob, fp, w.sampleStates, w.argbOut, w.counters, y0, y1, w.image, w.eyeGrid)
   const bool grids = w.lightGrids || w.eyeGrid.cellStart != nullptr;
-  if (w.triBvh)
-  {
-    if (!multi && grids) RFX_LAUNCH_BLOB(false, true, true);
-    else if (!multi) RFX_LAUNCH_BLOB(false, false, true);
-    else if (grids) RFX_LAUNCH_BLOB(true, true, true);
-    else RFX_LAUNCH_BLOB(true, false, true);
-  }
-  else if (!multi && grids) RFX_LAUNCH_BLOB(false, true, false);
-  else if (!multi) RFX_LAUNCH_BLOB(false, false, false);
-  else if (grids) RFX_LAUNCH_BLOB(true, true, false);
-  else RFX_LAUNCH_BLOB(true, false, false);
-#undef RFX_LAUNCH_BLOB
+  withFlag(multi, [&](auto M) { withFlag(grids, [&](auto G) { withFlag(w.triBvh, [&](auto T) { withFlag(w.far, [&](auto F) {
+    k_trace_blob<decltype(M)::value, decltype(G)::value, decltype(T)::value, decltype(F)::value><<<grid, BLOB_THREADS, 0, st>>>(blob, fp, w.sampleStates, w.argbOut, w.counters, y0, y1, w.image, w.eyeGrid);
+  }); }); }); });
   return 1;
 }
 
@@ -1128,19 +1170,21 @@ int launchTraceBlobAny(const TraceWork & w, cudaStream_t st)
   }
   if (nThreads == 0) return 0;
   const uint32_t blocks = (uint32_t)((nThreads + BLOB_THREADS - 1) / BLOB_THREADS);
-  const auto kAny = w.triBvh ? k_trace_blob_any<true> : k_trace_blob_any<false>;
-  kAny<<<blocks, BLOB_THREADS, 0, st>>>(reinterpret_cast<const unsigned char *>(w.sceneBlob), fp, w.sampleStates, w.image, w.argbOut, w.sigOut,
-                                        w.counters, tiled, w.eyeGrid);
+  withFlag(w.triBvh, [&](auto T) { withFlag(w.far, [&](auto F) {
+    k_trace_blob_any<decltype(T)::value, decltype(F)::value><<<blocks, BLOB_THREADS, 0, st>>>(reinterpret_cast<const unsigned char *>(w.sceneBlob), fp, w.sampleStates, w.image,
+                                                                       w.argbOut, w.sigOut, w.counters, tiled, w.eyeGrid);
+  }); });
   return 1;
 }
 
 int launchTraceBlobRays(const void * sceneBlob, int n, const float * origins, const float * rays, int reflNum,
-                        const uint32_t * sampleStates, float * rgbOut, unsigned long long * counters, cudaStream_t st, bool triBvh)
+                        const uint32_t * sampleStates, float * rgbOut, unsigned long long * counters, cudaStream_t st, bool triBvh, bool far)
 {
   if (n <= 0) return 0;
-  const auto kRays = triBvh ? k_trace_blob_rays<true> : k_trace_blob_rays<false>;
-  kRays<<<(n + BLOB_THREADS - 1) / BLOB_THREADS, BLOB_THREADS, 0, st>>>(reinterpret_cast<const unsigned char *>(sceneBlob), n, origins, rays, reflNum,
-                                                                                    sampleStates, rgbOut, counters);
+  withFlag(triBvh, [&](auto T) { withFlag(far, [&](auto F) {
+    k_trace_blob_rays<decltype(T)::value, decltype(F)::value><<<(n + BLOB_THREADS - 1) / BLOB_THREADS, BLOB_THREADS, 0, st>>>(reinterpret_cast<const unsigned char *>(sceneBlob), n,
+                                                                                                       origins, rays, reflNum, sampleStates, rgbOut, counters);
+  }); });
   return 1;
 }
 

@@ -85,6 +85,14 @@ struct SceneHeader
   const float4 * triLeaf;           // 3 float4 per slot, then the pair nodes
   const float4 * triPairs;
   int triRoot;
+  // Scenes with a plane and a hierarchy (rfx_scene.cpp farGrowthSpheres): a drop point on a plane can lie outside the box of ray origins
+  // the margins were sized for.  A query whose origin o lies outside a reach box grows every box of that hierarchy by
+  // grow * (L1 distance of o from the reach box); from inside it grows nothing.  Only the kernels instantiated with FAR read these.
+  float sphReach[6];                // lo xyz, hi xyz: the box the sphere margins assume (every origin and every centre)
+  float triReach[6];                // the same for the triangle margins (sphReach joined with every effective triangle)
+  float growS, growT;               // growth per unit of distance, rounded upwards
+  const int * triAlways;            // plane scenes: triangles no margin can hold from far origins (slivers, non-finite), sorted-array
+  int nTriAlways;                   // positions, tested one by one after the triangle walk; they are not in the hierarchy
 };
 
 // Small scenes travel as a kernel parameter (constant bank): see rfx_trace_small.cu

@@ -152,6 +152,13 @@ def mesh_scene(n_u, n_v, spheres=0, floor=None, skybox=None):
     return base
 
 
+def with_ground_plane(scene, y=-0.05, refl=0.6, mtype=MT_METAL):
+    """The same scene over an unbounded ground plane y = ``y`` facing up (a little below the floor triangles of :func:`synthetic_scene`):
+    a reflective plane sends bounces from points far outside the objects' box back into the scene."""
+    objs = list(scene["objects"]) + [("plane", (0.0, float(y), 0.0), (0.0, 1.0, 0.0), mtype, (0.55, 0.6, 0.65), float(refl), 0.0)]
+    return dict(scene, objects=objs)
+
+
 def expand_meshes(scene):
     """The same scene with every "mesh" object replaced by its triangles, in order (untextured "tri" objects)."""
     objs = []
