@@ -294,4 +294,183 @@ __device__ __forceinline__ uint32_t packArgb(float r, float g, float b)   // Col
 
 #define RFX_SIG(h, ev) ((h) = ((h) ^ (uint32_t)(ev)) * 16777619u)
 
+// =====================================================================================================================
+// the pixel loop of Render::renderNext (Render.cpp:136-215), shared by the K2 kernels of both scene families
+// =====================================================================================================================
+// primary ray through the point (px, py) of the image plane, relative to the image centre (Render.cpp:184-186)
+__device__ __forceinline__ V3 primaryRay(const FrameParams & fp, float px, float py)
+{
+  return mk((px * fp.view[0] + py * fp.view[1]) + fp.rz * fp.view[2],
+            (px * fp.view[3] + py * fp.view[4]) + fp.rz * fp.view[5],
+            (px * fp.view[6] + py * fp.view[7]) + fp.rz * fp.view[8]);
+}
+
+// additive jitter of the pixel with index rel inside the slice: two draws per pixel, Render.cpp:177-178
+__device__ __forceinline__ void pixelJitter(const FrameParams & fp, uint32_t rel, float & rndx, float & rndy)
+{
+  uint32_t s = lcgJump(fp.seedRender, 2u * rel);
+  s = 214013u * s + 2531011u; rndx = divExact(float((int)((s >> 16) & 0x7FFFu)), 32767.0f, RFX_RCP_32767);
+  s = 214013u * s + 2531011u; rndy = divExact(float((int)((s >> 16) & 0x7FFFu)), 32767.0f, RFX_RCP_32767);
+}
+
+// The sn * sn Scene::trace calls of one pixel (Render.cpp:174-196) in the reference's order, ssx outer and ssy inner, so that
+// the sum is formed in the same order; then finColor /= float(s*s).  x / 1.0f == x exactly, so sn == 1 skips every divide.
+// block: block preview (Render.cpp:158-173: sn == 1, no sub-pixel offset, the colour is the call's own).  Call k uses the random
+// state st[k], read through the read-only cache when ldg is set.  trace(ray, randDir, events) is one Scene::trace call.
+// Returns the pixel's colour; adds the calls' bounce-loop iterations and shadow rays to bounces and shadow, and raises longest
+// to the iterations of the longest call.
+template <typename Trace>
+__device__ __forceinline__ V3 samplePixel(const FrameParams & fp, float rx, float ry, float rndx, float rndy, int sn, bool block, const uint32_t * st,
+                                          bool ldg, uint32_t & bounces, uint32_t & shadow, uint32_t & longest, Trace trace)
+{
+  V3 fin = mk(0.0f, 0.0f, 0.0f);
+  const int nCalls = sn * sn;
+  int ssx = 0, ssy = 0;
+#pragma unroll 1
+  for (int call = 0; call < nCalls; call++)
+  {
+    uint32_t s = ldg ? __ldg(st + call) : st[call];
+    V3 rd;
+    rngTriple(s, rd.x, rd.y, rd.z);
+    float px = rx, py = ry;
+    if (!block)
+    {
+      // (rx + float(ssx)/s) + rndx, Render.cpp:184
+      const float offx = sn == 1 ? 0.0f : float(ssx) / float(sn);
+      const float offy = sn == 1 ? 0.0f : float(ssy) / float(sn);
+      px = (rx + offx) + rndx;
+      py = (ry + offy) + rndy;
+    }
+    const V3 ray = primaryRay(fp, px, py);
+    uint32_t ev = 0;
+    const V3 c = trace(ray, rd, ev);
+    fin = block ? c : vadd(fin, c);
+    bounces += ev & 0xFFFFu; shadow += ev >> 16;
+    longest = max(longest, ev & 0xFFFFu);
+    if (++ssy == sn) { ssy = 0; ssx++; }
+  }
+  if (sn != 1)   // Color::operator/=, Color.cpp:50-61 (its guard |s*s| > 2^-63 always holds)
+  {
+    const float sq = float(nCalls);
+    fin = mk(fin.x / sq, fin.y / sq, fin.z / sq);
+  }
+  return fin;
+}
+
+// One-sample framebuffer store of a warp's pixel tile (tileW pixels wide).  The four lanes of a tile row hold four consecutive
+// pixels; the first of them stores all four as one 128-bit word when all four are in the image (16-byte aligned when W is a
+// multiple of 4 and the frame is), so a warp writes a 4x8 tile with 8 STG.128 and L2 merges them into lines.  out: the lane's
+// pixel (any address when !valid).
+__device__ __forceinline__ void storeTileRow(uint32_t * out, uint32_t packed, bool valid, uint32_t W, uint32_t tileW)
+{
+  const uint32_t lane = threadIdx.x & 31u;
+  const uint32_t p1 = __shfl_down_sync(0xffffffffu, packed, 1), p2 = __shfl_down_sync(0xffffffffu, packed, 2), p3 = __shfl_down_sync(0xffffffffu, packed, 3);
+  const uint32_t validMask = __ballot_sync(0xffffffffu, valid);
+  const bool rowOfFour = tileW % 4u == 0u && (W & 3u) == 0u && ((validMask >> (lane & ~3u)) & 0xFu) == 0xFu;
+  if (rowOfFour)
+  {
+    if ((lane & 3u) == 0u) *reinterpret_cast<uint4 *>(out) = make_uint4(packed, p1, p2, p3);
+  }
+  else if (valid) *out = packed;
+}
+
+// event counters: one striped atomic pair per warp
+__device__ __forceinline__ void flushCounters(unsigned long long * __restrict__ counters, uint32_t nBounces, uint32_t nShadow, uint32_t warpId)
+{
+  if (!counters) return;   // uniform
+  __syncwarp();
+  const uint32_t wb = __reduce_add_sync(0xffffffffu, nBounces);
+  const uint32_t ws = __reduce_add_sync(0xffffffffu, nShadow);
+  if ((threadIdx.x & 31u) == 0u)
+  {
+    const uint32_t slot = warpId & 31u;
+    atomicAdd(&counters[slot * 2], (unsigned long long)wb);
+    atomicAdd(&counters[slot * 2 + 1], (unsigned long long)ws);
+  }
+}
+
+// General K2 body: every mode of Render::renderNext — block preview, grid SSAA, additive jitter, arbitrary pixel slices, float
+// image, signatures — one lane per pixel or per block origin.  tiled: the slice is whole rows and each warp renders one tile of
+// tileW x (32 / tileW) pixels; threads: the CTA size.  pixelTrace(x, y) returns the Scene::trace call of pixel (x, y),
+// trace(ray, randDir, events, sig), where sig is the pixel's hit-path signature.
+template <typename PixelTrace>
+__device__ __forceinline__ void renderAny(const FrameParams & fp, const uint32_t * __restrict__ sampleStates, float * __restrict__ image,
+                                          uint32_t * __restrict__ argbOut, uint32_t * __restrict__ sigOut,
+                                          unsigned long long * __restrict__ counters, int tiled, uint32_t tileW, uint32_t threads,
+                                          PixelTrace pixelTrace)
+{
+  uint32_t nBounces = 0, nShadow = 0;
+  const uint64_t gid = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+
+  // ---- which pixel does this lane own, and how many Scene::trace calls does it make
+  const bool blockMode = fp.sampleNum < 0;                 // block preview, Render.cpp:158-173
+  const uint32_t blk = blockMode ? (uint32_t)(-fp.sampleNum) : 1u;
+  const int sn = blockMode ? 1 : fp.sampleNum;             // grid SSAA factor, Render.cpp:174-196
+  uint32_t x, y;
+  bool valid;
+  uint64_t firstState;                                     // index of this lane's first ranked random state
+  if (blockMode)
+  {
+    // gid enumerates block origins in scan order starting at rank fp.firstRank
+    const uint32_t bw = (fp.W + blk - 1) / blk;
+    const uint64_t k = fp.firstRank + gid;
+    y = (uint32_t)(k / bw) * blk; x = (uint32_t)(k % bw) * blk;
+    valid = y < fp.H && ((uint64_t)y * fp.W + x) < fp.p1;
+    firstState = gid;
+  }
+  else if (tiled)
+  {
+    // row-aligned slice (a whole frame, a band of rows, or this GPU's strips of a split frame): one pixel tile per warp
+    const uint32_t tileH = 32u / tileW;
+    const uint32_t tilesX = (fp.W + (tileW - 1u)) / tileW;
+    const uint32_t y0 = (uint32_t)(fp.p0 / fp.W), y1 = (uint32_t)(fp.p1 / fp.W);
+    const uint32_t warp = (uint32_t)(gid >> 5), lane = threadIdx.x & 31u;
+    x = (warp % tilesX) * tileW + (lane % tileW);
+    y = y0 + (warp / tilesX) * tileH + (lane / tileW);
+    if (fp.stripWorld)
+    {
+      const uint32_t k = y / fp.stripRows;
+      y = (k * fp.stripWorld + fp.stripRank) * fp.stripRows + (y % fp.stripRows);
+    }
+    valid = x < fp.W && y < y1;
+    firstState = (((uint64_t)y * fp.W + x) - fp.p0) * (uint64_t)(sn * sn);
+  }
+  else
+  {
+    const uint64_t p = fp.p0 + gid;
+    valid = p < fp.p1;
+    y = (uint32_t)(p / fp.W); x = (uint32_t)(p % fp.W);
+    firstState = gid * (uint64_t)(sn * sn);
+  }
+
+  if (valid)
+  {
+    const uint64_t p = (uint64_t)y * fp.W + x;
+    float rndx = 0, rndy = 0;
+    if (fp.jitter && !blockMode) pixelJitter(fp, (uint32_t)(p - fp.p0), rndx, rndy);
+    uint32_t sig = 2166136261u, longest = 0;
+    const auto trace = pixelTrace(x, y);
+    const V3 fin = samplePixel(fp, float(x) - fp.wHalf, float(y) - fp.hHalf, rndx, rndy, sn, blockMode, sampleStates + firstState, false,
+                               nBounces, nShadow, longest, [&](V3 ray, V3 rd, uint32_t & ev) { return trace(ray, rd, ev, sig); });
+    const uint32_t ex = min(x + blk, fp.W), ey = min(y + blk, fp.H);
+    const uint32_t packed = packArgb(fin.x, fin.y, fin.z);
+#pragma unroll 1
+    for (uint32_t qy = y; qy < ey; qy++)
+#pragma unroll 1
+      for (uint32_t qx = x; qx < ex; qx++)
+      {
+        const uint64_t q = (uint64_t)qy * fp.W + qx;
+        if (image)
+        {
+          float * px = image + q * 3;
+          if (fp.accumulate && !blockMode) { px[0] = px[0] + fin.x; px[1] = px[1] + fin.y; px[2] = px[2] + fin.z; }
+          else { px[0] = fin.x; px[1] = fin.y; px[2] = fin.z; }
+        }
+        if (argbOut) argbOut[q] = packed;
+        if (sigOut) sigOut[q] = sig;
+      }
+  }
+  flushCounters(counters, nBounces, nShadow, blockIdx.x * (threads / 32) + (threadIdx.x >> 5));
+}
+
 } // namespace rfx

@@ -3,6 +3,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <type_traits>
 #include "rfx_types.h"
 
 namespace rfx
@@ -142,6 +143,40 @@ PrimaryCull makePrimaryCull(const SmallScene & sc, const FrameParams & fp);
 struct PrimaryCamera { double c[3][3], eye[3], rz, wHalf, hHalf, W, H; bool ok; };   // ok = false: no bounds (camera not orthonormal): whole image
 PrimaryCamera makePrimaryCamera(const FrameParams & fp);
 int4 primarySphereBounds(const PrimaryCamera & cam, const float4 & sphere);   // x0, x1, y0, y1 inclusive; x0 > x1: no pixel
+
+// rows a launch over `rows` whole rows enumerates: all of them, or in a split frame (fp.stripWorld > 0) the rows of this rank's
+// strips, full strips plus the (possibly shorter) last strip, rounded up to whole strips
+inline uint64_t ownedRows(const FrameParams & fp, uint64_t rows)
+{
+  if (!fp.stripWorld) return rows;
+  const uint64_t nStrips = (rows + fp.stripRows - 1) / fp.stripRows;
+  const uint64_t mine = nStrips > fp.stripRank ? (nStrips - fp.stripRank + fp.stripWorld - 1) / fp.stripWorld : 0;
+  return mine * fp.stripRows;
+}
+
+// threads of a general K2 kernel (k_trace_small_any, k_trace_blob_any) for this work, 0 = nothing to render.  tiled = 1: the slice
+// is whole rows and each warp renders a tile of tileW x (32 / tileW) pixels; tiled = 0: one thread per pixel or block origin
+inline uint64_t anyThreads(const FrameParams & fp, uint32_t tileW, int & tiled)
+{
+  tiled = 0;
+  if (fp.sampleNum <= 0)
+  {
+    const uint32_t a = (uint32_t)(-fp.sampleNum);
+    const uint32_t bw = (fp.W + a - 1) / a, bh = (fp.H + a - 1) / a;
+    return (uint64_t)bw * bh - fp.firstRank;   // upper bound; threads past p1 exit
+  }
+  if (fp.p0 % fp.W != 0 || fp.p1 % fp.W != 0) return fp.p1 - fp.p0;
+  tiled = 1;
+  const uint64_t rows = ownedRows(fp, (fp.p1 - fp.p0) / fp.W), tileH = 32u / tileW;
+  return (uint64_t)((fp.W + tileW - 1) / tileW) * ((rows + tileH - 1) / tileH) * 32u;
+}
+
+// calls f(std::true_type()) or f(std::false_type()): a run-time flag picks a kernel instantiation
+template <typename F> inline void withFlag(bool b, F && f)
+{
+  if (b) f(std::true_type());
+  else f(std::false_type());
+}
 
 // ---- K3: resolve (imagePixel + argb) ---------------------------------------------------------------------------
 int launchResolve(const float * image, uint64_t nPixels, int additiveCounter, float * rgbfOut, uint32_t * argbOut, cudaStream_t st);

@@ -32,8 +32,6 @@
 #include "rfx_kernels.h"
 #include "rfx_device.cuh"
 
-#include <type_traits>
-
 namespace rfx
 {
 
@@ -723,20 +721,6 @@ __device__ __forceinline__ V3 tracePath(const BlobView & sc, int * __restrict__ 
   return pix;
 }
 
-__device__ __forceinline__ void flushBlobCounters(unsigned long long * __restrict__ counters, uint32_t nBounces, uint32_t nShadow, uint32_t warpId)
-{
-  if (!counters) return;   // uniform
-  __syncwarp();
-  const uint32_t wb = __reduce_add_sync(0xffffffffu, nBounces);
-  const uint32_t ws = __reduce_add_sync(0xffffffffu, nShadow);
-  if ((threadIdx.x & 31u) == 0u)
-  {
-    const uint32_t slot = warpId & 31u;
-    atomicAdd(&counters[slot * 2], (unsigned long long)wb);
-    atomicAdd(&counters[slot * 2 + 1], (unsigned long long)ws);
-  }
-}
-
 // K2 for row-aligned slices of blob scenes.  MULTI = false: one sample per pixel, no jitter (the batch path of the bench).
 // MULTI = true: the same tiling for grid SSAA (Render.cpp:174-196: the thread walks its s*s samples in the reference's ssx, ssy
 // order so the sum is formed in the same order) and additive jitter / accumulation (Render.cpp:177-178, :196-207).
@@ -765,9 +749,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob
     if (!MULTI)
     {
       uint32_t s = __ldg(sampleStates + (q - y0 * fp.W));
-      const V3 ray = mk((rx * fp.view[0] + ry * fp.view[1]) + fp.rz * fp.view[2],
-                        (rx * fp.view[3] + ry * fp.view[4]) + fp.rz * fp.view[5],
-                        (rx * fp.view[6] + ry * fp.view[7]) + fp.rz * fp.view[8]);
+      const V3 ray = primaryRay(fp, rx, ry);
       V3 rd;
       rngTriple(s, rd.x, rd.y, rd.z);
       uint32_t events = 0, sig = 0;
@@ -779,33 +761,13 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob
       const int sn = fp.sampleNum;
       const uint32_t rel = q - y0 * fp.W;                                // pixel index inside the slice
       float rndx = 0, rndy = 0;
-      if (fp.jitter)
-      {
-        uint32_t s = lcgJump(fp.seedRender, 2u * rel);                   // two draws per pixel, Render.cpp:177-178
-        s = 214013u * s + 2531011u; rndx = divExact(float((int)((s >> 16) & 0x7FFFu)), 32767.0f, RFX_RCP_32767);
-        s = 214013u * s + 2531011u; rndy = divExact(float((int)((s >> 16) & 0x7FFFu)), 32767.0f, RFX_RCP_32767);
-      }
-      c = mk(0.0f, 0.0f, 0.0f);
-      const uint32_t * st = sampleStates + (size_t)rel * (size_t)(sn * sn);
-#pragma unroll 1
-      for (int k = 0; k < sn * sn; k++)
-      {
-        const int ssx = k / sn, ssy = k - ssx * sn;
-        uint32_t s = __ldg(st + k);
-        V3 rd;
-        rngTriple(s, rd.x, rd.y, rd.z);
-        const float px = (rx + float(ssx) / float(sn)) + rndx;           // Render.cpp:184
-        const float py = (ry + float(ssy) / float(sn)) + rndy;
-        const V3 ray = mk((px * fp.view[0] + py * fp.view[1]) + fp.rz * fp.view[2],
-                          (px * fp.view[3] + py * fp.view[4]) + fp.rz * fp.view[5],
-                          (px * fp.view[6] + py * fp.view[7]) + fp.rz * fp.view[8]);
-        uint32_t events = 0, sig = 0;
-        const V3 one = tracePath<false, GRIDS, TRIS, FAR>(sc, stackMem + threadIdx.x, eye, ray, fp.reflNum, rd, events, sig, eg, eyeCell);
-        nBounces += events & 0xFFFFu; nShadow += events >> 16;
-        c = vadd(c, one);
-      }
-      const float sq = float(sn * sn);
-      if (fabsf(sq) > RFX_VSN) c = mk(c.x / sq, c.y / sq, c.z / sq);     // Color::operator/=, Color.cpp:50-61
+      if (fp.jitter) pixelJitter(fp, rel, rndx, rndy);
+      uint32_t longest = 0;
+      c = samplePixel(fp, rx, ry, rndx, rndy, sn, false, sampleStates + (size_t)rel * (size_t)(sn * sn), true, nBounces, nShadow, longest,
+                      [&](V3 ray, V3 rd, uint32_t & events) {
+        uint32_t sig = 0;
+        return tracePath<false, GRIDS, TRIS, FAR>(sc, stackMem + threadIdx.x, eye, ray, fp.reflNum, rd, events, sig, eg, eyeCell);
+      });
     }
     packed = packArgb(c.x, c.y, c.z);
     qOut = q;
@@ -816,19 +778,9 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob
       else { px[0] = c.x; px[1] = c.y; px[2] = c.z; }
     }
   }
-  if (argbOut)
-  {
-    // framebuffer: one 128-bit store per tile row (see k_trace_small)
-    const uint32_t p1 = __shfl_down_sync(0xffffffffu, packed, 1), p2 = __shfl_down_sync(0xffffffffu, packed, 2), p3 = __shfl_down_sync(0xffffffffu, packed, 3);
-    const uint32_t validMask = __ballot_sync(0xffffffffu, valid);
-    if ((fp.W & 3u) == 0u && ((validMask >> (lane & ~3u)) & 0xFu) == 0xFu)
-    {
-      if ((lane & 3u) == 0u) *reinterpret_cast<uint4 *>(argbOut + qOut) = make_uint4(packed, p1, p2, p3);
-    }
-    else if (valid) argbOut[qOut] = packed;
-  }
+  if (argbOut) storeTileRow(argbOut + qOut, packed, valid, fp.W, BLOB_TILE_W);
 
-  flushBlobCounters(counters, nBounces, nShadow, (blockIdx.y * gridDim.x + blockIdx.x) * (BLOB_THREADS / 32) + warp);
+  flushCounters(counters, nBounces, nShadow, (blockIdx.y * gridDim.x + blockIdx.x) * (BLOB_THREADS / 32) + warp);
 }
 
 // ---- wavefront pair for one-sample ARGB frames (the batch path of the bench) -------------------------------------------------
@@ -873,9 +825,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_blob_wave_
     state0 = s;
     const float rx = float(x) - fp.wHalf;                                // Render.cpp:154-155
     const float ry = float(y) - fp.hHalf;
-    qd = mk((rx * fp.view[0] + ry * fp.view[1]) + fp.rz * fp.view[2],
-            (rx * fp.view[3] + ry * fp.view[4]) + fp.rz * fp.view[5],
-            (rx * fp.view[6] + ry * fp.view[7]) + fp.rz * fp.view[8]);
+    qd = primaryRay(fp, rx, ry);
     V3 rd;
     rngTriple(s, rd.x, rd.y, rd.z);
     uint32_t sig = 0;
@@ -902,7 +852,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_blob_wave_
       r[3] = make_uint4(rel, events, state0, 0u);
     }
   }
-  flushBlobCounters(counters, nBounces, nShadow, (blockIdx.y * gridDim.x + blockIdx.x) * (BLOB_THREADS / 32) + warp);
+  flushCounters(counters, nBounces, nShadow, (blockIdx.y * gridDim.x + blockIdx.x) * (BLOB_THREADS / 32) + warp);
 }
 
 template <int THREADS, bool SMEM, bool TRIS = false, bool FAR = false>
@@ -935,7 +885,7 @@ __global__ void __launch_bounds__(THREADS, SMEM ? 2 : RFX_BLOB_MINBLOCKS) k_blob
   V3 qo = mk(0.0f, 0.0f, 0.0f), qd = qo, mul = qo, pix = qo;
   uint32_t events = 0, sig = 0;
   traceBlob<false, MODE_QUEUE, THREADS, SMEM, false, TRIS, FAR>(sc, stackMem + threadIdx.x, qo, qd, reflNum, qo, mul, pix, events, sig, &feed);
-  flushBlobCounters(counters, feed.doneBounces, feed.doneShadow, blockIdx.x * (THREADS / 32) + (threadIdx.x >> 5));
+  flushCounters(counters, feed.doneBounces, feed.doneShadow, blockIdx.x * (THREADS / 32) + (threadIdx.x >> 5));
 }
 
 // ---- general kernel: every mode of Render::renderNext for blob scenes (arbitrary pixel slices, block preview, signatures; grid SSAA,
@@ -949,110 +899,14 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob
 {
   __shared__ int stackMem[BLOB_STACK * BLOB_THREADS];
   const BlobView sc = blobView(sceneBlob);
-  uint32_t nBounces = 0, nShadow = 0;
   const V3 eye = mk(fp.eye[0], fp.eye[1], fp.eye[2]);
-  const uint64_t gid = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const EyeGrid * eg = eyeGrid.cellStart != nullptr ? &eyeGrid : nullptr;
-
-  // ---- which pixel does this lane own, and how many Scene::trace calls does it make
-  const bool blockMode = fp.sampleNum < 0;                 // block preview, Render.cpp:158-173
-  const uint32_t blk = blockMode ? (uint32_t)(-fp.sampleNum) : 1u;
-  const int sn = blockMode ? 1 : fp.sampleNum;             // grid SSAA factor, Render.cpp:174-196
-  uint32_t x, y;
-  bool valid;
-  uint64_t firstState;                                     // index of this lane's first ranked random state
-  if (blockMode)
-  {
-    // gid enumerates block origins in scan order starting at rank fp.firstRank
-    const uint32_t bw = (fp.W + blk - 1) / blk;
-    const uint64_t k = fp.firstRank + gid;
-    y = (uint32_t)(k / bw) * blk; x = (uint32_t)(k % bw) * blk;
-    valid = y < fp.H && ((uint64_t)y * fp.W + x) < fp.p1;
-    firstState = gid;
-  }
-  else if (tiled)
-  {
-    // row-aligned slice (a whole frame or a band of rows): one pixel tile per warp
-    const uint32_t tilesX = (fp.W + (BLOB_TILE_W - 1u)) / BLOB_TILE_W;
-    const uint32_t y0 = (uint32_t)(fp.p0 / fp.W), y1 = (uint32_t)(fp.p1 / fp.W);
-    const uint32_t warp = (uint32_t)(gid >> 5), lane = threadIdx.x & 31u;
-    x = (warp % tilesX) * BLOB_TILE_W + (lane % BLOB_TILE_W);
-    y = y0 + (warp / tilesX) * BLOB_TILE_H + (lane / BLOB_TILE_W);
-    valid = x < fp.W && y < y1;
-    firstState = (((uint64_t)y * fp.W + x) - fp.p0) * (uint64_t)(sn * sn);
-  }
-  else
-  {
-    const uint64_t p = fp.p0 + gid;
-    valid = p < fp.p1;
-    y = (uint32_t)(p / fp.W); x = (uint32_t)(p % fp.W);
-    firstState = gid * (uint64_t)(sn * sn);
-  }
-
-  if (valid)
-  {
-    const uint64_t p = (uint64_t)y * fp.W + x;
-    const float rx = float(x) - fp.wHalf;
-    const float ry = float(y) - fp.hHalf;
-    float rndx = 0, rndy = 0;
-    if (fp.jitter && !blockMode)
-    {
-      uint32_t s = lcgJump(fp.seedRender, (uint32_t)(2 * (p - fp.p0)));      // two draws per pixel, Render.cpp:177-178
-      s = 214013u * s + 2531011u; rndx = divExact(float((int)((s >> 16) & 0x7FFFu)), 32767.0f, RFX_RCP_32767);
-      s = 214013u * s + 2531011u; rndy = divExact(float((int)((s >> 16) & 0x7FFFu)), 32767.0f, RFX_RCP_32767);
-    }
-    V3 fin = mk(0.0f, 0.0f, 0.0f);
-    uint32_t sig = 2166136261u;
+  renderAny(fp, sampleStates, image, argbOut, sigOut, counters, tiled, BLOB_TILE_W, BLOB_THREADS, [&](uint32_t x, uint32_t y) {
     const int eyeCell = eg ? (int)((y >> eyeGrid.shift) * (uint32_t)eyeGrid.nx + (x >> eyeGrid.shift)) : -1;
-    const uint32_t * st = sampleStates + firstState;
-    const int nCalls = sn * sn;
-    int ssx = 0, ssy = 0;
-#pragma unroll 1
-    for (int call = 0; call < nCalls; call++)
-    {
-      uint32_t s = st[call];
-      V3 rd;
-      rngTriple(s, rd.x, rd.y, rd.z);
-      float px = rx, py = ry;
-      if (!blockMode)
-      {
-        // (rx + float(ssx)/s) + rndx, Render.cpp:184
-        px = (rx + float(ssx) / float(sn)) + rndx;
-        py = (ry + float(ssy) / float(sn)) + rndy;
-      }
-      const V3 ray = mk((px * fp.view[0] + py * fp.view[1]) + fp.rz * fp.view[2],
-                        (px * fp.view[3] + py * fp.view[4]) + fp.rz * fp.view[5],
-                        (px * fp.view[6] + py * fp.view[7]) + fp.rz * fp.view[8]);
-      uint32_t events = 0;
-      const V3 c = tracePath<true, true, TRIS, FAR>(sc, stackMem + threadIdx.x, eye, ray, fp.reflNum, rd, events, sig, eg, eyeCell);
-      nBounces += events & 0xFFFFu; nShadow += events >> 16;
-      fin = blockMode ? c : vadd(fin, c);
-      if (++ssy == sn) { ssy = 0; ssx++; }                  // ssx outer, ssy inner: the reference's summation order
-    }
-    if (!blockMode)
-    {
-      const float sq = float(sn * sn);
-      if (fabsf(sq) > RFX_VSN) fin = mk(fin.x / sq, fin.y / sq, fin.z / sq);   // Color::operator/=, Color.cpp:50-61
-    }
-    const uint32_t ex = min(x + blk, fp.W), ey = min(y + blk, fp.H);
-    const uint32_t packed = packArgb(fin.x, fin.y, fin.z);
-#pragma unroll 1
-    for (uint32_t qy = y; qy < ey; qy++)
-#pragma unroll 1
-      for (uint32_t qx = x; qx < ex; qx++)
-      {
-        const uint64_t q = (uint64_t)qy * fp.W + qx;
-        if (image)
-        {
-          float * px = image + q * 3;
-          if (fp.accumulate && !blockMode) { px[0] = px[0] + fin.x; px[1] = px[1] + fin.y; px[2] = px[2] + fin.z; }
-          else { px[0] = fin.x; px[1] = fin.y; px[2] = fin.z; }
-        }
-        if (argbOut) argbOut[q] = packed;
-        if (sigOut) sigOut[q] = sig;
-      }
-  }
-  flushBlobCounters(counters, nBounces, nShadow, blockIdx.x * (BLOB_THREADS / 32) + (threadIdx.x >> 5));
+    return [&, eyeCell](V3 ray, V3 rd, uint32_t & events, uint32_t & sig) {
+      return tracePath<true, true, TRIS, FAR>(sc, stackMem + threadIdx.x, eye, ray, fp.reflNum, rd, events, sig, eg, eyeCell);
+    };
+  });
 }
 
 // ---- Scene::trace for an explicit ray list (rfx_trace_rays): ray i uses sampleStates[i]
@@ -1075,14 +929,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob
                                   mk(rays[3 * i], rays[3 * i + 1], rays[3 * i + 2]), reflNum, rd, events, sig);
     rgbOut[3 * i] = c.x; rgbOut[3 * i + 1] = c.y; rgbOut[3 * i + 2] = c.z;
   }
-  flushBlobCounters(counters, events & 0xFFFFu, events >> 16, blockIdx.x * (BLOB_THREADS / 32) + (threadIdx.x >> 5));
-}
-
-// calls f(std::true_type()) or f(std::false_type()): a run-time flag picks a kernel instantiation
-template <typename F> inline void withFlag(bool b, F && f)
-{
-  if (b) f(std::true_type());
-  else f(std::false_type());
+  flushCounters(counters, events & 0xFFFFu, events >> 16, blockIdx.x * (BLOB_THREADS / 32) + (threadIdx.x >> 5));
 }
 
 } // namespace
@@ -1150,24 +997,8 @@ int launchTraceBlobFast(const TraceWork & w, cudaStream_t st, void * queueRecord
 int launchTraceBlobAny(const TraceWork & w, cudaStream_t st)
 {
   const FrameParams & fp = w.fp;
-  uint64_t nThreads;
-  int tiled = 0;
-  if (fp.sampleNum > 0)
-  {
-    nThreads = fp.p1 - fp.p0;
-    if (fp.p0 % fp.W == 0 && fp.p1 % fp.W == 0)
-    {
-      tiled = 1;
-      const uint64_t rows = (fp.p1 - fp.p0) / fp.W;
-      nThreads = (uint64_t)((fp.W + BLOB_TILE_W - 1) / BLOB_TILE_W) * ((rows + BLOB_TILE_H - 1) / BLOB_TILE_H) * 32u;
-    }
-  }
-  else
-  {
-    const uint32_t a = (uint32_t)(-fp.sampleNum);
-    const uint32_t bw = (fp.W + a - 1) / a, bh = (fp.H + a - 1) / a;
-    nThreads = (uint64_t)bw * bh - fp.firstRank;   // upper bound; threads past p1 exit
-  }
+  int tiled;
+  const uint64_t nThreads = anyThreads(fp, BLOB_TILE_W, tiled);
   if (nThreads == 0) return 0;
   const uint32_t blocks = (uint32_t)((nThreads + BLOB_THREADS - 1) / BLOB_THREADS);
   withFlag(w.triBvh, [&](auto T) { withFlag(w.far, [&](auto F) {

@@ -620,21 +620,6 @@ PrimaryCull makePrimaryCull(const SmallScene & sc, const FrameParams & fp)
 
 // ---- K2 ----------------------------------------------------------------------------------------------------------------
 
-__device__ __forceinline__ void flushCounters(unsigned long long * __restrict__ counters, uint32_t nBounces, uint32_t nShadow, uint32_t warpId)
-{
-  if (!counters) return;   // uniform
-  // event counters: one striped atomic pair per warp
-  __syncwarp();
-  const uint32_t wb = __reduce_add_sync(0xffffffffu, nBounces);
-  const uint32_t ws = __reduce_add_sync(0xffffffffu, nShadow);
-  if ((threadIdx.x & 31) == 0 && counters)
-  {
-    const uint32_t slot = warpId & 31u;
-    atomicAdd(&counters[slot * 2], (unsigned long long)wb);
-    atomicAdd(&counters[slot * 2 + 1], (unsigned long long)ws);
-  }
-}
-
 #ifdef RFX_CTA_TIMES
 // debug build (tools/cta_times.py): start/end time and SM of every CTA of the last fast-kernel launch
 __device__ unsigned long long g_ctaTimes[1 << 16][3];
@@ -751,9 +736,7 @@ __global__ void __launch_bounds__(SMALL_THREADS, MULTI ? 7 : RFX_SMALL_MINBLOCKS
         }
         const float rx = float(x) - fp.wHalf;                            // Render.cpp:154-155
         const float ry = float(y) - fp.hHalf;
-        const V3 ray = mk((rx * fp.view[0] + ry * fp.view[1]) + fp.rz * fp.view[2],
-                          (rx * fp.view[3] + ry * fp.view[4]) + fp.rz * fp.view[5],
-                          (rx * fp.view[6] + ry * fp.view[7]) + fp.rz * fp.view[8]);
+        const V3 ray = primaryRay(fp, rx, ry);
         uint32_t ev = 0, sig = 0;
         const V3 c = traceSmall<false, FEAT, RFX_PRIMARY_CULL != 0, BATCH>(sc, mk(fp.eye[0], fp.eye[1], fp.eye[2]), ray, fp.reflNum, rd, ev, sig,
                                                                          range,
@@ -771,9 +754,7 @@ __global__ void __launch_bounds__(SMALL_THREADS, MULTI ? 7 : RFX_SMALL_MINBLOCKS
       }
       if (BATCH && f < 0) { __syncwarp(); continue; }                    // every lane of the tile starts frame 0 together
       // Framebuffer store of the one-sample path.
-      //  * Frame in local HBM: the four lanes of a tile row hold four consecutive pixels; the first of them stores all four as one
-      //    128-bit word (16-byte aligned when W is a multiple of 4 and the frame is), so a warp writes its 4x8 tile with 8 STG.128;
-      //    L2 merges them into lines.
+      //  * Frame in local HBM: one 128-bit store per tile row (storeTileRow).
       //  * Split frame (rfx_render_strips): argbOut may be ANOTHER GPU's framebuffer (peer mapping), and then every store
       //    instruction leaves this GPU as NVLink write packets.  Eight 16-byte pieces per instruction (one per tile row) throttled
       //    the 7-to-1 gather of an 8K frame to 0.70 ms against 0.48 ms with local stores (profiles/r2_s2), so a tile group that lies
@@ -782,18 +763,7 @@ __global__ void __launch_bounds__(SMALL_THREADS, MULTI ? 7 : RFX_SMALL_MINBLOCKS
       //    (For local frames the staging costs 0.8 % — measured — so they keep the direct stores: STRIPS is a template parameter and
       //    the whole-frame instantiations carry none of this.)
       if (staged) sStage[(lane / RFX_TILE_W) * STAGE_STRIDE + warp * RFX_TILE_W + (lane % RFX_TILE_W)] = packed;
-      else
-      {
-        uint32_t * out = argbOut + (BATCH ? (size_t)f * frameStride : 0) + (valid ? q : 0u);
-        const uint32_t p1 = __shfl_down_sync(0xffffffffu, packed, 1), p2 = __shfl_down_sync(0xffffffffu, packed, 2), p3 = __shfl_down_sync(0xffffffffu, packed, 3);
-        const uint32_t validMask = __ballot_sync(0xffffffffu, valid);
-        const bool rowOfFour = RFX_TILE_W % 4u == 0u && (fp.W & 3u) == 0u && ((validMask >> (lane & ~3u)) & 0xFu) == 0xFu;
-        if (rowOfFour)
-        {
-          if ((lane & 3u) == 0u) *reinterpret_cast<uint4 *>(out) = make_uint4(packed, p1, p2, p3);
-        }
-        else if (valid) *out = packed;
-      }
+      else storeTileRow(argbOut + (BATCH ? (size_t)f * frameStride : 0) + (valid ? q : 0u), packed, valid, fp.W, RFX_TILE_W);
     }
   }
   if (valid && MULTI)
@@ -801,45 +771,13 @@ __global__ void __launch_bounds__(SMALL_THREADS, MULTI ? 7 : RFX_SMALL_MINBLOCKS
     const uint32_t q = y * fp.W + x;
     const uint32_t rel = q - y0 * fp.W;                                  // pixel index inside the slice
     const int sn = fp.sampleNum;
-    const int nCalls = sn * sn;
-    const uint32_t * st = sampleStates + (uint64_t)rel * (uint64_t)nCalls;
-    const float rx = float(x) - fp.wHalf;
-    const float ry = float(y) - fp.hHalf;
     float rndx = 0, rndy = 0;
-    if (fp.jitter)
-    {
-      uint32_t s = lcgJump(fp.seedRender, 2u * rel);                     // two draws per pixel, Render.cpp:177-178
-      s = 214013u * s + 2531011u; rndx = divExact(float((int)((s >> 16) & 0x7FFFu)), 32767.0f, RFX_RCP_32767);
-      s = 214013u * s + 2531011u; rndy = divExact(float((int)((s >> 16) & 0x7FFFu)), 32767.0f, RFX_RCP_32767);
-    }
-    V3 fin = mk(0.0f, 0.0f, 0.0f);
-    int ssx = 0, ssy = 0;
-#pragma unroll 1
-    for (int call = 0; call < nCalls; call++)
-    {
-      uint32_t s = __ldg(st + call);
-      V3 rd;
-      rngTriple(s, rd.x, rd.y, rd.z);
-      // (rx + float(ssx)/s) + rndx, Render.cpp:184; x / 1.0f == x exactly, so sn == 1 skips the divides
-      const float offx = sn == 1 ? 0.0f : float(ssx) / float(sn);
-      const float offy = sn == 1 ? 0.0f : float(ssy) / float(sn);
-      const float px = (rx + offx) + rndx;
-      const float py = (ry + offy) + rndy;
-      const V3 ray = mk((px * fp.view[0] + py * fp.view[1]) + fp.rz * fp.view[2],
-                        (px * fp.view[3] + py * fp.view[4]) + fp.rz * fp.view[5],
-                        (px * fp.view[6] + py * fp.view[7]) + fp.rz * fp.view[8]);
-      uint32_t ev = 0, sig = 0;
-      const V3 c = traceSmall<false, FEAT, RFX_PRIMARY_CULL != 0>(sc, mk(fp.eye[0], fp.eye[1], fp.eye[2]), ray, fp.reflNum, rd, ev, sig, first);
-      fin = vadd(fin, c);
-      nBounces += ev & 0xFFFFu; nShadow += ev >> 16;
-      events = max(events, ev & 0xFFFFu);
-      if (++ssy == sn) { ssy = 0; ssx++; }                  // ssx outer, ssy inner: the reference's summation order
-    }
-    if (sn != 1)   // finColor /= float(s*s): dividing by 1.0f is the identity (Color.cpp:50-61)
-    {
-      const float sq = float(nCalls);
-      fin = mk(fin.x / sq, fin.y / sq, fin.z / sq);
-    }
+    if (fp.jitter) pixelJitter(fp, rel, rndx, rndy);
+    const V3 fin = samplePixel(fp, float(x) - fp.wHalf, float(y) - fp.hHalf, rndx, rndy, sn, false, sampleStates + (uint64_t)rel * (uint64_t)(sn * sn), true,
+                               nBounces, nShadow, events, [&](V3 ray, V3 rd, uint32_t & ev) {
+      uint32_t sig = 0;
+      return traceSmall<false, FEAT, RFX_PRIMARY_CULL != 0>(sc, mk(fp.eye[0], fp.eye[1], fp.eye[2]), ray, fp.reflNum, rd, ev, sig, first);
+    });
     if (image)
     {
       float * px = image + (uint64_t)q * 3;
@@ -894,115 +832,10 @@ __global__ void __launch_bounds__(SMALL_THREADS, RFX_ANY_MINBLOCKS) k_trace_smal
                                                                uint32_t * __restrict__ argbOut, uint32_t * __restrict__ sigOut,
                                                                unsigned long long * __restrict__ counters, int tiled)
 {
-  uint32_t nBounces = 0, nShadow = 0;
   const V3 eye = mk(fp.eye[0], fp.eye[1], fp.eye[2]);
-  const uint64_t gid = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-
-  // ---- which pixel does this lane own, and how many Scene::trace calls does it make -------------------------------
-  const bool blockMode = fp.sampleNum < 0;                 // block preview, Render.cpp:158-173
-  const uint32_t blk = blockMode ? (uint32_t)(-fp.sampleNum) : 1u;
-  const int sn = blockMode ? 1 : fp.sampleNum;             // grid SSAA factor, Render.cpp:174-196
-  uint32_t x, y;
-  bool valid;
-  uint64_t firstState;                                     // index of this lane's first ranked random state
-  if (blockMode)
-  {
-    // gid enumerates block origins in scan order starting at rank fp.firstRank
-    const uint32_t bw = (fp.W + blk - 1) / blk;
-    const uint64_t k = fp.firstRank + gid;
-    y = (uint32_t)(k / bw) * blk; x = (uint32_t)(k % bw) * blk;
-    valid = y < fp.H && ((uint64_t)y * fp.W + x) < fp.p1;
-    firstState = gid;
-  }
-  else if (tiled)
-  {
-    // row-aligned slice (a whole frame or a band of rows): one pixel tile per warp
-    const uint32_t tilesX = (fp.W + (RFX_TILE_W - 1u)) / RFX_TILE_W;
-    const uint32_t y0 = (uint32_t)(fp.p0 / fp.W), y1 = (uint32_t)(fp.p1 / fp.W);
-    const uint32_t warp = (uint32_t)(gid >> 5), lane = threadIdx.x & 31u;
-    x = (warp % tilesX) * RFX_TILE_W + (lane % RFX_TILE_W);
-    y = y0 + (warp / tilesX) * RFX_TILE_H + (lane / RFX_TILE_W);
-    if (fp.stripWorld)
-    {
-      const uint32_t k = y / fp.stripRows;
-      y = (k * fp.stripWorld + fp.stripRank) * fp.stripRows + (y % fp.stripRows);
-    }
-    valid = x < fp.W && y < y1;
-    firstState = (((uint64_t)y * fp.W + x) - fp.p0) * (uint64_t)(sn * sn);
-  }
-  else
-  {
-    const uint64_t p = fp.p0 + gid;
-    valid = p < fp.p1;
-    y = (uint32_t)(p / fp.W); x = (uint32_t)(p % fp.W);
-    firstState = gid * (uint64_t)(sn * sn);
-  }
-
-  if (valid)
-  {
-    const uint64_t p = (uint64_t)y * fp.W + x;
-    const float rx = float(x) - fp.wHalf;
-    const float ry = float(y) - fp.hHalf;
-    float rndx = 0, rndy = 0;
-    if (fp.jitter && !blockMode)
-    {
-      uint32_t s = lcgJump(fp.seedRender, (uint32_t)(2 * (p - fp.p0)));      // two draws per pixel, Render.cpp:177-178
-      s = 214013u * s + 2531011u; rndx = divExact(float((int)((s >> 16) & 0x7FFFu)), 32767.0f, RFX_RCP_32767);
-      s = 214013u * s + 2531011u; rndy = divExact(float((int)((s >> 16) & 0x7FFFu)), 32767.0f, RFX_RCP_32767);
-    }
-    V3 fin = mk(0.0f, 0.0f, 0.0f);
-    uint32_t sig = 2166136261u;
-    const uint32_t * st = sampleStates + firstState;
-    const int nCalls = sn * sn;
-    int ssx = 0, ssy = 0;
-#pragma unroll 1
-    for (int call = 0; call < nCalls; call++)
-    {
-      uint32_t s = st[call];
-      V3 rd;
-      rngTriple(s, rd.x, rd.y, rd.z);
-      float px = rx, py = ry;
-      if (!blockMode)
-      {
-        // (rx + float(ssx)/s) + rndx, Render.cpp:184; x / 1.0f == x exactly, so sn == 1 skips the divides
-        const float offx = sn == 1 ? 0.0f : float(ssx) / float(sn);
-        const float offy = sn == 1 ? 0.0f : float(ssy) / float(sn);
-        px = (rx + offx) + rndx;
-        py = (ry + offy) + rndy;
-      }
-      const V3 ray = mk((px * fp.view[0] + py * fp.view[1]) + fp.rz * fp.view[2],
-                        (px * fp.view[3] + py * fp.view[4]) + fp.rz * fp.view[5],
-                        (px * fp.view[6] + py * fp.view[7]) + fp.rz * fp.view[8]);
-      uint32_t events = 0;
-      const V3 c = traceSmall<true, F_ALL>(sc, eye, ray, fp.reflNum, rd, events, sig);
-      nBounces += events & 0xFFFFu; nShadow += events >> 16;
-      fin = blockMode ? c : vadd(fin, c);
-      if (++ssy == sn) { ssy = 0; ssx++; }                  // ssx outer, ssy inner: the reference's summation order
-    }
-    if (sn != 1)   // finColor /= float(s*s): dividing by 1.0f is the identity (Color.cpp:50-61)
-    {
-      const float sq = float(sn * sn);
-      fin = mk(fin.x / sq, fin.y / sq, fin.z / sq);
-    }
-    const uint32_t ex = min(x + blk, fp.W), ey = min(y + blk, fp.H);
-    const uint32_t packed = packArgb(fin.x, fin.y, fin.z);
-#pragma unroll 1
-    for (uint32_t qy = y; qy < ey; qy++)
-#pragma unroll 1
-      for (uint32_t qx = x; qx < ex; qx++)
-      {
-        const uint64_t q = (uint64_t)qy * fp.W + qx;
-        if (image)
-        {
-          float * px = image + q * 3;
-          if (fp.accumulate && !blockMode) { px[0] = px[0] + fin.x; px[1] = px[1] + fin.y; px[2] = px[2] + fin.z; }
-          else { px[0] = fin.x; px[1] = fin.y; px[2] = fin.z; }
-        }
-        if (argbOut) argbOut[q] = packed;
-        if (sigOut) sigOut[q] = sig;
-      }
-  }
-  flushCounters(counters, nBounces, nShadow, blockIdx.x * (SMALL_THREADS / 32) + (threadIdx.x >> 5));
+  renderAny(fp, sampleStates, image, argbOut, sigOut, counters, tiled, RFX_TILE_W, SMALL_THREADS, [&](uint32_t, uint32_t) {
+    return [&](V3 ray, V3 rd, uint32_t & events, uint32_t & sig) { return traceSmall<true, F_ALL>(sc, eye, ray, fp.reflNum, rd, events, sig); };
+  });
 }
 
 // rows the fast kernel enumerates for this work (0 = does not qualify): whole rows, grid sampling (not block preview), no signatures
@@ -1015,14 +848,7 @@ static uint64_t fastRows(const TraceWork & w)
   // the 128-bit framebuffer stores need a 16-byte aligned frame (rows of a W % 4 == 0 image then stay aligned); a caller's
   // offset sub-buffer that is only 4-byte aligned takes the general kernel's scalar stores
   if (w.argbOut && (fp.W & 3u) == 0u && (reinterpret_cast<uintptr_t>(w.argbOut) & 15u) != 0u) return 0;
-  uint64_t rows = (fp.p1 - fp.p0) / fp.W;
-  if (fp.stripWorld)
-  {
-    // rows owned by this rank: full strips plus the (possibly shorter) last strip, rounded up to whole strips
-    const uint64_t nStrips = (rows + fp.stripRows - 1) / fp.stripRows;
-    const uint64_t mine = nStrips > fp.stripRank ? (nStrips - fp.stripRank + fp.stripWorld - 1) / fp.stripWorld : 0;
-    rows = mine * fp.stripRows;
-  }
+  const uint64_t rows = ownedRows(fp, (fp.p1 - fp.p0) / fp.W);
   if ((rows + RFX_TILE_H - 1) / RFX_TILE_H > 65535u) return 0;
   return rows;
 }
@@ -1051,67 +877,30 @@ int launchTraceSmall(const SmallScene & sc, const TraceWork & w, cudaStream_t st
 {
   if (fastGrid) *fastGrid = 0;
   const FrameParams & fp = w.fp;
-  uint64_t nThreads;
-  int tiled = 0;
-  if (fp.sampleNum > 0)
+  if (fastGridSize(w))
   {
-    if (fp.p0 % fp.W == 0 && fp.p1 % fp.W == 0)
-    {
-      tiled = 1;
-      uint64_t rows = (fp.p1 - fp.p0) / fp.W;
-      if (fp.stripWorld)
-      {
-        // rows owned by this rank: full strips plus the (possibly shorter) last strip, rounded up to whole strips
-        const uint64_t nStrips = (rows + fp.stripRows - 1) / fp.stripRows;
-        const uint64_t mine = nStrips > fp.stripRank ? (nStrips - fp.stripRank + fp.stripWorld - 1) / fp.stripWorld : 0;
-        rows = mine * fp.stripRows;
-      }
-      if (rows == 0) return 0;
-      if (fastGridSize(w))
-      {
-        const dim3 grid = fastGrid3(w, fastRows(w));
-        if (fastGrid) *fastGrid = grid.x * grid.y;
-        // scene features decide the instantiation: texel-free, plane-free, single-light scenes run the lean one
-        bool texels = false;
-        for (int i = 0; i < SMALL_MAX_TEX; i++) texels = texels || sc.tex[i].px != nullptr;
-        const bool lean = !texels && sc.nP == 0 && sc.nL <= 1;
-        const bool multi = fp.sampleNum != 1 || fp.jitter || w.image != nullptr;
-        const uint32_t y0 = (uint32_t)(fp.p0 / fp.W), y1 = (uint32_t)(fp.p1 / fp.W);
-        const PrimaryCull pc = RFX_PRIMARY_CULL ? makePrimaryCull(sc, fp) : PrimaryCull();
-#define RFX_LAUNCH_SMALL(F, M, S, IMG) k_trace_small<F, M, S><<<grid, SMALL_THREADS, 0, st>>>(sc, fp, w.sampleStates, w.argbOut, w.counters, y0, y1, w.order, IMG, pc, 1u)
-        if (w.frames > 1)   // the caller checked fastBatchOk
-        {
-          if (lean) k_trace_small<0, false, false, true><<<grid, SMALL_THREADS, 0, st>>>(sc, fp, w.sampleStates, w.argbOut, w.counters, y0, y1, w.order, nullptr, pc, w.frames);
-          else k_trace_small<F_ALL, false, false, true><<<grid, SMALL_THREADS, 0, st>>>(sc, fp, w.sampleStates, w.argbOut, w.counters, y0, y1, w.order, nullptr, pc, w.frames);
-        }
-        else if (fp.stripWorld)
-        {
-          if (lean && !multi) RFX_LAUNCH_SMALL(0, false, true, nullptr);
-          else if (!multi) RFX_LAUNCH_SMALL(F_ALL, false, true, nullptr);
-          else if (lean) RFX_LAUNCH_SMALL(0, true, true, w.image);
-          else RFX_LAUNCH_SMALL(F_ALL, true, true, w.image);
-        }
-        else
-        {
-          if (lean && !multi) RFX_LAUNCH_SMALL(0, false, false, nullptr);
-          else if (!multi) RFX_LAUNCH_SMALL(F_ALL, false, false, nullptr);
-          else if (lean) RFX_LAUNCH_SMALL(0, true, false, w.image);
-          else RFX_LAUNCH_SMALL(F_ALL, true, false, w.image);
-        }
-#undef RFX_LAUNCH_SMALL
-        return 1;
-      }
-      nThreads = (uint64_t)((fp.W + RFX_TILE_W - 1) / RFX_TILE_W) * ((rows + RFX_TILE_H - 1) / RFX_TILE_H) * 32;
-    }
+    const dim3 grid = fastGrid3(w, fastRows(w));
+    if (fastGrid) *fastGrid = grid.x * grid.y;
+    // scene features decide the instantiation: texel-free, plane-free, single-light scenes run the lean one
+    bool texels = false;
+    for (int i = 0; i < SMALL_MAX_TEX; i++) texels = texels || sc.tex[i].px != nullptr;
+    const bool lean = !texels && sc.nP == 0 && sc.nL <= 1;
+    const bool multi = fp.sampleNum != 1 || fp.jitter || w.image != nullptr;
+    const uint32_t y0 = (uint32_t)(fp.p0 / fp.W), y1 = (uint32_t)(fp.p1 / fp.W);
+    const PrimaryCull pc = RFX_PRIMARY_CULL ? makePrimaryCull(sc, fp) : PrimaryCull();
+    if (w.frames > 1)   // the caller checked fastBatchOk
+      withFlag(lean, [&](auto L) {
+        k_trace_small<decltype(L)::value ? 0 : F_ALL, false, false, true><<<grid, SMALL_THREADS, 0, st>>>(sc, fp, w.sampleStates, w.argbOut, w.counters, y0, y1, w.order, nullptr, pc, w.frames);
+      });
     else
-      nThreads = fp.p1 - fp.p0;
+      withFlag(lean, [&](auto L) { withFlag(multi, [&](auto M) { withFlag(fp.stripWorld != 0, [&](auto S) {
+        k_trace_small<decltype(L)::value ? 0 : F_ALL, decltype(M)::value, decltype(S)::value><<<grid, SMALL_THREADS, 0, st>>>(sc, fp, w.sampleStates, w.argbOut, w.counters, y0, y1,
+                                                                                                    w.order, decltype(M)::value ? w.image : nullptr, pc, 1u);
+      }); }); });
+    return 1;
   }
-  else
-  {
-    const uint32_t a = (uint32_t)(-fp.sampleNum);
-    const uint32_t bw = (fp.W + a - 1) / a, bh = (fp.H + a - 1) / a;
-    nThreads = (uint64_t)bw * bh - fp.firstRank;   // upper bound; threads past p1 exit
-  }
+  int tiled;
+  const uint64_t nThreads = anyThreads(fp, RFX_TILE_W, tiled);
   if (nThreads == 0) return 0;
   const uint32_t blocks = (uint32_t)((nThreads + SMALL_THREADS - 1) / SMALL_THREADS);
   k_trace_small_any<<<blocks, SMALL_THREADS, 0, st>>>(sc, fp, w.sampleStates, w.image, w.argbOut, w.sigOut, w.counters, tiled);
