@@ -370,6 +370,14 @@ class Context:
         self._ck(self.L.rfx_read_rgbf(self.h, out.ctypes.data_as(_fp)), "rfx_read_rgbf")
         return out
 
+    def read_image(self, divide=True):
+        """rfx_read_image: (float image [H, W, 3], ARGB [H, W]).  divide=False reads the raw sums of the additive passes, as
+        Render::copyImage packs them; divide=True divides by the additive counter as imagePixel does."""
+        rgbf = np.empty((self.H, self.W, 3), np.float32)
+        argb = np.empty((self.H, self.W), np.uint32)
+        self._ck(self.L.rfx_read_image(self.h, rgbf.ctypes.data_as(_fp), argb.ctypes.data_as(_u32p), 1 if divide else 0), "rfx_read_image")
+        return rgbf, argb
+
     def read_pixel(self, x, y):
         out = (C.c_float * 3)()
         self._ck(self.L.rfx_read_pixel(self.h, x, y, out), "rfx_read_pixel")

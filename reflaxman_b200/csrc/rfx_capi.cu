@@ -933,12 +933,18 @@ int rfx_render_strips(rfx_ctx * ctx, uint32_t strip_rows, uint32_t world, uint32
   if ((rc = profileStart(ctx, st, evStop)) != RFX_OK) return rc;
   if ((rc = armTileOrder(ctx, w, st)) != RFX_OK) return rc;
   {
-    const int nl = launchTraceSmall(ctx->image.small, w, st);
-    ctx->stats.kernel_launches += nl; ctx->stats.launches_small_fast += nl;
+    uint32_t fastGrid = 0;   // 0: the fast kernel declined (a 4-byte aligned frame) and the general kernel ran
+    const int nl = launchTraceSmall(ctx->image.small, w, st, &fastGrid);
+    ctx->stats.kernel_launches += nl;
+    (fastGrid ? ctx->stats.launches_small_fast : ctx->stats.launches_small_any) += nl;
   }
   if (evStop) CK(cudaEventRecord(evStop, st));
   CK(cudaGetLastError());
-  ctx->stats.samples += calls / world;
+  // the Scene::trace calls of this rank's own rows: its whole strips, less what the frame cuts off its last strip
+  const uint32_t nStrips = (ctx->H + strip_rows - 1) / strip_rows;
+  uint64_t ownRows = ownedRows(w.fp, ctx->H);
+  if ((nStrips - 1) % world == rank) ownRows -= (uint64_t)nStrips * strip_rows - ctx->H;
+  ctx->stats.samples += ownRows * ctx->W * perPixel;
   ctx->cursor = total;
   ctx->inProgress = false;
   return RFX_OK;
