@@ -95,6 +95,14 @@ RFX_API int rfx_add_triangle(rfx_ctx * ctx, const float v[9], int mtype, const f
  * objects (rfx_set_triangle_texture applies to each). */
 RFX_API int rfx_add_mesh(rfx_ctx * ctx, uint32_t n_vertices, const float * xyz, uint32_t n_tris, const uint32_t * idx, int mtype,
                          const float rgb[3], float reflectivity, float transparency);
+/* Replace the vertex positions of a mesh added by rfx_add_mesh.  first = the object index rfx_add_mesh returned; xyz = n_vertices x 3
+ * floats, n_vertices as given to rfx_add_mesh (the index list, the material and any rfx_set_triangle_texture stay).  Every later output
+ * is bit-identical to that of a scene built with the same calls but rfx_add_mesh(xyz).  Returns 1 when the device scene was updated in
+ * place (queued on the stream the renders use, no synchronisation: the triangles are set up and the triangle hierarchy is refitted on
+ * the GPU, keeping the hierarchy's topology), 0 when the scene will be re-flattened on the host at the next render instead (the scene
+ * fits the constant bank, a re-flatten is pending anyway, or the new vertices leave the box the hierarchies or the light grids were
+ * built for), or a negative error code: RFX_ERR_ARG for NULL xyz or a first that does not start a mesh of this scene. */
+RFX_API int rfx_update_mesh(rfx_ctx * ctx, int first, const float * xyz);
 RFX_API int rfx_set_triangle_texture(rfx_ctx * ctx, int object, int texture, const float uv[6]); /* Triangle::setTexture, Triangle.cpp:110-120 (u1,v1,u2,v2,u3,v3) */
 RFX_API int rfx_add_plane(rfx_ctx * ctx, const float pos[3], const float norm[3], int mtype, const float rgb[3],
                           float reflectivity, float transparency);                              /* Plane::Plane, Plane.cpp:9-14 (no Scene::addPlane exists upstream) */

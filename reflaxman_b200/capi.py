@@ -45,6 +45,7 @@ SYMBOLS = [
     ("rfx_add_sphere", C.c_int, [C.c_void_p, _fp, C.c_float, C.c_int, _fp, C.c_float, C.c_float]),
     ("rfx_add_triangle", C.c_int, [C.c_void_p, _fp, C.c_int, _fp, C.c_float, C.c_float]),
     ("rfx_add_mesh", C.c_int, [C.c_void_p, C.c_uint32, _fp, C.c_uint32, _u32p, C.c_int, _fp, C.c_float, C.c_float]),
+    ("rfx_update_mesh", C.c_int, [C.c_void_p, C.c_int, _fp]),
     ("rfx_set_triangle_texture", C.c_int, [C.c_void_p, C.c_int, C.c_int, _fp]),
     ("rfx_add_plane", C.c_int, [C.c_void_p, _fp, _fp, C.c_int, _fp, C.c_float, C.c_float]),
     ("rfx_add_texture_argb", C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, _u32p]),
@@ -239,6 +240,7 @@ class Context:
             raise RfxError("rfx_create failed (%d): %s" % (rc, self.L.rfx_last_error(None).decode()))
         self.h = h
         self.W = self.H = 0
+        self._mesh_vertices = {}   # first object index of each mesh -> its vertex count
 
     def close(self):
         if getattr(self, "h", None):
@@ -258,9 +260,12 @@ class Context:
 
     # ---- scene -----------------------------------------------------------------------------------------------
     def load_scene(self, scene):
-        """Issue a scenes.py dict through the scene-building calls, in the reference's order (Render.cpp:32-54)."""
+        """Issue a scenes.py dict through the scene-building calls, in the reference's order (Render.cpp:32-54).  Returns the first
+        object index of each "mesh" entry, in order (what :meth:`update_mesh` takes)."""
         rgb, p = scene["ambient"]
         self._ck(self.L.rfx_scene_reset(self.h, _f(rgb)[1], C.c_float(p)), "rfx_scene_reset")
+        self._mesh_vertices = {}
+        meshes = []
         tex_ids = []
         for t in scene["textures"]:
             tex_ids.append(self.add_texture(t))
@@ -279,19 +284,31 @@ class Context:
                     self._ck(self.L.rfx_set_triangle_texture(self.h, idx, tex_ids[tex], _f(uv)[1]), "rfx_set_triangle_texture")
             elif ob[0] == "mesh":
                 _, xyz, idx, mt, col, refl, tr = ob
-                self.add_mesh(xyz, idx, mt, col, refl, tr)
+                meshes.append(self.add_mesh(xyz, idx, mt, col, refl, tr))
             elif ob[0] == "plane":
                 _, pos, nrm, mt, col, refl, tr = ob
                 self._ck(self.L.rfx_add_plane(self.h, _f(pos)[1], _f(nrm)[1], mt, _f(col)[1], C.c_float(refl), C.c_float(tr)), "rfx_add_plane")
             else:
                 raise ValueError(ob[0])
+        return meshes
 
     def add_mesh(self, xyz, idx, mtype, rgb, refl, transp):
         """rfx_add_mesh: xyz [N][3] vertices, idx [M][3] vertex indices; returns the object index of the first of the M triangles."""
         v = np.ascontiguousarray(xyz, dtype=np.float32).reshape(-1, 3)
         ix = np.ascontiguousarray(idx, dtype=np.uint32).reshape(-1, 3)
-        return self._ck(self.L.rfx_add_mesh(self.h, v.shape[0], v.ctypes.data_as(_fp), ix.shape[0], ix.ctypes.data_as(_u32p), mtype,
-                                            _f(rgb)[1], C.c_float(refl), C.c_float(transp)), "rfx_add_mesh")
+        first = self._ck(self.L.rfx_add_mesh(self.h, v.shape[0], v.ctypes.data_as(_fp), ix.shape[0], ix.ctypes.data_as(_u32p), mtype,
+                                             _f(rgb)[1], C.c_float(refl), C.c_float(transp)), "rfx_add_mesh")
+        self._mesh_vertices[first] = v.shape[0]
+        return first
+
+    def update_mesh(self, first, xyz):
+        """rfx_update_mesh: new vertices xyz [N][3] for the mesh whose first triangle is object ``first`` (N as given to add_mesh).
+        True: the device scene was updated in place; False: the scene is re-flattened on the host at the next render."""
+        v = np.ascontiguousarray(xyz, dtype=np.float32).reshape(-1, 3)
+        n = self._mesh_vertices.get(first)
+        if n is not None and v.shape[0] != n:
+            raise ValueError("update_mesh: %d vertices given, the mesh has %d" % (v.shape[0], n))
+        return self._ck(self.L.rfx_update_mesh(self.h, first, v.ctypes.data_as(_fp)), "rfx_update_mesh") == 1
 
     def add_texture(self, argb):
         if argb is None:

@@ -91,7 +91,15 @@ struct rfx_ctx
   uint64_t eyeGridBuilds = 0;
   DevArray<float4> dTriNodes;               // hierarchy over the triangles: leaf slots, then pair nodes
   DevArray<int> dTriPrims;
-  DevArray<int> dTriAlways;                 // plane scenes: triangles tested after the triangle walk (SceneHeader::triAlways)
+  DevArray<int> dTriAlways;                 // plane scenes: triangles tested after the triangle walk (SceneHeader::triAlways); with meshes
+                                            // room for every triangle (rfx_update_mesh appends slivers)
+  // mesh updates on the device (rfx_update_mesh, MeshUpdate): uploaded by uploadScene for blob scenes with meshes
+  DevArray<uint32_t> dMeshIdx;              // every mesh's index list (SceneImage::meshIdx)
+  DevArray<int> dTriSlot, dLeafParent, dPairParent;
+  DevArray<unsigned char> dInAlways;        // per triangle: appended to triAlways since the flatten
+  DevArray<uint32_t> dArrive;               // per pair node: refit arrival counters
+  DevArray<unsigned long long> dMeshRed;    // [14]: an update's reduction record (MeshUpdate::red), then its value at the flatten
+  DevArray<float> dVerts;                   // the vertices of the mesh being updated
 
   // ---- camera + render state (reference Render.h:9-27); the eye is scene.eye
   float view[9] = { 1, 0, 0, 0, 1, 0, 0, 0, 1 }, fov = 1.0f;
@@ -195,6 +203,7 @@ int uploadScene(rfx_ctx * ctx, cudaStream_t st)
 
   SceneImage & img = ctx->image;
   int rc;
+  refreshMeshes(ctx->scene);
   if ((rc = buildSceneImage(ctx->scene, img, ctx->err)) != RFX_OK) return rc;
   SceneHeader & h = *reinterpret_cast<SceneHeader *>(img.blob.data());
   h.byteLut = ctx->dLut.p;
@@ -225,6 +234,26 @@ int uploadScene(rfx_ctx * ctx, cudaStream_t st)
     h.triPrims = ctx->dTriPrims.p;
     h.triLeaf = ctx->dTriNodes.p;
     h.triPairs = ctx->dTriNodes.p + img.triBvh.leafFloat4;
+  }
+  const bool meshUpdates = !img.meshes.empty() && !img.smallOk;   // rfx_update_mesh can update this scene on the device
+  std::vector<unsigned long long> red;
+  if (meshUpdates)
+  {
+    if ((rc = upload(ctx, ctx->dMeshIdx, img.meshIdx, st)) != RFX_OK) return rc;
+    if (!img.triSlot.empty())
+    {
+      const size_t nTris = img.triSlot.size();
+      if ((rc = upload(ctx, ctx->dTriSlot, img.triSlot, st)) != RFX_OK || (rc = upload(ctx, ctx->dLeafParent, img.leafParent, st)) != RFX_OK ||
+          (rc = upload(ctx, ctx->dPairParent, img.pairParent, st)) != RFX_OK || (rc = ensure(ctx, ctx->dArrive, std::max<size_t>(img.pairParent.size(), 1))) != RFX_OK ||
+          (rc = ensure(ctx, ctx->dInAlways, nTris)) != RFX_OK || (rc = ensure(ctx, ctx->dTriAlways, nTris)) != RFX_OK)
+        return rc;
+      CK(cudaMemsetAsync(ctx->dInAlways.p, 0, nTris, st));
+      red.assign(14, 0);
+      for (int k = 0; k < 6; k++) red[7 + k] = orderedCode(img.triUnion[k]);
+      red[13] = orderedCode(0.0);
+      if ((rc = upload(ctx, ctx->dMeshRed, red, st)) != RFX_OK) return rc;
+      if (img.far) h.triAlways = ctx->dTriAlways.p;
+    }
   }
   if (!img.triAlways.empty())
   {
@@ -470,6 +499,36 @@ int renderRange(rfx_ctx * ctx, uint64_t p0, uint64_t p1, uint32_t * argbOut, boo
   return RFX_OK;
 }
 
+void meshBox(HostMesh & m)
+{
+  float * b = m.box;
+  for (int k = 0; k < 3; k++) { b[k] = FLT_MAX; b[3 + k] = -FLT_MAX; }
+  for (size_t i = 0; i < m.xyz.size(); i++) { b[i % 3] = std::min(b[i % 3], m.xyz[i]); b[3 + i % 3] = std::max(b[3 + i % 3], m.xyz[i]); }
+}
+
+// Whether the structures of the last flatten still serve the scene after mesh m moved (rfx_update_mesh updates it on the device):
+// a blob scene whose hierarchies' margins were sized for a reach box that still holds m's vertices (every drop point on them), and
+// whose light grids were built for a drop-point box that still holds every object.
+bool deviceUpdateValid(const rfx_ctx * ctx, const HostMesh & m)
+{
+  const SceneImage & img = ctx->image;
+  if (img.smallOk || img.meshes.size() != ctx->scene.meshes.size()) return false;
+  if (img.bvhDepth > 0 || img.triBvhTris > 0)
+    for (int k = 0; k < 3; k++)
+      if (!(m.box[k] >= img.reach[k] && m.box[3 + k] <= img.reach[3 + k])) return false;
+  if (img.lightGridsBuilt)
+  {
+    double b[6];
+    memcpy(b, img.dropBase, sizeof(b));
+    for (const HostMesh & o : ctx->scene.meshes)
+      for (int k = 0; k < 3; k++) { b[k] = std::min(b[k], (double)o.box[k]); b[3 + k] = std::max(b[3 + k], (double)o.box[3 + k]); }
+    padDropBox(b);
+    for (int k = 0; k < 3; k++)
+      if (!(b[k] >= img.gridBox[k] && b[3 + k] <= img.gridBox[3 + k])) return false;
+  }
+  return true;
+}
+
 int checkStatus(rfx_ctx * ctx)
 {
   int status = 0;
@@ -591,7 +650,7 @@ int rfx_scene_reset(rfx_ctx * ctx, const float ambient_rgb[3], float ambient_pow
   CK(cudaSetDevice(ctx->device));
   CK(cudaDeviceSynchronize());
   for (HostTex & t : ctx->scene.tex) if (t.dev) cudaFree(t.dev);
-  ctx->scene.tex.clear(); ctx->scene.objs.clear(); ctx->scene.lights.clear();
+  ctx->scene.tex.clear(); ctx->scene.objs.clear(); ctx->scene.lights.clear(); ctx->scene.meshes.clear();
   ctx->scene.skyTex = -1;
   for (int i = 0; i < 3; i++) { ctx->scene.extraOrigins[i] = FLT_MAX; ctx->scene.extraOrigins[3 + i] = -FLT_MAX; }
   for (int i = 0; i < 3; i++)
@@ -641,12 +700,7 @@ int rfx_add_triangle(rfx_ctx * ctx, const float v[9], int mtype, const float rgb
   memset(&o, 0, sizeof(o));
   o.kind = 1;
   o.mat = makeMaterial(mtype, rgb, refl, transp, (int)ctx->scene.objs.size());
-  const H3 v0 = { v[0], v[1], v[2] }, v1 = { v[3], v[4], v[5] }, v2 = { v[6], v[7], v[8] };
-  const H3 n = hnormalize(hcross(hsub(v1, v0), hsub(v2, v0)));  // Triangle.cpp:13
-  const H3 nn = { -n.x, -n.y, -n.z };
-  invertColumns(hsub(v2, v0), hsub(v1, v0), nn, o.tri.ax);      // Triangle.cpp:19-20
-  o.tri.v0[0] = v0.x; o.tri.v0[1] = v0.y; o.tri.v0[2] = v0.z;
-  o.tri.n[0] = n.x; o.tri.n[1] = n.y; o.tri.n[2] = n.z;
+  setupTriangle(v, o.tri);                                      // Triangle.cpp:11-21
   memcpy(o.triVerts, v, sizeof(o.triVerts));
   ctx->scene.objs.push_back(o);
   ctx->sceneDirty = true;
@@ -669,7 +723,62 @@ int rfx_add_mesh(rfx_ctx * ctx, uint32_t n_vertices, const float * xyz, uint32_t
     const int rc = rfx_add_triangle(ctx, v, mtype, rgb, refl, transp);
     if (rc < 0) return rc;
   }
+  HostMesh m;
+  m.first = first;
+  m.idx.assign(idx, idx + 3 * (size_t)n_tris);
+  m.xyz.assign(xyz, xyz + 3 * (size_t)n_vertices);
+  meshBox(m);
+  ctx->scene.meshes.push_back(std::move(m));
   return first;
+}
+
+int rfx_update_mesh(rfx_ctx * ctx, int first, const float * xyz)
+{
+  if (!ctx || !xyz) return fail(ctx, RFX_ERR_ARG, "rfx_update_mesh: NULL argument");
+  HostScene & s = ctx->scene;
+  size_t mi = 0;
+  while (mi < s.meshes.size() && s.meshes[mi].first != first) mi++;
+  if (mi == s.meshes.size()) return fail(ctx, RFX_ERR_ARG, "rfx_update_mesh: first does not start a mesh of this scene");
+  HostMesh & m = s.meshes[mi];
+  memcpy(m.xyz.data(), xyz, m.xyz.size() * sizeof(float));
+  meshBox(m);
+  m.stale = true;   // the host records follow at the next flatten (refreshMeshes)
+  if (ctx->sceneDirty || !deviceUpdateValid(ctx, m)) { ctx->sceneDirty = true; return 0; }
+
+  const SceneImage & img = ctx->image;
+  const SceneImage::MeshImage & im = img.meshes[mi];
+  CK(cudaSetDevice(ctx->device));
+  // the stream the renders use: the update is ordered after the frames already queued there
+  cudaStream_t st = ctx->lastStream ? ctx->lastStream : ctx->stream;
+  int rc;
+  if ((rc = useStream(ctx, st)) != RFX_OK || (rc = ensure(ctx, ctx->dVerts, m.xyz.size())) != RFX_OK) return rc;
+  CK(cudaMemcpyAsync(ctx->dVerts.p, m.xyz.data(), m.xyz.size() * sizeof(float), cudaMemcpyHostToDevice, st));   // (staged before the call returns)
+  ctx->stats.h2d_bytes += m.xyz.size() * sizeof(float);
+  const SceneHeader & h = *reinterpret_cast<const SceneHeader *>(img.blob.data());
+  MeshUpdate u;
+  memset(&u, 0, sizeof(u));
+  u.tris = reinterpret_cast<Triangle *>(ctx->dBlob.p + h.offTris);
+  u.header = reinterpret_cast<SceneHeader *>(ctx->dBlob.p);
+  u.xyz = ctx->dVerts.p;
+  u.idx = ctx->dMeshIdx.p + im.idxOff;
+  u.triBase = im.triBase; u.nTris = (int)im.nTris;
+  if (!img.triSlot.empty())
+  {
+    u.triLeaf = ctx->dTriNodes.p; u.triPairs = ctx->dTriNodes.p + img.triBvh.leafFloat4;
+    u.triPrims = ctx->dTriPrims.p; u.triSlot = ctx->dTriSlot.p;
+    u.leafParent = ctx->dLeafParent.p; u.pairParent = ctx->dPairParent.p;
+    u.arrive = ctx->dArrive.p;
+    u.nLeaves = (int)img.leafParent.size();
+    u.red = ctx->dMeshRed.p;
+    u.far = img.far;
+    u.triAlways = ctx->dTriAlways.p;
+    u.inAlways = ctx->dInAlways.p;
+    CK(cudaMemcpyAsync(ctx->dMeshRed.p, ctx->dMeshRed.p + 7, 7 * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, st));
+    if (!img.pairParent.empty()) CK(cudaMemsetAsync(ctx->dArrive.p, 0, img.pairParent.size() * sizeof(uint32_t), st));
+  }
+  ctx->stats.kernel_launches += launchMeshUpdate(u, st);
+  CK(cudaGetLastError());
+  return 1;
 }
 
 int rfx_set_triangle_texture(rfx_ctx * ctx, int object, int texture, const float uv[6])

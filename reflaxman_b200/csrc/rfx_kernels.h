@@ -178,7 +178,30 @@ template <typename F> inline void withFlag(bool b, F && f)
   else f(std::false_type());
 }
 
-// ---- K3: resolve (imagePixel + argb) ---------------------------------------------------------------------------
+// ---- mesh updates (rfx_mesh.cu, rfx_update_mesh) ------------------------------------------------------------------
+// k_mesh_setup sets up one mesh's triangles from new vertices into the blob and the hierarchy's leaf slots; k_tri_refit then
+// recomputes every leaf's box and the pair nodes bottom-up.  The hierarchy keeps the topology of the last flatten.
+struct MeshUpdate
+{
+  Triangle * tris;              // the blob's sorted triangle array
+  SceneHeader * header;         // the blob's header (triReach, growT, nTriAlways of plane scenes)
+  const float * xyz;            // the mesh's new vertices (device)
+  const uint32_t * idx;         // its index list (device), 3 per triangle
+  int triBase, nTris;           // its triangles' positions in the sorted array
+  // the triangle hierarchy (triLeaf == NULL: none, only the blob is written)
+  float4 * triLeaf, * triPairs;
+  const int * triPrims, * triSlot;          // slot -> sorted position, sorted position -> slot (-1: none)
+  const int * leafParent, * pairParent;     // 2 * parent pair node + side, -1: root
+  uint32_t * arrive;                        // per pair node, zero before the refit
+  int nLeaves;
+  unsigned long long * red;                 // [7] orderedCode: union box lo xyz (min), hi xyz (max), largest kappa (max)
+  bool far;                                 // plane scene: slivers leave the hierarchy for triAlways
+  int * triAlways;                          // capacity: every triangle
+  unsigned char * inAlways;                 // per sorted position: already appended to triAlways since the flatten
+};
+int launchMeshUpdate(const MeshUpdate & u, cudaStream_t st);   // returns the number of kernels launched
+
+// ---- K3: resolve (imagePixel + argb)---------------------------------------------------------------------------
 int launchResolve(const float * image, uint64_t nPixels, int additiveCounter, float * rgbfOut, uint32_t * argbOut, cudaStream_t st);
 int launchClear(float * image, uint64_t nFloats, cudaStream_t st);
 

@@ -11,23 +11,6 @@
 namespace rfx
 {
 
-void invertColumns(H3 u, H3 v, H3 n, float out[9])
-{
-  const float _11 = u.x, _12 = v.x, _13 = n.x, _21 = u.y, _22 = v.y, _23 = n.y, _31 = u.z, _32 = v.z, _33 = n.z;
-  const float d = (_11 * (_22 * _33 - _32 * _23) + _21 * (_32 * _13 - _12 * _33)) + _31 * (_12 * _23 - _13 * _22);
-  if (fabsf(d) > VSN)
-  {
-    out[0] = (_22 * _33 - _23 * _32) / d; out[1] = (_13 * _32 - _12 * _33) / d; out[2] = (_12 * _23 - _13 * _22) / d;
-    out[3] = (_23 * _31 - _21 * _33) / d; out[4] = (_11 * _33 - _13 * _31) / d; out[5] = (_13 * _21 - _11 * _23) / d;
-    out[6] = (_21 * _32 - _22 * _31) / d; out[7] = (_12 * _31 - _11 * _32) / d; out[8] = (_11 * _22 - _12 * _21) / d;
-  }
-  else
-  {
-    const float id[9] = { 1, 0, 0, 0, 1, 0, 0, 0, 1 };
-    memcpy(out, id, sizeof(id));
-  }
-}
-
 Material makeMaterial(int mtype, const float rgb[3], float refl, float transp, int order)
 {
   Material m;
@@ -58,14 +41,6 @@ namespace
 {
 
 template <typename T> inline size_t align16(T v) { return ((size_t)v + 15) & ~(size_t)15; }
-
-// a triangle as 3 float4 for the intersection loops (SmallScene::triPk, the leaf slots of the triangle hierarchy)
-void packTriangle(const Triangle & t, float4 w[3])
-{
-  w[0] = make_float4(t.v0[0], t.v0[1], t.v0[2], t.ax[6]);
-  w[1] = make_float4(t.ax[7], t.ax[8], t.ax[0], t.ax[1]);
-  w[2] = make_float4(t.ax[2], t.ax[3], t.ax[4], t.ax[5]);
-}
 
 // ---- bounding-volume hierarchies over the spheres and over the triangles of big scenes (SURVEY f-3) ---------------------------
 // Median split on the widest centroid axis, leaves of <= 4 primitives, each primitive's box inflated by its margin.  A hierarchy
@@ -147,12 +122,27 @@ void writePairNode(const std::vector<BvhNode> & nodes, const std::vector<int> & 
 
 // [leaf slots | pair nodes] of a hierarchy built by buildBvhRec.  Every leaf is 4 slots of slotFloat4 float4s: writeSlot(position in
 // the sorted primitive array, slot) fills a used one, unused ones keep pad — which the device's leaf test never accepts — so a whole
-// leaf is tested without indirection.
+// leaf is tested without indirection.  parents (optional): per leaf and per pair node, 2 * (its parent's pair node) + side, -1 for the
+// root (the bottom-up refit of rfx_mesh.cu).
 template <typename WriteSlot>
-void packBvh(const std::vector<BvhNode> & nodes, const std::vector<BvhPrim> & prims, int slotFloat4, float pad, WriteSlot writeSlot, PackedBvh & out)
+void packBvh(const std::vector<BvhNode> & nodes, const std::vector<BvhPrim> & prims, int slotFloat4, float pad, WriteSlot writeSlot, PackedBvh & out,
+             std::vector<int> * leafParent = nullptr, std::vector<int> * pairParent = nullptr)
 {
   std::vector<int> ref;
   const size_t nLeaves = bvhRefs(nodes, ref), nInner = nodes.size() - nLeaves;
+  if (leafParent)
+  {
+    leafParent->assign(nLeaves, -1);
+    pairParent->assign(nInner, -1);
+    for (size_t i = 0; i < nodes.size(); i++)
+      if (nodes[i].b >= 0)
+        for (int side = 0; side < 2; side++)
+        {
+          const int c = side ? nodes[i].b : nodes[i].a;
+          if (nodes[c].b < 0) (*leafParent)[(~ref[c]) / 4] = 2 * ref[i] + side;
+          else (*pairParent)[ref[c]] = 2 * ref[i] + side;
+        }
+  }
   out.leafFloat4 = nLeaves * 4 * slotFloat4;
   out.nodes.assign(out.leafFloat4 + nInner * 4, make_float4(pad, pad, pad, pad));
   out.prims.assign(nLeaves * 4, -1);
@@ -204,63 +194,21 @@ void packBvh(const std::vector<BvhNode> & nodes, const std::vector<BvhPrim> & pr
 double buildTriBoxes(int n, const float * tris, const float reach[6], float * boxes, bool farOrigins = false, double triReach[6] = nullptr,
                      double * kappaMax = nullptr)
 {
-  const double u = 1.0 / 16777216.0;
-  std::vector<double> e((size_t)n * 8);   // per triangle: E's box (lo xyz, hi xyz), |A|, kappa (negative: no finite E)
+  std::vector<TriExtent> e((size_t)n);
   double ulo[3] = { reach[0], reach[1], reach[2] }, uhi[3] = { reach[3], reach[4], reach[5] };
   for (int i = 0; i < n; i++)
   {
     const float * t = tris + 12 * (size_t)i;
-    double M[9], A[9];
-    bool ok = true;
-    for (int k = 0; k < 9; k++) { M[k] = t[3 + k]; ok = ok && std::isfinite(M[k]); }
-    for (int k = 0; k < 3; k++) ok = ok && std::isfinite((double)t[k]);
-    double det = 0;
-    if (ok)
-    {
-      A[0] = M[4] * M[8] - M[5] * M[7]; A[1] = M[2] * M[7] - M[1] * M[8]; A[2] = M[1] * M[5] - M[2] * M[4];
-      A[3] = M[5] * M[6] - M[3] * M[8]; A[4] = M[0] * M[8] - M[2] * M[6]; A[5] = M[2] * M[3] - M[0] * M[5];
-      A[6] = M[3] * M[7] - M[4] * M[6]; A[7] = M[1] * M[6] - M[0] * M[7]; A[8] = M[0] * M[4] - M[1] * M[3];
-      det = M[0] * A[0] + M[1] * A[3] + M[2] * A[6];
-      ok = std::isfinite(det) && det != 0.0;
-    }
-    double * r = &e[8 * (size_t)i];
-    r[7] = -1.0;
-    if (!ok) continue;
-    double na = 0, kappa = 0;
-    for (int k = 0; k < 9; k++) { A[k] /= det; na += A[k] * A[k]; }
-    na = sqrt(na);
-    for (int k = 0; k < 3; k++)   // |column k of A| * |row k of M|
-      kappa += sqrt(A[k] * A[k] + A[3 + k] * A[3 + k] + A[6 + k] * A[6 + k]) * sqrt(M[3 * k] * M[3 * k] + M[3 * k + 1] * M[3 * k + 1] + M[3 * k + 2] * M[3 * k + 2]);
-    bool fin = std::isfinite(na) && std::isfinite(kappa);
-    for (int k = 0; k < 3; k++)
-    {
-      const double v0 = t[k], pa = v0 + A[3 * k], pb = v0 + A[3 * k + 1];   // v0, v0 + a, v0 + b (a, b: columns 0 and 1 of A)
-      r[k] = std::min(v0, std::min(pa, pb)); r[3 + k] = std::max(v0, std::max(pa, pb));
-      fin = fin && std::isfinite(r[k]) && std::isfinite(r[3 + k]);
-    }
-    if (!fin) continue;
-    r[6] = na; r[7] = kappa;
-    for (int k = 0; k < 3; k++) { ulo[k] = std::min(ulo[k], r[k]); uhi[k] = std::max(uhi[k], r[3 + k]); }
+    triExtent(t, t + 3, e[i]);
+    if (e[i].kappa < 0.0) continue;
+    for (int k = 0; k < 3; k++) { ulo[k] = std::min(ulo[k], e[i].lo[k]); uhi[k] = std::max(uhi[k], e[i].hi[k]); }
   }
-  const double dx = uhi[0] - ulo[0], dy = uhi[1] - ulo[1], dz = uhi[2] - ulo[2];
-  const double R = sqrt(dx * dx + dy * dy + dz * dz);
-  auto down = [](double v) { float f = (float)v; if ((double)f > v) f = nextafterf(f, -FLT_MAX); return f; };
-  auto up = [](double v) { float f = (float)v; if ((double)f < v) f = nextafterf(f, FLT_MAX); return f; };
+  const double R = boxDiagonal(ulo, uhi);
   double kmax = 0.0;
   for (int i = 0; i < n; i++)
   {
-    const double * r = &e[8 * (size_t)i];
-    float * b = boxes + 6 * (size_t)i;
-    if (!(r[7] >= 0.0) || !(16.0 * u * r[7] <= 0.5))
-    {
-      for (int k = 0; k < 3; k++)
-        if (farOrigins) { b[k] = -std::numeric_limits<float>::infinity(); b[3 + k] = std::numeric_limits<float>::infinity(); }
-        else { b[k] = down(ulo[k]); b[3 + k] = up(uhi[k]); }
-      continue;
-    }
-    kmax = std::max(kmax, r[7]);
-    const double m = 64.0 * u * (r[7] * R + r[6]) + 1e-6 * R;
-    for (int k = 0; k < 3; k++) { b[k] = down(r[k] - m); b[3 + k] = up(r[3 + k] + m); }
+    triBox(e[i], ulo, uhi, R, farOrigins, boxes + 6 * (size_t)i);
+    if (triBoxed(e[i])) kmax = std::max(kmax, e[i].kappa);
   }
   if (triReach)
     for (int k = 0; k < 3; k++) { triReach[k] = ulo[k]; triReach[3 + k] = uhi[k]; }
@@ -285,19 +233,8 @@ double buildTriBoxes(int n, const float * tris, const float reach[6], float * bo
 //   triangles have no such bound: in plane scenes they stay out of the hierarchy and every query tests them after the walk.
 // The device widens the slab interval of every box by G |1/d_k| per axis (G = grow * delta_1, rounded upwards; the bounds rounded
 // outwards), which is the fused slab test of the box grown by G on every side, with the same clamped reciprocals.
-float roundUp(double v) { float f = (float)v; if ((double)f < v) f = nextafterf(f, FLT_MAX); return f; }
+// (farGrowthTris, roundUp and roundOutwards: rfx_tri_setup.h, shared with the device refit)
 float farGrowthSpheres() { return roundUp(4.0 * 7.7e-4 + 1e-6); }
-float farGrowthTris(double kappaMax) { return roundUp(64.0 / 16777216.0 * kappaMax + 1e-6); }
-
-// a box (lo xyz, hi xyz) rounded outwards to float
-void roundOutwards(const double in[6], float out[6])
-{
-  for (int k = 0; k < 3; k++)
-  {
-    out[k] = (float)in[k]; if ((double)out[k] > in[k]) out[k] = nextafterf(out[k], -FLT_MAX);
-    out[3 + k] = (float)in[3 + k]; if ((double)out[3 + k] < in[3 + k]) out[3 + k] = nextafterf(out[3 + k], FLT_MAX);
-  }
-}
 
 // the box of a sphere in the hierarchy: centre -/+ (r + sphereMargin(r, R)); returns the margin
 float sphereBox(const float c[3], float r, double R, float lo[3], float hi[3])
@@ -449,9 +386,9 @@ void buildLightGrids(const std::vector<Light> & lights, const std::vector<const 
         bhi[k] = std::max(bhi[k], (double)t->triVerts[3 * v + k]);
       }
   {
-    const double ex = bhi[0] - blo[0], ey = bhi[1] - blo[1], ez = bhi[2] - blo[2];
-    const double pad = 1e-3 * sqrt(ex * ex + ey * ey + ez * ez) + 1e-5 * (fabs(blo[0]) + fabs(blo[1]) + fabs(blo[2]) + fabs(bhi[0]) + fabs(bhi[1]) + fabs(bhi[2]));
-    for (int k = 0; k < 3; k++) { blo[k] -= pad; bhi[k] += pad; }
+    double b[6] = { blo[0], blo[1], blo[2], bhi[0], bhi[1], bhi[2] };
+    padDropBox(b);
+    for (int k = 0; k < 3; k++) { blo[k] = b[k]; bhi[k] = b[3 + k]; img.gridBox[k] = b[k]; img.gridBox[3 + k] = b[3 + k]; }
   }
   img.grids.assign(lights.size(), LightGrid());
   img.gridCellOff.assign(lights.size(), 0);
@@ -471,6 +408,28 @@ void buildLightGrids(const std::vector<Light> & lights, const std::vector<const 
 }
 
 } // namespace
+
+void padDropBox(double b[6])
+{
+  const double ex = b[3] - b[0], ey = b[4] - b[1], ez = b[5] - b[2];
+  const double pad = 1e-3 * sqrt(ex * ex + ey * ey + ez * ez) + 1e-5 * (fabs(b[0]) + fabs(b[1]) + fabs(b[2]) + fabs(b[3]) + fabs(b[4]) + fabs(b[5]));
+  for (int k = 0; k < 3; k++) { b[k] -= pad; b[3 + k] += pad; }
+}
+
+void refreshMeshes(HostScene & s)
+{
+  for (HostMesh & m : s.meshes)
+  {
+    if (!m.stale) continue;
+    for (size_t k = 0; k < m.idx.size() / 3; k++)
+    {
+      HostObj & o = s.objs[m.first + k];
+      for (int j = 0; j < 3; j++) memcpy(o.triVerts + 3 * j, &m.xyz[3 * (size_t)m.idx[3 * k + j]], 12);
+      setupTriangle(o.triVerts, o.tri);
+    }
+    m.stale = false;
+  }
+}
 
 int buildSceneImage(const HostScene & s, SceneImage & img, std::string & err)
 {
@@ -514,6 +473,7 @@ int buildSceneImage(const HostScene & s, SceneImage & img, std::string & err)
   img.grids.clear(); img.gridCells.clear(); img.gridSpheres.clear(); img.gridIndex.clear();
   img.lightGridsBuilt = 0; img.bvhDepth = 0; img.bvhFloat4 = 0; img.triBvhTris = 0; img.bvhSpheres = 0;
   img.triAlways.clear(); img.far = false;
+  img.meshes.clear(); img.meshIdx.clear(); img.triSlot.clear(); img.leafParent.clear(); img.pairParent.clear();
   memset(img.reach, 0, sizeof(img.reach));
   img.spheres.resize(sph.size());
   for (size_t i = 0; i < sph.size(); i++) img.spheres[i] = make_float4(sph[i]->center[0], sph[i]->center[1], sph[i]->center[2], sph[i]->sqRadius);
@@ -619,13 +579,50 @@ int buildSceneImage(const HostScene & s, SceneImage & img, std::string & err)
     {
       // leaf slots of 3 float4 each (the layout of SmallScene::triPk), all zero in the unused ones, which the exact test's gate
       // |rz| > 2^-63 rejects
-      packBvh(nodes, prims, 3, 0.0f, [&](int i, float4 * w) { packTriangle(tri[i]->tri, w); }, img.triBvh);
+      const bool meshes = !s.meshes.empty();
+      packBvh(nodes, prims, 3, 0.0f, [&](int i, float4 * w) { packTriangle(tri[i]->tri, w); }, img.triBvh,
+              meshes ? &img.leafParent : nullptr, meshes ? &img.pairParent : nullptr);
+      if (meshes)
+      {
+        img.triSlot.assign(tri.size(), -1);
+        for (size_t j = 0; j < img.triBvh.prims.size(); j++)
+          if (img.triBvh.prims[j] >= 0) img.triSlot[img.triBvh.prims[j]] = (int)j;
+        memcpy(img.triUnion, triReach, sizeof(img.triUnion));
+      }
       h.triRoot = img.triBvh.root;
       img.triBvhTris = tri.size();
       img.triAlways = always;
       h.nTriAlways = (int)always.size();
       roundOutwards(triReach, h.triReach);
       h.growT = farGrowthTris(kappaMax);
+    }
+  }
+  if (!s.meshes.empty())
+  {
+    // where each mesh's triangles sit in the sorted triangle array (a mesh's triangles are consecutive objects)
+    std::vector<int> triOf(s.objs.size(), -1);
+    for (size_t i = 0; i < tri.size(); i++) triOf[tri[i] - s.objs.data()] = (int)i;
+    std::vector<char> inMesh(tri.size(), 0);
+    for (const HostMesh & m : s.meshes)
+    {
+      SceneImage::MeshImage mi = { triOf[m.first], (uint32_t)(m.idx.size() / 3), img.meshIdx.size() };
+      img.meshes.push_back(mi);
+      img.meshIdx.insert(img.meshIdx.end(), m.idx.begin(), m.idx.end());
+      memset(&inMesh[mi.triBase], 1, mi.nTris);
+    }
+    if (img.lightGridsBuilt)   // the drop-point box without the meshes (rfx_update_mesh adds their current boxes to it)
+    {
+      double * b = img.dropBase;
+      for (int k = 0; k < 3; k++) { b[k] = 1e300; b[3 + k] = -1e300; }
+      for (size_t i = 0; i < sph.size(); i++)
+        for (int k = 0; k < 3; k++)
+        {
+          b[k] = std::min(b[k], (double)sph[i]->center[k] - fabs((double)sph[i]->radius));
+          b[3 + k] = std::max(b[3 + k], (double)sph[i]->center[k] + fabs((double)sph[i]->radius));
+        }
+      for (size_t i = 0; i < tri.size(); i++)
+        if (!inMesh[i])
+          for (int v = 0; v < 9; v++) { b[v % 3] = std::min(b[v % 3], (double)tri[i]->triVerts[v]); b[3 + v % 3] = std::max(b[3 + v % 3], (double)tri[i]->triVerts[v]); }
     }
   }
   if (farOrigins && (img.bvhSpheres || img.triBvhTris))

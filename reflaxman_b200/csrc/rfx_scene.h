@@ -5,7 +5,7 @@
 // once per object/frame; it is compiled with -ffp-contract=off so every operation is the same IEEE binary32 operation the reference's
 // build performs (reference Triangle.cpp:11-21,110-120; Matrix33.cpp:10-15,49-79; Skybox.cpp:21-37; Material.cpp:8-14; Render.cpp:148-150).
 #pragma once
-#include "rfx_types.h"
+#include "rfx_tri_setup.h"
 
 #include <float.h>
 #include <math.h>
@@ -15,21 +15,8 @@
 namespace rfx
 {
 
-const float VSN = 1.08420217248550443e-19f;   // sqrtf(FLT_MIN), reference trace_math.h:17
-
 inline float clampf(float v, float lo, float hi) { return v < lo ? lo : v > hi ? hi : v; }
 
-struct H3 { float x, y, z; };
-inline H3 hsub(H3 a, H3 b) { return { a.x - b.x, a.y - b.y, a.z - b.z }; }
-inline H3 hcross(H3 a, H3 b) { return { a.y * b.z - a.z * b.y, a.z * b.x - a.x * b.z, a.x * b.y - a.y * b.x }; }   // Vector3.cpp:136-141
-inline H3 hnormalize(H3 a)   // trace_math.cpp:3-12
-{
-  const float l = sqrtf((a.x * a.x + a.y * a.y) + a.z * a.z);
-  if (l > VSN) return { a.x / l, a.y / l, a.z / l };
-  return a;
-}
-// Matrix33(u, v, n) columns + invert(), reference Matrix33.cpp:10-15, 49-79
-void invertColumns(H3 u, H3 v, H3 n, float out[9]);
 Material makeMaterial(int mtype, const float rgb[3], float refl, float transp, int order);   // Material.cpp:8-14
 
 struct HostTex { uint32_t w = 0, h = 0; std::vector<uint32_t> px; uint32_t * dev = nullptr; bool uploaded = false; };
@@ -43,11 +30,23 @@ struct HostObj
   Plane plane;
 };
 
+// A mesh of rfx_add_mesh: its triangles are objs[first, first + idx.size() / 3).  rfx_update_mesh replaces xyz and marks it stale:
+// the triangles' host records (triVerts, tri) are recomputed from xyz before the next flatten (refreshMeshes).
+struct HostMesh
+{
+  int first = 0;
+  std::vector<uint32_t> idx;                // 3 per triangle
+  std::vector<float> xyz;                   // the current vertices, 3 per vertex
+  float box[6];                             // their box (lo xyz, hi xyz)
+  bool stale = false;
+};
+
 struct HostScene
 {
   float ambient[3] = { 0, 0, 0 }, ambientPower = 0, env[3] = { 0, 0, 0 };
   std::vector<Light> lights;
   std::vector<HostObj> objs;
+  std::vector<HostMesh> meshes;
   std::vector<HostTex> tex;                 // uploaded before the image is built: TexRef and SmallScene carry their device pointers
   int skyTex = -1;
   int bvhMode = 0;                          // 0 auto (spheres > 32, triangles > 32), 1 always, 2 never — tests compare them
@@ -89,7 +88,24 @@ struct SceneImage
   uint64_t bvhSpheres = 0;                  // spheres under the sphere hierarchy (0: list walk)
   std::vector<int> triAlways;               // SceneHeader::triAlways (plane scenes: triangles tested after the walk)
   bool far = false;                         // the scene has a plane and a hierarchy: the kernels instantiated with FAR
+  // What rfx_update_mesh needs to set up mesh triangles and refit the triangle hierarchy on the device (rfx_mesh.cu) without a
+  // re-flatten.  meshes[i] is scene.meshes[i] as flattened: its triangles sit at [triBase, triBase + nTris) of the sorted triangle
+  // array, its index list at meshIdx[idxOff ...].
+  struct MeshImage { int triBase; uint32_t nTris; size_t idxOff; };
+  std::vector<MeshImage> meshes;
+  std::vector<uint32_t> meshIdx;
+  std::vector<int> triSlot;                 // per triangle of the sorted array: its leaf slot in triBvh, -1 (none); empty: no hierarchy
+  std::vector<int> leafParent, pairParent;  // triBvh: per leaf / pair node, 2 * (parent pair node) + side (0: a, 1: b); -1: the root
+  double triUnion[6] = { 0, 0, 0, 0, 0, 0 };  // the box R is the diagonal of in the triangle margins: reach joined with every E
+  double gridBox[6] = { 0, 0, 0, 0, 0, 0 };   // the padded drop-point box the light grids were built for (when lightGridsBuilt)
+  double dropBase[6] = { 0, 0, 0, 0, 0, 0 };  // the un-padded drop-point box of everything except the meshes' triangles
 };
+
+// the drop-point box (lo xyz, hi xyz) padded for the rounding of a drop point, as the light grids take it
+void padDropBox(double b[6]);
+
+// recompute the host records (triVerts, tri.v0/ax/n) of the stale meshes' triangles from their current vertices
+void refreshMeshes(HostScene & s);
 
 // flattens the host scene into img, rebuilt in place: its arrays keep their memory from the last image (a re-flatten of a big scene then
 // touches no fresh pages).  RFX_ERR_ARG (with err, img unchanged) when the blob outgrows its 32-bit offsets.

@@ -121,9 +121,8 @@ def synthetic_scene(n_side=32, floor=None, skybox=None, seed=0x9E3779B9, back_wa
     }
 
 
-def torus_mesh(n_u, n_v, major=2.2, minor=0.6, center=(0.0, 2.6, 0.0), tilt=1.0):
-    """An indexed torus of 2 * n_u * n_v triangles: n_u segments around the ring, n_v around the tube, the ring's axis tilted by
-    ``tilt`` radians about x.  Returns (xyz float32 [n_u * n_v, 3], idx uint32 [2 * n_u * n_v, 3]); the triangles face outwards."""
+def _torus_vertices(n_u, n_v, major, minor, center, tilt):
+    """vertices of :func:`torus_mesh`; ``minor``: the tube radius, a scalar or one per (u, v) vertex [n_u, n_v]"""
     u = 2.0 * np.pi * np.arange(n_u) / n_u
     v = 2.0 * np.pi * np.arange(n_v) / n_v
     uu, vv = np.meshgrid(u, v, indexing="ij")
@@ -131,7 +130,13 @@ def torus_mesh(n_u, n_v, major=2.2, minor=0.6, center=(0.0, 2.6, 0.0), tilt=1.0)
     x, y, z = ring * np.cos(uu), minor * np.sin(vv), ring * np.sin(uu)
     c, s = math.cos(tilt), math.sin(tilt)
     y, z = c * y - s * z, s * y + c * z
-    xyz = np.stack([x + center[0], y + center[1], z + center[2]], axis=-1).reshape(-1, 3).astype(np.float32)
+    return np.stack([x + center[0], y + center[1], z + center[2]], axis=-1).reshape(-1, 3).astype(np.float32)
+
+
+def torus_mesh(n_u, n_v, major=2.2, minor=0.6, center=(0.0, 2.6, 0.0), tilt=1.0):
+    """An indexed torus of 2 * n_u * n_v triangles: n_u segments around the ring, n_v around the tube, the ring's axis tilted by
+    ``tilt`` radians about x.  Returns (xyz float32 [n_u * n_v, 3], idx uint32 [2 * n_u * n_v, 3]); the triangles face outwards."""
+    xyz = _torus_vertices(n_u, n_v, major, minor, center, tilt)
     i, j = np.meshgrid(np.arange(n_u), np.arange(n_v), indexing="ij")
     a = i * n_v + j
     b = ((i + 1) % n_u) * n_v + j
@@ -139,6 +144,14 @@ def torus_mesh(n_u, n_v, major=2.2, minor=0.6, center=(0.0, 2.6, 0.0), tilt=1.0)
     d = i * n_v + (j + 1) % n_v
     idx = np.stack([np.stack([a, cc, b], axis=-1), np.stack([a, d, cc], axis=-1)], axis=2).reshape(-1, 3).astype(np.uint32)
     return xyz, idx
+
+
+def torus_wave(n_u, n_v, phase, amplitude=0.25, waves=3, major=2.2, minor=0.6, center=(0.0, 2.6, 0.0), tilt=1.0):
+    """The vertices of :func:`torus_mesh` (same count and order: its index list applies) with a wave travelling around the ring on
+    the tube radius: minor * (1 + amplitude * sin(waves * u - phase)) at ring angle u.  Stepping ``phase`` animates the torus."""
+    u = 2.0 * np.pi * np.arange(n_u) / n_u
+    r = minor * (1.0 + amplitude * np.sin(waves * u - phase))
+    return _torus_vertices(n_u, n_v, major, np.repeat(r[:, None], n_v, axis=1), center, tilt)
 
 
 def mesh_scene(n_u, n_v, spheres=0, floor=None, skybox=None):
