@@ -103,6 +103,15 @@ RFX_API int rfx_add_mesh(rfx_ctx * ctx, uint32_t n_vertices, const float * xyz, 
  * fits the constant bank, a re-flatten is pending anyway, or the new vertices leave the box the hierarchies or the light grids were
  * built for), or a negative error code: RFX_ERR_ARG for NULL xyz or a first that does not start a mesh of this scene. */
 RFX_API int rfx_update_mesh(rfx_ctx * ctx, int first, const float * xyz);
+/* Move / resize spheres added by rfx_add_sphere.  objects = n object indices, each a sphere of this scene; spheres = n x (cx, cy, cz,
+ * radius).  Afterwards every output is bit-identical to that of a scene built with the same calls but rfx_add_sphere(new centre, new
+ * radius) (material, insertion order and tie-breaks stay).  A repeated object: the later entry wins.  Returns 1 when the device scene
+ * was updated in place (queued on the stream the renders use, no synchronisation: the sphere records are written and the sphere
+ * hierarchy is refitted on the GPU, keeping its topology; the light grids are rebuilt on the host and uploaded), 0 when the scene will
+ * be re-flattened on the host at the next render instead (the scene fits the constant bank, a re-flatten is pending anyway, or a
+ * sphere leaves the box the hierarchies or the light grids were built for), or RFX_ERR_ARG (NULL pointer, n = 0, an index that is not
+ * a sphere of this scene); an error changes nothing. */
+RFX_API int rfx_update_spheres(rfx_ctx * ctx, uint32_t n, const int32_t * objects, const float * spheres);
 RFX_API int rfx_set_triangle_texture(rfx_ctx * ctx, int object, int texture, const float uv[6]); /* Triangle::setTexture, Triangle.cpp:110-120 (u1,v1,u2,v2,u3,v3) */
 RFX_API int rfx_add_plane(rfx_ctx * ctx, const float pos[3], const float norm[3], int mtype, const float rgb[3],
                           float reflectivity, float transparency);                              /* Plane::Plane, Plane.cpp:9-14 (no Scene::addPlane exists upstream) */

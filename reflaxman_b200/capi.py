@@ -46,6 +46,7 @@ SYMBOLS = [
     ("rfx_add_triangle", C.c_int, [C.c_void_p, _fp, C.c_int, _fp, C.c_float, C.c_float]),
     ("rfx_add_mesh", C.c_int, [C.c_void_p, C.c_uint32, _fp, C.c_uint32, _u32p, C.c_int, _fp, C.c_float, C.c_float]),
     ("rfx_update_mesh", C.c_int, [C.c_void_p, C.c_int, _fp]),
+    ("rfx_update_spheres", C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(C.c_int32), _fp]),
     ("rfx_set_triangle_texture", C.c_int, [C.c_void_p, C.c_int, C.c_int, _fp]),
     ("rfx_add_plane", C.c_int, [C.c_void_p, _fp, _fp, C.c_int, _fp, C.c_float, C.c_float]),
     ("rfx_add_texture_argb", C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, _u32p]),
@@ -309,6 +310,17 @@ class Context:
         if n is not None and v.shape[0] != n:
             raise ValueError("update_mesh: %d vertices given, the mesh has %d" % (v.shape[0], n))
         return self._ck(self.L.rfx_update_mesh(self.h, first, v.ctypes.data_as(_fp)), "rfx_update_mesh") == 1
+
+    def update_spheres(self, objects, spheres):
+        """rfx_update_spheres: objects [n] sphere object indices, spheres [n][4] rows of their new (cx, cy, cz, r); a repeated object
+        takes its last row.  True: the device scene was updated in place; False: the scene is re-flattened on the host at the next
+        render."""
+        ob = np.ascontiguousarray(objects, dtype=np.int32).reshape(-1)
+        sp = np.ascontiguousarray(spheres, dtype=np.float32)
+        if sp.ndim != 2 or sp.shape[1] != 4 or sp.shape[0] != ob.shape[0]:
+            raise ValueError("update_spheres: %d objects need [%d, 4] spheres, got %s" % (ob.shape[0], ob.shape[0], sp.shape))
+        return self._ck(self.L.rfx_update_spheres(self.h, ob.shape[0], ob.ctypes.data_as(C.POINTER(C.c_int32)), sp.ctypes.data_as(_fp)),
+                        "rfx_update_spheres") == 1
 
     def add_texture(self, argb):
         if argb is None:

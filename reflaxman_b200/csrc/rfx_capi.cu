@@ -100,6 +100,13 @@ struct rfx_ctx
   DevArray<uint32_t> dArrive;               // per pair node: refit arrival counters
   DevArray<unsigned long long> dMeshRed;    // [14]: an update's reduction record (MeshUpdate::red), then its value at the flatten
   DevArray<float> dVerts;                   // the vertices of the mesh being updated
+  // sphere updates on the device (rfx_update_spheres, SphereUpdate): uploaded by uploadScene for blob scenes with spheres
+  DevArray<float> dSphRadius;               // per sphere: its radius (SceneImage::sphRadius)
+  DevArray<int> dSphSlot, dSphLeafParent, dSphPairParent;
+  DevArray<uint32_t> dSphArrive;            // per pair node of the sphere hierarchy: refit arrival counters
+  DevArray<SphereMove> dSphMoves;           // the moved spheres of an update
+  std::vector<SphereMove> sphMoves;         // ... their host records (alive until the next update)
+  std::vector<char> sphMoved;               // per sphere: scratch of the update's duplicate resolution
 
   // ---- camera + render state (reference Render.h:9-27); the eye is scene.eye
   float view[9] = { 1, 0, 0, 0, 1, 0, 0, 0, 1 }, fov = 1.0f;
@@ -254,6 +261,15 @@ int uploadScene(rfx_ctx * ctx, cudaStream_t st)
       if ((rc = upload(ctx, ctx->dMeshRed, red, st)) != RFX_OK) return rc;
       if (img.far) h.triAlways = ctx->dTriAlways.p;
     }
+  }
+  if (!img.smallOk && !img.spheres.empty())   // rfx_update_spheres can update this scene on the device
+  {
+    if ((rc = upload(ctx, ctx->dSphRadius, img.sphRadius, st)) != RFX_OK) return rc;
+    if (!img.sphSlot.empty() &&
+        ((rc = upload(ctx, ctx->dSphSlot, img.sphSlot, st)) != RFX_OK || (rc = upload(ctx, ctx->dSphLeafParent, img.sphLeafParent, st)) != RFX_OK ||
+         (rc = upload(ctx, ctx->dSphPairParent, img.sphPairParent, st)) != RFX_OK ||
+         (rc = ensure(ctx, ctx->dSphArrive, std::max<size_t>(img.sphPairParent.size(), 1))) != RFX_OK))
+      return rc;
   }
   if (!img.triAlways.empty())
   {
@@ -506,6 +522,23 @@ void meshBox(HostMesh & m)
   for (size_t i = 0; i < m.xyz.size(); i++) { b[i % 3] = std::min(b[i % 3], m.xyz[i]); b[3 + i % 3] = std::max(b[3 + i % 3], m.xyz[i]); }
 }
 
+// Whether the light grids (if any) were built for a drop-point box that still holds every object: the triangles outside meshes,
+// the spheres (their current box: sph, or img.dropSpheres) and the meshes' current boxes.
+bool gridBoxHolds(const rfx_ctx * ctx, const double * sph = nullptr)
+{
+  const SceneImage & img = ctx->image;
+  if (!img.lightGridsBuilt) return true;
+  if (!sph) sph = img.dropSpheres;
+  double b[6];
+  for (int k = 0; k < 3; k++) { b[k] = std::min(img.dropTris[k], sph[k]); b[3 + k] = std::max(img.dropTris[3 + k], sph[3 + k]); }
+  for (const HostMesh & o : ctx->scene.meshes)
+    for (int k = 0; k < 3; k++) { b[k] = std::min(b[k], (double)o.box[k]); b[3 + k] = std::max(b[3 + k], (double)o.box[3 + k]); }
+  padDropBox(b);
+  for (int k = 0; k < 3; k++)
+    if (!(b[k] >= img.gridBox[k] && b[3 + k] <= img.gridBox[3 + k])) return false;
+  return true;
+}
+
 // Whether the structures of the last flatten still serve the scene after mesh m moved (rfx_update_mesh updates it on the device):
 // a blob scene whose hierarchies' margins were sized for a reach box that still holds m's vertices (every drop point on them), and
 // whose light grids were built for a drop-point box that still holds every object.
@@ -516,17 +549,7 @@ bool deviceUpdateValid(const rfx_ctx * ctx, const HostMesh & m)
   if (img.bvhDepth > 0 || img.triBvhTris > 0)
     for (int k = 0; k < 3; k++)
       if (!(m.box[k] >= img.reach[k] && m.box[3 + k] <= img.reach[3 + k])) return false;
-  if (img.lightGridsBuilt)
-  {
-    double b[6];
-    memcpy(b, img.dropBase, sizeof(b));
-    for (const HostMesh & o : ctx->scene.meshes)
-      for (int k = 0; k < 3; k++) { b[k] = std::min(b[k], (double)o.box[k]); b[3 + k] = std::max(b[3 + k], (double)o.box[3 + k]); }
-    padDropBox(b);
-    for (int k = 0; k < 3; k++)
-      if (!(b[k] >= img.gridBox[k] && b[3 + k] <= img.gridBox[3 + k])) return false;
-  }
-  return true;
+  return gridBoxHolds(ctx);
 }
 
 int checkStatus(rfx_ctx * ctx)
@@ -778,6 +801,112 @@ int rfx_update_mesh(rfx_ctx * ctx, int first, const float * xyz)
   }
   ctx->stats.kernel_launches += launchMeshUpdate(u, st);
   CK(cudaGetLastError());
+  return 1;
+}
+
+int rfx_update_spheres(rfx_ctx * ctx, uint32_t n, const int32_t * objects, const float * spheres)
+{
+  if (!ctx || !objects || !spheres || n == 0) return fail(ctx, RFX_ERR_ARG, "rfx_update_spheres: NULL argument or no sphere");
+  HostScene & s = ctx->scene;
+  for (uint32_t i = 0; i < n; i++)
+    if (objects[i] < 0 || objects[i] >= (int)s.objs.size() || s.objs[objects[i]].kind != 0)
+      return fail(ctx, RFX_ERR_ARG, "rfx_update_spheres: object " + std::to_string(objects[i]) + " is not a sphere of this scene");
+  // the host records, as rfx_add_sphere makes them (a later entry for the same object overwrites an earlier one)
+  for (uint32_t i = 0; i < n; i++)
+  {
+    HostObj & o = s.objs[objects[i]];
+    float radius = spheres[4 * i + 3];
+    if (radius <= VSN) radius = VSN;                            // Scene.cpp:33-34
+    memcpy(o.center, spheres + 4 * i, sizeof(o.center));
+    o.sqRadius = radius * radius;                               // Sphere.cpp:19
+    o.radius = radius;
+  }
+  if (ctx->sceneDirty || ctx->image.smallOk) { ctx->sceneDirty = true; return 0; }
+  SceneImage & img = ctx->image;
+  // the hierarchies' margins were sized for a reach box that must still hold every moved sphere (every drop point on it, its centre)
+  if (img.bvhDepth > 0 || img.triBvhTris > 0)
+    for (uint32_t i = 0; i < n; i++)
+    {
+      const HostObj & o = s.objs[objects[i]];
+      for (int k = 0; k < 3; k++)
+        if (!((double)o.center[k] - fabs((double)o.radius) >= img.reach[k] && (double)o.center[k] + fabs((double)o.radius) <= img.reach[3 + k]))
+        {
+          ctx->sceneDirty = true;
+          return 0;
+        }
+    }
+  double sphBox[6];
+  if (img.lightGridsBuilt)
+  {
+    sphereDropBox(s, img, sphBox);
+    if (!gridBoxHolds(ctx, sphBox)) { ctx->sceneDirty = true; return 0; }
+  }
+
+  // the moved spheres, once each, with their final records
+  ctx->sphMoved.assign(img.spheres.size(), 0);
+  ctx->sphMoves.clear();
+  for (uint32_t i = n; i-- > 0;)
+  {
+    const int pos = (int)(std::lower_bound(img.sphObj.begin(), img.sphObj.end(), objects[i]) - img.sphObj.begin());
+    if (ctx->sphMoved[pos]) continue;
+    ctx->sphMoved[pos] = 1;
+    const HostObj & o = s.objs[objects[i]];
+    SphereMove m;
+    memset(&m, 0, sizeof(m));
+    m.rec = make_float4(o.center[0], o.center[1], o.center[2], o.sqRadius);
+    m.pos = pos; m.radius = o.radius;
+    ctx->sphMoves.push_back(m);
+    img.spheres[pos] = m.rec;                                  // the eye grid's records
+    img.sphRadius[pos] = o.radius;
+  }
+  CK(cudaSetDevice(ctx->device));
+  // the stream the renders use: the update is ordered after the frames already queued there
+  cudaStream_t st = ctx->lastStream ? ctx->lastStream : ctx->stream;
+  int rc;
+  if ((rc = useStream(ctx, st)) != RFX_OK || (rc = upload(ctx, ctx->dSphMoves, ctx->sphMoves, st)) != RFX_OK) return rc;
+  const SceneHeader & h = *reinterpret_cast<const SceneHeader *>(img.blob.data());
+  SphereUpdate u;
+  memset(&u, 0, sizeof(u));
+  u.moves = ctx->dSphMoves.p; u.nMoves = (int)ctx->sphMoves.size();
+  u.spheres = reinterpret_cast<float4 *>(ctx->dBlob.p + h.offSpheres);
+  u.radius = ctx->dSphRadius.p;
+  if (!img.sphSlot.empty())
+  {
+    u.leafSph = ctx->dBvhNodes.p; u.pairs = ctx->dBvhNodes.p + img.sphBvh.leafFloat4;
+    u.prims = ctx->dBvhPrims.p; u.slot = ctx->dSphSlot.p;
+    u.leafParent = ctx->dSphLeafParent.p; u.pairParent = ctx->dSphPairParent.p;
+    u.arrive = ctx->dSphArrive.p;
+    u.nLeaves = (int)img.sphLeafParent.size();
+    u.R = img.sphR;
+    if (!img.sphPairParent.empty()) CK(cudaMemsetAsync(ctx->dSphArrive.p, 0, img.sphPairParent.size() * sizeof(uint32_t), st));
+  }
+  ctx->stats.kernel_launches += launchSphereUpdate(u, st);
+  CK(cudaGetLastError());
+
+  // The light grids are rebuilt for the new spheres over the box they were built for (which still holds every drop point): cells and
+  // items first, then the headers, whose pointers move when an array grows.  The copies follow the frames queued on the stream.
+  if (img.lightGridsBuilt)
+  {
+    memcpy(img.dropSpheres, sphBox, sizeof(sphBox));
+    rebuildLightGrids(s, img);
+    if (!img.grids.empty())
+    {
+      if ((rc = upload(ctx, ctx->dGridCells, img.gridCells, st)) != RFX_OK || (rc = upload(ctx, ctx->dGridSpheres, img.gridSpheres, st)) != RFX_OK ||
+          (rc = upload(ctx, ctx->dGridIndex, img.gridIndex, st)) != RFX_OK) return rc;
+      for (size_t li = 0; li < img.grids.size(); li++)
+        if (img.grids[li].nx)
+        {
+          img.grids[li].cellStart = ctx->dGridCells.p + img.gridCellOff[li];
+          img.grids[li].itemSphere = ctx->dGridSpheres.p + img.gridItemOff[li];
+          img.grids[li].itemIndex = ctx->dGridIndex.p + img.gridItemOff[li];
+        }
+    }
+    else   // (not seen: whether a light gets a grid depends on the light and the box alone) no grid: every light walks the hierarchy
+      img.grids.assign(s.lights.size(), LightGrid());
+    if ((rc = upload(ctx, ctx->dLightGrids, img.grids, st)) != RFX_OK) return rc;
+  }
+  // the eye grid is binned again from img.spheres at the next render
+  ctx->eyeValid = false;
   return 1;
 }
 

@@ -201,6 +201,32 @@ struct MeshUpdate
 };
 int launchMeshUpdate(const MeshUpdate & u, cudaStream_t st);   // returns the number of kernels launched
 
+// ---- sphere updates (rfx_mesh.cu, rfx_update_spheres) -----------------------------------------------------------------------
+// k_sphere_scatter writes the moved spheres' records into the blob's sphere array and the hierarchy's leaf slots; k_sphere_refit then
+// recomputes every leaf's box and the pair nodes bottom-up, as k_tri_refit does.  The hierarchy keeps the topology of the last flatten.
+struct SphereMove
+{
+  float4 rec;                   // (cx, cy, cz, r^2), as rfx_add_sphere stores it
+  int pos;                      // the sphere's position in the sorted sphere array
+  float radius;
+  int pad[2];
+};
+struct SphereUpdate
+{
+  const SphereMove * moves;     // device, one per moved sphere (no duplicates)
+  int nMoves;
+  float4 * spheres;             // the blob's sorted sphere array
+  float * radius;               // per sphere: its radius
+  // the sphere hierarchy (leafSph == NULL: none, only the blob is written)
+  float4 * leafSph, * pairs;
+  const int * prims, * slot;                // slot -> sphere, sphere -> slot
+  const int * leafParent, * pairParent;     // 2 * parent pair node + side, -1: root
+  uint32_t * arrive;                        // per pair node, zero before the refit
+  int nLeaves;
+  double R;                                 // the margins' R of the last flatten
+};
+int launchSphereUpdate(const SphereUpdate & u, cudaStream_t st);   // returns the number of kernels launched
+
 // ---- K3: resolve (imagePixel + argb)---------------------------------------------------------------------------
 int launchResolve(const float * image, uint64_t nPixels, int additiveCounter, float * rgbfOut, uint32_t * argbOut, cudaStream_t st);
 int launchClear(float * image, uint64_t nFloats, cudaStream_t st);

@@ -1,5 +1,6 @@
 // rfx_mesh.cu — rfx_update_mesh on the device: set up a mesh's triangles from new vertices (k_mesh_setup) and refit the triangle
-// hierarchy over the new boxes (k_tri_refit), without a host re-flatten.
+// hierarchy over the new boxes (k_tri_refit), without a host re-flatten.  rfx_update_spheres likewise: write the moved spheres' records
+// (k_sphere_scatter) and refit the sphere hierarchy (k_sphere_refit).
 //
 // Both kernels run the host's own per-triangle code (rfx_tri_setup.h: the reference's constructor, the box arithmetic of
 // buildTriBoxes), compiled with --fmad=false, so every triangle record and every box is the one a host flatten of the same triangles
@@ -8,7 +9,7 @@
 // effective triangles: it only grows until the next flatten, which keeps every margin sufficient.  A union box is an exact min / max,
 // so a refit with unchanged vertices reproduces the host's packed hierarchy bit for bit.
 #include "rfx_kernels.h"
-#include "rfx_tri_setup.h"
+#include "rfx_sphere_box.h"
 
 namespace rfx
 {
@@ -18,6 +19,32 @@ namespace
 
 constexpr int SETUP_THREADS = 256;
 constexpr int REFIT_THREADS = 128;
+
+// The climb of a bottom-up refit, from a leaf whose box is (lo, hi) and whose parent ref is p (2 * pair node + side, -1: root): the
+// thread writes its box into its side of the parent pair node (xyz lanes only: the w lanes hold the child refs); the second thread to
+// arrive at a pair node unions its two children's boxes and carries on.  Returns true in the one thread that completed the root.
+__device__ __forceinline__ bool refitClimb(float lo[3], float hi[3], int p, float4 * pairs, const int * pairParent, uint32_t * arrive)
+{
+  while (p >= 0)
+  {
+    const int node = p >> 1, side = p & 1;
+    float * mine = reinterpret_cast<float *>(pairs + 4 * (size_t)node + 2 * side);   // {lo.xyz, ref} {hi.xyz, ref}
+    mine[0] = lo[0]; mine[1] = lo[1]; mine[2] = lo[2];
+    mine[4] = hi[0]; mine[5] = hi[1]; mine[6] = hi[2];
+    __threadfence();
+    if (atomicAdd(arrive + node, 1u) == 0) return false;   // the sibling's thread finishes this node
+    __threadfence();
+    const volatile float * other = reinterpret_cast<const volatile float *>(pairs + 4 * (size_t)node + 2 * (side ^ 1));
+    for (int k = 0; k < 3; k++)
+    {
+      const float ol = other[k], oh = other[4 + k];
+      lo[k] = ol < lo[k] ? ol : lo[k];
+      hi[k] = hi[k] < oh ? oh : hi[k];
+    }
+    p = pairParent[node];
+  }
+  return true;
+}
 
 // One thread per mesh triangle: the triangle record in the blob (v0, ax, n; the texture fields stay), its leaf slot (packTriangle
 // layout), and the block's union of the new effective triangles, folded into u.red with one atomic per component.
@@ -118,25 +145,7 @@ __global__ void __launch_bounds__(REFIT_THREADS) k_tri_refit(const MeshUpdate u)
     if (triBoxed(e)) kmax = dmax(kmax, e.kappa);
   }
   if (u.far) atomicMax(u.red + 6, orderedCode(kmax));
-  int p = u.leafParent[leaf];
-  while (p >= 0)
-  {
-    const int node = p >> 1, side = p & 1;
-    float * mine = reinterpret_cast<float *>(u.triPairs + 4 * (size_t)node + 2 * side);   // {lo.xyz, ref} {hi.xyz, ref}
-    mine[0] = lo[0]; mine[1] = lo[1]; mine[2] = lo[2];
-    mine[4] = hi[0]; mine[5] = hi[1]; mine[6] = hi[2];
-    __threadfence();
-    if (atomicAdd(u.arrive + node, 1u) == 0) return;   // the sibling's thread finishes this node
-    __threadfence();
-    const volatile float * other = reinterpret_cast<const volatile float *>(u.triPairs + 4 * (size_t)node + 2 * (side ^ 1));
-    for (int k = 0; k < 3; k++)
-    {
-      const float ol = other[k], oh = other[4 + k];
-      lo[k] = ol < lo[k] ? ol : lo[k];
-      hi[k] = hi[k] < oh ? oh : hi[k];
-    }
-    p = u.pairParent[node];
-  }
+  if (!refitClimb(lo, hi, u.leafParent[leaf], u.triPairs, u.pairParent, u.arrive)) return;
   // the root is complete: every leaf's kappa is in red[6]
   if (u.far)
   {
@@ -147,7 +156,48 @@ __global__ void __launch_bounds__(REFIT_THREADS) k_tri_refit(const MeshUpdate u)
   }
 }
 
+// One thread per moved sphere: its record into the blob's sphere array (the list walk), its radius, and its leaf slot.
+__global__ void __launch_bounds__(SETUP_THREADS) k_sphere_scatter(const SphereUpdate u)
+{
+  const int k = blockIdx.x * SETUP_THREADS + threadIdx.x;
+  if (k >= u.nMoves) return;
+  const SphereMove m = u.moves[k];
+  u.spheres[m.pos] = m.rec;
+  u.radius[m.pos] = m.radius;
+  if (u.leafSph) u.leafSph[u.slot[m.pos]] = m.rec;
+}
+
+// One thread per leaf: the union of its spheres' boxes (sphereBox at the flatten's R, in slot order as the host build takes them),
+// then the climb to the root.  The leaf slots keep the records (unused slots: NaN); only the pair nodes hold boxes.
+__global__ void __launch_bounds__(REFIT_THREADS) k_sphere_refit(const SphereUpdate u)
+{
+  const int leaf = blockIdx.x * REFIT_THREADS + threadIdx.x;
+  if (leaf >= u.nLeaves) return;
+  float lo[3] = { FLT_MAX, FLT_MAX, FLT_MAX }, hi[3] = { -FLT_MAX, -FLT_MAX, -FLT_MAX };
+  for (int s = 0; s < 4; s++)
+  {
+    const int j = 4 * leaf + s;
+    const int pos = u.prims[j];
+    if (pos < 0) continue;
+    const float4 q = u.leafSph[j];
+    const float c[3] = { q.x, q.y, q.z };
+    float blo[3], bhi[3];
+    sphereBox(c, u.radius[pos], u.R, blo, bhi);
+    for (int k = 0; k < 3; k++) { lo[k] = blo[k] < lo[k] ? blo[k] : lo[k]; hi[k] = hi[k] < bhi[k] ? bhi[k] : hi[k]; }
+  }
+  refitClimb(lo, hi, u.leafParent[leaf], u.pairs, u.pairParent, u.arrive);
+}
+
 } // namespace
+
+int launchSphereUpdate(const SphereUpdate & u, cudaStream_t st)
+{
+  if (u.nMoves <= 0) return 0;
+  k_sphere_scatter<<<(u.nMoves + SETUP_THREADS - 1) / SETUP_THREADS, SETUP_THREADS, 0, st>>>(u);
+  if (!u.leafSph) return 1;
+  k_sphere_refit<<<(u.nLeaves + REFIT_THREADS - 1) / REFIT_THREADS, REFIT_THREADS, 0, st>>>(u);
+  return 2;
+}
 
 int launchMeshUpdate(const MeshUpdate & u, cudaStream_t st)
 {

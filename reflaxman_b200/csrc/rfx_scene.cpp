@@ -53,17 +53,7 @@ struct BvhPrim
   float lo[3], hi[3];       // the box: spheres c -/+ r -/+ m, triangles buildTriBoxes
 };
 
-// Box margin of a sphere of radius r when every ray origin and every centre lies in a box of diagonal R.  The hierarchy must never
-// cull a sphere the reference's exact test (Sphere.cpp:49-57) would report, and that test is noisy: with v = origin - centre,
-// disc = b*b - 4a*c carries an absolute rounding error of at most ~40 * 2^-24 * a|v|^2 (three-term dot products, the square, the
-// product), while a ray that misses the sphere by m has disc = 4a(r^2 - m^2).  A "noise hit" therefore needs m^2 - r^2 < 6e-7 |v|^2,
-// i.e. m - r < min(3e-7 |v|^2 / r, 7.7e-4 |v|), and |v| <= R.  The margin is twice that bound, plus 1e-6 R for the device's slab test
-// (fused arithmetic with clamped reciprocals: a box plane moves by at most 2^-22 |origin| along its axis).
-float sphereMargin(float r, double R)
-{
-  const double noise = std::min(3e-7 * R * R / std::max((double)r, 1e-30), 7.7e-4 * R);
-  return (float)(2.0 * noise + 1e-6 * R);
-}
+// (sphereMargin and sphereBox, the boxes of the spheres: rfx_sphere_box.h, shared with the device refit)
 
 int buildBvhRec(std::vector<BvhNode> & nodes, std::vector<BvhPrim> & prims, int begin, int end, int depth, int & maxDepth)
 {
@@ -236,14 +226,6 @@ double buildTriBoxes(int n, const float * tris, const float reach[6], float * bo
 // (farGrowthTris, roundUp and roundOutwards: rfx_tri_setup.h, shared with the device refit)
 float farGrowthSpheres() { return roundUp(4.0 * 7.7e-4 + 1e-6); }
 
-// the box of a sphere in the hierarchy: centre -/+ (r + sphereMargin(r, R)); returns the margin
-float sphereBox(const float c[3], float r, double R, float lo[3], float hi[3])
-{
-  const float m = sphereMargin(r, R);
-  for (int k = 0; k < 3; k++) { lo[k] = c[k] - r - m; hi[k] = c[k] + r + m; }
-  return m;
-}
-
 // ---- shadow-ray candidate grids (LightGrid) ---------------------------------------------------------------------------------------
 // A shadow ray (Scene.cpp:129) runs from a drop point P — a point of some object, so inside the objects' bounding box B — to
 // L + radius * randDir, |randDir| <= 1.  For a light far from the scene all those rays are nearly parallel to l = (L - centre(B)) / |..|:
@@ -365,9 +347,32 @@ bool buildLightGrid(const Light & L, const std::vector<const HostObj *> & sph, c
   return true;
 }
 
-// The grids of every far light, concatenated into img.  B: the box of every drop point — all objects (with planes present no grid is
-// built: a drop point on a plane can lie anywhere), padded for the rounding of a drop point.  prims: the sphere
-// hierarchy's, in the order its build left them.
+// The grids of every far light over the drop-point box (blo, bhi), concatenated into img.  prims: the sphere hierarchy's, in the order
+// its build left them (its slot order).
+void fillLightGrids(const std::vector<Light> & lights, const std::vector<const HostObj *> & sph, const std::vector<BvhPrim> & prims,
+                    const double blo[3], const double bhi[3], SceneImage & img)
+{
+  img.grids.assign(lights.size(), LightGrid());
+  img.gridCellOff.assign(lights.size(), 0);
+  img.gridItemOff.assign(lights.size(), 0);
+  img.gridCells.clear(); img.gridSpheres.clear(); img.gridIndex.clear();
+  img.lightGridsBuilt = 0;
+  for (size_t li = 0; li < lights.size(); li++)
+  {
+    LightGridHost lg;
+    if (!buildLightGrid(lights[li], sph, prims, blo, bhi, lg)) continue;
+    img.grids[li] = lg.g;
+    img.gridCellOff[li] = img.gridCells.size(); img.gridItemOff[li] = img.gridSpheres.size();
+    img.gridCells.insert(img.gridCells.end(), lg.cellStart.begin(), lg.cellStart.end());
+    img.gridSpheres.insert(img.gridSpheres.end(), lg.spheres.begin(), lg.spheres.end());
+    img.gridIndex.insert(img.gridIndex.end(), lg.index.begin(), lg.index.end());
+    img.lightGridsBuilt++;
+  }
+  if (!img.lightGridsBuilt) img.grids.clear();
+}
+
+// The grids of every far light.  B: the box of every drop point — all objects (with planes present no grid is built: a drop point on
+// a plane can lie anywhere), padded for the rounding of a drop point.
 void buildLightGrids(const std::vector<Light> & lights, const std::vector<const HostObj *> & sph, const std::vector<const HostObj *> & tri,
                      const std::vector<BvhPrim> & prims, SceneImage & img)
 {
@@ -390,21 +395,7 @@ void buildLightGrids(const std::vector<Light> & lights, const std::vector<const 
     padDropBox(b);
     for (int k = 0; k < 3; k++) { blo[k] = b[k]; bhi[k] = b[3 + k]; img.gridBox[k] = b[k]; img.gridBox[3 + k] = b[3 + k]; }
   }
-  img.grids.assign(lights.size(), LightGrid());
-  img.gridCellOff.assign(lights.size(), 0);
-  img.gridItemOff.assign(lights.size(), 0);
-  for (size_t li = 0; li < lights.size(); li++)
-  {
-    LightGridHost lg;
-    if (!buildLightGrid(lights[li], sph, prims, blo, bhi, lg)) continue;
-    img.grids[li] = lg.g;
-    img.gridCellOff[li] = img.gridCells.size(); img.gridItemOff[li] = img.gridSpheres.size();
-    img.gridCells.insert(img.gridCells.end(), lg.cellStart.begin(), lg.cellStart.end());
-    img.gridSpheres.insert(img.gridSpheres.end(), lg.spheres.begin(), lg.spheres.end());
-    img.gridIndex.insert(img.gridIndex.end(), lg.index.begin(), lg.index.end());
-    img.lightGridsBuilt++;
-  }
-  if (!img.lightGridsBuilt) img.grids.clear();
+  fillLightGrids(lights, sph, prims, blo, bhi, img);
 }
 
 } // namespace
@@ -414,6 +405,39 @@ void padDropBox(double b[6])
   const double ex = b[3] - b[0], ey = b[4] - b[1], ez = b[5] - b[2];
   const double pad = 1e-3 * sqrt(ex * ex + ey * ey + ez * ez) + 1e-5 * (fabs(b[0]) + fabs(b[1]) + fabs(b[2]) + fabs(b[3]) + fabs(b[4]) + fabs(b[5]));
   for (int k = 0; k < 3; k++) { b[k] -= pad; b[3 + k] += pad; }
+}
+
+void sphereDropBox(const HostScene & s, const SceneImage & img, double b[6])
+{
+  for (int k = 0; k < 3; k++) { b[k] = 1e300; b[3 + k] = -1e300; }
+  for (int i : img.sphObj)
+  {
+    const HostObj & o = s.objs[i];
+    for (int k = 0; k < 3; k++)
+    {
+      b[k] = std::min(b[k], (double)o.center[k] - fabs((double)o.radius));
+      b[3 + k] = std::max(b[3 + k], (double)o.center[k] + fabs((double)o.radius));
+    }
+  }
+}
+
+void rebuildLightGrids(const HostScene & s, SceneImage & img)
+{
+  std::vector<const HostObj *> sph(img.sphObj.size());
+  for (size_t i = 0; i < sph.size(); i++) sph[i] = &s.objs[img.sphObj[i]];
+  std::vector<BvhPrim> prims;
+  prims.reserve(sph.size());
+  for (int p : img.sphBvh.prims)
+    if (p >= 0)
+    {
+      BvhPrim q;
+      memset(&q, 0, sizeof(q));
+      q.index = p;
+      q.m = sphereMargin(sph[p]->radius, img.sphR);
+      prims.push_back(q);
+    }
+  const double blo[3] = { img.gridBox[0], img.gridBox[1], img.gridBox[2] }, bhi[3] = { img.gridBox[3], img.gridBox[4], img.gridBox[5] };
+  fillLightGrids(s.lights, sph, prims, blo, bhi, img);
 }
 
 void refreshMeshes(HostScene & s)
@@ -474,9 +498,18 @@ int buildSceneImage(const HostScene & s, SceneImage & img, std::string & err)
   img.lightGridsBuilt = 0; img.bvhDepth = 0; img.bvhFloat4 = 0; img.triBvhTris = 0; img.bvhSpheres = 0;
   img.triAlways.clear(); img.far = false;
   img.meshes.clear(); img.meshIdx.clear(); img.triSlot.clear(); img.leafParent.clear(); img.pairParent.clear();
+  img.sphSlot.clear(); img.sphLeafParent.clear(); img.sphPairParent.clear(); img.sphR = 0.0;
   memset(img.reach, 0, sizeof(img.reach));
-  img.spheres.resize(sph.size());
-  for (size_t i = 0; i < sph.size(); i++) img.spheres[i] = make_float4(sph[i]->center[0], sph[i]->center[1], sph[i]->center[2], sph[i]->sqRadius);
+  img.spheres.resize(sph.size()); img.sphObj.resize(sph.size()); img.sphRadius.resize(sph.size());
+  for (size_t i = 0; i < sph.size(); i++)
+  {
+    img.spheres[i] = make_float4(sph[i]->center[0], sph[i]->center[1], sph[i]->center[2], sph[i]->sqRadius);
+    img.sphObj[i] = (int)(sph[i] - s.objs.data());
+    img.sphRadius[i] = sph[i]->radius;
+  }
+  // the constant-bank form (built at the end) holds the whole scene
+  const bool fitsSmall = sph.size() <= (size_t)SMALL_MAX_SPHERES && tri.size() <= (size_t)SMALL_MAX_TRIS && pla.size() <= (size_t)SMALL_MAX_PLANES &&
+                         s.lights.size() <= (size_t)SMALL_MAX_LIGHTS && s.tex.size() <= (size_t)SMALL_MAX_TEX;
 
   // automatic mode: more than 32 spheres; mode 1: any.  The box margins below are sized for ray origins inside a bounded reach box;
   // next to an (unbounded) plane a drop point can lie anywhere, and a query from outside the box grows the boxes it tests by an
@@ -540,7 +573,16 @@ int buildSceneImage(const HostScene & s, SceneImage & img, std::string & err)
     {
       // leaf slots of one (cx, cy, cz, r^2) each, NaN in the unused ones (their discriminant is NaN: never a hit)
       const float qnan = std::numeric_limits<float>::quiet_NaN();
-      packBvh(nodes, prims, 1, qnan, [&](int i, float4 * w) { w[0] = img.spheres[i]; }, img.sphBvh);
+      // blob scenes: the parents for the refit of rfx_update_spheres (rfx_mesh.cu)
+      packBvh(nodes, prims, 1, qnan, [&](int i, float4 * w) { w[0] = img.spheres[i]; }, img.sphBvh,
+              fitsSmall ? nullptr : &img.sphLeafParent, fitsSmall ? nullptr : &img.sphPairParent);
+      if (!fitsSmall)
+      {
+        img.sphSlot.assign(sph.size(), -1);
+        for (size_t j = 0; j < img.sphBvh.prims.size(); j++)
+          if (img.sphBvh.prims[j] >= 0) img.sphSlot[img.sphBvh.prims[j]] = (int)j;
+      }
+      img.sphR = R;
       img.bvhDepth = maxDepth;
       img.bvhFloat4 = (uint32_t)img.sphBvh.nodes.size();
       h.bvhRoot = img.sphBvh.root;
@@ -597,12 +639,12 @@ int buildSceneImage(const HostScene & s, SceneImage & img, std::string & err)
       h.growT = farGrowthTris(kappaMax);
     }
   }
+  std::vector<char> inMesh(tri.size(), 0);
   if (!s.meshes.empty())
   {
     // where each mesh's triangles sit in the sorted triangle array (a mesh's triangles are consecutive objects)
     std::vector<int> triOf(s.objs.size(), -1);
     for (size_t i = 0; i < tri.size(); i++) triOf[tri[i] - s.objs.data()] = (int)i;
-    std::vector<char> inMesh(tri.size(), 0);
     for (const HostMesh & m : s.meshes)
     {
       SceneImage::MeshImage mi = { triOf[m.first], (uint32_t)(m.idx.size() / 3), img.meshIdx.size() };
@@ -610,20 +652,15 @@ int buildSceneImage(const HostScene & s, SceneImage & img, std::string & err)
       img.meshIdx.insert(img.meshIdx.end(), m.idx.begin(), m.idx.end());
       memset(&inMesh[mi.triBase], 1, mi.nTris);
     }
-    if (img.lightGridsBuilt)   // the drop-point box without the meshes (rfx_update_mesh adds their current boxes to it)
-    {
-      double * b = img.dropBase;
-      for (int k = 0; k < 3; k++) { b[k] = 1e300; b[3 + k] = -1e300; }
-      for (size_t i = 0; i < sph.size(); i++)
-        for (int k = 0; k < 3; k++)
-        {
-          b[k] = std::min(b[k], (double)sph[i]->center[k] - fabs((double)sph[i]->radius));
-          b[3 + k] = std::max(b[3 + k], (double)sph[i]->center[k] + fabs((double)sph[i]->radius));
-        }
-      for (size_t i = 0; i < tri.size(); i++)
-        if (!inMesh[i])
-          for (int v = 0; v < 9; v++) { b[v % 3] = std::min(b[v % 3], (double)tri[i]->triVerts[v]); b[3 + v % 3] = std::max(b[3 + v % 3], (double)tri[i]->triVerts[v]); }
-    }
+  }
+  if (img.lightGridsBuilt)   // the drop-point box in parts (rfx_update_mesh and rfx_update_spheres check their current union)
+  {
+    double * b = img.dropTris;
+    for (int k = 0; k < 3; k++) { b[k] = 1e300; b[3 + k] = -1e300; }
+    for (size_t i = 0; i < tri.size(); i++)
+      if (!inMesh[i])
+        for (int v = 0; v < 9; v++) { b[v % 3] = std::min(b[v % 3], (double)tri[i]->triVerts[v]); b[3 + v % 3] = std::max(b[3 + v % 3], (double)tri[i]->triVerts[v]); }
+    sphereDropBox(s, img, img.dropSpheres);
   }
   if (farOrigins && (img.bvhSpheres || img.triBvhTris))
   {
@@ -660,8 +697,7 @@ int buildSceneImage(const HostScene & s, SceneImage & img, std::string & err)
   // constant-bank form (rfx_trace_small.cu)
   SmallScene & ss = img.small;
   memset(&ss, 0, sizeof(ss));
-  img.smallOk = sph.size() <= (size_t)SMALL_MAX_SPHERES && tri.size() <= (size_t)SMALL_MAX_TRIS && pla.size() <= (size_t)SMALL_MAX_PLANES &&
-                s.lights.size() <= (size_t)SMALL_MAX_LIGHTS && s.tex.size() <= (size_t)SMALL_MAX_TEX;
+  img.smallOk = fitsSmall;
   if (!img.smallOk) return RFX_OK;
   ss.nS = h.nSpheres; ss.nT = h.nTris; ss.nP = h.nPlanes; ss.nL = h.nLights;
   ss.skyTex = h.skyTex; ss.halfTileW = h.halfTileW; ss.halfTileH = h.halfTileH;

@@ -5,7 +5,7 @@
 // once per object/frame; it is compiled with -ffp-contract=off so every operation is the same IEEE binary32 operation the reference's
 // build performs (reference Triangle.cpp:11-21,110-120; Matrix33.cpp:10-15,49-79; Skybox.cpp:21-37; Material.cpp:8-14; Render.cpp:148-150).
 #pragma once
-#include "rfx_tri_setup.h"
+#include "rfx_sphere_box.h"
 
 #include <float.h>
 #include <math.h>
@@ -98,11 +98,30 @@ struct SceneImage
   std::vector<int> leafParent, pairParent;  // triBvh: per leaf / pair node, 2 * (parent pair node) + side (0: a, 1: b); -1: the root
   double triUnion[6] = { 0, 0, 0, 0, 0, 0 };  // the box R is the diagonal of in the triangle margins: reach joined with every E
   double gridBox[6] = { 0, 0, 0, 0, 0, 0 };   // the padded drop-point box the light grids were built for (when lightGridsBuilt)
-  double dropBase[6] = { 0, 0, 0, 0, 0, 0 };  // the un-padded drop-point box of everything except the meshes' triangles
+  // The un-padded drop-point boxes (when lightGridsBuilt) that, joined with the meshes' current boxes, must stay inside gridBox for the
+  // light grids to stay complete: the triangles outside meshes (fixed until the next flatten), and every sphere (rfx_update_spheres
+  // keeps it current).  Empty: lo > hi.
+  double dropTris[6] = { 0, 0, 0, 0, 0, 0 };
+  double dropSpheres[6] = { 0, 0, 0, 0, 0, 0 };
+  // What rfx_update_spheres needs to move spheres on the device (rfx_mesh.cu) without a re-flatten.  Spheres keep insertion order in
+  // the sorted array: sphObj[i] is the object index of sphere i (ascending).
+  std::vector<int> sphObj;
+  std::vector<float> sphRadius;             // per sphere: its radius (the margins of the sphere hierarchy)
+  std::vector<int> sphSlot;                 // per sphere: its leaf slot in sphBvh (the inverse of sphBvh.prims); empty: no hierarchy
+  std::vector<int> sphLeafParent, sphPairParent;   // sphBvh, as leafParent / pairParent (blob scenes with a sphere hierarchy)
+  double sphR = 0.0;                        // R of the sphere margins (the diagonal of reach)
 };
 
 // the drop-point box (lo xyz, hi xyz) padded for the rounding of a drop point, as the light grids take it
 void padDropBox(double b[6]);
+
+// the un-padded drop-point box (lo xyz, hi xyz) of the spheres of img, from their records in s
+void sphereDropBox(const HostScene & s, const SceneImage & img, double b[6]);
+
+// Rebuilds the light grids of img for the current spheres of s over the drop-point box they were built for (img.gridBox), with the
+// margins of the hierarchy's last flatten (img.sphR) and its prims in slot order, as buildSceneImage would build them for that box:
+// after rfx_update_spheres moved spheres within gridBox.  The device pointers of img.grids are left null.
+void rebuildLightGrids(const HostScene & s, SceneImage & img);
 
 // recompute the host records (triVerts, tri.v0/ax/n) of the stale meshes' triangles from their current vertices
 void refreshMeshes(HostScene & s);

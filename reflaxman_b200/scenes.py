@@ -172,6 +172,56 @@ def with_ground_plane(scene, y=-0.05, refl=0.6, mtype=MT_METAL):
     return dict(scene, objects=objs)
 
 
+def object_indices(scene):
+    """The object index the C ABI gives the first object of each entry of ``scene["objects"]`` (a "mesh" entry counts all its
+    triangles), as :meth:`capi.Context.load_scene` issues them."""
+    out, k = [], 0
+    for ob in scene["objects"]:
+        out.append(k)
+        k += len(np.asarray(ob[2]).reshape(-1, 3)) if ob[0] == "mesh" else 1
+    return out
+
+
+def sphere_bounce(scene, t, height=1.5, pulse=0.0):
+    """Every "sphere" entry of ``scene`` bouncing at time ``t``: returns (objects int32 [n], spheres float32 [n, 4] rows of
+    (cx, cy, cz, r)) for :meth:`capi.Context.update_spheres`.  Sphere k rises by height * |sin(t + phase_k)| above its loaded centre
+    (phase_k = 2.399963 k, the golden angle) and, with ``pulse``, its radius scales by 1 + pulse * sin(2 t + phase_k); a sphere that
+    grows rises by as much, so its lowest point never sinks below the loaded one (a sphere resting on the floor stays on it).  At t = 0
+    with pulse = 0 the rows are the loaded values bit for bit.  (For :func:`synthetic_scene`, height <= 4 with pulse <= 0.3 keeps every
+    sphere above the floor and below the back wall's top, y = 8: inside the box the hierarchies and the light grid were built for.)"""
+    objects, rows = [], []
+    for k, (ob, i) in enumerate((ob, i) for ob, i in zip(scene["objects"], object_indices(scene)) if ob[0] == "sphere"):
+        _, c, r, *_ = ob
+        objects.append(i)
+        rows.append((float(np.float32(c[0])), float(np.float32(c[1])), float(np.float32(c[2])), float(np.float32(r))))
+    if not rows:
+        return np.zeros(0, np.int32), np.zeros((0, 4), np.float32)
+    base = np.asarray(rows, np.float64)
+    phase = 2.399963 * np.arange(len(rows))
+    out = base.copy()
+    if pulse != 0.0:
+        out[:, 3] = base[:, 3] * (1.0 + pulse * np.sin(2.0 * t + phase))
+        out[:, 1] += np.maximum(out[:, 3] - base[:, 3], 0.0)
+    if t != 0.0:
+        out[:, 1] += height * np.abs(np.sin(t + phase))
+    return np.asarray(objects, np.int32), out.astype(np.float32)
+
+
+def with_spheres(scene, objects, spheres):
+    """The same scene with the "sphere" entries whose object index (:func:`object_indices`) is in ``objects`` moved to the matching
+    rows (cx, cy, cz, r) of ``spheres`` (a repeated index takes its last row): what rfx_update_spheres(objects, spheres) describes."""
+    new = {int(i): tuple(float(x) for x in np.asarray(row, np.float32)) for i, row in zip(np.asarray(objects).reshape(-1), np.asarray(spheres, np.float32).reshape(-1, 4))}
+    objs = []
+    for ob, i in zip(scene["objects"], object_indices(scene)):
+        if i in new:
+            if ob[0] != "sphere":
+                raise ValueError("object %d is not a sphere" % i)
+            cx, cy, cz, r = new[i]
+            ob = ("sphere", (cx, cy, cz), r) + tuple(ob[3:])
+        objs.append(ob)
+    return dict(scene, objects=objs)
+
+
 def expand_meshes(scene):
     """The same scene with every "mesh" object replaced by its triangles, in order (untextured "tri" objects)."""
     objs = []
