@@ -107,11 +107,21 @@ RFX_API int rfx_update_mesh(rfx_ctx * ctx, int first, const float * xyz);
  * radius).  Afterwards every output is bit-identical to that of a scene built with the same calls but rfx_add_sphere(new centre, new
  * radius) (material, insertion order and tie-breaks stay).  A repeated object: the later entry wins.  Returns 1 when the device scene
  * was updated in place (queued on the stream the renders use, no synchronisation: the sphere records are written and the sphere
- * hierarchy is refitted on the GPU, keeping its topology; the light grids are rebuilt on the host and uploaded), 0 when the scene will
+ * hierarchy is refitted on the GPU, keeping its topology; the light grids are rebuilt on the GPU), 0 when the scene will
  * be re-flattened on the host at the next render instead (the scene fits the constant bank, a re-flatten is pending anyway, or a
  * sphere leaves the box the hierarchies or the light grids were built for), or RFX_ERR_ARG (NULL pointer, n = 0, an index that is not
  * a sphere of this scene); an error changes nothing. */
 RFX_API int rfx_update_spheres(rfx_ctx * ctx, uint32_t n, const int32_t * objects, const float * spheres);
+/* Move, resize and recolour lights added by rfx_add_light.  lights = n light indices (as rfx_add_light returned them); records = n x
+ * (origin[3], radius, rgb[3], power): the arguments of rfx_add_light, with its clamps (radius <= VSN becomes VSN, the light's power is
+ * clamped to [0, 1]; the ambient term adds rgb * power unclamped).  Afterwards every output is bit-identical to that of a scene built
+ * with the same calls but rfx_add_light(new values).  A repeated light: the later entry wins.  Returns 1 when the device scene was
+ * updated in place (queued on the stream the renders use, no synchronisation: the light records and the ambient term are copied, and
+ * the candidate grid of each moved light that is far from the scene is built on the GPU; a light that comes near loses its grid), 0
+ * when the scene will be re-flattened on the host at the next render instead (the scene fits the constant bank, a re-flatten is pending
+ * anyway, or a light becomes far in a scene whose last flatten built no light grid), or RFX_ERR_ARG (NULL pointer, n = 0, an index
+ * outside [0, number of lights)); an error changes nothing. */
+RFX_API int rfx_update_lights(rfx_ctx * ctx, uint32_t n, const int32_t * lights, const float * records);
 RFX_API int rfx_set_triangle_texture(rfx_ctx * ctx, int object, int texture, const float uv[6]); /* Triangle::setTexture, Triangle.cpp:110-120 (u1,v1,u2,v2,u3,v3) */
 RFX_API int rfx_add_plane(rfx_ctx * ctx, const float pos[3], const float norm[3], int mtype, const float rgb[3],
                           float reflectivity, float transparency);                              /* Plane::Plane, Plane.cpp:9-14 (no Scene::addPlane exists upstream) */
@@ -137,6 +147,13 @@ RFX_API int rfx_skip_samples(rfx_ctx * ctx, uint64_t n_trace_calls);
  * 2^32-state cycle.  out[0] = triples on which they disagree (0 = the decisions are the reference's, by exhaustion),
  * out[1] = triples inside the guard band.  About 20 ms. */
 RFX_API int rfx_selftest_rng(rfx_ctx * ctx, uint64_t out[2]);
+/* diagnostic: synchronises, reads back the light grids on the device (the flatten's, or those rfx_update_lights and rfx_update_spheres
+ * built on the GPU) and rebuilds every light's grid on the host from the current lights and spheres, over the box the last flatten
+ * built its grids for.  out[0] = lights whose grids differ in any byte (header floats and sizes, cell offsets, items; pointers aside),
+ * or that have a grid on one side only; out[1] = lights with a grid on the device; out[2] = lights with a grid on the host.  A grid
+ * dropped because it did not fit its item region (option "light_grid_items") is not a difference.  All 0 when the last flatten built no
+ * light grid; RFX_ERR_ARG when the scene changed since its last flatten. */
+RFX_API int rfx_selftest_light_grids(rfx_ctx * ctx, uint64_t out[3]);
 /* diagnostic: every path of a frame starts at the eye (Render.cpp:154-156), so the fast kernel lets a warp's first pass over the
  * objects skip those whose screen bounds miss its 4x8 pixel tile.  This returns the bounds the library derives for the current
  * scene (constant-bank scenes only), camera and image size: out[4*i .. 4*i+3] = x0, x1, y0, y1 (inclusive; x0 > x1 = no pixel) of
@@ -242,7 +259,12 @@ RFX_API int rfx_enable_profiling(rfx_ctx * ctx, int on);
  * candidate spheres across the light's direction instead of walking the hierarchy (default 1).  "eye_grid": the same scenes take the
  * candidates of a path's first query (origin = eye) from a screen grid binned per camera out of the spheres' primary-ray bounds
  * (default 1).  Both grids list spheres only: triangles are tested after them, through their own hierarchy when the scene has one
- * (rfx_set_bvh_mode).  Scenes with a plane get no light grids (a shadow ray can start anywhere on the plane); their eye grid is built.  Frames are bit-identical under every setting. */
+ * (rfx_set_bvh_mode).  Scenes with a plane get no light grids (a shadow ray can start anywhere on the plane); their eye grid is built.
+ * "light_grid_items" (test hook): at most this many items per light grid (0 = no limit, the default).  Each light has fixed device
+ * regions for its grid, with room for twice the items of the flatten's largest grid; a grid built on the GPU (rfx_update_lights,
+ * rfx_update_spheres) that does not fit is dropped — its shadow queries walk the hierarchy, and stats.light_grids counts it out — and
+ * the next synchronising call (rfx_get_stats, rfx_synchronize) grows the regions for the later builds.  Frames are bit-identical under
+ * every setting. */
 RFX_API int rfx_set_option(rfx_ctx * ctx, const char * name, int64_t value);
 /* kernel selection: 0 = automatic (constant-bank kernels when the scene fits, the blob kernels otherwise),
  * 1 = constant-bank kernel if it fits, 2 = always the blob kernels (tile / wavefront kernels for row-aligned slices, the general

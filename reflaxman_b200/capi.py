@@ -47,6 +47,7 @@ SYMBOLS = [
     ("rfx_add_mesh", C.c_int, [C.c_void_p, C.c_uint32, _fp, C.c_uint32, _u32p, C.c_int, _fp, C.c_float, C.c_float]),
     ("rfx_update_mesh", C.c_int, [C.c_void_p, C.c_int, _fp]),
     ("rfx_update_spheres", C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(C.c_int32), _fp]),
+    ("rfx_update_lights", C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(C.c_int32), _fp]),
     ("rfx_set_triangle_texture", C.c_int, [C.c_void_p, C.c_int, C.c_int, _fp]),
     ("rfx_add_plane", C.c_int, [C.c_void_p, _fp, _fp, C.c_int, _fp, C.c_float, C.c_float]),
     ("rfx_add_texture_argb", C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, _u32p]),
@@ -56,6 +57,7 @@ SYMBOLS = [
     ("rfx_get_seeds", C.c_int, [C.c_void_p, _u32p]),
     ("rfx_skip_samples", C.c_int, [C.c_void_p, C.c_uint64]),
     ("rfx_selftest_rng", C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
+    ("rfx_selftest_light_grids", C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
     ("rfx_selftest_primary_bounds", C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     ("rfx_selftest_primary_bounds_host", C.c_int, [_fp, C.c_uint32, C.c_uint32, C.c_int, _fp, C.c_int, _fp, C.POINTER(C.c_int32)]),
     ("rfx_selftest_light_grid_host", C.c_int, [_fp, C.c_int, _fp, _fp, C.c_float, _fp, C.POINTER(C.c_int32), _u32p, C.c_uint64,
@@ -322,6 +324,24 @@ class Context:
         return self._ck(self.L.rfx_update_spheres(self.h, ob.shape[0], ob.ctypes.data_as(C.POINTER(C.c_int32)), sp.ctypes.data_as(_fp)),
                         "rfx_update_spheres") == 1
 
+    def update_lights(self, lights, records):
+        """rfx_update_lights: lights [n] light indices, records [n][8] rows of their new (origin[3], radius, rgb[3], power), as
+        rfx_add_light takes them; a repeated light takes its last row.  True: the device scene was updated in place (the grids of far
+        lights built on the GPU); False: the scene is re-flattened on the host at the next render."""
+        li = np.ascontiguousarray(lights, dtype=np.int32).reshape(-1)
+        rec = np.ascontiguousarray(records, dtype=np.float32)
+        if rec.ndim != 2 or rec.shape[1] != 8 or rec.shape[0] != li.shape[0]:
+            raise ValueError("update_lights: %d lights need [%d, 8] records, got %s" % (li.shape[0], li.shape[0], rec.shape))
+        return self._ck(self.L.rfx_update_lights(self.h, li.shape[0], li.ctypes.data_as(C.POINTER(C.c_int32)), rec.ctypes.data_as(_fp)),
+                        "rfx_update_lights") == 1
+
+    def light_grids_selftest(self):
+        """rfx_selftest_light_grids: (lights whose device grid differs from the host's rebuild, lights with a grid on the device, lights
+        with a grid on the host)"""
+        out = (C.c_uint64 * 3)()
+        self._ck(self.L.rfx_selftest_light_grids(self.h, out), "rfx_selftest_light_grids")
+        return int(out[0]), int(out[1]), int(out[2])
+
     def add_texture(self, argb):
         if argb is None:
             return self._ck(self.L.rfx_add_texture_argb(self.h, 0, 0, None), "rfx_add_texture_argb")
@@ -493,7 +513,8 @@ class Context:
         self._ck(self.L.rfx_enable_profiling(self.h, 1 if on else 0), "rfx_enable_profiling")
 
     def set_option(self, name, value):
-        """tuning / test hook (include/reflax_c.h): "max_calls_per_launch", "copy_streams"; results never depend on it"""
+        """tuning / test hook (include/reflax_c.h): "max_calls_per_launch", "copy_streams", "light_grid_items", ...; results never
+        depend on it"""
         self._ck(self.L.rfx_set_option(self.h, name.encode(), int(value)), "rfx_set_option")
 
     def force_path(self, path):

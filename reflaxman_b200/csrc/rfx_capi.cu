@@ -15,6 +15,8 @@
 #include <string>
 #include <vector>
 #include <algorithm>
+#include <memory>
+#include <stddef.h>
 
 using namespace rfx;
 
@@ -74,11 +76,22 @@ struct rfx_ctx
   DevArray<float4> dBvhNodes;               // big scenes only: the hierarchy over the spheres, leaf slots then pair nodes
   DevArray<int> dBvhPrims;
   bool blobSmemBvh = true;                  // rfx_set_option "blob_smem_bvh"
-  // shadow-ray candidate grids of the far lights (LightGrid, rfx_types.h): one allocation each for the headers, the cell offsets and the items
+  // shadow-ray candidate grids of the far lights (LightGrid, rfx_types.h): a header per light, and per light fixed regions of
+  // LIGHT_GRID_CELLS cell offsets and gridItemAlloc items, which the flatten's grids are uploaded into and the device builder
+  // (rfx_light_grid.cu) writes: light i's cells at dGridCells + i * LIGHT_GRID_CELLS, its items at i * gridItemAlloc
   DevArray<LightGrid> dLightGrids;
   DevArray<uint32_t> dGridCells;
   DevArray<float4> dGridSpheres;
   DevArray<int> dGridIndex;
+  size_t gridItemAlloc = 0;                 // items per light region: twice the flatten's largest grid (at least 1024), grown on demand
+  uint32_t gridItemCap = 0;                 // items a device build may write: gridItemAlloc, or fewer under gridItemLimit
+  int64_t gridItemLimit = 0;                // rfx_set_option "light_grid_items" (test hook; 0: none)
+  std::vector<char> lightGrid;              // per light: it has a grid now (the flatten built one, or its last update found it far)
+  DevArray<uint32_t> dGridFlags;            // [1 + nLights]: the largest item count of a build that did not fit, then per light: dropped
+  DevArray<double> dLgDisc, dLgBlockSum;    // the builder's scratch (LightGridBuild)
+  DevArray<uint32_t> dLgSpan;
+  DevArray<unsigned long long> dLgRed;
+  DevArray<LightGridDims> dLgDims;
   // candidate spheres of the first query of a path per 32x32-pixel screen cell (EyeGrid, rfx_kernels.h), rebuilt when the camera,
   // the image size or the scene changes
   DevArray<uint32_t> dEyeCells;
@@ -189,6 +202,13 @@ template <typename T> int upload(rfx_ctx * ctx, DevArray<T> & a, const std::vect
   return RFX_OK;
 }
 
+void setGridItemCap(rfx_ctx * ctx)
+{
+  size_t cap = ctx->gridItemAlloc;
+  if (ctx->gridItemLimit > 0) cap = std::min<size_t>(cap, (size_t)ctx->gridItemLimit);
+  ctx->gridItemCap = (uint32_t)std::min<size_t>(cap, UINT32_MAX);
+}
+
 // flatten the host scene (rfx_scene.cpp) and upload it
 int uploadScene(rfx_ctx * ctx, cudaStream_t st)
 {
@@ -221,19 +241,55 @@ int uploadScene(rfx_ctx * ctx, cudaStream_t st)
     h.bvhLeafSph = ctx->dBvhNodes.p;
     h.bvhPairs = ctx->dBvhNodes.p + img.sphBvh.leafFloat4;
   }
+  ctx->lightGrid.assign(ctx->scene.lights.size(), 0);
+  std::vector<LightGrid> headers(img.grids);   // (alive until the synchronisation below)
+  std::vector<uint32_t> flags;
+  std::vector<unsigned long long> lgRed;
   if (!img.grids.empty())
   {
-    if ((rc = upload(ctx, ctx->dGridCells, img.gridCells, st)) != RFX_OK || (rc = upload(ctx, ctx->dGridSpheres, img.gridSpheres, st)) != RFX_OK ||
-        (rc = upload(ctx, ctx->dGridIndex, img.gridIndex, st)) != RFX_OK) return rc;
-    for (size_t li = 0; li < img.grids.size(); li++)
-      if (img.grids[li].nx)
+    // each light's grid into its regions (cellStart offsets are relative to the light's own items)
+    const size_t nL = img.grids.size();
+    size_t largest = 0;
+    for (size_t li = 0; li < nL; li++)
+      if (img.grids[li].nx) largest = std::max<size_t>(largest, img.gridCells[img.gridCellOff[li] + (size_t)img.grids[li].nx * img.grids[li].ny]);
+    if ((rc = ensure(ctx, ctx->dGridCells, nL * LIGHT_GRID_CELLS)) != RFX_OK || (rc = ensure(ctx, ctx->dGridSpheres, nL * std::max<size_t>(2 * largest, 1024))) != RFX_OK ||
+        (rc = ensure(ctx, ctx->dGridIndex, nL * std::max<size_t>(2 * largest, 1024))) != RFX_OK) return rc;
+    ctx->gridItemAlloc = std::min(ctx->dGridSpheres.cap, ctx->dGridIndex.cap) / nL;
+    setGridItemCap(ctx);
+    flags.assign(1 + nL, 0);
+    for (size_t li = 0; li < nL; li++)
+    {
+      if (!img.grids[li].nx) continue;
+      ctx->lightGrid[li] = 1;
+      const size_t nCells = (size_t)img.grids[li].nx * img.grids[li].ny + 1, nItems = img.gridCells[img.gridCellOff[li] + nCells - 1];
+      if (nItems > ctx->gridItemCap)   // (only under the "light_grid_items" hook) dropped, as a device build that does not fit
       {
-        img.grids[li].cellStart = ctx->dGridCells.p + img.gridCellOff[li];
-        img.grids[li].itemSphere = ctx->dGridSpheres.p + img.gridItemOff[li];   // cellStart offsets are relative to the light's own items
-        img.grids[li].itemIndex = ctx->dGridIndex.p + img.gridItemOff[li];
+        headers[li] = LightGrid();
+        flags[0] = std::max<uint32_t>(flags[0], (uint32_t)nItems); flags[1 + li] = 1;
+        continue;
       }
-    if ((rc = upload(ctx, ctx->dLightGrids, img.grids, st)) != RFX_OK) return rc;
+      LightGrid & g = headers[li];
+      g.cellStart = ctx->dGridCells.p + li * LIGHT_GRID_CELLS;
+      g.itemSphere = ctx->dGridSpheres.p + li * ctx->gridItemAlloc;
+      g.itemIndex = ctx->dGridIndex.p + li * ctx->gridItemAlloc;
+      CK(cudaMemcpyAsync((void *)g.cellStart, &img.gridCells[img.gridCellOff[li]], nCells * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+      if (nItems)
+      {
+        CK(cudaMemcpyAsync((void *)g.itemSphere, &img.gridSpheres[img.gridItemOff[li]], nItems * sizeof(float4), cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync((void *)g.itemIndex, &img.gridIndex[img.gridItemOff[li]], nItems * sizeof(int), cudaMemcpyHostToDevice, st));
+      }
+      ctx->stats.h2d_bytes += nCells * sizeof(uint32_t) + nItems * (sizeof(float4) + sizeof(int));
+    }
+    if ((rc = upload(ctx, ctx->dLightGrids, headers, st)) != RFX_OK || (rc = upload(ctx, ctx->dGridFlags, flags, st)) != RFX_OK) return rc;
     h.lightGrids = ctx->dLightGrids.p;
+    if (!img.smallOk)   // the device builder's scratch (rfx_update_lights, rfx_update_spheres)
+    {
+      const size_t nSlots = img.sphBvh.prims.size();
+      lgRed = { orderedCode(1e300), orderedCode(-1e300), orderedCode(1e300), orderedCode(-1e300), 0ull };
+      if ((rc = ensure(ctx, ctx->dLgDisc, 3 * nSlots)) != RFX_OK || (rc = ensure(ctx, ctx->dLgSpan, 2 * nSlots)) != RFX_OK ||
+          (rc = ensure(ctx, ctx->dLgBlockSum, nSlots / LIGHT_GRID_SUM_BLOCK + 1)) != RFX_OK || (rc = ensure(ctx, ctx->dLgDims, 1)) != RFX_OK ||
+          (rc = upload(ctx, ctx->dLgRed, lgRed, st)) != RFX_OK) return rc;
+    }
   }
   if (!img.triBvh.nodes.empty())
   {
@@ -425,7 +481,7 @@ TraceWork traceWork(const rfx_ctx * ctx, uint64_t p0, uint64_t p1, uint64_t firs
   w.argbOut = argbOut;
   w.sigOut = ctx->sigOn ? ctx->dSig.p : nullptr;
   w.counters = ctx->dCounters.p;
-  w.lightGrids = ctx->image.lightGridsBuilt > 0;
+  w.lightGrids = ctx->image.lightGridsBuilt > 0 && std::count(ctx->lightGrid.begin(), ctx->lightGrid.end(), 1) > 0;   // (the lights with a grid now)
   w.triBvh = ctx->image.triBvhTris > 0;
   w.far = ctx->image.far;
   return w;
@@ -537,6 +593,97 @@ bool gridBoxHolds(const rfx_ctx * ctx, const double * sph = nullptr)
   for (int k = 0; k < 3; k++)
     if (!(b[k] >= img.gridBox[k] && b[3 + k] <= img.gridBox[3 + k])) return false;
   return true;
+}
+
+// Light li's grid after it or the spheres moved (a scene whose flatten built grids): built on the device over the flatten's box when the
+// light is far from it, else a NULL header.  Queued on st.
+int updateLightGrid(rfx_ctx * ctx, size_t li, cudaStream_t st)
+{
+  const SceneImage & img = ctx->image;
+  const double blo[3] = { img.gridBox[0], img.gridBox[1], img.gridBox[2] }, bhi[3] = { img.gridBox[3], img.gridBox[4], img.gridBox[5] };
+  LightFrame f;
+  ctx->lightGrid[li] = lightFrame(ctx->scene.lights[li], blo, bhi, f);
+  if (!ctx->lightGrid[li])
+  {
+    CK(cudaMemsetAsync(ctx->dLightGrids.p + li, 0, sizeof(LightGrid), st));
+    CK(cudaMemsetAsync(ctx->dGridFlags.p + 1 + li, 0, sizeof(uint32_t), st));
+    return RFX_OK;
+  }
+  const SceneHeader & h = *reinterpret_cast<const SceneHeader *>(img.blob.data());
+  LightGridBuild b;
+  memset(&b, 0, sizeof(b));
+  b.f = f;
+  b.spheres = reinterpret_cast<const float4 *>(ctx->dBlob.p + h.offSpheres);
+  b.radius = ctx->dSphRadius.p;
+  b.prims = ctx->dBvhPrims.p;
+  b.nSlots = (int)img.sphBvh.prims.size();
+  b.nPrims = img.bvhSpheres;
+  b.R = img.sphR;
+  b.header = ctx->dLightGrids.p + li;
+  b.cells = ctx->dGridCells.p + li * LIGHT_GRID_CELLS;
+  b.itemSphere = ctx->dGridSpheres.p + li * ctx->gridItemAlloc;
+  b.itemIndex = ctx->dGridIndex.p + li * ctx->gridItemAlloc;
+  b.itemCap = ctx->gridItemCap;
+  b.need = ctx->dGridFlags.p;
+  b.dropped = ctx->dGridFlags.p + 1 + li;
+  b.disc = ctx->dLgDisc.p; b.span = ctx->dLgSpan.p; b.blockSum = ctx->dLgBlockSum.p; b.red = ctx->dLgRed.p; b.dims = ctx->dLgDims.p;
+  ctx->stats.kernel_launches += launchLightGridBuild(b, st);
+  CK(cudaGetLastError());
+  return RFX_OK;
+}
+
+// At a synchronising call: a device build that did not fit its item region (LightGridBuild::need) grows every light's regions for the
+// later builds.  The grids already built move with their regions; the dropped one returns at its light's next build.
+int growLightGrids(rfx_ctx * ctx)
+{
+  const SceneImage & img = ctx->image;
+  if (ctx->sceneDirty || !img.lightGridsBuilt || !ctx->dGridFlags.p) return RFX_OK;   // (a pending flatten sizes its own regions)
+  uint32_t need = 0;
+  CK(cudaMemcpy(&need, ctx->dGridFlags.p, sizeof(need), cudaMemcpyDeviceToHost));
+  if (need <= ctx->gridItemAlloc) return RFX_OK;
+  const size_t nL = ctx->scene.lights.size(), old = ctx->gridItemAlloc, alloc = (size_t)need + need / 2;
+  DevArray<float4> sp;
+  DevArray<int> ix;
+  CK(sp.alloc(nL * alloc));
+  CK(ix.alloc(nL * alloc));
+  CK(cudaMemcpy2D(sp.p, alloc * sizeof(float4), ctx->dGridSpheres.p, old * sizeof(float4), old * sizeof(float4), nL, cudaMemcpyDeviceToDevice));
+  CK(cudaMemcpy2D(ix.p, alloc * sizeof(int), ctx->dGridIndex.p, old * sizeof(int), old * sizeof(int), nL, cudaMemcpyDeviceToDevice));
+  std::vector<LightGrid> hdr(nL);
+  CK(cudaMemcpy(hdr.data(), ctx->dLightGrids.p, nL * sizeof(LightGrid), cudaMemcpyDeviceToHost));
+  for (size_t li = 0; li < nL; li++)
+    if (hdr[li].cellStart) { hdr[li].itemSphere = sp.p + li * alloc; hdr[li].itemIndex = ix.p + li * alloc; }
+  CK(cudaMemcpy(ctx->dLightGrids.p, hdr.data(), nL * sizeof(LightGrid), cudaMemcpyHostToDevice));
+  CK(cudaFree(ctx->dGridSpheres.p)); CK(cudaFree(ctx->dGridIndex.p));
+  ctx->dGridSpheres.p = sp.p; ctx->dGridSpheres.cap = sp.cap; sp.p = nullptr; sp.cap = 0;
+  ctx->dGridIndex.p = ix.p; ctx->dGridIndex.cap = ix.cap; ix.p = nullptr; ix.cap = 0;
+  ctx->gridItemAlloc = alloc;
+  setGridItemCap(ctx);
+  CK(cudaMemset(ctx->dGridFlags.p, 0, sizeof(uint32_t)));
+  return RFX_OK;
+}
+
+// lights whose shadow queries use a grid: the headers on the device that are not NULL (after a synchronisation)
+int countLightGrids(rfx_ctx * ctx, uint64_t & n)
+{
+  n = 0;
+  if (!ctx->image.lightGridsBuilt || ctx->image.grids.empty()) return RFX_OK;
+  std::vector<LightGrid> hdr(ctx->image.grids.size());
+  CK(cudaMemcpy(hdr.data(), ctx->dLightGrids.p, hdr.size() * sizeof(LightGrid), cudaMemcpyDeviceToHost));
+  for (const LightGrid & g : hdr) n += g.cellStart != nullptr;
+  return RFX_OK;
+}
+
+// recompute envColor from the lights' current colours and powers as Scene's constructor and addLight do (Scene.cpp:12,54): the
+// ambient term, then colour * (unclamped) power added light after light in insertion order
+void recomputeEnv(HostScene & s)
+{
+  for (int k = 0; k < 3; k++) s.env[k] = s.ambient[k] * s.ambientPower;
+  for (size_t i = 0; i < s.lights.size(); i++)
+  {
+    const Light & L = s.lights[i];
+    const float rgb[3] = { L.r, L.g, L.b };
+    for (int k = 0; k < 3; k++) s.env[k] = s.env[k] + rgb[k] * s.lightPower[i];
+  }
 }
 
 // Whether the structures of the last flatten still serve the scene after mesh m moved (rfx_update_mesh updates it on the device):
@@ -673,7 +820,7 @@ int rfx_scene_reset(rfx_ctx * ctx, const float ambient_rgb[3], float ambient_pow
   CK(cudaSetDevice(ctx->device));
   CK(cudaDeviceSynchronize());
   for (HostTex & t : ctx->scene.tex) if (t.dev) cudaFree(t.dev);
-  ctx->scene.tex.clear(); ctx->scene.objs.clear(); ctx->scene.lights.clear(); ctx->scene.meshes.clear();
+  ctx->scene.tex.clear(); ctx->scene.objs.clear(); ctx->scene.lights.clear(); ctx->scene.lightPower.clear(); ctx->scene.meshes.clear();
   ctx->scene.skyTex = -1;
   for (int i = 0; i < 3; i++) { ctx->scene.extraOrigins[i] = FLT_MAX; ctx->scene.extraOrigins[3 + i] = -FLT_MAX; }
   for (int i = 0; i < 3; i++)
@@ -696,8 +843,60 @@ int rfx_add_light(rfx_ctx * ctx, const float o[3], float radius, const float rgb
   l.r = rgb[0]; l.g = rgb[1]; l.b = rgb[2];
   l.power = clampf(power, 0.0f, 1.0f);                          // OmniLight.cpp:13
   ctx->scene.lights.push_back(l);
+  ctx->scene.lightPower.push_back(power);
   ctx->sceneDirty = true;
   return (int)ctx->scene.lights.size() - 1;
+}
+
+int rfx_update_lights(rfx_ctx * ctx, uint32_t n, const int32_t * lights, const float * records)
+{
+  if (!ctx || !lights || !records || n == 0) return fail(ctx, RFX_ERR_ARG, "rfx_update_lights: NULL argument or no light");
+  HostScene & s = ctx->scene;
+  for (uint32_t i = 0; i < n; i++)
+    if (lights[i] < 0 || lights[i] >= (int)s.lights.size())
+      return fail(ctx, RFX_ERR_ARG, "rfx_update_lights: light " + std::to_string(lights[i]) + " is not a light of this scene");
+  // the host records, as rfx_add_light makes them (a later entry for the same light overwrites an earlier one)
+  std::vector<char> moved(s.lights.size(), 0);
+  for (uint32_t i = 0; i < n; i++)
+  {
+    const float * r = records + 8 * (size_t)i;
+    Light & l = s.lights[lights[i]];
+    float radius = r[3];
+    if (radius <= VSN) radius = VSN;                              // Scene.cpp:51-52
+    l.ox = r[0]; l.oy = r[1]; l.oz = r[2]; l.radius = radius;
+    l.r = r[4]; l.g = r[5]; l.b = r[6];
+    l.power = clampf(r[7], 0.0f, 1.0f);                           // OmniLight.cpp:13
+    s.lightPower[lights[i]] = r[7];
+    moved[lights[i]] = 1;
+  }
+  recomputeEnv(s);
+  if (ctx->sceneDirty || ctx->image.smallOk) { ctx->sceneDirty = true; return 0; }
+  SceneImage & img = ctx->image;
+  SceneHeader & h = *reinterpret_cast<SceneHeader *>(img.blob.data());
+  // Light positions enter neither the reach box nor the hierarchies' margins nor the eye grid: only the light grids can change.  A
+  // light that becomes far in a scene whose flatten built no grid (no header array on the device) re-flattens the scene.
+  if (!img.lightGridsBuilt && img.bvhDepth > 0 && s.lightGridsOn && h.nPlanes == 0)
+  {
+    const double blo[3] = { img.gridBox[0], img.gridBox[1], img.gridBox[2] }, bhi[3] = { img.gridBox[3], img.gridBox[4], img.gridBox[5] };
+    LightFrame f;
+    for (size_t li = 0; li < moved.size(); li++)
+      if (moved[li] && lightFrame(s.lights[li], blo, bhi, f)) { ctx->sceneDirty = true; return 0; }
+  }
+  CK(cudaSetDevice(ctx->device));
+  // the stream the renders use: the update is ordered after the frames already queued there
+  cudaStream_t st = ctx->lastStream ? ctx->lastStream : ctx->stream;
+  int rc;
+  if ((rc = useStream(ctx, st)) != RFX_OK) return rc;
+  // the records and envColor into the blob (the host copy first: the copies read from it, staged before they return)
+  memcpy(img.blob.data() + h.offLights, s.lights.data(), sizeof(Light) * s.lights.size());
+  memcpy(h.env, s.env, sizeof(h.env));
+  CK(cudaMemcpyAsync(ctx->dBlob.p + h.offLights, img.blob.data() + h.offLights, sizeof(Light) * s.lights.size(), cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(ctx->dBlob.p + offsetof(SceneHeader, env), h.env, sizeof(h.env), cudaMemcpyHostToDevice, st));
+  ctx->stats.h2d_bytes += sizeof(Light) * s.lights.size() + sizeof(h.env);
+  if (img.lightGridsBuilt)
+    for (size_t li = 0; li < moved.size(); li++)
+      if (moved[li] && (rc = updateLightGrid(ctx, li, st)) != RFX_OK) return rc;
+  return 1;
 }
 
 int rfx_add_sphere(rfx_ctx * ctx, const float c[3], float radius, int mtype, const float rgb[3], float refl, float transp)
@@ -883,27 +1082,13 @@ int rfx_update_spheres(rfx_ctx * ctx, uint32_t n, const int32_t * objects, const
   ctx->stats.kernel_launches += launchSphereUpdate(u, st);
   CK(cudaGetLastError());
 
-  // The light grids are rebuilt for the new spheres over the box they were built for (which still holds every drop point): cells and
-  // items first, then the headers, whose pointers move when an array grows.  The copies follow the frames queued on the stream.
+  // The grids of the lights that have one are rebuilt on the device for the new spheres, over the box they were built for (which still
+  // holds every drop point).  Re-binning into the old cells would miss spheres that moved out of a grid's rectangle.
   if (img.lightGridsBuilt)
   {
     memcpy(img.dropSpheres, sphBox, sizeof(sphBox));
-    rebuildLightGrids(s, img);
-    if (!img.grids.empty())
-    {
-      if ((rc = upload(ctx, ctx->dGridCells, img.gridCells, st)) != RFX_OK || (rc = upload(ctx, ctx->dGridSpheres, img.gridSpheres, st)) != RFX_OK ||
-          (rc = upload(ctx, ctx->dGridIndex, img.gridIndex, st)) != RFX_OK) return rc;
-      for (size_t li = 0; li < img.grids.size(); li++)
-        if (img.grids[li].nx)
-        {
-          img.grids[li].cellStart = ctx->dGridCells.p + img.gridCellOff[li];
-          img.grids[li].itemSphere = ctx->dGridSpheres.p + img.gridItemOff[li];
-          img.grids[li].itemIndex = ctx->dGridIndex.p + img.gridItemOff[li];
-        }
-    }
-    else   // (not seen: whether a light gets a grid depends on the light and the box alone) no grid: every light walks the hierarchy
-      img.grids.assign(s.lights.size(), LightGrid());
-    if ((rc = upload(ctx, ctx->dLightGrids, img.grids, st)) != RFX_OK) return rc;
+    for (size_t li = 0; li < s.lights.size(); li++)
+      if (ctx->lightGrid[li] && (rc = updateLightGrid(ctx, li, st)) != RFX_OK) return rc;
   }
   // the eye grid is binned again from img.spheres at the next render
   ctx->eyeValid = false;
@@ -1012,6 +1197,50 @@ int rfx_selftest_rng(rfx_ctx * ctx, uint64_t out[2])
   cudaFree(d);
   if (e != cudaSuccess) return fail(ctx, RFX_ERR_CUDA, std::string("rfx_selftest_rng: ") + cudaGetErrorString(e));
   out[0] = h[0]; out[1] = h[1];
+  return RFX_OK;
+}
+
+int rfx_selftest_light_grids(rfx_ctx * ctx, uint64_t out[3])
+{
+  if (!ctx || !out) return RFX_ERR_ARG;
+  if (ctx->sceneDirty) return fail(ctx, RFX_ERR_ARG, "rfx_selftest_light_grids: the scene changed since its last flatten");
+  CK(cudaSetDevice(ctx->device));
+  CK(cudaDeviceSynchronize());
+  out[0] = out[1] = out[2] = 0;
+  const SceneImage & img = ctx->image;
+  if (!img.lightGridsBuilt) return RFX_OK;
+  std::unique_ptr<SceneImage> ref(new SceneImage());
+  rebuildLightGrids(ctx->scene, img, *ref);
+  const size_t nL = ctx->scene.lights.size();
+  std::vector<LightGrid> hdr(nL);
+  std::vector<uint32_t> flags(1 + nL), cells;
+  std::vector<float4> sp;
+  std::vector<int> ix;
+  CK(cudaMemcpy(hdr.data(), ctx->dLightGrids.p, nL * sizeof(LightGrid), cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(flags.data(), ctx->dGridFlags.p, flags.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+  for (size_t li = 0; li < nL; li++)
+  {
+    const LightGrid & g = hdr[li];
+    const bool dev = g.cellStart != nullptr, host = !ref->grids.empty() && ref->grids[li].nx != 0;
+    out[1] += dev; out[2] += host;
+    if (!dev && host && flags[1 + li]) continue;   // dropped for want of room: its queries walk the hierarchy until a build fits
+    if (dev != host) { out[0]++; continue; }
+    if (!dev) continue;
+    const LightGrid & r = ref->grids[li];
+    const size_t nCells = (size_t)r.nx * r.ny + 1, off = ref->gridCellOff[li], nItems = ref->gridCells[off + nCells - 1];
+    if (memcmp(g.u, r.u, sizeof(g.u)) || memcmp(g.v, r.v, sizeof(g.v)) || g.nx != r.nx || g.ny != r.ny || nItems > ctx->gridItemAlloc) { out[0]++; continue; }
+    cells.resize(nCells); sp.resize(nItems); ix.resize(nItems);
+    CK(cudaMemcpy(cells.data(), g.cellStart, nCells * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+    if (nItems)
+    {
+      CK(cudaMemcpy(sp.data(), g.itemSphere, nItems * sizeof(float4), cudaMemcpyDeviceToHost));
+      CK(cudaMemcpy(ix.data(), g.itemIndex, nItems * sizeof(int), cudaMemcpyDeviceToHost));
+    }
+    const size_t io = ref->gridItemOff[li];
+    if (memcmp(cells.data(), &ref->gridCells[off], nCells * sizeof(uint32_t)) ||
+        (nItems && (memcmp(sp.data(), &ref->gridSpheres[io], nItems * sizeof(float4)) || memcmp(ix.data(), &ref->gridIndex[io], nItems * sizeof(int)))))
+      out[0]++;
+  }
   return RFX_OK;
 }
 
@@ -1516,6 +1745,8 @@ int rfx_synchronize(rfx_ctx * ctx)
   CK(cudaSetDevice(ctx->device));
   if (ctx->lastStream) CK(cudaStreamSynchronize(ctx->lastStream));
   CK(cudaStreamSynchronize(ctx->stream));
+  int rc;
+  if ((rc = growLightGrids(ctx)) != RFX_OK) return rc;
   return checkStatus(ctx);
 }
 
@@ -1540,7 +1771,8 @@ int rfx_get_stats(rfx_ctx * ctx, rfx_stats * out)
     ctx->stats.trace_kernels++;
   }
   ctx->evUsed = 0;
-  ctx->stats.light_grids = (uint64_t)ctx->image.lightGridsBuilt;
+  int rc;
+  if ((rc = countLightGrids(ctx, ctx->stats.light_grids)) != RFX_OK || (rc = growLightGrids(ctx)) != RFX_OK) return rc;
   ctx->stats.bvh_triangles = ctx->image.triBvhTris;
   ctx->stats.bvh_spheres = ctx->image.bvhSpheres;
   *out = ctx->stats;
@@ -1595,6 +1827,13 @@ int rfx_set_option(rfx_ctx * ctx, const char * name, int64_t value)
     if (value != 0 && value != 1) return fail(ctx, RFX_ERR_ARG, "rfx_set_option: light_grids must be 0 or 1");
     if (ctx->scene.lightGridsOn != (value != 0)) ctx->sceneDirty = true;
     ctx->scene.lightGridsOn = value != 0;
+    return RFX_OK;
+  }
+  if (!strcmp(name, "light_grid_items"))
+  {
+    if (value < 0) return fail(ctx, RFX_ERR_ARG, "rfx_set_option: light_grid_items must be >= 0 (0: no limit)");
+    ctx->gridItemLimit = value;
+    setGridItemCap(ctx);
     return RFX_OK;
   }
   if (!strcmp(name, "eye_grid"))

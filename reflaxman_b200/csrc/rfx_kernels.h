@@ -5,6 +5,7 @@
 #include <stdint.h>
 #include <type_traits>
 #include "rfx_types.h"
+#include "rfx_light_grid.h"
 
 namespace rfx
 {
@@ -226,6 +227,36 @@ struct SphereUpdate
   double R;                                 // the margins' R of the last flatten
 };
 int launchSphereUpdate(const SphereUpdate & u, cudaStream_t st);   // returns the number of kernels launched
+
+// ---- light grids on the device (rfx_light_grid.cu: rfx_update_lights, rfx_update_spheres) --------------------------------------------
+// One far light's LightGrid built from the spheres of the blob, byte for byte what rfx_scene.cpp buildLightGrid builds for them, into the
+// light's fixed regions (cells, items).  A grid with more items than itemCap is dropped: its header is NULL and *dropped set, *need
+// raised to its item count.  A light without a grid (no disc, an empty extent, no finite bound) gets a NULL header.
+struct LightGridBuild
+{
+  LightFrame f;                 // the light over the grid box (lightFrame, on the host)
+  const float4 * spheres;       // the blob's sorted sphere array
+  const float * radius;         // per sphere: its radius
+  const int * prims;            // the sphere hierarchy's leaf slots: the sphere of each slot, -1 unused
+  int nSlots;
+  uint64_t nPrims;              // used slots (every sphere)
+  double R;                     // the margins' R of the last flatten
+  LightGrid * header;           // the light's header in the device array
+  uint32_t * cells;             // the light's cell region [LIGHT_GRID_CELLS]
+  float4 * itemSphere;          // its item regions [itemCap]
+  int * itemIndex;
+  uint32_t itemCap;
+  uint32_t * need;              // raised to the item count of a grid that did not fit (read by the host at a synchronising call)
+  uint32_t * dropped;           // the light's last build did not fit
+  // scratch, shared by the builds on one stream
+  double * disc;                // 3 per slot: pu, pv, rho
+  uint32_t * span;              // 2 per slot: x0 | x1 << 16, y0 | y1 << 16 of the disc's cells (0xFFFF: none)
+  double * blockSum;            // one per LIGHT_GRID_SUM_BLOCK slots
+  unsigned long long * red;     // [5] orderedCode of ulo (min), uhi (max), vlo (min), vhi (max); non-zero: no finite bound.  Left at
+                                // (1e300, -1e300, 1e300, -1e300, 0) by each build for the next
+  LightGridDims * dims;         // nx == 0: no grid (or dropped)
+};
+int launchLightGridBuild(const LightGridBuild & b, cudaStream_t st);   // returns the number of kernels launched
 
 // ---- K3: resolve (imagePixel + argb)---------------------------------------------------------------------------
 int launchResolve(const float * image, uint64_t nPixels, int additiveCounter, float * rgbfOut, uint32_t * argbOut, cudaStream_t st);

@@ -246,69 +246,33 @@ struct LightGridHost
   std::vector<int> index;
 };
 
-bool buildLightGrid(const Light & L, const std::vector<const HostObj *> & sph, const std::vector<BvhPrim> & prims, const double blo[3], const double bhi[3], LightGridHost & out)
+// (lightFrame, lightDisc, lightGridDims, lightCellsOf, lightTouches and lightGridHeader: rfx_light_grid.h, shared with the device builder
+// of rfx_light_grid.cu.)  slots[i]: the leaf slot of prims[i] in the sphere hierarchy (ascending), which fixes the shape of rhoSum.
+bool buildLightGrid(const Light & L, const std::vector<const HostObj *> & sph, const std::vector<BvhPrim> & prims, const std::vector<int> & slots,
+                    const double blo[3], const double bhi[3], LightGridHost & out)
 {
-  const double cb[3] = { 0.5 * (blo[0] + bhi[0]), 0.5 * (blo[1] + bhi[1]), 0.5 * (blo[2] + bhi[2]) };
-  const double ext[3] = { bhi[0] - blo[0], bhi[1] - blo[1], bhi[2] - blo[2] };
-  const double diag = sqrt(ext[0] * ext[0] + ext[1] * ext[1] + ext[2] * ext[2]);
-  double l[3] = { (double)L.ox - cb[0], (double)L.oy - cb[1], (double)L.oz - cb[2] };
-  const double D = sqrt(l[0] * l[0] + l[1] * l[1] + l[2] * l[2]);
-  const double rad = fabs((double)L.radius) * (1.0 + 1e-5);
-  if (!(D < 1e300) || !(rad < 1e300) || !(diag > 0.0)) return false;
-  const double lateral = 0.5 * diag + rad;
-  if (!(D > 8.0 * lateral)) return false;                       // the light is inside or near the scene: its rays are no bundle
-  const double sigma = lateral / (D - lateral) * 1.001 + 1e-6;   // + the float evaluation of the ray on the device
-  for (int k = 0; k < 3; k++) l[k] /= D;
-  // plane axes
-  const int minAxis = fabs(l[0]) <= fabs(l[1]) && fabs(l[0]) <= fabs(l[2]) ? 0 : fabs(l[1]) <= fabs(l[2]) ? 1 : 2;
-  double e[3] = { 0, 0, 0 }; e[minAxis] = 1.0;
-  double u[3] = { l[1] * e[2] - l[2] * e[1], l[2] * e[0] - l[0] * e[2], l[0] * e[1] - l[1] * e[0] };
-  const double ul = sqrt(u[0] * u[0] + u[1] * u[1] + u[2] * u[2]);
-  for (int k = 0; k < 3; k++) u[k] /= ul;
-  const double v[3] = { l[1] * u[2] - l[2] * u[1], l[2] * u[0] - l[0] * u[2], l[0] * u[1] - l[1] * u[0] };
+  LightFrame f;
+  if (!lightFrame(L, blo, bhi, f)) return false;
   // per sphere: disc centre and radius on the plane
   const size_t n = prims.size();
   std::vector<double> pu(n), pv(n), rho(n);
-  double ulo = 1e300, uhi = -1e300, vlo = 1e300, vhi = -1e300, rhoSum = 0.0;
+  double ulo = 1e300, uhi = -1e300, vlo = 1e300, vhi = -1e300, rhoSum = 0.0, blockSum = 0.0;
+  int block = 0;
   for (size_t i = 0; i < n; i++)
   {
     const HostObj * o = sph[prims[i].index];
-    const double C[3] = { (double)o->center[0], (double)o->center[1], (double)o->center[2] };
-    const double r = fabs((double)o->radius), m = (double)prims[i].m;
-    const double infl = r + m + 1.01 * sigma * (diag + r);
-    // distance from C backwards along l to the boundary of B inflated by infl (C is inside B)
-    double sMax = 1e300;
-    for (int k = 0; k < 3; k++)
-    {
-      const double dk = -l[k];
-      if (dk > 1e-300) sMax = std::min(sMax, (bhi[k] + infl - C[k]) / dk);
-      else if (dk < -1e-300) sMax = std::min(sMax, (blo[k] - infl - C[k]) / dk);
-    }
-    if (!(sMax < 1e300)) return false;
-    sMax = std::max(sMax, 0.0);
-    rho[i] = (r + m + sigma * sMax) * 1.001 + 1e-5 * diag + 1e-6 * (fabs(cb[0]) + fabs(cb[1]) + fabs(cb[2]));   // + the float evaluation of the cell coordinates
-    pu[i] = u[0] * C[0] + u[1] * C[1] + u[2] * C[2];
-    pv[i] = v[0] * C[0] + v[1] * C[1] + v[2] * C[2];
+    if (!lightDisc(f, o->center, o->radius, prims[i].m, pu[i], pv[i], rho[i])) return false;
     ulo = std::min(ulo, pu[i] - rho[i]); uhi = std::max(uhi, pu[i] + rho[i]);
     vlo = std::min(vlo, pv[i] - rho[i]); vhi = std::max(vhi, pv[i] + rho[i]);
-    rhoSum += rho[i];
+    // lightRhoSum's shape (rfx_light_grid.h): a block's sum joins the total when the slots leave the block (an empty block adds 0)
+    if (slots[i] / LIGHT_GRID_SUM_BLOCK != block) { rhoSum += blockSum; blockSum = 0.0; block = slots[i] / LIGHT_GRID_SUM_BLOCK; }
+    blockSum += rho[i];
   }
-  if (n == 0 || !(uhi > ulo) || !(vhi > vlo)) return false;
-  const double cell = std::max(std::max(uhi - ulo, vhi - vlo) / 256.0, 0.75 * rhoSum / (double)n);
-  const int nx = (int)std::min(256.0, ceil((uhi - ulo) / cell)) + 1, ny = (int)std::min(256.0, ceil((vhi - vlo) / cell)) + 1;
-  const double inv = 1.0 / cell;
+  rhoSum += blockSum;
+  LightGridDims d;
+  if (!lightGridDims(ulo, uhi, vlo, vhi, rhoSum, n, d)) return false;
+  const int nx = d.nx, ny = d.ny;
   std::vector<uint32_t> count((size_t)nx * ny + 1, 0);
-  auto cellsOf = [&](size_t i, int & x0, int & x1, int & y0, int & y1)
-  {
-    x0 = std::max(0, (int)floor((pu[i] - rho[i] - ulo) * inv)); x1 = std::min(nx - 1, (int)floor((pu[i] + rho[i] - ulo) * inv));
-    y0 = std::max(0, (int)floor((pv[i] - rho[i] - vlo) * inv)); y1 = std::min(ny - 1, (int)floor((pv[i] + rho[i] - vlo) * inv));
-  };
-  auto touches = [&](size_t i, int x, int y)     // the disc against the cell's square
-  {
-    const double cx0 = ulo + x * cell, cy0 = vlo + y * cell;
-    const double dx = std::max(std::max(cx0 - pu[i], pu[i] - (cx0 + cell)), 0.0), dy = std::max(std::max(cy0 - pv[i], pv[i] - (cy0 + cell)), 0.0);
-    return dx * dx + dy * dy <= rho[i] * rho[i];
-  };
   for (int pass = 0; pass < 2; pass++)
   {
     if (pass == 1)
@@ -322,10 +286,10 @@ bool buildLightGrid(const Light & L, const std::vector<const HostObj *> & sph, c
     for (size_t i = 0; i < n; i++)
     {
       int x0, x1, y0, y1;
-      cellsOf(i, x0, x1, y0, y1);
+      lightCellsOf(d, pu[i], pv[i], rho[i], x0, x1, y0, y1);
       for (int y = y0; y <= y1; y++)
         for (int x = x0; x <= x1; x++)
-          if (touches(i, x, y))
+          if (lightTouches(d, pu[i], pv[i], rho[i], x, y))
           {
             const size_t c = (size_t)y * nx + x;
             if (pass == 0) count[c]++;
@@ -340,17 +304,15 @@ bool buildLightGrid(const Light & L, const std::vector<const HostObj *> & sph, c
     }
   }
   LightGrid & g = out.g;
-  for (int k = 0; k < 3; k++) { g.u[k] = (float)(u[k] * inv); g.v[k] = (float)(v[k] * inv); }
-  g.u[3] = (float)(-ulo * inv); g.v[3] = (float)(-vlo * inv);
-  g.nx = nx; g.ny = ny;
+  lightGridHeader(f, d, g);
   g.cellStart = nullptr; g.itemSphere = nullptr; g.itemIndex = nullptr;
   return true;
 }
 
 // The grids of every far light over the drop-point box (blo, bhi), concatenated into img.  prims: the sphere hierarchy's, in the order
-// its build left them (its slot order).
+// its build left them (its slot order), slots their leaf slots.
 void fillLightGrids(const std::vector<Light> & lights, const std::vector<const HostObj *> & sph, const std::vector<BvhPrim> & prims,
-                    const double blo[3], const double bhi[3], SceneImage & img)
+                    const std::vector<int> & slots, const double blo[3], const double bhi[3], SceneImage & img)
 {
   img.grids.assign(lights.size(), LightGrid());
   img.gridCellOff.assign(lights.size(), 0);
@@ -360,7 +322,7 @@ void fillLightGrids(const std::vector<Light> & lights, const std::vector<const H
   for (size_t li = 0; li < lights.size(); li++)
   {
     LightGridHost lg;
-    if (!buildLightGrid(lights[li], sph, prims, blo, bhi, lg)) continue;
+    if (!buildLightGrid(lights[li], sph, prims, slots, blo, bhi, lg)) continue;
     img.grids[li] = lg.g;
     img.gridCellOff[li] = img.gridCells.size(); img.gridItemOff[li] = img.gridSpheres.size();
     img.gridCells.insert(img.gridCells.end(), lg.cellStart.begin(), lg.cellStart.end());
@@ -369,6 +331,15 @@ void fillLightGrids(const std::vector<Light> & lights, const std::vector<const H
     img.lightGridsBuilt++;
   }
   if (!img.lightGridsBuilt) img.grids.clear();
+}
+
+// the used leaf slots of a packed sphere hierarchy, ascending: the slots of its prims in the order its build left them
+std::vector<int> usedSlots(const PackedBvh & bvh)
+{
+  std::vector<int> slots;
+  for (size_t j = 0; j < bvh.prims.size(); j++)
+    if (bvh.prims[j] >= 0) slots.push_back((int)j);
+  return slots;
 }
 
 // The grids of every far light.  B: the box of every drop point — all objects (with planes present no grid is built: a drop point on
@@ -395,7 +366,7 @@ void buildLightGrids(const std::vector<Light> & lights, const std::vector<const 
     padDropBox(b);
     for (int k = 0; k < 3; k++) { blo[k] = b[k]; bhi[k] = b[3 + k]; img.gridBox[k] = b[k]; img.gridBox[3 + k] = b[3 + k]; }
   }
-  fillLightGrids(lights, sph, prims, blo, bhi, img);
+  fillLightGrids(lights, sph, prims, usedSlots(img.sphBvh), blo, bhi, img);
 }
 
 } // namespace
@@ -421,7 +392,7 @@ void sphereDropBox(const HostScene & s, const SceneImage & img, double b[6])
   }
 }
 
-void rebuildLightGrids(const HostScene & s, SceneImage & img)
+void rebuildLightGrids(const HostScene & s, const SceneImage & img, SceneImage & out)
 {
   std::vector<const HostObj *> sph(img.sphObj.size());
   for (size_t i = 0; i < sph.size(); i++) sph[i] = &s.objs[img.sphObj[i]];
@@ -437,7 +408,7 @@ void rebuildLightGrids(const HostScene & s, SceneImage & img)
       prims.push_back(q);
     }
   const double blo[3] = { img.gridBox[0], img.gridBox[1], img.gridBox[2] }, bhi[3] = { img.gridBox[3], img.gridBox[4], img.gridBox[5] };
-  fillLightGrids(s.lights, sph, prims, blo, bhi, img);
+  fillLightGrids(s.lights, sph, prims, usedSlots(img.sphBvh), blo, bhi, out);
 }
 
 void refreshMeshes(HostScene & s)
@@ -833,10 +804,12 @@ int rfx_selftest_light_grid_host(const float light[4], int n_spheres, const floa
   memset(&L, 0, sizeof(L));
   L.ox = light[0]; L.oy = light[1]; L.oz = light[2]; L.radius = light[3];
   const double blo[3] = { box[0], box[1], box[2] }, bhi[3] = { box[3], box[4], box[5] };
+  std::vector<int> slots((size_t)n_spheres);
+  for (int i = 0; i < n_spheres; i++) slots[i] = i;                // (one leaf slot per sphere, in order)
   LightGridHost lg;
   counts[0] = counts[1] = 0;
   dims[0] = dims[1] = 0;
-  if (!buildLightGrid(L, sph, prims, blo, bhi, lg)) return RFX_OK;      // no grid for this light: dims stay 0
+  if (!buildLightGrid(L, sph, prims, slots, blo, bhi, lg)) return RFX_OK;      // no grid for this light: dims stay 0
   memcpy(uv, lg.g.u, 16); memcpy(uv + 4, lg.g.v, 16);
   dims[0] = lg.g.nx; dims[1] = lg.g.ny;
   counts[0] = lg.cellStart.size(); counts[1] = lg.index.size();

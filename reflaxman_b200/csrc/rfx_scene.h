@@ -5,7 +5,7 @@
 // once per object/frame; it is compiled with -ffp-contract=off so every operation is the same IEEE binary32 operation the reference's
 // build performs (reference Triangle.cpp:11-21,110-120; Matrix33.cpp:10-15,49-79; Skybox.cpp:21-37; Material.cpp:8-14; Render.cpp:148-150).
 #pragma once
-#include "rfx_sphere_box.h"
+#include "rfx_light_grid.h"
 
 #include <float.h>
 #include <math.h>
@@ -45,6 +45,7 @@ struct HostScene
 {
   float ambient[3] = { 0, 0, 0 }, ambientPower = 0, env[3] = { 0, 0, 0 };
   std::vector<Light> lights;
+  std::vector<float> lightPower;            // per light: its power as given (the record keeps it clamped; env adds it unclamped, Scene.cpp:54)
   std::vector<HostObj> objs;
   std::vector<HostMesh> meshes;
   std::vector<HostTex> tex;                 // uploaded before the image is built: TexRef and SmallScene carry their device pointers
@@ -78,7 +79,8 @@ struct SceneImage
   std::vector<float4> gridSpheres;          // every grid's items, light after light
   std::vector<int> gridIndex;
   std::vector<size_t> gridCellOff, gridItemOff;   // per light: where its cells / items start in the arrays above
-  int lightGridsBuilt = 0;
+  int lightGridsBuilt = 0;                  // lights the flatten built a grid for.  Not changed by later updates: > 0 means the device has a
+                                            // header per light and grid regions, and gridBox, dropTris, dropSpheres stay tracked
   SmallScene small;                         // constant-bank form of the same scene (rfx_trace_small.cu), when smallOk
   bool smallOk = false;
   float reach[6] = { 0, 0, 0, 0, 0, 0 };   // box of ray origins the hierarchies' margins were sized for (lo xyz, hi xyz)
@@ -118,10 +120,11 @@ void padDropBox(double b[6]);
 // the un-padded drop-point box (lo xyz, hi xyz) of the spheres of img, from their records in s
 void sphereDropBox(const HostScene & s, const SceneImage & img, double b[6]);
 
-// Rebuilds the light grids of img for the current spheres of s over the drop-point box they were built for (img.gridBox), with the
-// margins of the hierarchy's last flatten (img.sphR) and its prims in slot order, as buildSceneImage would build them for that box:
-// after rfx_update_spheres moved spheres within gridBox.  The device pointers of img.grids are left null.
-void rebuildLightGrids(const HostScene & s, SceneImage & img);
+// Builds into out's grid fields (grids, gridCells, gridSpheres, gridIndex, their offsets, lightGridsBuilt) the light grids of the
+// current lights and spheres of s over the drop-point box img's were built for (img.gridBox), with the margins of img's flatten
+// (img.sphR) and its prims in slot order, as buildSceneImage would build them for that box: the host reference of the grids
+// rfx_update_spheres and rfx_update_lights build on the device (rfx_selftest_light_grids).  The device pointers are left null.
+void rebuildLightGrids(const HostScene & s, const SceneImage & img, SceneImage & out);
 
 // recompute the host records (triVerts, tri.v0/ax/n) of the stale meshes' triangles from their current vertices
 void refreshMeshes(HostScene & s);

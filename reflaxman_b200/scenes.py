@@ -222,6 +222,37 @@ def with_spheres(scene, objects, spheres):
     return dict(scene, objects=objs)
 
 
+def with_lights(scene, lights, records):
+    """The same scene with the lights whose index is in ``lights`` replaced by the matching rows (origin[3], radius, rgb[3], power) of
+    ``records`` (a repeated index takes its last row): what rfx_update_lights(lights, records) describes."""
+    new = {int(i): tuple(float(x) for x in np.asarray(row, np.float32))
+           for i, row in zip(np.asarray(lights).reshape(-1), np.asarray(records, np.float32).reshape(-1, 8))}
+    out = list(scene["lights"])
+    for i, r in new.items():
+        if not 0 <= i < len(out):
+            raise ValueError("light %d is not a light of the scene" % i)
+        out[i] = ((r[0], r[1], r[2]), r[3], (r[4], r[5], r[6]), r[7])
+    return dict(scene, lights=out)
+
+
+def sun_orbit(scene, t, speed=1.0, swing=0.5):
+    """The scene's first light as a sun crossing the sky at time ``t``: returns (lights int32 [1], records float32 [1, 8]) for
+    :meth:`capi.Context.update_lights`.  The light keeps its distance from the origin, radius, colour and power; its azimuth about the
+    vertical axis turns by speed * t and its elevation swings by ``swing`` * sin(t / 2) around the loaded one (kept between 0.1 and 1.4
+    radians), so a light that is far from the scene stays far.  At t = 0 the record is the loaded light bit for bit."""
+    (o, r, c, p) = scene["lights"][0]
+    o64 = np.asarray(o, np.float32).astype(np.float64)
+    if t != 0.0:
+        dist = float(np.linalg.norm(o64))
+        el = math.asin(max(-1.0, min(1.0, o64[1] / dist)))
+        az = math.atan2(o64[2], o64[0])
+        el = min(1.4, max(0.1, el + swing * math.sin(0.5 * t)))
+        az += speed * t
+        o64 = np.array([dist * math.cos(el) * math.cos(az), dist * math.sin(el), dist * math.cos(el) * math.sin(az)])
+    rec = np.concatenate([o64, [r], np.asarray(c, np.float64), [p]]).astype(np.float32)
+    return np.zeros(1, np.int32), rec.reshape(1, 8)
+
+
 def expand_meshes(scene):
     """The same scene with every "mesh" object replaced by its triangles, in order (untextured "tri" objects)."""
     objs = []
