@@ -154,6 +154,13 @@ RFX_API int rfx_selftest_rng(rfx_ctx * ctx, uint64_t out[2]);
  * dropped because it did not fit its item region (option "light_grid_items") is not a difference.  All 0 when the last flatten built no
  * light grid; RFX_ERR_ARG when the scene changed since its last flatten. */
 RFX_API int rfx_selftest_light_grids(rfx_ctx * ctx, uint64_t out[3]);
+/* diagnostic: the screen grid of the first query (option "eye_grid") that the last blob render used — built on the GPU for every new
+ * camera, image size and sphere update (option "eye_grid_device") — against the host's binning (rfx_selftest_eye_grid_host) for that
+ * render's camera and the current spheres.  Synchronises.  out[0] = differences: dims, each cell offset, each item (sphere index or
+ * record), or a grid on one side only, 0 when identical; out[1] = items on the device (0: no grid, or its build was dropped for want of
+ * room — not a difference); out[2] = items on the host; out[3] = device builds dropped since the context was created.  RFX_ERR_ARG when
+ * the scene changed since its last flatten or no blob frame has been rendered since. */
+RFX_API int rfx_selftest_eye_grid(rfx_ctx * ctx, uint64_t out[4]);
 /* diagnostic: every path of a frame starts at the eye (Render.cpp:154-156), so the fast kernel lets a warp's first pass over the
  * objects skip those whose screen bounds miss its 4x8 pixel tile.  This returns the bounds the library derives for the current
  * scene (constant-bank scenes only), camera and image size: out[4*i .. 4*i+3] = x0, x1, y0, y1 (inclusive; x0 > x1 = no pixel) of
@@ -257,14 +264,18 @@ RFX_API int rfx_enable_profiling(rfx_ctx * ctx, int on);
  * constant-bank fast kernel records the tiles' cost classes on every k-th launch over the same grid and replays the last recording
  * in between (default 8).  "light_grids": scenes with a sphere hierarchy answer the shadow queries of far lights from a 2-D grid of
  * candidate spheres across the light's direction instead of walking the hierarchy (default 1).  "eye_grid": the same scenes take the
- * candidates of a path's first query (origin = eye) from a screen grid binned per camera out of the spheres' primary-ray bounds
+ * candidates of a path's first query (origin = eye) from a screen grid built per camera out of the spheres' primary-ray bounds
  * (default 1).  Both grids list spheres only: triangles are tested after them, through their own hierarchy when the scene has one
  * (rfx_set_bvh_mode).  Scenes with a plane get no light grids (a shadow ray can start anywhere on the plane); their eye grid is built.
  * "light_grid_items" (test hook): at most this many items per light grid (0 = no limit, the default).  Each light has fixed device
  * regions for its grid, with room for twice the items of the flatten's largest grid; a grid built on the GPU (rfx_update_lights,
  * rfx_update_spheres) that does not fit is dropped — its shadow queries walk the hierarchy, and stats.light_grids counts it out — and
- * the next synchronising call (rfx_get_stats, rfx_synchronize) grows the regions for the later builds.  Frames are bit-identical under
- * every setting. */
+ * the next synchronising call (rfx_get_stats, rfx_synchronize) grows the regions for the later builds.  "eye_grid_device": the eye grid
+ * is built on the GPU, queued on the render stream without a synchronisation, for every new camera, image size and sphere update (1, the
+ * default), or binned on the host and uploaded (0).  "eye_grid_items" (test hook): at most this many items in an eye grid built on the
+ * GPU (0 = no limit, the default).  Its item region is sized at the first build; a build that does not fit is dropped — that frame's
+ * first queries walk the hierarchy — and the next synchronising call grows the region, so the next render builds the grid again.
+ * Frames are bit-identical under every setting. */
 RFX_API int rfx_set_option(rfx_ctx * ctx, const char * name, int64_t value);
 /* kernel selection: 0 = automatic (constant-bank kernels when the scene fits, the blob kernels otherwise),
  * 1 = constant-bank kernel if it fits, 2 = always the blob kernels (tile / wavefront kernels for row-aligned slices, the general

@@ -10,10 +10,10 @@ import subprocess
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-SRC = [os.path.join(HERE, "csrc", f) for f in ("rfx_kernels.cu", "rfx_trace_small.cu", "rfx_trace_blob.cu", "rfx_mesh.cu", "rfx_light_grid.cu",
+SRC = [os.path.join(HERE, "csrc", f) for f in ("rfx_kernels.cu", "rfx_trace_small.cu", "rfx_trace_blob.cu", "rfx_mesh.cu", "rfx_light_grid.cu", "rfx_eye_grid.cu",
                                                "rfx_capi.cu", "rfx_scene.cpp")]
 HDR = [os.path.join(HERE, "csrc", f) for f in ("rfx_kernels.h", "rfx_types.h", "rfx_device.cuh", "rfx_scene.h", "rfx_tri_setup.h",
-                                               "rfx_sphere_box.h", "rfx_light_grid.h")] + [os.path.join(HERE, "..", "include", "reflax_c.h")]
+                                               "rfx_sphere_box.h", "rfx_light_grid.h", "rfx_eye_grid.h")] + [os.path.join(HERE, "..", "include", "reflax_c.h")]
 OUT = os.path.join(HERE, "libreflax_b200.so")
 
 NVCC_FLAGS = [

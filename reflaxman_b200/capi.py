@@ -58,6 +58,7 @@ SYMBOLS = [
     ("rfx_skip_samples", C.c_int, [C.c_void_p, C.c_uint64]),
     ("rfx_selftest_rng", C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
     ("rfx_selftest_light_grids", C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
+    ("rfx_selftest_eye_grid", C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
     ("rfx_selftest_primary_bounds", C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     ("rfx_selftest_primary_bounds_host", C.c_int, [_fp, C.c_uint32, C.c_uint32, C.c_int, _fp, C.c_int, _fp, C.POINTER(C.c_int32)]),
     ("rfx_selftest_light_grid_host", C.c_int, [_fp, C.c_int, _fp, _fp, C.c_float, _fp, C.POINTER(C.c_int32), _u32p, C.c_uint64,
@@ -341,6 +342,13 @@ class Context:
         out = (C.c_uint64 * 3)()
         self._ck(self.L.rfx_selftest_light_grids(self.h, out), "rfx_selftest_light_grids")
         return int(out[0]), int(out[1]), int(out[2])
+
+    def eye_grid_selftest(self):
+        """rfx_selftest_eye_grid: (differences between the eye grid the last blob render used and the host's binning, items on the
+        device (0: no grid or dropped), items on the host, device builds dropped since creation)"""
+        out = (C.c_uint64 * 4)()
+        self._ck(self.L.rfx_selftest_eye_grid(self.h, out), "rfx_selftest_eye_grid")
+        return int(out[0]), int(out[1]), int(out[2]), int(out[3])
 
     def add_texture(self, argb):
         if argb is None:

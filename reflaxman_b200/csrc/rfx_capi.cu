@@ -93,15 +93,26 @@ struct rfx_ctx
   DevArray<unsigned long long> dLgRed;
   DevArray<LightGridDims> dLgDims;
   // candidate spheres of the first query of a path per 32x32-pixel screen cell (EyeGrid, rfx_kernels.h), rebuilt when the camera,
-  // the image size or the scene changes
-  DevArray<uint32_t> dEyeCells;
+  // the image size, the scene or the spheres change: on the device (rfx_eye_grid.cu) into a fixed item region of eyeItemAlloc items
+  DevArray<uint32_t> dEyeCells;             // [nx * ny + 2]
   DevArray<float4> dEyeSpheres;
   DevArray<int> dEyeIndex;
+  size_t eyeItemAlloc = 0;                  // items of the region: sized at the first build, grown at a synchronising call after a drop
+  int64_t eyeItemLimit = 0;                 // rfx_set_option "eye_grid_items" (test hook; 0: none)
+  DevArray<uint32_t> dEyeFlags;             // [2]: the largest item count of a dropped build, builds dropped since creation
+  DevArray<int2> dEgSpan;                   // the builder's scratch (EyeGridBuild)
+  DevArray<uint32_t> dEgRows;
   EyeGrid eyeGrid = { nullptr, nullptr, nullptr, 0, 0, 0 };
-  uint32_t eyeKey[17] = { 0 }; uint64_t eyeSceneKey = 0; bool eyeValid = false;   // camera (eye, view, rz, wHalf, hHalf as bits) + W, H
+  uint32_t eyeKey[17] = { 0 }; uint64_t eyeSceneKey = 0, eyeSphereKey = 0; bool eyeValid = false;   // camera (eye, view, rz, wHalf, hHalf as bits) + W, H
   uint64_t sceneUploads = 0;                // bumped by uploadScene
+  uint64_t sphereUpdates = 0;               // bumped by rfx_update_spheres when it updates the device scene
   bool eyeGridOn = true;                    // rfx_set_option "eye_grid"
+  bool eyeGridDevice = true;                // rfx_set_option "eye_grid_device": 0 = binned on the host and uploaded
   uint64_t eyeGridBuilds = 0;
+  // the last blob render (rfx_selftest_eye_grid): its camera, and the grid it used
+  bool eyeRendered = false;
+  FrameParams eyeFp;
+  EyeGrid eyeUsed = { nullptr, nullptr, nullptr, 0, 0, 0 };
   DevArray<float4> dTriNodes;               // hierarchy over the triangles: leaf slots, then pair nodes
   DevArray<int> dTriPrims;
   DevArray<int> dTriAlways;                 // plane scenes: triangles tested after the triangle walk (SceneHeader::triAlways); with meshes
@@ -215,6 +226,7 @@ int uploadScene(rfx_ctx * ctx, cudaStream_t st)
   if (!ctx->sceneDirty) return RFX_OK;
   ctx->sceneUploads++;
   ctx->eyeValid = false;
+  ctx->eyeRendered = false;
 
   for (HostTex & t : ctx->scene.tex)
     if (!t.uploaded)
@@ -392,6 +404,8 @@ int skipSamples(rfx_ctx * ctx, uint64_t n, cudaStream_t st)
   return RFX_OK;
 }
 
+// The eye grid of the frame fp (EyeGrid), queued on st behind the kernels of the previous frame that still read the old one.  Cached
+// per camera, image size, scene upload and sphere update.
 int buildEyeGrid(rfx_ctx * ctx, const FrameParams & fp, cudaStream_t st)
 {
   ctx->eyeGrid.cellStart = nullptr;
@@ -400,25 +414,80 @@ int buildEyeGrid(rfx_ctx * ctx, const FrameParams & fp, cudaStream_t st)
   memcpy(key, fp.eye, 12); memcpy(key + 3, fp.view, 36);
   memcpy(key + 12, &fp.rz, 4); memcpy(key + 13, &fp.wHalf, 4); memcpy(key + 14, &fp.hHalf, 4);
   key[15] = fp.W; key[16] = fp.H;
-  if (ctx->eyeValid && ctx->eyeSceneKey == ctx->sceneUploads && !memcmp(key, ctx->eyeKey, sizeof(key)))
+  if (ctx->eyeValid && ctx->eyeSceneKey == ctx->sceneUploads && ctx->eyeSphereKey == ctx->sphereUpdates && !memcmp(key, ctx->eyeKey, sizeof(key)))
   {
     ctx->eyeGrid.cellStart = ctx->dEyeCells.p;
     return RFX_OK;
   }
   ctx->eyeValid = false;
-  int nx = 0, ny = 0;
-  std::vector<uint32_t> cells;
-  std::vector<float4> items;
-  std::vector<int> index;
-  if (!binEyeGrid(fp, ctx->image.spheres, nx, ny, cells, items, index)) return RFX_OK;
-  // the copies are ordered on the stream behind the kernels of the previous frame that still read the old grid
-  int rc;
-  if ((rc = upload(ctx, ctx->dEyeCells, cells, st)) != RFX_OK || (rc = upload(ctx, ctx->dEyeSpheres, items, st)) != RFX_OK ||
-      (rc = upload(ctx, ctx->dEyeIndex, index, st)) != RFX_OK) return rc;
+  int nx = 0, ny = 0, rc;
+  if (ctx->eyeGridDevice)
+  {
+    const PrimaryCamera cam = makePrimaryCamera(fp);
+    if (!eyeGridDims(cam, fp.W, fp.H, nx, ny)) return RFX_OK;
+    const size_t nS = ctx->image.spheres.size(), nCells = (size_t)nx * ny, words = (nS + 31) / 32;
+    if (!ctx->eyeItemAlloc) ctx->eyeItemAlloc = std::max<size_t>(8 * nS + 2 * nCells, 1 << 16);   // grown after a build that did not fit
+    if ((rc = ensure(ctx, ctx->dEyeCells, nCells + 2)) != RFX_OK || (rc = ensure(ctx, ctx->dEyeSpheres, ctx->eyeItemAlloc)) != RFX_OK ||
+        (rc = ensure(ctx, ctx->dEyeIndex, ctx->eyeItemAlloc)) != RFX_OK || (rc = ensure(ctx, ctx->dEgSpan, std::max<size_t>(nS, 1))) != RFX_OK ||
+        (rc = ensure(ctx, ctx->dEgRows, std::max<size_t>(ny * words, 1))) != RFX_OK) return rc;
+    if (!ctx->dEyeFlags.p)
+    {
+      CK(ctx->dEyeFlags.alloc(2));
+      CK(cudaMemsetAsync(ctx->dEyeFlags.p, 0, 2 * sizeof(uint32_t), st));
+    }
+    EyeGridBuild b;
+    memset(&b, 0, sizeof(b));
+    b.cam = cam; b.W = fp.W; b.H = fp.H; b.nx = nx; b.ny = ny;
+    b.spheres = reinterpret_cast<const float4 *>(ctx->dBlob.p + reinterpret_cast<const SceneHeader *>(ctx->image.blob.data())->offSpheres);
+    b.nSpheres = (int)nS;
+    b.cells = ctx->dEyeCells.p; b.itemSphere = ctx->dEyeSpheres.p; b.itemIndex = ctx->dEyeIndex.p;
+    size_t cap = std::min(ctx->dEyeSpheres.cap, ctx->dEyeIndex.cap);
+    if (ctx->eyeItemLimit > 0) cap = std::min<size_t>(cap, (size_t)ctx->eyeItemLimit);
+    b.itemCap = (uint32_t)std::min<size_t>(cap, UINT32_MAX);
+    b.flags = ctx->dEyeFlags.p;
+    b.xSpan = ctx->dEgSpan.p; b.rowMask = ctx->dEgRows.p; b.maskWords = (int)words;
+    const int nl = launchEyeGridBuild(b, st);
+    if (!nl) return fail(ctx, RFX_ERR_CUDA, "buildEyeGrid: the row masks could not be cleared");
+    ctx->stats.kernel_launches += nl;
+    CK(cudaGetLastError());
+  }
+  else
+  {
+    std::vector<uint32_t> cells;
+    std::vector<float4> items;
+    std::vector<int> index;
+    if (!binEyeGrid(fp, ctx->image.spheres, nx, ny, cells, items, index)) return RFX_OK;
+    cells.push_back(0u);                      // the drop word: the whole grid is uploaded
+    if ((rc = upload(ctx, ctx->dEyeCells, cells, st)) != RFX_OK || (rc = upload(ctx, ctx->dEyeSpheres, items, st)) != RFX_OK ||
+        (rc = upload(ctx, ctx->dEyeIndex, index, st)) != RFX_OK) return rc;
+  }
   ctx->eyeGrid.cellStart = ctx->dEyeCells.p; ctx->eyeGrid.itemSphere = ctx->dEyeSpheres.p; ctx->eyeGrid.itemIndex = ctx->dEyeIndex.p;
   ctx->eyeGrid.nx = nx; ctx->eyeGrid.ny = ny; ctx->eyeGrid.shift = EYE_GRID_SHIFT;
-  memcpy(ctx->eyeKey, key, sizeof(key)); ctx->eyeSceneKey = ctx->sceneUploads; ctx->eyeValid = true;
+  memcpy(ctx->eyeKey, key, sizeof(key)); ctx->eyeSceneKey = ctx->sceneUploads; ctx->eyeSphereKey = ctx->sphereUpdates; ctx->eyeValid = true;
   ctx->eyeGridBuilds++;
+  return RFX_OK;
+}
+
+// At a synchronising call: after a device build that did not fit its item region (EyeGridBuild::flags), grow the region and forget the
+// cached grid, so the next render builds it again.
+int growEyeGrid(rfx_ctx * ctx)
+{
+  if (!ctx->dEyeFlags.p) return RFX_OK;
+  uint32_t need = 0;
+  CK(cudaMemcpy(&need, ctx->dEyeFlags.p, sizeof(need), cudaMemcpyDeviceToHost));
+  if (!need) return RFX_OK;
+  ctx->eyeValid = false;
+  if (need > std::min(ctx->dEyeSpheres.cap, ctx->dEyeIndex.cap))
+  {
+    const size_t alloc = (size_t)need + need / 2;
+    CK(cudaFree(ctx->dEyeSpheres.p)); ctx->dEyeSpheres.p = nullptr; ctx->dEyeSpheres.cap = 0;
+    CK(cudaFree(ctx->dEyeIndex.p)); ctx->dEyeIndex.p = nullptr; ctx->dEyeIndex.cap = 0;
+    CK(ctx->dEyeSpheres.alloc(alloc));
+    CK(ctx->dEyeIndex.alloc(alloc));
+    ctx->eyeItemAlloc = alloc;
+    ctx->eyeRendered = false;                 // (the grid of the last render lived in the old region)
+  }
+  CK(cudaMemset(ctx->dEyeFlags.p, 0, sizeof(uint32_t)));
   return RFX_OK;
 }
 
@@ -555,6 +624,7 @@ int renderRange(rfx_ctx * ctx, uint64_t p0, uint64_t p1, uint32_t * argbOut, boo
         }
         if ((rc = buildEyeGrid(ctx, w.fp, st)) != RFX_OK) return rc;
         w.eyeGrid = ctx->eyeGrid;
+        ctx->eyeRendered = true; ctx->eyeFp = w.fp; ctx->eyeUsed = ctx->eyeGrid;
         int nl = ctx->forcePath == 3 ? 0 : launchTraceBlobFast(w, st, wavePixels ? ctx->dQueue.p : nullptr, ctx->dQueueCtl.p, (uint32_t)ctx->prop.multiProcessorCount * 8u,
                                                                ctx->blobWavefront, ctx->blobSmemBvh ? ctx->image.bvhFloat4 : 0u);
         if (nl) ctx->stats.launches_blob_fast += nl;
@@ -1090,8 +1160,8 @@ int rfx_update_spheres(rfx_ctx * ctx, uint32_t n, const int32_t * objects, const
     for (size_t li = 0; li < s.lights.size(); li++)
       if (ctx->lightGrid[li] && (rc = updateLightGrid(ctx, li, st)) != RFX_OK) return rc;
   }
-  // the eye grid is binned again from img.spheres at the next render
-  ctx->eyeValid = false;
+  // the eye grid is built again at the next render, from the blob's spheres (img.spheres on the host path)
+  ctx->sphereUpdates++;
   return 1;
 }
 
@@ -1240,6 +1310,47 @@ int rfx_selftest_light_grids(rfx_ctx * ctx, uint64_t out[3])
     if (memcmp(cells.data(), &ref->gridCells[off], nCells * sizeof(uint32_t)) ||
         (nItems && (memcmp(sp.data(), &ref->gridSpheres[io], nItems * sizeof(float4)) || memcmp(ix.data(), &ref->gridIndex[io], nItems * sizeof(int)))))
       out[0]++;
+  }
+  return RFX_OK;
+}
+
+int rfx_selftest_eye_grid(rfx_ctx * ctx, uint64_t out[4])
+{
+  if (!ctx || !out) return RFX_ERR_ARG;
+  if (ctx->sceneDirty) return fail(ctx, RFX_ERR_ARG, "rfx_selftest_eye_grid: the scene changed since its last flatten");
+  if (!ctx->eyeRendered) return fail(ctx, RFX_ERR_ARG, "rfx_selftest_eye_grid: no blob frame has been rendered since the last flatten");
+  CK(cudaSetDevice(ctx->device));
+  CK(cudaDeviceSynchronize());
+  out[0] = out[1] = out[2] = out[3] = 0;
+  uint32_t flags[2] = { 0, 0 };
+  if (ctx->dEyeFlags.p) CK(cudaMemcpy(flags, ctx->dEyeFlags.p, sizeof(flags), cudaMemcpyDeviceToHost));
+  out[3] = flags[1];
+  // the host's binning for the camera of that render and the current spheres (none where buildEyeGrid builds none)
+  int nx = 0, ny = 0;
+  std::vector<uint32_t> cells, dev;
+  std::vector<float4> items;
+  std::vector<int> index;
+  const bool host = ctx->eyeGridOn && ctx->image.bvhDepth > 0 && binEyeGrid(ctx->eyeFp, ctx->image.spheres, nx, ny, cells, items, index);
+  const EyeGrid & g = ctx->eyeUsed;
+  if (host) out[2] = cells.back();
+  if ((g.cellStart != nullptr) != host) { out[0]++; return RFX_OK; }
+  if (!host) return RFX_OK;
+  if (g.nx != nx || g.ny != ny || g.shift != EYE_GRID_SHIFT) { out[0]++; return RFX_OK; }
+  dev.resize(cells.size() + 1);
+  CK(cudaMemcpy(dev.data(), g.cellStart, dev.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+  if (dev.back() != 0u) return RFX_OK;                          // dropped for want of room: the first queries walked the hierarchy
+  const uint32_t nDev = dev[cells.size() - 1];
+  out[1] = nDev;
+  for (size_t c = 0; c < cells.size(); c++) out[0] += dev[c] != cells[c];
+  const size_t n = std::min<size_t>(nDev, cells.back());
+  out[0] += std::max<size_t>(nDev, cells.back()) - n;            // items on one side only
+  if (n)
+  {
+    std::vector<float4> sp(n);
+    std::vector<int> ix(n);
+    CK(cudaMemcpy(sp.data(), g.itemSphere, n * sizeof(float4), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(ix.data(), g.itemIndex, n * sizeof(int), cudaMemcpyDeviceToHost));
+    for (size_t k = 0; k < n; k++) out[0] += ix[k] != index[k] || memcmp(&sp[k], &items[k], sizeof(float4)) != 0;
   }
   return RFX_OK;
 }
@@ -1746,7 +1857,7 @@ int rfx_synchronize(rfx_ctx * ctx)
   if (ctx->lastStream) CK(cudaStreamSynchronize(ctx->lastStream));
   CK(cudaStreamSynchronize(ctx->stream));
   int rc;
-  if ((rc = growLightGrids(ctx)) != RFX_OK) return rc;
+  if ((rc = growLightGrids(ctx)) != RFX_OK || (rc = growEyeGrid(ctx)) != RFX_OK) return rc;
   return checkStatus(ctx);
 }
 
@@ -1772,7 +1883,8 @@ int rfx_get_stats(rfx_ctx * ctx, rfx_stats * out)
   }
   ctx->evUsed = 0;
   int rc;
-  if ((rc = countLightGrids(ctx, ctx->stats.light_grids)) != RFX_OK || (rc = growLightGrids(ctx)) != RFX_OK) return rc;
+  if ((rc = countLightGrids(ctx, ctx->stats.light_grids)) != RFX_OK || (rc = growLightGrids(ctx)) != RFX_OK ||
+      (rc = growEyeGrid(ctx)) != RFX_OK) return rc;
   ctx->stats.bvh_triangles = ctx->image.triBvhTris;
   ctx->stats.bvh_spheres = ctx->image.bvhSpheres;
   *out = ctx->stats;
@@ -1840,6 +1952,20 @@ int rfx_set_option(rfx_ctx * ctx, const char * name, int64_t value)
   {
     if (value != 0 && value != 1) return fail(ctx, RFX_ERR_ARG, "rfx_set_option: eye_grid must be 0 or 1");
     ctx->eyeGridOn = value != 0;
+    ctx->eyeValid = false;
+    return RFX_OK;
+  }
+  if (!strcmp(name, "eye_grid_device"))
+  {
+    if (value != 0 && value != 1) return fail(ctx, RFX_ERR_ARG, "rfx_set_option: eye_grid_device must be 0 or 1");
+    ctx->eyeGridDevice = value != 0;
+    ctx->eyeValid = false;
+    return RFX_OK;
+  }
+  if (!strcmp(name, "eye_grid_items"))
+  {
+    if (value < 0) return fail(ctx, RFX_ERR_ARG, "rfx_set_option: eye_grid_items must be >= 0 (0: no limit)");
+    ctx->eyeItemLimit = value;
     ctx->eyeValid = false;
     return RFX_OK;
   }

@@ -6,6 +6,7 @@
 #include <type_traits>
 #include "rfx_types.h"
 #include "rfx_light_grid.h"
+#include "rfx_eye_grid.h"
 
 namespace rfx
 {
@@ -76,11 +77,14 @@ struct TileOrder
   uint32_t capacity = 0;
 };
 
-// Blob scenes: candidate spheres of the FIRST query of a path (origin = eye) per screen cell of 2^shift x 2^shift pixels, rebuilt by the
-// host for every camera from the primary-ray screen bounds of the spheres; cellStart == NULL: none (the query walks the hierarchy)
+// Blob scenes: candidate spheres of the FIRST query of a path (origin = eye) per screen cell of 2^shift x 2^shift pixels, built for every
+// camera, image size and sphere update from the primary-ray screen bounds of the spheres: on the device (rfx_eye_grid.cu), or binned by the
+// host (option "eye_grid_device" 0).  cellStart == NULL: none (the query walks the hierarchy).  The dims are the host's; whether the items
+// fitted their region is known on the device only, so the kernels read the drop word after the offsets: non-zero, the build was dropped
+// and the first queries walk the hierarchy.
 struct EyeGrid
 {
-  const uint32_t * cellStart;   // [nx * ny + 1]
+  const uint32_t * cellStart;   // [nx * ny + 2]: the cells' item offsets, the item total, the drop word
   const float4 * itemSphere;    // (cx, cy, cz, r^2) per (cell, sphere)
   const int * itemIndex;        // position in the sorted sphere array
   int nx, ny, shift;
@@ -140,10 +144,7 @@ struct PrimaryCull
   int4 rect[SMALL_MAX_SPHERES + SMALL_MAX_TRIS];   // x0, x1, y0, y1 (inclusive, frame pixels); x0 > x1: no pixel
 };
 PrimaryCull makePrimaryCull(const SmallScene & sc, const FrameParams & fp);
-// the same bounds one sphere at a time (blob scenes bin them into the screen grid of the first query, EyeGrid)
-struct PrimaryCamera { double c[3][3], eye[3], rz, wHalf, hHalf, W, H; bool ok; };   // ok = false: no bounds (camera not orthonormal): whole image
-PrimaryCamera makePrimaryCamera(const FrameParams & fp);
-int4 primarySphereBounds(const PrimaryCamera & cam, const float4 & sphere);   // x0, x1, y0, y1 inclusive; x0 > x1: no pixel
+// (the same bounds one sphere at a time, which blob scenes bin into the screen grid of the first query: primarySphereBounds, rfx_eye_grid.h)
 
 // rows a launch over `rows` whole rows enumerates: all of them, or in a split frame (fp.stripWorld > 0) the rows of this rank's
 // strips, full strips plus the (possibly shorter) last strip, rounded up to whole strips
@@ -257,6 +258,28 @@ struct LightGridBuild
   LightGridDims * dims;         // nx == 0: no grid (or dropped)
 };
 int launchLightGridBuild(const LightGridBuild & b, cudaStream_t st);   // returns the number of kernels launched
+
+// ---- the eye grid on the device (rfx_eye_grid.cu) -----------------------------------------------------------------------------------------
+// The EyeGrid of one camera built from the spheres of the blob: exactly what rfx_scene.cpp binEyeGrid bins for them, into fixed regions.  A
+// grid with more items than itemCap is dropped: its drop word is set, flags[0] raised to its item count and flags[1] counts the drop.
+struct EyeGridBuild
+{
+  PrimaryCamera cam;            // makePrimaryCamera of the frame (ok: eyeGridDims gave nx, ny)
+  uint32_t W, H;
+  int nx, ny;
+  const float4 * spheres;       // the blob's sorted sphere array
+  int nSpheres;
+  uint32_t * cells;             // [nx * ny + 2] (EyeGrid::cellStart)
+  float4 * itemSphere;          // [itemCap]
+  int * itemIndex;
+  uint32_t itemCap;
+  uint32_t * flags;             // [2]: the largest item count of a dropped build, builds dropped (read by the host at a synchronising call)
+  // scratch
+  int2 * xSpan;                 // per sphere: the columns of cells its rectangle touches (x0 > x1: none)
+  uint32_t * rowMask;           // [ny][maskWords]: bit i of row y set when sphere i touches row y
+  int maskWords;                // (nSpheres + 31) / 32
+};
+int launchEyeGridBuild(const EyeGridBuild & b, cudaStream_t st);      // returns the number of kernels launched
 
 // ---- K3: resolve (imagePixel + argb)---------------------------------------------------------------------------
 int launchResolve(const float * image, uint64_t nPixels, int additiveCounter, float * rgbfOut, uint32_t * argbOut, cudaStream_t st);

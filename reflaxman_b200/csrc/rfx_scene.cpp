@@ -710,24 +710,14 @@ bool binEyeGrid(const FrameParams & fp, const std::vector<float4> & spheres, int
                 std::vector<float4> & items, std::vector<int> & index)
 {
   const PrimaryCamera cam = makePrimaryCamera(fp);
-  if (!cam.ok || fp.W == 0 || fp.H == 0) return false;
-  const int shift = EYE_GRID_SHIFT;
-  nx = (int)((fp.W + 31u) >> shift); ny = (int)((fp.H + 31u) >> shift);
-  if ((uint64_t)nx * ny > (1u << 22)) return false;
-  struct Span { int x0, x1, y0, y1; };
-  std::vector<Span> spans(spheres.size());
+  if (!eyeGridDims(cam, fp.W, fp.H, nx, ny)) return false;
+  std::vector<int4> spans(spheres.size());
   cells.assign((size_t)nx * ny + 1, 0);
   for (size_t i = 0; i < spheres.size(); i++)
   {
-    const int4 r = primarySphereBounds(cam, spheres[i]);
-    Span sp = { 1, 0, 1, 0 };
-    if (r.x <= r.y && r.z <= r.w && r.y >= 0 && r.w >= 0 && r.x < (int)fp.W && r.z < (int)fp.H)
-    {
-      sp.x0 = std::max(r.x, 0) >> shift; sp.x1 = std::min(r.y, (int)fp.W - 1) >> shift;
-      sp.y0 = std::max(r.z, 0) >> shift; sp.y1 = std::min(r.w, (int)fp.H - 1) >> shift;
-      for (int y = sp.y0; y <= sp.y1; y++)
-        for (int x = sp.x0; x <= sp.x1; x++) cells[(size_t)y * nx + x]++;
-    }
+    const int4 sp = eyeCellSpan(primarySphereBounds(cam, spheres[i]), fp.W, fp.H);   // x0, x1, y0, y1
+    for (int y = sp.z; y <= sp.w; y++)
+      for (int x = sp.x; x <= sp.y; x++) cells[(size_t)y * nx + x]++;
     spans[i] = sp;
   }
   uint32_t run = 0;
@@ -738,9 +728,9 @@ bool binEyeGrid(const FrameParams & fp, const std::vector<float4> & spheres, int
   std::vector<uint32_t> fill(cells.begin(), cells.end() - 1);
   for (size_t i = 0; i < spheres.size(); i++)
   {
-    const Span & sp = spans[i];
-    for (int y = sp.y0; y <= sp.y1; y++)
-      for (int x = sp.x0; x <= sp.x1; x++)
+    const int4 & sp = spans[i];
+    for (int y = sp.z; y <= sp.w; y++)
+      for (int x = sp.x; x <= sp.y; x++)
       {
         const uint32_t k = fill[(size_t)y * nx + x]++;
         items[k] = spheres[i];

@@ -138,7 +138,6 @@ FrameParams frameFromCamera(const float eye[3], const float view[9], float fov, 
 
 // candidates of the first query of a path (EyeGrid, rfx_kernels.h): the primary-ray screen bounds of spheres[i] = (cx, cy, cz, r^2)
 // binned into 2^EYE_GRID_SHIFT-pixel square cells; false: no grid for this camera
-constexpr int EYE_GRID_SHIFT = 5;      // 32x32-pixel cells: a 4x8 tile of the kernels lies in one cell
 bool binEyeGrid(const FrameParams & fp, const std::vector<float4> & spheres, int & nx, int & ny, std::vector<uint32_t> & cells,
                 std::vector<float4> & items, std::vector<int> & index);
 

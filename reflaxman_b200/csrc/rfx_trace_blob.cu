@@ -721,6 +721,12 @@ __device__ __forceinline__ V3 tracePath(const BlobView & sc, int * __restrict__ 
   return pix;
 }
 
+// whether the first queries use the eye grid: there is one, and its build was not dropped (the drop word after its cell offsets)
+__device__ __forceinline__ bool eyeGridLive(const EyeGrid & g)
+{
+  return g.cellStart != nullptr && __ldg(g.cellStart + (size_t)g.nx * (uint32_t)g.ny + 1) == 0u;
+}
+
 // K2 for row-aligned slices of blob scenes.  MULTI = false: one sample per pixel, no jitter (the batch path of the bench).
 // MULTI = true: the same tiling for grid SSAA (Render.cpp:174-196: the thread walks its s*s samples in the reference's ssx, ssy
 // order so the sum is formed in the same order) and additive jitter / accumulation (Render.cpp:177-178, :196-207).
@@ -737,7 +743,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob
   const uint32_t y = y0 + blockIdx.y * BLOB_TILE_H + (lane / BLOB_TILE_W);
   const bool valid = x < fp.W && y < y1;
   uint32_t nBounces = 0, nShadow = 0, packed = 0, qOut = 0;
-  const EyeGrid * eg = (GRIDS && eyeGrid.cellStart != nullptr) ? &eyeGrid : nullptr;
+  const EyeGrid * eg = (GRIDS && eyeGridLive(eyeGrid)) ? &eyeGrid : nullptr;
   const int eyeCell = eg ? (int)((y >> eyeGrid.shift) * (uint32_t)eyeGrid.nx + (x >> eyeGrid.shift)) : -1;
   if (valid)
   {
@@ -815,7 +821,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_blob_wave_
   uint32_t nBounces = 0, nShadow = 0, events = 0, rel = 0, state0 = 0;
   V3 qo = mk(fp.eye[0], fp.eye[1], fp.eye[2]), qd = qo, mul = mk(1.0f, 1.0f, 1.0f), pix = mk(0.0f, 0.0f, 0.0f);
   bool alive = false;
-  const EyeGrid * eg = (GRIDS && eyeGrid.cellStart != nullptr) ? &eyeGrid : nullptr;
+  const EyeGrid * eg = (GRIDS && eyeGridLive(eyeGrid)) ? &eyeGrid : nullptr;
   const int eyeCell = eg ? (int)((y >> eyeGrid.shift) * (uint32_t)eyeGrid.nx + (x >> eyeGrid.shift)) : -1;
   if (valid)
   {
@@ -900,7 +906,7 @@ __global__ void __launch_bounds__(BLOB_THREADS, RFX_BLOB_MINBLOCKS) k_trace_blob
   __shared__ int stackMem[BLOB_STACK * BLOB_THREADS];
   const BlobView sc = blobView(sceneBlob);
   const V3 eye = mk(fp.eye[0], fp.eye[1], fp.eye[2]);
-  const EyeGrid * eg = eyeGrid.cellStart != nullptr ? &eyeGrid : nullptr;
+  const EyeGrid * eg = eyeGridLive(eyeGrid) ? &eyeGrid : nullptr;
   renderAny(fp, sampleStates, image, argbOut, sigOut, counters, tiled, BLOB_TILE_W, BLOB_THREADS, [&](uint32_t x, uint32_t y) {
     const int eyeCell = eg ? (int)((y >> eyeGrid.shift) * (uint32_t)eyeGrid.nx + (x >> eyeGrid.shift)) : -1;
     return [&, eyeCell](V3 ray, V3 rd, uint32_t & events, uint32_t & sig) {

@@ -485,43 +485,8 @@ __device__ __forceinline__ V3 traceSmall(const SmallScene & sc, V3 origin, V3 ra
 // produced a hit, so nothing a path computes changes; later queries of the path (shadow rays, bounces) see every object.
 // tests/test_oracle.py::test_primary_bounds_are_conservative evaluates the kernel's float expressions on every pixel for
 // random cameras (inside spheres, under the floor, looking away) against rfx_selftest_primary_bounds.
-// (struct PrimaryCull: rfx_kernels.h)
-constexpr int CULL_LO = -(1 << 30), CULL_HI = 1 << 30;
-constexpr double CULL_PIX_MARGIN = 3.0;            // sub-samples and jitter reach < 2 pixels past the pixel origin (Render.cpp:177-184)
-
-static int4 cullFull() { return make_int4(CULL_LO, CULL_HI, CULL_LO, CULL_HI); }
-static int4 cullNone() { return make_int4(1, 0, 1, 0); }
-static int cullClamp(double v)
-{
-  if (!(v == v)) return 0;
-  return v <= (double)CULL_LO ? CULL_LO : v >= (double)CULL_HI ? CULL_HI : (int)v;
-}
-
-// A sphere: the tangent planes through the eye that contain the camera's y (x) axis bound its projection in x (y).  The test the
-// kernel runs is the float discriminant of Sphere.cpp:49-53, whose rounding noise lets a ray pass that misses the sphere by up to
-// sqrt(r^2 + 4e-7 |w|^2) - r: the radius is inflated by 1e-3 r + 1e-3 |w|.
-static int4 cullSphere(const double * c0, const double * c1, const double * c2, const double * eye, double rz, double wHalf, double hHalf, const float4 & s)
-{
-  const double w[3] = { (double)s.x - eye[0], (double)s.y - eye[1], (double)s.z - eye[2] };
-  const double wl = sqrt(w[0] * w[0] + w[1] * w[1] + w[2] * w[2]);
-  const double r = sqrt(s.w > 0.0f ? (double)s.w : 0.0);
-  if (!(wl < 1e300) || !(r < 1e300)) return cullFull();
-  const double rEff = r * 1.001 + 1e-3 * wl + 1e-30;
-  const double wx = c0[0] * w[0] + c0[1] * w[1] + c0[2] * w[2], wy = c1[0] * w[0] + c1[1] * w[1] + c1[2] * w[2], wz = c2[0] * w[0] + c2[1] * w[1] + c2[2] * w[2];
-  int out[4];
-  for (int ax = 0; ax < 2; ax++)
-  {
-    const double a = ax ? wy : wx, half = ax ? hHalf : wHalf;
-    const double d2 = sqrt(a * a + wz * wz);
-    if (d2 <= rEff) { out[2 * ax] = CULL_LO; out[2 * ax + 1] = CULL_HI; continue; }
-    const double th = atan2(a, wz), al = asin(rEff / d2), lim = 1.5707963267948966 - 1e-4;
-    const double lo = th - al, hi = th + al;
-    if (hi <= -lim || lo >= lim) return cullNone();          // behind the eye in this projection
-    out[2 * ax] = lo <= -lim ? CULL_LO : cullClamp(floor(rz * tan(lo) + half - CULL_PIX_MARGIN));
-    out[2 * ax + 1] = hi >= lim ? CULL_HI : cullClamp(ceil(rz * tan(hi) + half + CULL_PIX_MARGIN));
-  }
-  return make_int4(out[0], out[1], out[2], out[3]);
-}
+// (struct PrimaryCull: rfx_kernels.h; the sphere rectangles, cullSphere, and the helpers: rfx_eye_grid.h, which the screen grid of the
+// blob scenes' first query shares)
 
 // A triangle: the edges come back out of axTrans (its inverse holds v2-v0 | v1-v0 | -n), the triangle is widened in barycentric
 // space by the noise of u = ox + t*rx (Triangle.cpp:65-66), clipped against a near plane so close to the eye that what it cuts
@@ -582,28 +547,6 @@ static int4 cullTriangle(const double * c0, const double * c1, const double * c2
   if (!n) return cullNone();
   if (!(x0 == x0) || !(x1 == x1) || !(y0 == y0) || !(y1 == y1)) return cullFull();
   return make_int4(cullClamp(floor(x0 - CULL_PIX_MARGIN)), cullClamp(ceil(x1 + CULL_PIX_MARGIN)), cullClamp(floor(y0 - CULL_PIX_MARGIN)), cullClamp(ceil(y1 + CULL_PIX_MARGIN)));
-}
-
-PrimaryCamera makePrimaryCamera(const FrameParams & fp)
-{
-  // ray = rx * c0 + ry * c1 + rz * c2 (Render.cpp:154-156): the bounds need an orthonormal camera (Camera.cpp:24-36 builds one)
-  PrimaryCamera cam;
-  for (int j = 0; j < 3; j++) { cam.eye[j] = (double)fp.eye[j]; for (int i = 0; i < 3; i++) cam.c[j][i] = (double)fp.view[3 * i + j]; }
-  cam.rz = (double)fp.rz; cam.wHalf = (double)fp.wHalf; cam.hHalf = (double)fp.hHalf; cam.W = (double)fp.W; cam.H = (double)fp.H;
-  cam.ok = fp.rz > 0.0f && fp.rz < 1e30f && fabs(cam.eye[0]) < 1e30 && fabs(cam.eye[1]) < 1e30 && fabs(cam.eye[2]) < 1e30;
-  for (int a = 0; a < 3 && cam.ok; a++)
-    for (int b = 0; b < 3; b++)
-    {
-      const double dot = cam.c[a][0] * cam.c[b][0] + cam.c[a][1] * cam.c[b][1] + cam.c[a][2] * cam.c[b][2];
-      if (!(fabs(dot - (a == b ? 1.0 : 0.0)) < 1e-4)) cam.ok = false;
-    }
-  return cam;
-}
-
-int4 primarySphereBounds(const PrimaryCamera & cam, const float4 & sphere)
-{
-  if (!cam.ok) return cullFull();
-  return cullSphere(cam.c[0], cam.c[1], cam.c[2], cam.eye, cam.rz, cam.wHalf, cam.hHalf, sphere);
 }
 
 PrimaryCull makePrimaryCull(const SmallScene & sc, const FrameParams & fp)
